@@ -2,6 +2,7 @@
 """bench.py -- Schnorr verifications/sec on B200 (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 20] [--msg-len 8]
+                    [--dump-outputs DIR]
 
 Workload (config.workload): independent Signature::verify of 2^20 synthetic signatures per GPU,
 8-byte messages (BASELINE.json configs[2]; the metric's own configuration).  A step = one pass of the
@@ -57,7 +58,38 @@ def parse_args():
     ap.add_argument("--batch-log2n", type=int, default=None,
                     help="signatures per GPU of the batch side measurement (default 16 at 1 GPU = configs[3], "
                          "21 at N > 1 = configs[4]: 2^24 over 8 GPUs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the verdicts of the last timed step of both timed paths to DIR/<name>.npy (float32; "
+                         "a fixed sample of rows above 2^22 signatures over all GPUs), so that two builds can be "
+                         "compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours (the CPU arm sizes its inputs from the measured host rate)")
+    return args
+
+
+DUMP_MAX_ROWS = 1 << 22      # over all ranks: two float32 outputs per row -> at most 32 MiB (+ file headers) in all
+
+
+def dump_rows(n, k):
+    """The fixed sample of k of n rows that the dump keeps when a rank's output is longer than its share: sorted,
+    drawn from seed 0, a function of (n, k) alone (so a reader can recompute which signatures the files hold)."""
+    return np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+
+
+def dump_outputs(path, outputs, rank=0, world=1):
+    """Writes each output of this rank (one row per signature) as float32 to path/<name>.npy, or path/<name>_rank<r>.npy
+    when world > 1.  Each rank keeps at most DUMP_MAX_ROWS // world rows, the rows dump_rows(n, cap) when it has more,
+    so the dump of all ranks together stays under DUMP_MAX_ROWS rows whatever the size and the number of GPUs."""
+    os.makedirs(path, exist_ok=True)
+    n = len(next(iter(outputs.values())))
+    cap = DUMP_MAX_ROWS // world
+    rows = dump_rows(n, cap) if n > cap else slice(None)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + suffix + ".npy"), np.asarray(a)[rows].astype(np.float32))
 
 
 class ClockSampler:
@@ -259,9 +291,6 @@ def main():
         for _ in range(args.warmup):
             step_dev()
         stream.synchronize()
-    got = d_verdicts.cpu().numpy()
-    if not np.array_equal(got, expect):
-        raise SystemExit("rank %d: verdicts differ from the expected pattern (%d mismatches)" % (rank, int((got != expect).sum())))
 
     sampler = ClockSampler(local) if rank == 0 else None
     barrier()
@@ -280,6 +309,9 @@ def main():
     barrier()
     launches = eng.launch_count - launches0
     clocks = sampler.stop() if sampler else None
+    got = d_verdicts.cpu().numpy()          # the verdicts of the last timed step
+    if not np.array_equal(got, expect):
+        raise SystemExit("rank %d: verdicts differ from the expected pattern (%d mismatches)" % (rank, int((got != expect).sum())))
     dev_ms = ev[0].elapsed_time(ev[-1])
     t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -315,6 +347,11 @@ def main():
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     e2e_value = world * n * args.steps / (float(t.item()) * 1e-3)
+    e2e_got = h_out.numpy().copy()          # the verdicts of the last timed step
+    if not np.array_equal(e2e_got, expect):
+        raise SystemExit("rank %d: e2e verdicts differ" % rank)
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, {"verdicts": got, "e2e_verdicts": e2e_got}, rank, world)
 
     # ---- roofline of the dominant kernel (k_verify_fast; the exact pass over handed-back items is inside kernel_ms) ----
     peak_w, peak_ms = eng.imad_peak(1 << 15)
