@@ -79,6 +79,7 @@ def w_per_batch_signature(n: int, msg_len: int, plan=None) -> float:
 # ---- executed by the shipped kernels (host-build counter; pinned by the CPU test named above) ------------------------
 W_EXECUTED_FAST_L8 = 335892       # k_verify_fast, 8-byte message: products of the (X, Y, w) path incl. 2 permutations
 W_EXECUTED_EXACT_L8 = 529896      # k_verify (exact Jacobian path)
+W_EXECUTED_REG_L8 = 80219         # k_verify_reg (registered key, 8-byte message): 2 permutations + table additions
 W_EXECUTED_PER_PERMUTATION = 28000
 
 
@@ -134,4 +135,4 @@ if __name__ == "__main__":
     print(json.dumps({"w_per_verify_L8": w_per_verify(8), "w_per_verify_L80": w_per_verify(80), "w_per_hash_L8": w_per_hash(8),
                       "w_per_batch_signature_2^16_L8": w_per_batch_signature(1 << 16, 8), "plan_2^17_points": msm_plan(1 << 17),
                       "w_per_batch_signature_2^21_L8": w_per_batch_signature(1 << 21, 8), "plan_2^22_points": msm_plan(1 << 22),
-                      "w_executed_fast_L8": w_executed_fast(8), "source_sha256": source_sha256()}, indent=1))
+                      "w_executed_fast_L8": w_executed_fast(8), "w_executed_reg_L8": W_EXECUTED_REG_L8, "source_sha256": source_sha256()}, indent=1))

@@ -129,6 +129,34 @@ int schnorr_b200_verify_many_dev(schnorr_b200_ctx *ctx, size_t n, const uint8_t 
                                  const uint8_t *pk_inf, const uint8_t *msgs, const uint64_t *msg_off,
                                  uint8_t *verdicts);
 
+/* Registered key sets: Signature::verify (src/signature.rs:181-205, also PublicKey::verify_signature :170-176) for many
+ * signatures under a small, recurring set of public keys.  Registration does once per key what every verification
+ * otherwise repeats: the subgroup check [q]P == O and the doubling chain of h*P, kept as a table of 32 x 129 affine
+ * multiples of P (396 KB per key, on every device of the context).  A verification is then the challenge hash and about
+ * 52 table additions.
+ * Keys are public data: the tables are indexed by challenge digits and are not constant-time (DESIGN.md §7).
+ *
+ * keyset_create registers n_keys public keys (pk96 / pk_inf as in verify_many; pk_inf may be NULL) on every device of
+ * ctx.  status (optional, n_keys bytes): 0 = in the prime-order subgroup (the identity included), 1 = not (verify gives
+ * InvalidPublicKey), 3 = non-canonical limb (verify gives 3).  EARG for n_keys == 0 or n_keys >= 2^32.  Duplicate keys
+ * are allowed.  A set belongs to the context it was created on and must be destroyed before it. */
+typedef struct schnorr_b200_keyset schnorr_b200_keyset;
+int schnorr_b200_keyset_create(schnorr_b200_ctx *ctx, size_t n_keys, const uint8_t *pk96, const uint8_t *pk_inf,
+                               uint8_t *status, schnorr_b200_keyset **out);
+void schnorr_b200_keyset_destroy(schnorr_b200_keyset *ks);
+/* Signature::verify for n (signature, key, message) triples, key = key_idx[i] into the set: verdicts[i] is, byte for
+ * byte, what verify_many returns for sigs81[i], message i and that key.  An index outside the set gives verdict 3
+ * (indexing past the end of a slice panics in the reference).  A set from another context returns EARG.
+ * last_exact_count, last_kernel_ms and set_exact_only apply as for verify_many.  The host form shards a multi-device
+ * context in contiguous slices; the _dev form (device buffers, no synchronisation) needs a single-device context and a
+ * non-NULL msgs even when every message is empty. */
+int schnorr_b200_verify_registered_many(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                        const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
+                                        const uint64_t *msg_off, uint8_t *verdicts);
+int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                            const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
+                                            const uint64_t *msg_off, uint8_t *verdicts);
+
 /* KeyedSignature::from_bytes + KeyedSignature::verify over n 130-byte wire records
  * (49-byte compressed public key || 81-byte signature)   src/signature.rs:232-271, src/constants.rs:33
  * The key is decompressed on the device; a record whose key does not decode gets verdict 3. */

@@ -127,6 +127,46 @@ inline Result PublicKey::verify_signature(const Signature& signature, const std:
     return signature.verify(message, *this);
 }
 
+// Public keys registered once for many verifications (schnorr_b200_keyset_*): the subgroup check and the per-key
+// table are computed at construction; verify_signature(i, ...) gives what Signature::verify gives under keys[i].
+class KeySet {
+public:
+    KeySet(Engine& eng, const std::vector<PublicKey>& keys) : eng_(eng) {
+        size_t n = keys.size();
+        std::vector<uint8_t> pks(n * 96), inf(n);
+        for (size_t i = 0; i < n; i++) {
+            std::memcpy(&pks[i * 96], keys[i].xy.data(), 96);
+            inf[i] = keys[i].infinity;
+        }
+        status_.assign(n, 255);
+        eng_.check(schnorr_b200_keyset_create(eng_.get(), n, pks.data(), inf.data(), status_.data(), &ks_), "keyset_create");
+    }
+    explicit KeySet(const std::vector<PublicKey>& keys) : KeySet(Engine::instance(), keys) {}
+    ~KeySet() { schnorr_b200_keyset_destroy(ks_); }
+    KeySet(const KeySet&) = delete;
+    KeySet& operator=(const KeySet&) = delete;
+    schnorr_b200_keyset* get() const { return ks_; }
+    // per key: 0 = in the prime-order subgroup (identity included), 1 = not, 3 = non-canonical limb
+    const std::vector<uint8_t>& status() const { return status_; }
+    size_t size() const { return status_.size(); }
+    // an index outside the set throws, as indexing past the end of a slice panics
+    Result verify_signature(size_t index, const Signature& signature, const std::vector<uint8_t>& message) const {
+        auto sig = signature.to_bytes();
+        uint64_t off[2] = {0, message.size()};
+        uint32_t idx = index < size() ? (uint32_t)index : UINT32_MAX;
+        uint8_t verdict = 255;
+        eng_.check(schnorr_b200_verify_registered_many(eng_.get(), ks_, 1, sig.data(), &idx,
+                                                       message.empty() ? nullptr : message.data(), off, &verdict),
+                   "verify_registered_many");
+        return result_from_verdict(verdict);
+    }
+
+private:
+    Engine& eng_;
+    schnorr_b200_keyset* ks_ = nullptr;
+    std::vector<uint8_t> status_;
+};
+
 struct KeyedSignature {
     PublicKey public_key;
     Signature signature;

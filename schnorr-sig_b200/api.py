@@ -184,6 +184,31 @@ class Signature:
         return isinstance(other, Signature) and (self.x, self.e) == (other.x, other.e)
 
 
+class KeySet:
+    """Public keys registered once for many verifications (no reference counterpart: the reference verifies each
+    signature from scratch).  Registration runs the subgroup check of every key and builds its table on the GPU;
+    verify_signature then gives what Signature.verify gives for that key without repeating that per-key work.
+    `status[i]`: 0 = key i is in the prime-order subgroup (identity included), 1 = it is not, 3 = non-canonical limb."""
+
+    def __init__(self, public_keys):
+        keys = list(public_keys)
+        pks = np.frombuffer(b"".join(k.xy for k in keys), dtype=np.uint8).reshape(len(keys), 96)
+        inf = np.array([k.infinity for k in keys], dtype=np.uint8)
+        self._handle, self.status = default_engine().register_keys(pks, inf)
+
+    def __len__(self):
+        return self._handle.n_keys
+
+    def verify_signature(self, index: int, signature: Signature, message: bytes) -> Result:
+        """Signature::verify(message, &keys[index]); an index outside the set panics, as indexing a slice does."""
+        index = int(index)
+        idx = np.array([index if 0 <= index < 2**32 else 2**32 - 1], dtype=np.uint32)
+        sig = np.frombuffer(signature.to_bytes(), dtype=np.uint8).reshape(1, 81)
+        blob, off = _pack([message])
+        v = default_engine().verify_registered_many(self._handle, sig, idx, blob, off)
+        return _result_from_verdict(int(v[0]))
+
+
 class KeyedSignature:
     def __init__(self, public_key: PublicKey, signature: Signature):
         self.public_key = public_key

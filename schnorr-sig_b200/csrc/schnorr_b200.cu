@@ -5,7 +5,11 @@
 //   k_hash            K1  hash_message per thread
 //   k_verify          K2  Signature::verify per thread (challenge hash + subgroup check + h*P + e*G)
 //   k_keygen / k_sign K5  fixed-base multiplication; device signer for synthetic inputs
-//   k_gtab_*              builds the fixed-base table of G at context creation
+//   k_tab_*               signed-window tables of affine multiples: the fixed-base table of G at context creation,
+//                         the per-key tables of registered key sets
+//   k_keyset_register     registration of a key set (status + subgroup check per key)
+//   k_keyset_gather       key records of the items of a registered call (ahead of k_ingest)
+//   k_verify_reg          Signature::verify against registered keys (table additions, no doubling chain)
 //   k_imad_peak       K6  integer-multiply roofline calibration
 //   batch kernels     K3/K4  in batch.cuh (Pippenger MSM)
 // No CPU fallback exists: every entry point needs a live CUDA context.
@@ -20,6 +24,7 @@
 #include "../../include/cheetah_params.h"
 #include "../../include/schnorr_b200.h"
 #include "verify.cuh"
+#include "keyset.cuh"
 #include "dist.cuh"
 #include "debug_ops.cuh"
 #include "derive.cuh"
@@ -627,36 +632,109 @@ __global__ void __launch_bounds__(SIGN_THREADS) k_derive_public(size_t n, const 
 }
 
 // ------------------------------------------------------------------------------------------------
-// fixed-base table of G:  gtab[i][d] = d * 2^(13 i) * G  (affine), i < 20, 1 <= d <= 4096 (curve.cuh)
+// signed-window tables of affine multiples (keyset.cuh: tab_bases / tab_entry), for a list of base points:
+//   tab[p][i][d] = d * 2^(w i) * P_p,  i < windows,  d < 2^(w-1) + 1  (slot 0 unused)
+// The fixed-base table of G (curve.cuh: w = 13, 20 windows) and the per-key tables of registered key sets (KT_W).
+// skip[p] != 0 (skip may be NULL): no table for point p (its slots are left as they are).
 // ------------------------------------------------------------------------------------------------
-__global__ void k_gtab_bases(jac_pt* bases, fp6 gx, fp6 gy) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= GTAB_WINDOWS) return;
-    jac_pt p = jac_from_affine(gx, gy, false);
-#pragma unroll 1
-    for (int k = 0; k < GTAB_W * i; k++) jac_dbl_mem(&p);
-    bases[i] = p;
+__global__ void __launch_bounds__(128) k_tab_bases(size_t n_pts, const uint64_t* __restrict__ pts12, const uint8_t* __restrict__ skip,
+                                                   int w, int windows, jac_pt* __restrict__ bases) {
+    size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n_pts || (skip && skip[p])) return;
+    tab_bases(pts12 + 12 * p, w, windows, bases + p * windows);
 }
-__global__ void __launch_bounds__(128) k_gtab_fill(const jac_pt* __restrict__ bases, uint64_t* __restrict__ gtab) {
-    int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= GTAB_WINDOWS * GTAB_ENTRIES) return;
-    int i = t / GTAB_ENTRIES, b = t % GTAB_ENTRIES;
-    jac_pt base = bases[i];
-    jac_pt acc = jac_identity();
-#pragma unroll 1
-    for (int bit = GTAB_W - 1; bit >= 0; bit--) {
-        jac_dbl_mem(&acc);
-        if ((b >> bit) & 1) jac_add_mem(&acc, &base, false);
-    }
-    fp6 x, y;
-    bool inf;
-    jac_to_affine(acc, x, y, inf);  // slot 0 (the identity) is written as zeros and never read
-    uint64_t* o = gtab + (size_t)t * 12;
+__global__ void __launch_bounds__(128) k_tab_fill(size_t n_pts, const uint8_t* __restrict__ skip, int w, int windows,
+                                                  const jac_pt* __restrict__ bases, uint64_t* __restrict__ tab) {
+    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    size_t entries = ((size_t)1 << (w - 1)) + 1, per_pt = (size_t)windows * entries;
+    if (t >= n_pts * per_pt) return;
+    size_t p = t / per_pt;
+    if (skip && skip[p]) return;
+    tab_entry(bases[t / entries], w, (int)(t % entries), tab + t * 12);
+}
+
+// ------------------------------------------------------------------------------------------------
+// registered key sets (keyset.cuh)
+// ------------------------------------------------------------------------------------------------
+// one thread per key: status (canonical limbs, exact subgroup check) and skip = no table (status != 0 or identity)
+__global__ void __launch_bounds__(128) k_keyset_register(size_t n_keys, const uint64_t* __restrict__ pk12,
+                                                         const uint8_t* __restrict__ pk_inf, uint8_t* __restrict__ status,
+                                                         uint8_t* __restrict__ skip) {
+    size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_keys) return;
+    bool inf = pk_inf[k] != 0;
+    jac_pt d;
+    uint8_t st = keyset_key_status(pk12 + 12 * k, inf, &d);
+    status[k] = st;
+    skip[k] = st != KEY_OK || inf;
+}
+// per item: the key record of key_idx[i] for k_ingest.  An index outside the set gets all-ones limbs, which k_ingest
+// flags as malformed (verdict 3: indexing past the end of a slice panics in the reference).
+__global__ void __launch_bounds__(128) k_keyset_gather(size_t n, const uint32_t* __restrict__ key_idx, size_t n_keys,
+                                                       const uint64_t* __restrict__ ks_pk12, const uint8_t* __restrict__ ks_inf,
+                                                       uint64_t* __restrict__ pk12, uint8_t* __restrict__ pk_inf) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t k = key_idx[i];
+    bool in = k < n_keys;
 #pragma unroll
-    for (int k = 0; k < 6; k++) {
-        o[k] = x.c[k];
-        o[6 + k] = y.c[k];
+    for (int c = 0; c < 12; c++) pk12[12 * i + c] = in ? ks_pk12[12 * (size_t)k + c] : ~0ULL;
+    pk_inf[i] = in ? ks_inf[k] : 0;
+}
+
+// Signature::verify against registered keys: the shape of k_verify_fast (block-agreed challenge hash, stand-in inputs
+// for threads without work, the same verdicts and hand-back list), with h*P from the key's table instead of the
+// doubling chain and no subgroup check (the key's status).  Items handed back are finished by k_verify, which reads
+// the key k_keyset_gather placed in the planes.
+__global__ void __launch_bounds__(VERIFY_THREADS) k_verify_reg(soa_batch in, const uint32_t* __restrict__ key_idx,
+                                                               const uint8_t* __restrict__ key_status,
+                                                               const uint64_t* __restrict__ ktab,
+                                                               const uint8_t* __restrict__ msgs,
+                                                               const uint64_t* __restrict__ msg_off,
+                                                               const uint64_t* __restrict__ gtab,
+                                                               uint8_t* __restrict__ verdicts,
+                                                               uint32_t* __restrict__ work_list,
+                                                               uint32_t* __restrict__ work_count) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool live = i < in.n;
+    uint8_t fl = live ? in.flags[i] : FL_MALFORMED;
+    // a record that is not malformed has an index inside the set (k_keyset_gather)
+    bool keyed = !(fl & (FL_MALFORMED | FL_PK_INF));
+    uint32_t k = keyed ? key_idx[i] : 0;
+    uint8_t st = keyed ? key_status[k] : KEY_OK;
+    bool work = keyed && st == KEY_OK;
+    uint64_t off = work ? msg_off[i] : 0, len = work ? msg_off[i + 1] - off : 0;
+    hash_vote hv = block_hash_vote(work ? hash_message_permutations(len) : -1, off, len);
+    fp6 sx = fp6_zero(), px, py;
+    scalar e = sc_zero();
+    if (work) {
+        sx = load_fp6_planes(in.planes, 0, in.n, i);
+        e = load_scalar_planes(in.planes, 3, in.n, i);
+        px = load_fp6_planes(in.planes, 5, in.n, i);
+        py = load_fp6_planes(in.planes, 8, in.n, i);
+    } else {  // 1 * G, the first entry of the fixed-base table
+        const uint64_t* g = gtab + (size_t)1 * GTAB_ENTRY_U64;
+#pragma unroll
+        for (int c = 0; c < 6; c++) {
+            px.c[c] = g[c];
+            py.c[c] = g[6 + c];
+        }
     }
+    bool x_ok = !(fl & FL_X_BAD);
+    scalar h = sc_zero();
+    if (hv.any) {  // block-uniform
+        h = challenge_scalar(sx, px, py, false, msgs + off, len, hv.sync);
+        if (!x_ok || !work) h = sc_zero();
+    }
+    jf_pt r;
+    int fr = verify_core_reg(h, e, ktab + (size_t)k * KT_KEY_U64, gtab, &r);
+    if (!live) return;
+    uint8_t v;
+    if (fl & FL_MALFORMED) v = VERDICT_MALFORMED;
+    else if (fl & FL_PK_INF) v = VERDICT_NEEDS_EXACT;   // the identity key is the exact kernel's business
+    else v = reg_verdict(st, x_ok, fr, r, sx);
+    verdicts[i] = v;
+    if (v == VERDICT_NEEDS_EXACT) work_list[atomicAdd(work_count, 1u)] = (uint32_t)i;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -731,6 +809,17 @@ __global__ void __launch_bounds__(256) k_imad_peak(int iters, uint64_t* sink) {
 // host side
 // ------------------------------------------------------------------------------------------------
 static inline unsigned grid_for(size_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
+
+// tables of n_pts base points (k_tab_bases / k_tab_fill); bases: n_pts * windows Jacobian points of scratch
+static int build_tables(schnorr_b200_ctx* ctx, size_t n_pts, const uint64_t* pts12, const uint8_t* skip, int w, int windows,
+                        jac_pt* bases, uint64_t* tab) {
+    size_t threads = n_pts * (size_t)windows * (((size_t)1 << (w - 1)) + 1);
+    k_tab_bases<<<grid_for(n_pts, 128), 128, 0, ctx->stream>>>(n_pts, pts12, skip, w, windows, bases);
+    k_tab_fill<<<grid_for(threads, 128), 128, 0, ctx->stream>>>(n_pts, skip, w, windows, bases, tab);
+    ctx->launches += 2;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
 
 static int alloc_soa(schnorr_b200_ctx* ctx, size_t n, soa_batch* b) {
     void *p, *f, *sf;
@@ -886,15 +975,15 @@ int schnorr_b200_create(int device, schnorr_b200_ctx** out) {
     CREATE_TRY(cudaMemcpyToSymbol(c_q_wnaf5, CHEETAH_Q_WNAF5, sizeof(CHEETAH_Q_WNAF5)));  // the tail of the symbol stays zero
     CREATE_TRY(cudaMemcpyToSymbol(c_q_wnaf4, CHEETAH_Q_WNAF4, 256));
     CREATE_TRY(cudaMalloc(&ctx->gtab, GTAB_U64 * sizeof(uint64_t)));
-    jac_pt* bases = nullptr;
-    CREATE_TRY(cudaMalloc(&bases, sizeof(jac_pt) * GTAB_WINDOWS));
-    fp6 gx, gy;
-    memcpy(gx.c, CHEETAH_GX, 48);
-    memcpy(gy.c, CHEETAH_GY, 48);
-    k_gtab_bases<<<1, 32, 0, ctx->stream>>>(bases, gx, gy);
-    k_gtab_fill<<<(GTAB_WINDOWS * GTAB_ENTRIES + 127) / 128, 128, 0, ctx->stream>>>(bases, ctx->gtab);
-    ctx->launches += 2;
-    CREATE_TRY(cudaGetLastError());
+    jac_pt* bases = nullptr;  // the GTAB_WINDOWS bases, then G itself (12 limbs)
+    CREATE_TRY(cudaMalloc(&bases, sizeof(jac_pt) * GTAB_WINDOWS + 96));
+    uint64_t* g12 = reinterpret_cast<uint64_t*>(bases + GTAB_WINDOWS);
+    CREATE_TRY(cudaMemcpyAsync(g12, CHEETAH_GX, 48, cudaMemcpyHostToDevice, ctx->stream));
+    CREATE_TRY(cudaMemcpyAsync(g12 + 6, CHEETAH_GY, 48, cudaMemcpyHostToDevice, ctx->stream));
+    if (build_tables(ctx, 1, g12, nullptr, GTAB_W, GTAB_WINDOWS, bases, ctx->gtab)) {
+        cudaFree(bases);
+        return fail(SCHNORR_B200_ECUDA);
+    }
     CREATE_TRY(cudaStreamSynchronize(ctx->stream));
     cudaFree(bases);
 #undef CREATE_TRY
@@ -1270,6 +1359,193 @@ int schnorr_b200_verify_keyed_many(schnorr_b200_ctx* ctx, size_t n, const uint8_
     CUDA_TRY(ctx, cudaMemcpyAsync(verdicts, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return SCHNORR_B200_OK;
+}
+
+} // extern "C"
+
+// ---- registered key sets (keyset.cuh) ---------------------------------------------------------
+// On a multi-device context the set holds one single-device set per shard (`shards`), each with its own table.
+struct schnorr_b200_keyset {
+    schnorr_b200_ctx* ctx = nullptr;  // the context the set was created on
+    int device = 0;
+    size_t n_keys = 0;
+    uint64_t* pk12 = nullptr;   // [n_keys][12] the registered records, gathered per item ahead of k_ingest
+    uint8_t* pk_inf = nullptr;  // [n_keys]
+    uint8_t* status = nullptr;  // [n_keys] KEY_OK / KEY_NOT_TORSION_FREE / KEY_MALFORMED
+    uint64_t* ktab = nullptr;   // [n_keys][KT_KEY_U64]; zeros for keys without a table
+    std::vector<schnorr_b200_keyset*> shards;
+};
+
+static void keyset_free(schnorr_b200_keyset* ks) {
+    for (schnorr_b200_keyset* sh : ks->shards) keyset_free(sh);
+    if (ks->pk12 || ks->ktab) {
+        cudaSetDevice(ks->device);
+        cudaFree(ks->pk12);   // pk_inf and status live in the same allocation
+        cudaFree(ks->ktab);
+    }
+    delete ks;
+}
+
+// registration on one device: copies the records, k_keyset_register, the tables of the keys with status 0
+static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const uint8_t* pk96, const uint8_t* pk_inf,
+                        uint8_t* status) {
+    const size_t n = ks->n_keys;
+    ks->device = ctx->device;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    void* rec;
+    CUDA_TRY(ctx, cudaMalloc(&rec, n * 96 + 2 * n));
+    ks->pk12 = (uint64_t*)rec;
+    ks->pk_inf = (uint8_t*)rec + n * 96;
+    ks->status = ks->pk_inf + n;
+    CUDA_TRY(ctx, cudaMalloc(&ks->ktab, n * KT_KEY_U64 * sizeof(uint64_t)));
+    CUDA_TRY(ctx, cudaMemsetAsync(ks->ktab, 0, n * KT_KEY_U64 * sizeof(uint64_t), ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk12, pk96, n * 96, cudaMemcpyHostToDevice, ctx->stream));
+    if (pk_inf) CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk_inf, pk_inf, n, cudaMemcpyHostToDevice, ctx->stream));
+    else CUDA_TRY(ctx, cudaMemsetAsync(ks->pk_inf, 0, n, ctx->stream));
+    void* tmp;  // skip flags, then the table bases
+    size_t skip_bytes = (n + 15) / 16 * 16;
+    if (int rc = ensure_scratch(ctx, SL_D, skip_bytes + n * KT_WINDOWS * sizeof(jac_pt), &tmp)) return rc;
+    uint8_t* skip = (uint8_t*)tmp;
+    k_keyset_register<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, ks->pk12, ks->pk_inf, ks->status, skip);
+    ctx->launches += 1;
+    if (int rc = build_tables(ctx, n, ks->pk12, skip, KT_W, KT_WINDOWS, (jac_pt*)((uint8_t*)tmp + skip_bytes), ks->ktab)) return rc;
+    if (status) CUDA_TRY(ctx, cudaMemcpyAsync(status, ks->status, n, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+// Calls of at most this many items run verify_many's kernels (launch_verify) on the gathered records: at these sizes
+// its block-per-signature kernel wins on latency.  Measured on a B200 (1000 W, 1965 MHz; profiles/r3_registered.md):
+// 1 / 128 / 384 signatures 0.47 / 0.47 / 0.58 ms there against 0.59 / 0.60 / 0.60 ms in k_verify_reg, 512 signatures
+// 0.61 against 0.60 ms.
+static constexpr size_t REG_SMALL_MAX = 384;
+
+// the fast kernel over an ingested batch of registered items, then the exact kernel over the items it handed back;
+// exact_only and small calls go through launch_verify (same verdicts: the planes hold each item's key record)
+static int launch_verify_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, const soa_batch& soa,
+                                    const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
+    cudaStream_t st = ctx->stream;
+    if (ctx->exact_only || soa.n <= REG_SMALL_MAX) return launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, 0, soa.n, st);
+    void* wl;
+    if (int rc = ensure_scratch(ctx, SL_M, 4 * (soa.n + schnorr_b200_ctx::MAX_CHUNKS), &wl)) return rc;
+    uint32_t* counter = (uint32_t*)wl;
+    uint32_t* list = counter + schnorr_b200_ctx::MAX_CHUNKS;
+    CUDA_TRY(ctx, cudaMemsetAsync(counter, 0, 4, st));
+    ctx->exact_counters_used = 1;
+    unsigned grid = grid_for(soa.n, VERIFY_THREADS);
+    k_verify_reg<<<grid, VERIFY_THREADS, 0, st>>>(soa, key_idx, ks->status, ks->ktab, msgs, msg_off, ctx->gtab, verdicts, list, counter);
+    k_verify<<<grid, VERIFY_THREADS, 0, st>>>(soa, msgs, msg_off, ctx->gtab, verdicts, list, counter);
+    ctx->launches += 2;
+    return 0;
+}
+
+// device buffers, single-device context, arguments checked by the caller
+static int verify_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                 const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    void *d_pk, *d_inf;
+    if (int rc = ensure_scratch(ctx, SL_E, n * 96, &d_pk)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_I, n, &d_inf)) return rc;
+    soa_batch soa;
+    if (int rc = alloc_soa(ctx, n, &soa)) return rc;
+    k_keyset_gather<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, key_idx, ks->n_keys, ks->pk12, ks->pk_inf, (uint64_t*)d_pk,
+                                                              (uint8_t*)d_inf);
+    k_ingest<<<grid_for(n, INGEST_THREADS), INGEST_THREADS, 0, ctx->stream>>>(n, sigs81, (uint8_t*)d_pk, (uint8_t*)d_inf, soa);
+    ctx->launches += 2;
+    cudaEventRecord(ctx->ev_k0, ctx->stream);
+    if (int rc = launch_verify_registered(ctx, ks, soa, key_idx, msgs, msg_off, verdicts)) return rc;
+    cudaEventRecord(ctx->ev_k1, ctx->stream);
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+
+// host buffers, single-device context: staged with cudaMemcpyAsync, verdicts copied back, synchronised
+static int verify_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                  const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    size_t mb = msg_off[n];
+    void *d_sig, *d_idx, *d_m, *d_off, *d_out;
+    if (int rc = stage_in(ctx, SL_D, sigs81, n * 81, &d_sig)) return rc;
+    if (int rc = stage_in(ctx, SL_J, key_idx, n * 4, &d_idx)) return rc;
+    if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
+    if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
+    if (int rc = verify_registered_dev(ctx, ks, n, (uint8_t*)d_sig, (uint32_t*)d_idx, (uint8_t*)d_m, (uint64_t*)d_off,
+                                       (uint8_t*)d_out))
+        return rc;
+    CUDA_TRY(ctx, cudaMemcpyAsync(verdicts, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+#define CHECK_KEYSET(ctx, ks)                                                   \
+    do {                                                                        \
+        if ((ks)->ctx != (ctx)) {                                               \
+            (ctx)->err = "the key set was created on another context";          \
+            return SCHNORR_B200_EARG;                                           \
+        }                                                                       \
+    } while (0)
+
+extern "C" {
+
+int schnorr_b200_keyset_create(schnorr_b200_ctx* ctx, size_t n_keys, const uint8_t* pk96, const uint8_t* pk_inf,
+                               uint8_t* status, schnorr_b200_keyset** out) {
+    if (!out) return SCHNORR_B200_EARG;
+    *out = nullptr;
+    if (!ctx || !pk96 || n_keys == 0 || (uint64_t)n_keys >= ((uint64_t)1 << 32)) return SCHNORR_B200_EARG;
+    schnorr_b200_keyset* ks = new schnorr_b200_keyset();
+    ks->ctx = ctx;
+    ks->n_keys = n_keys;
+    int rc = 0;
+    if (ctx->shards.empty()) {
+        rc = keyset_build(ctx, ks, pk96, pk_inf, status);
+    } else {  // one table per device; the status comes from the first (every shard computes the same)
+        for (size_t k = 0; k < ctx->shards.size() && rc == 0; k++) {
+            schnorr_b200_keyset* sh = new schnorr_b200_keyset();
+            sh->ctx = ctx->shards[k];
+            sh->n_keys = n_keys;
+            ks->shards.push_back(sh);
+            rc = keyset_build(ctx->shards[k], sh, pk96, pk_inf, k == 0 ? status : nullptr);
+            if (rc) ctx->err = "device " + std::to_string(ctx->shards[k]->device) + ": " + ctx->shards[k]->err;
+        }
+    }
+    if (rc) {
+        keyset_free(ks);
+        return rc;
+    }
+    *out = ks;
+    return SCHNORR_B200_OK;
+}
+
+void schnorr_b200_keyset_destroy(schnorr_b200_keyset* ks) {
+    if (ks) keyset_free(ks);
+}
+
+int schnorr_b200_verify_registered_many(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                        const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
+    if (!ctx || !ks || (n && (!sigs81 || !key_idx || !msg_off || !verdicts))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n == 0) return SCHNORR_B200_OK;
+    CHECK_MSG_OFF(ctx, n, msg_off);
+    if (msg_off[n] && !msgs) return SCHNORR_B200_EARG;
+    if (ctx->shards.empty()) return verify_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, verdicts);
+    auto sl = multi_slices(ctx, n);
+    return multi_run(ctx, sl, [&](int k, shard_slice s) {
+        auto off = rebase_offsets(msg_off, s.lo, s.hi);
+        return verify_registered_host(ctx->shards[k], ks->shards[k], s.hi - s.lo, sigs81 + 81 * s.lo, key_idx + s.lo,
+                                      msgs ? msgs + msg_off[s.lo] : nullptr, off.data(), verdicts + s.lo);
+    });
+}
+
+int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                            const uint8_t* sigs81, const uint32_t* key_idx, const uint8_t* msgs,
+                                            const uint64_t* msg_off, uint8_t* verdicts) {
+    // msgs is required too: the offset table lives on the device, so whether every message is empty is not known here
+    if (!ctx || !ks || (n && (!sigs81 || !key_idx || !msgs || !msg_off || !verdicts))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    NOT_ON_MULTI(ctx);
+    if (n == 0) return SCHNORR_B200_OK;
+    return verify_registered_dev(ctx, ks, n, sigs81, key_idx, msgs, msg_off, verdicts);
 }
 
 // ---- keygen / sign ---------------------------------------------------------------------------

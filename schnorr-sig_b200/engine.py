@@ -181,6 +181,41 @@ class Engine:
                     "verify_keyed_many")
         return out
 
+    # ---- registered key sets -------------------------------------------------------------
+    def register_keys(self, pk96, pk_inf=None):
+        """Registers public keys (subgroup check + per-key table on every device) -> (KeySetHandle, status uint8[n_keys]):
+        status 0 = in the prime-order subgroup (identity included), 1 = not, 3 = non-canonical limb."""
+        pk96 = _u8(pk96, 96)
+        n = pk96.shape[0]
+        inf = None if pk_inf is None else _u8(pk_inf)
+        self._check_inf(n, inf)
+        status = np.full(n, 255, dtype=np.uint8)
+        h = C.c_void_p()
+        self._check(self._L.schnorr_b200_keyset_create(self._h, n, _ptr(pk96), _ptr(inf), _ptr(status), C.byref(h)),
+                    "keyset_create")
+        return KeySetHandle(self, h, n), status
+
+    def verify_registered_many(self, keyset, sigs81, key_idx, msgs, off):
+        """Signature::verify of sigs81[i] over message i under key key_idx[i] of `keyset` -> verdicts (those of
+        verify_many; 3 for an index outside the set)."""
+        sigs81, msgs = _u8(sigs81, 81), _u8(msgs)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = sigs81.shape[0]
+        if key_idx.ndim != 1:
+            raise ValueError("key_idx must be one-dimensional")
+        self._check_offsets(n, key_idx.shape[0], off, msgs)
+        out = np.full(n, 255, dtype=np.uint8)
+        self._check(self._L.schnorr_b200_verify_registered_many(self._h, keyset.handle, n, _ptr(sigs81), _ptr(key_idx),
+                                                                _ptr(msgs), _ptr(off), _ptr(out)), "verify_registered_many")
+        return out
+
+    def verify_registered_many_dev(self, keyset, n, sigs81, key_idx, msgs, off, verdicts):
+        """Device buffers (key_idx: n uint32), enqueued on the engine's stream, no synchronisation."""
+        self._check(self._L.schnorr_b200_verify_registered_many_dev(self._h, keyset.handle, n, _ptr(sigs81), _ptr(key_idx),
+                                                                    _ptr(msgs), _ptr(off), _ptr(verdicts)),
+                    "verify_registered_many_dev")
+
     def verify_batch(self, sigs81, pk96, pk_inf, msgs, off, rand32):
         """-> (verdict, lhs97, rhs97)"""
         sigs81, pk96, msgs, rand32 = _u8(sigs81, 81), _u8(pk96, 96), _u8(msgs), _u8(rand32, 32)
@@ -365,6 +400,30 @@ class Engine:
     def batch_finish_dev(self, n_partials, partials192, result216):
         self._check(self._L.schnorr_b200_batch_finish_dev(self._h, n_partials, _ptr(partials192), _ptr(result216)),
                     "batch_finish_dev")
+
+
+class KeySetHandle:
+    """A registered key set (schnorr_b200_keyset) of one Engine; keeps the engine alive and frees the tables on close."""
+
+    def __init__(self, engine, handle, n_keys):
+        self.engine, self._h, self.n_keys = engine, handle, n_keys
+
+    @property
+    def handle(self):
+        if self._h is None or not self._h.value:
+            raise ValueError("the key set has been closed")
+        return self._h
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            self.engine._L.schnorr_b200_keyset_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 _DEFAULT = {}
