@@ -202,6 +202,39 @@ int schnorr_b200_locate_invalid_dev(schnorr_b200_ctx *ctx, size_t n, const uint8
                                     const uint8_t *pk_inf, const uint8_t *msgs, const uint64_t *msg_off,
                                     const uint8_t *rand32, uint8_t *flags);
 
+/* verify_batch (src/batch.rs:31-130) against a registered key set: item i is signature sigs81[i] over message i under
+ * key key_idx[i] of ks.  *verdict, lhs97 and rhs97 are, byte for byte, those of verify_batch on the gathered key records
+ * pk96[i] = keys[key_idx[i]] (the same group elements, the same affine encodings); an index outside the set makes the
+ * batch malformed (verdict 3), as does an item under a key of status 3.  Batch semantics are kept (src/batch.rs:102-106):
+ * no subgroup check on the keys, identity keys contribute nothing.
+ * The key side of the batch equation is summed per key, sum_i (s_i h_i) P_key(i) = sum_k c_k P_k: one product with the
+ * key's table per distinct key instead of one MSM point per signature, so the MSM runs over the n points R_i only.  That
+ * reduction of c_k mod q is valid only for keys with [q]P = O: a set that holds a key of status 1 runs every batch on
+ * the per-signature points (still the same result) -- register only the keys of status 0 to get the aggregated path.
+ * Batches of at most batch_small_max signatures, or with fewer than set_registered_batch_threshold signatures per key
+ * of the set, also take the per-signature points.  The host form shards a multi-device context in contiguous slices
+ * (one partial per shard from that device's copy of the set, finished on the first device); the _dev form (device
+ * buffers, no synchronisation, result216 as in verify_batch_dev) needs a single-device context and a non-NULL msgs. */
+int schnorr_b200_verify_batch_registered(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                         const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
+                                         const uint64_t *msg_off, const uint8_t *rand32, int *verdict, uint8_t *lhs97,
+                                         uint8_t *rhs97);
+int schnorr_b200_verify_batch_registered_dev(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                             const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
+                                             const uint64_t *msg_off, const uint8_t *rand32, uint8_t *result216);
+/* locate_invalid (above) against a registered key set: the flags and *n_bad of locate_invalid on the gathered key
+ * records; an index outside the set gets flag 3.  Runs on the first device.           src/batch.rs:102-129 */
+int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                           const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
+                                           const uint64_t *msg_off, const uint8_t *rand32, uint8_t *flags,
+                                           uint64_t *n_bad);
+/* MSM points of the last batch verification on this context (all devices of a multi-device context): 2n for
+ * verify_batch, n for a registered batch summed per key, 0 for the block-per-signature form of small batches. */
+int schnorr_b200_last_batch_points(const schnorr_b200_ctx *ctx, uint64_t *points);
+/* Registered batches sum the key side per key when they hold at least `min_signatures_per_key` signatures per key of
+ * the set (0: whenever the other rules allow it).  Default 64 (measured crossover, profiles/r4_registered_batch.md). */
+int schnorr_b200_set_registered_batch_threshold(schnorr_b200_ctx *ctx, size_t min_signatures_per_key);
+
 /* PublicKey::from(&PrivateKey) = BASEPOINT_TABLE * sk                      src/public.rs:26-32 */
 int schnorr_b200_keygen(schnorr_b200_ctx *ctx, size_t n, const uint8_t *sk32, uint8_t *pk96, uint8_t *pk_inf);
 int schnorr_b200_keygen_dev(schnorr_b200_ctx *ctx, size_t n, const uint8_t *sk32, uint8_t *pk96, uint8_t *pk_inf);

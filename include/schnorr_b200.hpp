@@ -160,8 +160,26 @@ public:
                    "verify_registered_many");
         return result_from_verdict(verdict);
     }
+    // verify_batch(signatures, [keys[i] for i in indices], messages, rng) with the key side summed per key of the set
+    // (schnorr_b200_verify_batch_registered); an index outside the set makes the batch malformed, which throws
+    Result verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                        const std::vector<std::vector<uint8_t>>& messages,
+                        const std::function<void(uint8_t*, size_t)>& rng) const;
+    // indices of the items whose own term of the batch equation fails (schnorr_b200_locate_invalid_registered); a
+    // malformed item or an index outside the set throws
+    std::vector<size_t> locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                       const std::vector<std::vector<uint8_t>>& messages,
+                                       const std::function<void(uint8_t*, size_t)>& rng) const;
 
 private:
+    struct BatchInputs {
+        std::vector<uint8_t> sigs, rand, blob;
+        std::vector<uint32_t> idx;
+        std::vector<uint64_t> off;
+    };
+    BatchInputs batch_inputs(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                             const std::vector<std::vector<uint8_t>>& messages,
+                             const std::function<void(uint8_t*, size_t)>& rng) const;
     Engine& eng_;
     schnorr_b200_keyset* ks_ = nullptr;
     std::vector<uint8_t> status_;
@@ -202,6 +220,58 @@ inline Result verify_batch(const std::vector<Signature>& signatures, const std::
                                         off.data(), rand.data(), &verdict, nullptr, nullptr),
               "verify_batch");
     return result_from_verdict(verdict);
+}
+
+inline KeySet::BatchInputs KeySet::batch_inputs(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                                const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
+    if (signatures.size() != indices.size())
+        throw std::logic_error("We should have the same number of signatures than public keys");
+    if (messages.size() != indices.size())
+        throw std::logic_error("We should have the same number of messages than public keys");
+    size_t n = signatures.size();
+    BatchInputs in;
+    in.sigs.resize(n * 81);
+    in.rand.resize(n * 32);
+    in.idx.resize(n);
+    in.off.assign(n + 1, 0);
+    for (size_t i = 0; i < n; i++) {
+        auto b = signatures[i].to_bytes();
+        std::memcpy(&in.sigs[i * 81], b.data(), 81);
+        in.idx[i] = indices[i] < size() ? (uint32_t)indices[i] : UINT32_MAX;
+        in.blob.insert(in.blob.end(), messages[i].begin(), messages[i].end());
+        in.off[i + 1] = in.blob.size();
+    }
+    rng(in.rand.data(), in.rand.size());
+    for (size_t i = 0; i < n; i++) in.rand[i * 32 + 31] &= 0x3f;
+    return in;
+}
+
+inline Result KeySet::verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                   const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
+    BatchInputs in = batch_inputs(indices, signatures, messages, rng);
+    int verdict = -1;
+    eng_.check(schnorr_b200_verify_batch_registered(eng_.get(), ks_, in.idx.size(), in.sigs.data(), in.idx.data(),
+                                                    in.blob.empty() ? nullptr : in.blob.data(), in.off.data(), in.rand.data(),
+                                                    &verdict, nullptr, nullptr),
+               "verify_batch_registered");
+    return result_from_verdict(verdict);
+}
+
+inline std::vector<size_t> KeySet::locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                                  const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
+    BatchInputs in = batch_inputs(indices, signatures, messages, rng);
+    size_t n = in.idx.size();
+    std::vector<uint8_t> flags(n, 0);
+    eng_.check(schnorr_b200_locate_invalid_registered(eng_.get(), ks_, n, in.sigs.data(), in.idx.data(),
+                                                      in.blob.empty() ? nullptr : in.blob.data(), in.off.data(),
+                                                      in.rand.data(), flags.data(), nullptr),
+               "locate_invalid_registered");
+    std::vector<size_t> bad;
+    for (size_t i = 0; i < n; i++) {
+        if (flags[i] == 3) throw std::logic_error("called `Option::unwrap()` on a `None` value (non-canonical encoding)");
+        if (flags[i]) bad.push_back(i);
+    }
+    return bad;
 }
 
 }  // namespace schnorr_sig

@@ -44,6 +44,11 @@ _SIGNATURES = {
     "schnorr_b200_verify_batch_dev": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 7),
     "schnorr_b200_locate_invalid": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 7 + [C.POINTER(C.c_uint64)]),
     "schnorr_b200_locate_invalid_dev": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 7),
+    "schnorr_b200_verify_batch_registered": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 5 + [C.POINTER(C.c_int), _u8p, _u8p]),
+    "schnorr_b200_verify_batch_registered_dev": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 6),
+    "schnorr_b200_locate_invalid_registered": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 6 + [C.POINTER(C.c_uint64)]),
+    "schnorr_b200_last_batch_points": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
+    "schnorr_b200_set_registered_batch_threshold": (C.c_int, [C.c_void_p, _sz]),
     "schnorr_b200_batch_partial_dev": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 7),
     "schnorr_b200_batch_finish_dev": (C.c_int, [C.c_void_p, _sz, _u8p, _u8p]),
     "schnorr_b200_batch_finish": (C.c_int, [C.c_void_p, _sz, _u8p, C.POINTER(C.c_int), _u8p, _u8p]),

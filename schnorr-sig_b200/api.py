@@ -208,6 +208,41 @@ class KeySet:
         v = default_engine().verify_registered_many(self._handle, sig, idx, blob, off)
         return _result_from_verdict(int(v[0]))
 
+    def _batch_inputs(self, indices, signatures, messages, rng):
+        n = len(signatures)
+        assert len(indices) == n, "We should have the same number of signatures than public keys"
+        assert len(messages) == n, "We should have the same number of messages than public keys"
+        idx = np.array([int(i) if 0 <= int(i) < 2**32 else 2**32 - 1 for i in indices], dtype=np.uint32)
+        sigs = np.frombuffer(b"".join(s.to_bytes() for s in signatures), dtype=np.uint8).reshape(n, 81)
+        blob, off = _pack(messages)
+        rng = rng or OsRng()
+        rand = np.zeros((n, 32), dtype=np.uint8)
+        for i in range(n):
+            rand[i] = np.frombuffer(_random_scalar(rng).to_bytes(32, "little"), dtype=np.uint8)
+        return sigs, idx, blob, off, rand
+
+    def verify_batch(self, indices, signatures, messages, rng=None) -> Result:
+        """verify_batch(signatures, [keys[i] for i in indices], messages, rng) (src/batch.rs:31-130) with the key side of
+        the batch equation summed per key of the set; an index outside the set gives the malformed-batch error."""
+        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng)
+        v, _lhs, _rhs = default_engine().verify_batch_registered(self._handle, sigs, idx, blob, off, rand)
+        return _result_from_verdict(v)
+
+    def locate_invalid(self, indices, signatures, messages, rng=None):
+        """locate_invalid(signatures, [keys[i] for i in indices], messages, rng): [(index, SignatureError), ...] in batch
+        semantics; a malformed item or an index outside the set panics."""
+        if len(signatures) == 0:
+            assert len(indices) == 0 and len(messages) == 0
+            return []
+        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng)
+        flags = default_engine().locate_invalid_registered(self._handle, sigs, idx, blob, off, rand)
+        out = []
+        for i in np.nonzero(flags)[0]:
+            if flags[i] == MALFORMED:
+                raise PanicError("item %d has a key index outside the set or a non-canonical or undecodable encoding" % i)
+            out.append((int(i), SignatureError(SignatureError.InvalidSignature)))
+        return out
+
 
 class KeyedSignature:
     def __init__(self, public_key: PublicKey, signature: Signature):

@@ -1039,15 +1039,137 @@ __global__ void __launch_bounds__(SMALL_REDUCE_THREADS) k_batch_small_reduce(siz
     }
 }
 
+// ---- batches against a registered key set (keyset.cuh) ---------------------------------------------------------------
+// k_batch_prepare writes t_i = s_i h_i mod q into scalars [n, 2n) (zero for identity keys and malformed items).  Instead
+// of putting every -P_i into the MSM, the key side sums the t_i per key and adds c_k (-P_k) from the key's table, so the
+// MSM runs over the n points R_i only.  The three kernels below run on the second stream, beside the MSM.
+//
+// Per key: the exact integer sum of its t_i as 64-bit column sums of the eight 32-bit limbs (keyset_sum_reduce).  Lanes
+// of a warp with the same key add their limbs first (16-bit halves: 32 of them fit a 32-bit reduction), then one atomic
+// per group and limb.  Integer addition commutes: the sums do not depend on the order of the atomics.  A malformed item
+// (an index outside the set among them) never addresses the accumulator; its t_i is zero anyway.
+static constexpr int KEYSUM_THREADS = 256;
+__global__ void __launch_bounds__(KEYSUM_THREADS) k_keyset_scalar_sum(soa_batch in, const uint32_t* __restrict__ key_idx,
+                                                                      const uint32_t* __restrict__ scalars,
+                                                                      unsigned long long* __restrict__ cols) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    size_t n = in.n;
+    int lane = threadIdx.x & 31;
+    bool live = i < n && !(in.flags[i] & FL_MALFORMED);   // every lane stays for the warp-wide match below
+    uint32_t k = live ? key_idx[i] : 0xffffffffu;           // a live index is inside the set (k_keyset_gather)
+    uint4 a = make_uint4(0, 0, 0, 0), b = a;
+    if (live) {
+        const uint4* t = reinterpret_cast<const uint4*>(scalars + (n + i) * 8);
+        a = t[0];
+        b = t[1];
+    }
+    uint32_t v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+    unsigned grp = __match_any_sync(0xffffffffu, k);
+    bool leader = lane == __ffs(grp) - 1;
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+        unsigned lo = __reduce_add_sync(grp, v[j] & 0xffffu), hi = __reduce_add_sync(grp, v[j] >> 16);
+        if (live && leader) atomicAdd(&cols[(size_t)k * 8 + j], (unsigned long long)lo + ((unsigned long long)hi << 16));
+    }
+}
+
+// c_k (-P_k) for every key with a non-zero sum: one warp per key, lane i adds window i of the key's table
+// (keyset_window_term), a shuffle tree of exact additions folds the 32 addends (the pattern of warp_fixed_base_affine).
+// Warps stride over the keys and keep a running sum; each block writes the sum of its warps as one Jacobian term
+// (18 u64, the layout k_batch_small_reduce adds up).  A zero sum needs no table: keys without one (the identity, status
+// KEY_MALFORMED) only ever have zero sums, because their items contribute t_i = 0 or nothing.
+static_assert(KT_WINDOWS <= 32, "one window per lane");
+static constexpr int KEYTERM_THREADS = 128;
+__global__ void __launch_bounds__(KEYTERM_THREADS) k_keyset_batch_term(size_t n_keys, const unsigned long long* __restrict__ cols,
+                                                                       const uint64_t* __restrict__ ktab,
+                                                                       uint64_t* __restrict__ terms) {
+    __shared__ jac_pt s_warp[KEYTERM_THREADS / 32];
+    int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t wpb = KEYTERM_THREADS / 32;
+    jf_pt acc = jf_identity();   // lane 0: the running sum of this warp's keys
+#pragma unroll 1
+    for (size_t k = blockIdx.x * wpb + warp; k < n_keys; k += gridDim.x * wpb) {
+        uint64_t col[8];
+#pragma unroll
+        for (int j = 0; j < 8; j++) col[j] = cols[k * 8 + j];
+        scalar c = keyset_sum_reduce(col);
+        if (sc_is_zero(c)) continue;   // warp-uniform
+        jf_pt t = lane < KT_WINDOWS ? keyset_window_term(c, lane, ktab + k * KT_KEY_U64) : jf_identity();
+#pragma unroll 1
+        for (int d = 16; d >= 1; d >>= 1) {
+            jf_pt o = shfl_down_jf(t, d);
+            if (lane + d >= 32) o.w = 0;
+            jf_add_exact(&t, &o);
+        }
+        if (lane == 0) jf_add_exact(&acc, &t);
+    }
+    if (lane == 0) store_jf_as_jac(&s_warp[warp], acc);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+#pragma unroll 1
+        for (int w = 1; w < KEYTERM_THREADS / 32; w++) {
+            jf_pt t = load_jac_as_jf(&s_warp[w]);
+            jf_add_exact(&acc, &t);
+        }
+        store_jf_as_jac(reinterpret_cast<jac_pt*>(terms) + blockIdx.x, acc);
+    }
+}
+
+// out = a + b as 192-byte partials: point sum (exact), scalar sum mod q, bad flags or-ed.  Joins the MSM partial of a
+// registered batch and its key side.  out may alias a or b.
+__global__ void __launch_bounds__(32) k_partial_add(const uint64_t* __restrict__ a, const uint64_t* __restrict__ b,
+                                                    uint64_t* out) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    jac_pt p, q;
+#pragma unroll
+    for (int c = 0; c < 6; c++) {
+        p.X.c[c] = a[c];
+        p.Y.c[c] = a[6 + c];
+        p.Z.c[c] = a[12 + c];
+        q.X.c[c] = b[c];
+        q.Y.c[c] = b[6 + c];
+        q.Z.c[c] = b[12 + c];
+    }
+    scalar lin = sc_add(sc_from_u64x4(a[18], a[19], a[20], a[21]), sc_from_u64x4(b[18], b[19], b[20], b[21]));
+    uint64_t bad = (a[22] | b[22]) != 0;
+    jac_add_mem(&p, &q, false);
+#pragma unroll
+    for (int c = 0; c < 6; c++) {
+        out[c] = p.X.c[c];
+        out[6 + c] = p.Y.c[c];
+        out[12 + c] = p.Z.c[c];
+    }
+#pragma unroll
+    for (int c = 0; c < 4; c++) out[18 + c] = sc_u64(lin, c);
+    out[22] = bad;
+    out[23] = 0;
+}
+
+// key side of a registered batch (batch_partial_impl): the device buffers and the geometry of its launches
+struct reg_batch {
+    const uint32_t* key_idx;   // [n] device
+    size_t n_keys;
+    const uint64_t* ktab;      // the set's tables on this device
+    unsigned long long* cols;  // [n_keys][8] column sums (zeroed by batch_partial_impl)
+    uint64_t* terms;           // [term_blocks][18]
+    unsigned term_blocks;
+    uint64_t* key_partial;     // 192 B
+    uint64_t* msm_partial;     // 192 B
+    const uint32_t* zero;      // 64 zero bytes: the key partial's scalar sum and bad flag
+};
+
 // ---- host orchestration ----------------------------------------------------------------------
 // rhs_pre (optional, device, 13 x u64): single-device batches get (sum s_i e_i) G computed on the second stream beside the
 // MSM; the caller's finish kernel must wait on ctx->ev_aux
+// reg (optional): a batch against a registered key set (pk96 = the gathered records of its items): the MSM runs over the
+// n points R_i, the key terms c_k (-P_k) are computed on the second stream beside it and added to the MSM's partial
 static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
                               const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off,
-                              const uint8_t* rand32, uint8_t* partial192, uint64_t* rhs_pre = nullptr) {
+                              const uint8_t* rand32, uint8_t* partial192, uint64_t* rhs_pre = nullptr,
+                              const reg_batch* reg = nullptr) {
     soa_batch soa;
     if (int rc = alloc_soa(ctx, n, &soa)) return rc;
-    if (n <= ctx->batch_small_max) {   // one thread block per signature (latency), see k_batch_small
+    if (n <= ctx->batch_small_max && !reg) {   // one thread block per signature (latency), see k_batch_small
         void *d_terms, *d_lin, *d_small;
         if (int rc = ensure_scratch(ctx, SL_D, n * 18 * 8, &d_terms)) return rc;
         if (int rc = ensure_scratch(ctx, SL_F, n * 32 + 512 * 32, &d_lin)) return rc;
@@ -1076,12 +1198,13 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
         ctx->last_msm_c = 4;
         ctx->last_msm_K = SMALL_WINDOWS;
         ctx->last_msm_T = 0;
+        ctx->last_batch_points = 0;
         ctx->launches += 5;
         CUDA_TRY(ctx, cudaGetLastError());
         return SCHNORR_B200_OK;
     }
-    size_t npts = 2 * n;
-    if (npts >= 0x7fffffffu) {
+    size_t npts = reg ? n : 2 * n;   // k_batch_prepare writes 2n points and scalars either way
+    if (2 * n >= 0x7fffffffu) {
         ctx->err = "batch too large for 31-bit point indices";
         return SCHNORR_B200_EARG;
     }
@@ -1092,8 +1215,8 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     }
     size_t nslots = (size_t)pl.K * (pl.B + 1);
     void *d_pts, *d_sc, *d_lin, *d_cnt, *d_sorted, *d_buckets, *d_small;
-    if (int rc = ensure_scratch(ctx, SL_D, npts * 96, &d_pts)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, npts * 32, &d_sc)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_D, 2 * n * 96, &d_pts)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_E, 2 * n * 32, &d_sc)) return rc;
     if (int rc = ensure_scratch(ctx, SL_F, n * 32 + 512 * 32, &d_lin)) return rc;
     size_t scan_tiles_max = (nslots + SCAN_TILE - 1) / SCAN_TILE;
     if (int rc = ensure_scratch(ctx, SL_G, nslots * 4 * 3 + 4 * scan_tiles_max + 64, &d_cnt)) return rc;
@@ -1111,6 +1234,7 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     ctx->last_msm_c = pl.c;
     ctx->last_msm_K = pl.K;
     ctx->last_msm_T = T;
+    ctx->last_batch_points = npts;
     size_t nseg = ((max_entries + T - 1) / T + 127) / 128 * 128;
     void* d_parts;
     size_t max_long = nseg / MSM_LONG_SPAN + 1;  // buckets that can span >= MSM_LONG_SPAN segments
@@ -1131,6 +1255,7 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     cudaStream_t st = ctx->stream;
     CUDA_TRY(ctx, cudaMemsetAsync(d_cnt, 0, nslots * 4 * 3, st));
     CUDA_TRY(ctx, cudaMemsetAsync(d_small, 0, 64, st));
+    if (reg) CUDA_TRY(ctx, cudaMemsetAsync(reg->cols, 0, reg->n_keys * 8 * sizeof(unsigned long long), st));
     k_ingest<<<grid_for(n, INGEST_THREADS), INGEST_THREADS, 0, st>>>(n, sigs81, pk96, pk_inf, soa);
     uint32_t* h_pre = nullptr;
     // Challenges on six lanes per signature (k_batch_challenge_dist) ahead of a hash-free k_batch_prepare: up to a few
@@ -1148,12 +1273,23 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     if (sum_blocks > 256) sum_blocks = 256;
     k_scalar_sum<<<sum_blocks, 256, 0, st>>>(lin, n, lin_part);
     k_scalar_sum<<<1, 256, 0, st>>>(lin_part, (size_t)sum_blocks, lin_total);
-    if (rhs_pre) {
+    if (rhs_pre || reg) {
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_chunk[1], st));
         CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_chunk[1], 0));
-        k_lin_times_g<<<1, 32, 0, ctx->aux_stream>>>(lin_total, ctx->gtab, rhs_pre);
+        if (rhs_pre) {
+            k_lin_times_g<<<1, 32, 0, ctx->aux_stream>>>(lin_total, ctx->gtab, rhs_pre);
+            ctx->launches += 1;
+        }
+        if (reg) {   // the key side: per-key scalar sums, key terms, their sum as a partial
+            k_keyset_scalar_sum<<<grid_for(n, KEYSUM_THREADS), KEYSUM_THREADS, 0, ctx->aux_stream>>>(soa, reg->key_idx,
+                                                                                                  (uint32_t*)d_sc, reg->cols);
+            k_keyset_batch_term<<<reg->term_blocks, KEYTERM_THREADS, 0, ctx->aux_stream>>>(reg->n_keys, reg->cols, reg->ktab,
+                                                                                            reg->terms);
+            k_batch_small_reduce<<<1, SMALL_REDUCE_THREADS, 0, ctx->aux_stream>>>(reg->term_blocks, reg->terms, reg->zero,
+                                                                                   (const int*)reg->zero, reg->key_partial);
+            ctx->launches += 3;
+        }
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_aux, ctx->aux_stream));
-        ctx->launches += 1;
     }
     k_msm_count<<<grid_for(npts, 256), 256, 0, st>>>((uint32_t*)d_sc, npts, pl, counts);
     unsigned scan_tiles = (unsigned)((nslots + SCAN_TILE - 1) / SCAN_TILE);
@@ -1174,11 +1310,22 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
         pl, T, offsets, counts, (seg_partial*)d_parts, buckets, long_list, long_count);
     k_msm_window_sum<<<grid_for((size_t)pl.K * pl.chunks, DIST_SIGS_PER_BLOCK), DIST_THREADS, 0, st>>>(pl, buckets, chunk_out);
     k_msm_window_fold<<<pl.K, FOLD_THREADS, 0, st>>>(pl, chunk_out, windows);
-    k_msm_horner<<<1, 32, 0, st>>>(pl, windows, lin_total, bad, (uint64_t*)partial192);
+    k_msm_horner<<<1, 32, 0, st>>>(pl, windows, lin_total, bad, reg ? reg->msm_partial : (uint64_t*)partial192);
     ctx->launches += 14;
+    if (reg) {
+        CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_aux, 0));
+        k_partial_add<<<1, 32, 0, st>>>(reg->msm_partial, reg->key_partial, (uint64_t*)partial192);
+        ctx->launches += 1;
+    }
     CUDA_TRY(ctx, cudaGetLastError());
     return SCHNORR_B200_OK;
 }
+
+// multi.cuh: a batch over every device of a multi-device context; partial(k, slice, rebased offsets, partial192) reduces
+// the non-empty slice of shard k to its partial on that shard's device
+template <typename F>
+static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* msg_off, int* verdict, uint8_t* lhs97,
+                              uint8_t* rhs97, F partial);
 
 extern "C" {
 
@@ -1189,6 +1336,7 @@ int schnorr_b200_batch_partial_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_
     NOT_ON_MULTI(ctx);
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     if (n == 0) {  // empty slice: identity point, zero scalar
+        ctx->last_batch_points = 0;
         uint64_t h[24] = {0};
         h[0] = 1;
         h[6] = 1;
@@ -1415,15 +1563,16 @@ static int batch_partial_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
                               (uint8_t*)d_rand, partial, rhs_pre);
 }
 
-static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
-                              const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
-                              int* verdict, uint8_t* lhs97, uint8_t* rhs97);
-
 int schnorr_b200_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
                               const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
                               int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
     if (!ctx || !verdict || (n && (!sigs81 || !pk96 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
-    if (!ctx->shards.empty()) return multi_verify_batch(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, verdict, lhs97, rhs97);
+    if (!ctx->shards.empty())
+        return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
+            return batch_partial_host(ctx->shards[k], s.hi - s.lo, sigs81 + 81 * s.lo, pk96 + 96 * s.lo,
+                                      pk_inf ? pk_inf + s.lo : nullptr, msgs ? msgs + msg_off[s.lo] : nullptr, off,
+                                      rand32 + 32 * s.lo, partial);
+        });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     void* d_res;
     if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;

@@ -143,4 +143,57 @@ SB_DEV uint8_t reg_verdict(uint8_t status, bool x_ok, int fr, const jf_pt& r, co
     return fp6_eq(r.X, fp6_scale(sig_x, fp_sqr_nc(r.w))) ? VERDICT_OK : VERDICT_INVALID_SIGNATURE;
 }
 
+// ---- batch verification against registered keys (src/batch.rs:84-130) -------------------------------------------
+// The key side of the batch equation collapses to one term per distinct key:
+//     sum_i t_i (-P_key(i)) = sum_k c_k (-P_k),   t_i = s_i h_i mod q,   c_k = sum_{i: key(i) = k} t_i mod q.
+// Reducing the sum mod q is only valid for keys with [q]P_k = O (status KEY_OK): a set that holds a key of status
+// KEY_NOT_TORSION_FREE runs its batches on the per-signature points instead (schnorr_b200.h).
+//
+// c_k from the 64-bit column sums col[j] = sum_i limb_j(t_i) of the eight 32-bit limbs.  Every column is below
+// n 2^32 with n < 2^32 items, so the carry chain stays within 64 bits and the value is lo + hi 2^256 with hi < 2^32:
+// c = (lo mod q) + hi 2^256 mod q, the second term a Montgomery product of hi with 2^512 mod q.
+SB_DEV scalar keyset_sum_reduce(const uint64_t* col) {
+    scalar lo, hi = sc_zero(), r2;
+    uint64_t carry = 0;
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+        uint64_t v = col[j] + carry;  // col[j] <= (2^32 - 1)^2 and carry < 2^32: no wrap
+        lo.l[j] = (uint32_t)v;
+        carry = v >> 32;
+    }
+    hi.l[0] = (uint32_t)carry;
+#pragma unroll
+    for (int j = 0; j < 8; j++) r2.l[j] = SB_CONST_R2(j);
+    return sc_add(sc_from_u256(lo), sc_montmul(hi, r2));
+}
+
+// The addend of window `window` (< KT_WINDOWS) of c (-P) from the key's table: the signed digit recoded as in
+// jf_table_accumulate, entry |d| of that window, negated for a positive digit.  The identity (w = 0) for d = 0.
+SB_DEV jf_pt keyset_window_term(const scalar& c, int window, const uint64_t* __restrict__ ktab_key) {
+    int carry = 0, d = 0;
+    bool neg = false;
+#pragma unroll 1
+    for (int i = 0; i <= window; i++) {
+        int raw = (int)sc_bits(c, KT_W * i, KT_W) + carry;
+        neg = raw > (1 << (KT_W - 1));
+        carry = neg ? 1 : 0;
+        d = neg ? (1 << KT_W) - raw : raw;
+    }
+    jf_pt t;
+    t.X = fp6_one();
+    t.Y = fp6_one();
+    t.w = 0;
+    if (d) {
+        const uint64_t* ent = ktab_key + ((size_t)window * KT_ENTRIES + d) * 12;
+#pragma unroll
+        for (int k = 0; k < 6; k++) {
+            t.X.c[k] = ent[k];
+            t.Y.c[k] = ent[6 + k];
+        }
+        if (!neg) t.Y = fp6_neg(t.Y);
+        t.w = 1;
+    }
+    return t;
+}
+
 }  // namespace sb

@@ -115,11 +115,12 @@ static int multi_sign_many(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sk32,
     });
 }
 
-// verify_batch over all devices: per-shard partials, one peer copy each, finish on the first device.
-// A batch always uses every shard slice it is given (an empty slice contributes the identity).
-static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
-                              const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
-                              int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+// verify_batch (and its registered-key-set form) over all devices: per-shard partials from `partial_fn`, one peer copy
+// each, finish on the first device.  A batch always uses every shard slice it is given (an empty slice contributes the
+// identity).
+template <typename F>
+static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* msg_off, int* verdict, uint8_t* lhs97,
+                              uint8_t* rhs97, F partial_fn) {
     if (n) CHECK_MSG_OFF(ctx, n, msg_off);
     auto sl = multi_slices(ctx, n);
     size_t g = sl.size();
@@ -150,8 +151,7 @@ static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
             r = batch_partial_host(sh, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, partial);
         } else {
             auto off = rebase_offsets(msg_off, s.lo, s.hi);
-            r = batch_partial_host(sh, cn, sigs81 + 81 * s.lo, pk96 + 96 * s.lo, pk_inf ? pk_inf + s.lo : nullptr,
-                                   msgs ? msgs + msg_off[s.lo] : nullptr, off.data(), rand32 + 32 * s.lo, partial);
+            r = partial_fn(k, s, off.data(), partial);
             // `off` must outlive the asynchronous copy that reads it: synchronise before it goes out of scope
             if (r == 0 && cudaStreamSynchronize(sh->stream) != cudaSuccess) r = SCHNORR_B200_ECUDA;
         }
@@ -169,6 +169,9 @@ static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
         return (int)SCHNORR_B200_OK;
     });
     if (rc) return rc;
+    ctx->last_batch_points = 0;
+    for (size_t k = 0; k < g; k++)
+        if (sl[k].hi > sl[k].lo) ctx->last_batch_points += ctx->shards[k]->last_batch_points;
     CUDA_TRY(root, cudaSetDevice(root->device));
     if (int r = schnorr_b200_batch_finish_dev(root, g, gathered, res)) {
         ctx->err = root->err;

@@ -35,8 +35,18 @@ using namespace sb;
 // context
 // ------------------------------------------------------------------------------------------------
 static constexpr size_t GTAB_U64 = (size_t)GTAB_WINDOWS * GTAB_ENTRIES * 12;
+// Batches against a registered key set sum the key side per key (one table product per key instead of one MSM point
+// per signature) when they hold at least this many signatures per key of the set; others run the per-signature
+// pipeline on the gathered key records (schnorr_b200_set_registered_batch_threshold).  Measured on a B200 (1000 W,
+// 1965 MHz; profiles/r4_registered_batch.md), summed per key against per signature: 64 per key wins at every size
+// (2^12 / 64 keys 0.89 against 0.91 ms, 2^16 / 1024 keys 2.31 against 2.51 ms, 2^20 / 16 384 keys 20.9 against
+// 23.0 ms), 16 per key loses (2^10 / 64 keys 0.82 against 0.80 ms), 4 per key loses (2^16 / 16 384 keys 2.83
+// against 2.51 ms): the key terms of a warp per key cost more than the MSM points they remove.
+static constexpr size_t REG_BATCH_MIN_PER_KEY = 64;
 
-enum scratch_slot { SL_A = 0, SL_B, SL_C, SL_D, SL_E, SL_F, SL_G, SL_H, SL_I, SL_J, SL_K, SL_L, SL_M, SL_COUNT };
+// N, O: batches against registered key sets (gathered key records; key-side accumulators and terms), which run
+// batch_partial_impl (A-G, I-L) on inputs staged in H or M
+enum scratch_slot { SL_A = 0, SL_B, SL_C, SL_D, SL_E, SL_F, SL_G, SL_H, SL_I, SL_J, SL_K, SL_L, SL_M, SL_N, SL_O, SL_COUNT };
 
 struct schnorr_b200_ctx {
     int device = 0;
@@ -57,6 +67,8 @@ struct schnorr_b200_ctx {
     uint32_t msm_t_override = 0;
     int last_msm_c = 0, last_msm_K = 0;             // Pippenger geometry of the last batch call (schnorr_b200_last_batch_plan)
     uint32_t last_msm_T = 0;
+    uint64_t last_batch_points = 0;                 // MSM points of the last batch call (schnorr_b200_last_batch_points)
+    size_t reg_batch_min_per_key = REG_BATCH_MIN_PER_KEY;
     size_t dist_max = 10240;                        // calls up to this many signatures use the six-lanes-per-signature kernel
     size_t one_max = 512;                           // ... and up to this many the block-per-signature kernel (one.cuh)
     size_t batch_dist_max = (size_t)1 << 18;        // batches up to this size hash their challenges on six lanes per signature
@@ -1124,6 +1136,17 @@ int schnorr_b200_last_batch_plan(const schnorr_b200_ctx* ctx, int* window_bits, 
     if (segment_len) *segment_len = c->last_msm_T;
     return SCHNORR_B200_OK;
 }
+int schnorr_b200_last_batch_points(const schnorr_b200_ctx* ctx, uint64_t* points) {
+    if (!ctx || !points) return SCHNORR_B200_EARG;
+    *points = ctx->last_batch_points;
+    return SCHNORR_B200_OK;
+}
+int schnorr_b200_set_registered_batch_threshold(schnorr_b200_ctx* ctx, size_t min_signatures_per_key) {
+    if (!ctx) return SCHNORR_B200_EARG;
+    ctx->reg_batch_min_per_key = min_signatures_per_key;
+    for (schnorr_b200_ctx* sh : ctx->shards) sh->reg_batch_min_per_key = min_signatures_per_key;
+    return SCHNORR_B200_OK;
+}
 int schnorr_b200_last_exact_count(schnorr_b200_ctx* ctx, uint64_t* count) {
     if (!ctx || !count) return SCHNORR_B200_EARG;
     *count = 0;
@@ -1373,6 +1396,7 @@ struct schnorr_b200_keyset {
     uint8_t* pk_inf = nullptr;  // [n_keys]
     uint8_t* status = nullptr;  // [n_keys] KEY_OK / KEY_NOT_TORSION_FREE / KEY_MALFORMED
     uint64_t* ktab = nullptr;   // [n_keys][KT_KEY_U64]; zeros for keys without a table
+    bool any_not_torsion_free = false;  // a key of status KEY_NOT_TORSION_FREE: batches use the per-signature points
     std::vector<schnorr_b200_keyset*> shards;
 };
 
@@ -1496,16 +1520,17 @@ int schnorr_b200_keyset_create(schnorr_b200_ctx* ctx, size_t n_keys, const uint8
     schnorr_b200_keyset* ks = new schnorr_b200_keyset();
     ks->ctx = ctx;
     ks->n_keys = n_keys;
+    std::vector<uint8_t> st(n_keys);
     int rc = 0;
     if (ctx->shards.empty()) {
-        rc = keyset_build(ctx, ks, pk96, pk_inf, status);
+        rc = keyset_build(ctx, ks, pk96, pk_inf, st.data());
     } else {  // one table per device; the status comes from the first (every shard computes the same)
         for (size_t k = 0; k < ctx->shards.size() && rc == 0; k++) {
             schnorr_b200_keyset* sh = new schnorr_b200_keyset();
             sh->ctx = ctx->shards[k];
             sh->n_keys = n_keys;
             ks->shards.push_back(sh);
-            rc = keyset_build(ctx->shards[k], sh, pk96, pk_inf, k == 0 ? status : nullptr);
+            rc = keyset_build(ctx->shards[k], sh, pk96, pk_inf, k == 0 ? st.data() : nullptr);
             if (rc) ctx->err = "device " + std::to_string(ctx->shards[k]->device) + ": " + ctx->shards[k]->err;
         }
     }
@@ -1513,6 +1538,11 @@ int schnorr_b200_keyset_create(schnorr_b200_ctx* ctx, size_t n_keys, const uint8
         keyset_free(ks);
         return rc;
     }
+    bool off_subgroup = false;
+    for (uint8_t v : st) off_subgroup |= v == KEY_NOT_TORSION_FREE;
+    ks->any_not_torsion_free = off_subgroup;
+    for (schnorr_b200_keyset* sh : ks->shards) sh->any_not_torsion_free = off_subgroup;
+    if (status) memcpy(status, st.data(), n_keys);
     *out = ks;
     return SCHNORR_B200_OK;
 }
@@ -1546,6 +1576,176 @@ int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx* ctx, const schnorr
     NOT_ON_MULTI(ctx);
     if (n == 0) return SCHNORR_B200_OK;
     return verify_registered_dev(ctx, ks, n, sigs81, key_idx, msgs, msg_off, verdicts);
+}
+
+}  // extern "C"
+
+// ---- batch verification against a registered key set (src/batch.rs:84-130) -------------------------------------------
+// The key side aggregated per key (batch.cuh: k_keyset_scalar_sum, k_keyset_batch_term, keyset.cuh) needs [q]P_k = O for
+// every key, and pays up to one table product per key of the set for the n MSM points it saves.  Otherwise the items'
+// key records are gathered and the batch runs the per-signature pipeline unchanged, as do batches small enough for
+// the block-per-signature kernel (k_batch_small, the latency form).
+static bool reg_batch_aggregates(const schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n) {
+    return n > ctx->batch_small_max && !ks->any_not_torsion_free && n / ks->n_keys >= ctx->reg_batch_min_per_key;
+}
+
+// one 192-byte partial of a registered batch on device buffers (single-device context, arguments checked)
+static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                    const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
+                                    uint8_t* partial192, uint64_t* rhs_pre) {
+    if (n == 0) return schnorr_b200_batch_partial_dev(ctx, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, partial192);
+    cudaStream_t st = ctx->stream;
+    const size_t sz_pk = (n * 96 + 255) & ~(size_t)255;
+    void* d_pk;
+    if (int rc = ensure_scratch(ctx, SL_N, sz_pk + n, &d_pk)) return rc;
+    uint8_t* d_inf = (uint8_t*)d_pk + sz_pk;
+    k_keyset_gather<<<grid_for(n, 128), 128, 0, st>>>(n, key_idx, ks->n_keys, ks->pk12, ks->pk_inf, (uint64_t*)d_pk, d_inf);
+    ctx->launches += 1;
+    if (!reg_batch_aggregates(ctx, ks, n))
+        return batch_partial_impl(ctx, n, sigs81, (uint8_t*)d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre);
+    // key side: column sums | per-block key terms | key partial | MSM partial | 64 zero bytes
+    size_t max_blocks = (size_t)2 * ctx->sm_count, want = (ks->n_keys + KEYTERM_THREADS / 32 - 1) / (KEYTERM_THREADS / 32);
+    unsigned blocks = (unsigned)(want < max_blocks ? want : max_blocks);
+    const size_t sz_cols = ks->n_keys * 8 * sizeof(unsigned long long), sz_terms = ((size_t)blocks * sizeof(jac_pt) + 255) & ~(size_t)255;
+    void* d_key;
+    if (int rc = ensure_scratch(ctx, SL_O, sz_cols + sz_terms + 192 + 192 + 64, &d_key)) return rc;
+    uint8_t* p = (uint8_t*)d_key;
+    reg_batch rb;
+    rb.key_idx = key_idx;
+    rb.n_keys = ks->n_keys;
+    rb.ktab = ks->ktab;
+    rb.cols = (unsigned long long*)p;
+    rb.terms = (uint64_t*)(p + sz_cols);
+    rb.term_blocks = blocks;
+    rb.key_partial = (uint64_t*)(p + sz_cols + sz_terms);
+    rb.msm_partial = rb.key_partial + 24;
+    rb.zero = (const uint32_t*)(rb.msm_partial + 24);
+    CUDA_TRY(ctx, cudaMemsetAsync((void*)rb.zero, 0, 64, st));
+    return batch_partial_impl(ctx, n, sigs81, (uint8_t*)d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre, &rb);
+}
+
+// host inputs (offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
+static int batch_partial_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                         const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
+                                         const uint8_t* rand32, uint8_t* partial, uint64_t* rhs_pre) {
+    if (n == 0) return batch_partial_registered(ctx, ks, 0, nullptr, nullptr, nullptr, nullptr, nullptr, partial, nullptr);
+    size_t mb = msg_off[n];
+    size_t sz_sig = (n * 81 + 255) & ~(size_t)255, sz_idx = (n * 4 + 255) & ~(size_t)255, sz_m = (mb + 255) & ~(size_t)255,
+           sz_off = ((n + 1) * 8 + 255) & ~(size_t)255;
+    void* blob;
+    if (int rc = ensure_scratch(ctx, SL_H, sz_sig + sz_idx + sz_m + sz_off + n * 32, &blob)) return rc;
+    uint8_t* p = (uint8_t*)blob;
+    uint8_t* d_sig = p; p += sz_sig;
+    uint8_t* d_idx = p; p += sz_idx;
+    uint8_t* d_m = p; p += sz_m;
+    uint8_t* d_off = p; p += sz_off;
+    uint8_t* d_rand = p;
+    cudaStream_t st = ctx->stream;
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_sig, sigs81, n * 81, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_idx, key_idx, n * 4, cudaMemcpyHostToDevice, st));
+    if (mb) CUDA_TRY(ctx, cudaMemcpyAsync(d_m, msgs, mb, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_off, msg_off, (n + 1) * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_rand, rand32, n * 32, cudaMemcpyHostToDevice, st));
+    return batch_partial_registered(ctx, ks, n, d_sig, (uint32_t*)d_idx, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
+}
+
+extern "C" {
+
+int schnorr_b200_verify_batch_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                         const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
+                                         const uint8_t* rand32, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    if (!ctx || !ks || !verdict || (n && (!sigs81 || !key_idx || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n) {
+        CHECK_MSG_OFF(ctx, n, msg_off);
+        if (msg_off[n] && !msgs) return SCHNORR_B200_EARG;
+    }
+    if (!ctx->shards.empty())
+        return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
+            return batch_partial_registered_host(ctx->shards[k], ks->shards[k], s.hi - s.lo, sigs81 + 81 * s.lo, key_idx + s.lo,
+                                                 msgs ? msgs + msg_off[s.lo] : nullptr, off, rand32 + 32 * s.lo, partial, nullptr);
+        });
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    void* d_res;
+    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
+    uint8_t* res = (uint8_t*)d_res + 64;
+    uint8_t* partial = res + RESULT_BYTES;
+    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;   // (sum s e) G computed beside the MSM
+    if (int rc = batch_partial_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand32, partial, rhs_pre)) return rc;
+    if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
+    k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, res, rhs_pre);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return read_result(ctx, res, verdict, lhs97, rhs97);
+}
+
+int schnorr_b200_verify_batch_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                             const uint8_t* sigs81, const uint32_t* key_idx, const uint8_t* msgs,
+                                             const uint64_t* msg_off, const uint8_t* rand32, uint8_t* result216) {
+    if (!ctx || !ks || !result216 || (n && (!sigs81 || !key_idx || !msgs || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    NOT_ON_MULTI(ctx);
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    void* d_res;
+    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
+    uint8_t* partial = (uint8_t*)d_res + 64 + RESULT_BYTES;
+    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;
+    if (int rc = batch_partial_registered(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand32, partial, rhs_pre)) return rc;
+    if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
+    k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, result216, rhs_pre);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return SCHNORR_B200_OK;
+}
+
+// localisation on the first device: the inputs staged in slot M, the items' key records gathered into slot N, then the
+// per-signature bisection of schnorr_b200_locate_invalid_dev (which uses neither slot)
+int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                           const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
+                                           const uint8_t* rand32, uint8_t* flags, uint64_t* n_bad) {
+    if (!ctx || !ks || (n && (!sigs81 || !key_idx || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n_bad) *n_bad = 0;
+    if (n == 0) return SCHNORR_B200_OK;
+    CHECK_MSG_OFF(ctx, n, msg_off);
+    size_t mb = msg_off[n];
+    if (mb && !msgs) return SCHNORR_B200_EARG;
+    schnorr_b200_ctx* c = ctx->shards.empty() ? ctx : ctx->shards[0];
+    const schnorr_b200_keyset* kc = ks->shards.empty() ? ks : ks->shards[0];
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    size_t sz_sig = (n * 81 + 255) & ~(size_t)255, sz_idx = (n * 4 + 255) & ~(size_t)255, sz_m = (mb + 255) & ~(size_t)255,
+           sz_off = ((n + 1) * 8 + 255) & ~(size_t)255, sz_rand = (n * 32 + 255) & ~(size_t)255;
+    void *blob, *recs;
+    const size_t sz_pk = (n * 96 + 255) & ~(size_t)255;
+    if (int rc = ensure_scratch(c, SL_M, sz_sig + sz_idx + sz_m + sz_off + sz_rand + n, &blob)) return rc;
+    if (int rc = ensure_scratch(c, SL_N, sz_pk + n, &recs)) return rc;
+    uint8_t* p = (uint8_t*)blob;
+    uint8_t* d_sig = p; p += sz_sig;
+    uint8_t* d_idx = p; p += sz_idx;
+    uint8_t* d_m = p; p += sz_m;
+    uint8_t* d_off = p; p += sz_off;
+    uint8_t* d_rand = p; p += sz_rand;
+    uint8_t* d_flags = p;
+    uint8_t* d_pk = (uint8_t*)recs;
+    uint8_t* d_inf = d_pk + sz_pk;
+    cudaStream_t st = c->stream;
+    CUDA_TRY(c, cudaMemcpyAsync(d_sig, sigs81, n * 81, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(c, cudaMemcpyAsync(d_idx, key_idx, n * 4, cudaMemcpyHostToDevice, st));
+    if (mb) CUDA_TRY(c, cudaMemcpyAsync(d_m, msgs, mb, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(c, cudaMemcpyAsync(d_off, msg_off, (n + 1) * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(c, cudaMemcpyAsync(d_rand, rand32, n * 32, cudaMemcpyHostToDevice, st));
+    k_keyset_gather<<<grid_for(n, 128), 128, 0, st>>>(n, (uint32_t*)d_idx, kc->n_keys, kc->pk12, kc->pk_inf, (uint64_t*)d_pk, d_inf);
+    c->launches += 1;
+    int rc = schnorr_b200_locate_invalid_dev(c, n, d_sig, d_pk, d_inf, d_m, (const uint64_t*)d_off, d_rand, d_flags);
+    if (rc) {
+        if (c != ctx) ctx->err = c->err;
+        return rc;
+    }
+    CUDA_TRY(c, cudaMemcpyAsync(flags, d_flags, n, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    if (n_bad)
+        for (size_t i = 0; i < n; i++) *n_bad += flags[i] != 0;
+    return SCHNORR_B200_OK;
 }
 
 // ---- keygen / sign ---------------------------------------------------------------------------

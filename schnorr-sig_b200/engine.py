@@ -126,6 +126,18 @@ class Engine:
         """Batches up to this size hash their challenges on six lanes per signature (0 = never)."""
         self._check(self._L.schnorr_b200_set_batch_dist_threshold(self._h, int(max_signatures)), "set_batch_dist_threshold")
 
+    def last_batch_points(self) -> int:
+        """MSM points of the last batch call: 2n for verify_batch, n for a registered batch summed per key, 0 for the
+        block-per-signature form of small batches."""
+        c = C.c_uint64(0)
+        self._check(self._L.schnorr_b200_last_batch_points(self._h, C.byref(c)), "last_batch_points")
+        return int(c.value)
+
+    def set_registered_batch_threshold(self, min_signatures_per_key: int):
+        """Registered batches sum the key side per key from this many signatures per key of the set (0 = always)."""
+        self._check(self._L.schnorr_b200_set_registered_batch_threshold(self._h, int(min_signatures_per_key)),
+                    "set_registered_batch_threshold")
+
     def last_exact_count(self) -> int:
         """Items of the last verify_many* call that the fast path handed to the exact kernel."""
         c = C.c_uint64(0)
@@ -232,6 +244,41 @@ class Engine:
                                                       _ptr(off), _ptr(rand32), C.byref(verdict), _ptr(lhs), _ptr(rhs)),
                     "verify_batch")
         return verdict.value, lhs, rhs
+
+    def _registered_batch_args(self, sigs81, key_idx, msgs, off, rand32):
+        sigs81, msgs, rand32 = _u8(sigs81, 81), _u8(msgs), _u8(rand32, 32)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = sigs81.shape[0]
+        if key_idx.ndim != 1:
+            raise ValueError("key_idx must be one-dimensional")
+        self._check_offsets(n, key_idx.shape[0], off, msgs)
+        if rand32.shape[0] != n:
+            raise AssertionError("one randomiser per signature")
+        return n, sigs81, key_idx, msgs, off, rand32
+
+    def verify_batch_registered(self, keyset, sigs81, key_idx, msgs, off, rand32):
+        """verify_batch of sigs81[i] over message i under key key_idx[i] of `keyset` -> (verdict, lhs97, rhs97), those of
+        verify_batch on the gathered keys (3 when an index is outside the set)."""
+        n, sigs81, key_idx, msgs, off, rand32 = self._registered_batch_args(sigs81, key_idx, msgs, off, rand32)
+        verdict = C.c_int(-1)
+        lhs = np.zeros(97, dtype=np.uint8)
+        rhs = np.zeros(97, dtype=np.uint8)
+        self._check(self._L.schnorr_b200_verify_batch_registered(self._h, keyset.handle, n, _ptr(sigs81), _ptr(key_idx),
+                                                                 _ptr(msgs), _ptr(off), _ptr(rand32), C.byref(verdict),
+                                                                 _ptr(lhs), _ptr(rhs)), "verify_batch_registered")
+        return verdict.value, lhs, rhs
+
+    def locate_invalid_registered(self, keyset, sigs81, key_idx, msgs, off, rand32):
+        """locate_invalid against a registered key set -> uint8[n] (3 for an index outside the set)."""
+        n, sigs81, key_idx, msgs, off, rand32 = self._registered_batch_args(sigs81, key_idx, msgs, off, rand32)
+        flags = np.zeros(n, dtype=np.uint8)
+        nb = C.c_uint64(0)
+        self._check(self._L.schnorr_b200_locate_invalid_registered(self._h, keyset.handle, n, _ptr(sigs81), _ptr(key_idx),
+                                                                   _ptr(msgs), _ptr(off), _ptr(rand32), _ptr(flags),
+                                                                   C.byref(nb)), "locate_invalid_registered")
+        assert int(nb.value) == int(np.count_nonzero(flags))
+        return flags
 
     def locate_invalid(self, sigs81, pk96, pk_inf, msgs, off, rand32):
         """Failed-batch localisation in batch semantics -> uint8[n]: 0 clean, 2 bad, 3 malformed (see the header)."""
@@ -391,6 +438,13 @@ class Engine:
         """Whole single-device batch on device buffers; result216 (device) = verdict | lhs97 | rhs97 (see the header)."""
         self._check(self._L.schnorr_b200_verify_batch_dev(self._h, n, _ptr(sigs81), _ptr(pk96), _ptr(pk_inf), _ptr(msgs),
                                                           _ptr(off), _ptr(rand32), _ptr(result216)), "verify_batch_dev")
+
+    def verify_batch_registered_dev(self, keyset, n, sigs81, key_idx, msgs, off, rand32, result216):
+        """Registered batch on device buffers (key_idx: n uint32), enqueued on the engine's stream, no synchronisation;
+        result216 as in verify_batch_dev."""
+        self._check(self._L.schnorr_b200_verify_batch_registered_dev(self._h, keyset.handle, n, _ptr(sigs81), _ptr(key_idx),
+                                                                     _ptr(msgs), _ptr(off), _ptr(rand32), _ptr(result216)),
+                    "verify_batch_registered_dev")
 
     def batch_partial_dev(self, n, sigs81, pk96, pk_inf, msgs, off, rand32, partial192):
         self._check(self._L.schnorr_b200_batch_partial_dev(self._h, n, _ptr(sigs81), _ptr(pk96), _ptr(pk_inf),
