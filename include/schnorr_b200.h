@@ -157,6 +157,38 @@ int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx *ctx, const schnorr
                                             const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
                                             const uint64_t *msg_off, uint8_t *verdicts);
 
+/* Compressed keys against a registered key set.  Registration also builds a sorted table of the set's encodings
+ * (PublicKey::to_bytes of key k, src/public.rs:49-51, exactly as schnorr_b200_compress writes it), searched on the device
+ * by binary search: at most log2(n_keys) + 1 probes whatever keys were registered.  Key k is FINDABLE when decompressing
+ * its encoding (PublicKey::from_bytes, src/public.rs:54-56) gives back its registered record byte for byte (the same 96
+ * bytes, the same identity flag).  Keys of status 3, points off the curve and an identity registered with non-zero
+ * coordinates are therefore not findable; keys of status 1 are.
+ *
+ * keyset_lookup: key_idx[i] = the smallest findable index whose encoding equals keys49[i] exactly, or 0xFFFFFFFF (any
+ * other 49 bytes miss, including undecodable encodings, flag bytes with bits 0x3f set and non-canonical limbs).  The
+ * indices feed verify_registered_many and verify_batch_registered.  The host form runs on the first device of a
+ * multi-device context; the _dev form (device buffers, no synchronisation) needs a single-device context. */
+int schnorr_b200_keyset_lookup(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n, const uint8_t *keys49,
+                               uint32_t *key_idx);
+int schnorr_b200_keyset_lookup_dev(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n, const uint8_t *keys49,
+                                   uint32_t *key_idx);
+/* KeyedSignature::from_bytes + KeyedSignature::verify (src/signature.rs:232-271) over n 130-byte wire records, against
+ * a registered key set: verdicts[i] is, byte for byte, what verify_keyed_many returns for record i.  A record whose key
+ * bytes are the encoding of a findable key k takes the registered path of verify_registered_many with key k (the
+ * decompressed key IS key k's record, so the verdict is verify_many's); every other record is decompressed and verified
+ * as verify_keyed_many does (verdict 3 where the key does not decode).  Calls of at most 384 records run
+ * verify_keyed_many.  Records whose key is not in the set cost more than in verify_keyed_many (the exact kernel): the
+ * host form reads the miss count and runs verify_many on the decoded records when more than 40 % of them miss; the
+ * _dev form does not synchronise and always takes the lookup path.  last_exact_count (misses count as exact items),
+ * last_kernel_ms and set_exact_only apply.  The host form shards a multi-device context in contiguous slices, each with
+ * that device's copy of the set; the _dev form needs a single-device context and a non-NULL msgs. */
+int schnorr_b200_verify_keyed_registered_many(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                              const uint8_t *keyed130, const uint8_t *msgs, const uint64_t *msg_off,
+                                              uint8_t *verdicts);
+int schnorr_b200_verify_keyed_registered_many_dev(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                                  const uint8_t *keyed130, const uint8_t *msgs, const uint64_t *msg_off,
+                                                  uint8_t *verdicts);
+
 /* KeyedSignature::from_bytes + KeyedSignature::verify over n 130-byte wire records
  * (49-byte compressed public key || 81-byte signature)   src/signature.rs:232-271, src/constants.rs:33
  * The key is decompressed on the device; a record whose key does not decode gets verdict 3. */

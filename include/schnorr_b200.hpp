@@ -70,6 +70,7 @@ inline Result result_from_verdict(int v) {
 }
 
 struct Signature;
+struct KeyedSignature;
 
 // PublicKey(AffinePoint): affine x || y little-endian limbs + identity flag (src/public.rs:24)
 struct PublicKey {
@@ -160,6 +161,26 @@ public:
                    "verify_registered_many");
         return result_from_verdict(verdict);
     }
+    // index of the key whose encoding is exactly `key49` and which decompresses to its registered record (the smallest
+    // such index; schnorr_b200_keyset_lookup), nullopt when there is none
+    std::optional<uint32_t> index_of(const std::array<uint8_t, PUBLIC_KEY_LENGTH>& key49) const {
+        uint32_t idx = UINT32_MAX;
+        eng_.check(schnorr_b200_keyset_lookup(eng_.get(), ks_, 1, key49.data(), &idx), "keyset_lookup");
+        if (idx == UINT32_MAX) return std::nullopt;
+        return idx;
+    }
+    std::optional<uint32_t> index_of(const PublicKey& key) const { return index_of(key.to_bytes()); }
+    // KeyedSignature::verify(message) (schnorr_b200_verify_keyed_registered_many): the registered path when the key is
+    // in the set, what KeyedSignature::verify gives otherwise; a key or scalar that does not decode throws
+    Result verify_keyed(const std::array<uint8_t, KEYED_SIGNATURE_LENGTH>& keyed, const std::vector<uint8_t>& message) const {
+        uint64_t off[2] = {0, message.size()};
+        uint8_t verdict = 255;
+        eng_.check(schnorr_b200_verify_keyed_registered_many(eng_.get(), ks_, 1, keyed.data(),
+                                                             message.empty() ? nullptr : message.data(), off, &verdict),
+                   "verify_keyed_registered_many");
+        return result_from_verdict(verdict);
+    }
+    Result verify_keyed(const KeyedSignature& keyed, const std::vector<uint8_t>& message) const;
     // verify_batch(signatures, [keys[i] for i in indices], messages, rng) with the key side summed per key of the set
     // (schnorr_b200_verify_batch_registered); an index outside the set makes the batch malformed, which throws
     Result verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
@@ -189,7 +210,19 @@ struct KeyedSignature {
     PublicKey public_key;
     Signature signature;
     Result verify(const std::vector<uint8_t>& message) const { return signature.verify(message, public_key); }
+    std::array<uint8_t, KEYED_SIGNATURE_LENGTH> to_bytes() const {
+        std::array<uint8_t, KEYED_SIGNATURE_LENGTH> out{};
+        auto k = public_key.to_bytes();
+        auto s = signature.to_bytes();
+        std::memcpy(out.data(), k.data(), PUBLIC_KEY_LENGTH);
+        std::memcpy(out.data() + PUBLIC_KEY_LENGTH, s.data(), SIGNATURE_LENGTH);
+        return out;
+    }
 };
+
+inline Result KeySet::verify_keyed(const KeyedSignature& keyed, const std::vector<uint8_t>& message) const {
+    return verify_keyed(keyed.to_bytes(), message);
+}
 
 // rng(buf, len) fills len random bytes (CryptoRng + RngCore).  One full-width random scalar is drawn
 // per signature (src/batch.rs:75-78); 32 bytes with the top two bits cleared are uniform below 2^254 < q.

@@ -38,6 +38,10 @@ _SIGNATURES = {
     "schnorr_b200_keyset_destroy": (None, [C.c_void_p]),
     "schnorr_b200_verify_registered_many": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 5),
     "schnorr_b200_verify_registered_many_dev": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 5),
+    "schnorr_b200_keyset_lookup": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _u8p, _u8p]),
+    "schnorr_b200_keyset_lookup_dev": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _u8p, _u8p]),
+    "schnorr_b200_verify_keyed_registered_many": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 4),
+    "schnorr_b200_verify_keyed_registered_many_dev": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 4),
     "schnorr_b200_verify_keyed_many":(C.c_int, [C.c_void_p, _sz] + [_u8p] * 4),
     "schnorr_b200_verify_keyed_many_dev": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 4),
     "schnorr_b200_verify_batch": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 6 + [C.POINTER(C.c_int), _u8p, _u8p]),

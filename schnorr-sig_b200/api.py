@@ -208,6 +208,24 @@ class KeySet:
         v = default_engine().verify_registered_many(self._handle, sig, idx, blob, off)
         return _result_from_verdict(int(v[0]))
 
+    def index_of(self, public_key):
+        """Index of `public_key` (a PublicKey or its 49-byte encoding) in the set: the smallest index of a key whose
+        encoding is exactly those bytes and which decompresses to its registered record; None when there is none."""
+        b = public_key.to_bytes() if isinstance(public_key, PublicKey) else bytes(public_key)
+        assert len(b) == PUBLIC_KEY_LENGTH
+        k = int(default_engine().keyset_lookup(self._handle, np.frombuffer(b, dtype=np.uint8).reshape(1, 49))[0])
+        return None if k == 0xFFFFFFFF else k
+
+    def verify_keyed(self, keyed, message: bytes) -> Result:
+        """KeyedSignature::verify(message) for a KeyedSignature or its 130 bytes: the registered path when the key is in
+        the set, what KeyedSignature.verify gives otherwise; a record whose key or scalar does not decode panics."""
+        b = keyed.to_bytes() if isinstance(keyed, KeyedSignature) else bytes(keyed)
+        assert len(b) == KEYED_SIGNATURE_LENGTH
+        blob, off = _pack([message])
+        v = default_engine().verify_keyed_registered_many(self._handle, np.frombuffer(b, dtype=np.uint8).reshape(1, 130),
+                                                           blob, off)
+        return _result_from_verdict(int(v[0]))
+
     def _batch_inputs(self, indices, signatures, messages, rng):
         n = len(signatures)
         assert len(indices) == n, "We should have the same number of signatures than public keys"

@@ -8,6 +8,8 @@
 // Public keys are public data: the tables are indexed by the challenge digits and are not constant-time (DESIGN.md §7).
 // Written once and instantiated by the CUDA kernels (schnorr_b200.cu) and by the host test build (tests/hostsim).
 #pragma once
+#include <algorithm>
+
 #include "verify.cuh"
 
 namespace sb {
@@ -141,6 +143,86 @@ SB_DEV uint8_t reg_verdict(uint8_t status, bool x_ok, int fr, const jf_pt& r, co
     if (!x_ok) return VERDICT_MALFORMED;
     if (fr == FAST_EXCEPTIONAL) return VERDICT_NEEDS_EXACT;
     return fp6_eq(r.X, fp6_scale(sig_x, fp_sqr_nc(r.w))) ? VERDICT_OK : VERDICT_INVALID_SIGNATURE;
+}
+
+// ---- lookup of compressed keys (KeyedSignature records, src/signature.rs:232-271) --------------------------------
+// The encoding of a registered key is compress(pk, inf), the 49 bytes k_compress writes: the x limbs (zeros for the
+// identity) and the flag byte.  A key is findable when decompressing its encoding (src/public.rs:54-56) gives back its
+// registered record exactly, so a hit can take the registered record in place of the decompressed one.  That one rule
+// leaves out non-canonical limbs (they do not decode), points off the curve (y does not round-trip) and an identity
+// registered with non-zero coordinates.  The lookup table holds the findable encodings sorted by keyset_cmp, one entry
+// per distinct encoding (the smallest index); a query is a binary search: log2(entries) + 1 probes whatever the keys.
+static constexpr uint32_t KEYSET_MISS = 0xFFFFFFFFu;
+struct keyset_entry {  // 64 bytes: one aligned line pair per probe
+    uint64_t x[6];
+    uint32_t flag;
+    uint32_t index;
+    uint64_t pad;
+};
+static_assert(sizeof(keyset_entry) == 64, "lookup entries are 64 bytes");
+
+// the encoding of (pk12, inf) into x6 / flag; returns whether the key is findable
+SB_DEV bool keyset_encode(const uint64_t* pk12, bool inf, uint64_t* x6, uint8_t& flag) {
+    fp6 x, y;
+#pragma unroll
+    for (int k = 0; k < 6; k++) {
+        x.c[k] = inf ? 0 : pk12[k];
+        y.c[k] = pk12[6 + k];
+        x6[k] = x.c[k];
+    }
+    flag = compress_flags(y, inf);
+    fp6 ox, oy;
+    bool oinf;
+    bool same = decompress_point(x, flag, ox, oy, oinf) && oinf == inf;
+#pragma unroll
+    for (int k = 0; k < 6; k++) same &= ox.c[k] == pk12[k] && oy.c[k] == pk12[6 + k];
+    return same;
+}
+
+// order of the lookup table: limbs from the most significant, then the flag byte (< 0: the query sorts first).
+// Also compiled for the host, where the table is sorted (keyset_sort_entries).
+#if defined(__CUDACC__)
+__host__ __device__ __forceinline__
+#else
+static inline
+#endif
+int keyset_cmp(const uint64_t* x6, uint32_t flag, const keyset_entry* e) {
+#pragma unroll
+    for (int k = 5; k >= 0; k--) {
+        uint64_t v = e->x[k];
+        if (x6[k] != v) return x6[k] < v ? -1 : 1;
+    }
+    return flag == e->flag ? 0 : (flag < e->flag ? -1 : 1);
+}
+
+// index of the registered key whose encoding is exactly (x6, flag), or KEYSET_MISS: a lower-bound search over the
+// n_entries entries of `tab`
+SB_DEV uint32_t keyset_lookup(const keyset_entry* __restrict__ tab, uint32_t n_entries, const uint64_t* x6, uint32_t flag) {
+    uint32_t lo = 0, len = n_entries;
+#pragma unroll 1
+    while (len > 0) {
+        uint32_t half = len >> 1;
+        if (keyset_cmp(x6, flag, tab + lo + half) > 0) {
+            lo += half + 1;
+            len -= half + 1;
+        } else {
+            len = half;
+        }
+    }
+    return lo < n_entries && keyset_cmp(x6, flag, tab + lo) == 0 ? tab[lo].index : KEYSET_MISS;
+}
+
+// Host side of the table build: `entries` holds one entry per findable key (any order); sorts them and keeps the
+// smallest index of every encoding.  Returns the number of entries kept at the front.
+static inline size_t keyset_sort_entries(keyset_entry* entries, size_t n) {
+    std::sort(entries, entries + n, [](const keyset_entry& a, const keyset_entry& b) {
+        int c = keyset_cmp(a.x, a.flag, &b);
+        return c != 0 ? c < 0 : a.index < b.index;
+    });
+    size_t m = 0;
+    for (size_t i = 0; i < n; i++)
+        if (m == 0 || keyset_cmp(entries[i].x, entries[i].flag, &entries[m - 1]) != 0) entries[m++] = entries[i];
+    return m;
 }
 
 // ---- batch verification against registered keys (src/batch.rs:84-130) -------------------------------------------

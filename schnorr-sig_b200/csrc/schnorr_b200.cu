@@ -10,6 +10,10 @@
 //   k_keyset_register     registration of a key set (status + subgroup check per key)
 //   k_keyset_gather       key records of the items of a registered call (ahead of k_ingest)
 //   k_verify_reg          Signature::verify against registered keys (table additions, no doubling chain)
+//   k_keyset_encode       the lookup table of a key set's compressed encodings (sorted on the host)
+//   k_keyset_lookup       compressed keys -> indices into a registered key set (binary search)
+//   k_keyed_split_lookup  KeyedSignature records against a registered key set: registered record on a hit, decompressed
+//                         key on a miss, ahead of k_ingest
 //   k_imad_peak       K6  integer-multiply roofline calibration
 //   batch kernels     K3/K4  in batch.cuh (Pippenger MSM)
 // No CPU fallback exists: every entry point needs a live CUDA context.
@@ -693,11 +697,79 @@ __global__ void __launch_bounds__(128) k_keyset_gather(size_t n, const uint32_t*
     for (int c = 0; c < 12; c++) pk12[12 * i + c] = in ? ks_pk12[12 * (size_t)k + c] : ~0ULL;
     pk_inf[i] = in ? ks_inf[k] : 0;
 }
+// one thread per key: the key's lookup entry (keyset_encode) and whether it is findable
+__global__ void __launch_bounds__(128) k_keyset_encode(size_t n_keys, const uint64_t* __restrict__ pk12,
+                                                       const uint8_t* __restrict__ pk_inf, keyset_entry* __restrict__ entries,
+                                                       uint8_t* __restrict__ findable) {
+    size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_keys) return;
+    keyset_entry e;
+    uint8_t flag;
+    findable[k] = keyset_encode(pk12 + 12 * k, pk_inf[k] != 0, e.x, flag) ? 1 : 0;
+    e.flag = flag;
+    e.index = (uint32_t)k;
+    e.pad = 0;
+    entries[k] = e;
+}
+// 49-byte compressed keys -> index of the registered key with exactly that encoding, or KEYSET_MISS
+__global__ void __launch_bounds__(128) k_keyset_lookup(size_t n, const uint8_t* __restrict__ keys49,
+                                                       const keyset_entry* __restrict__ lut, uint32_t n_lut,
+                                                       uint32_t* __restrict__ key_idx) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint8_t* rec = keys49 + 49 * i;
+    uint64_t x[6];
+#pragma unroll
+    for (int k = 0; k < 6; k++) x[k] = load_u64_le(rec + 8 * k);
+    key_idx[i] = keyset_lookup(lut, n_lut, x, rec[48]);
+}
+// Front end of a keyed call against a registered set (KeyedSignature records, src/signature.rs:237-271): the
+// signature bytes, then the key searched in the set.  A hit writes the registered record (as k_keyset_gather) and the
+// key index; a miss decompresses the key as k_split_keyed does and writes KEYSET_MISS.  *miss_count += the misses.
+__global__ void __launch_bounds__(128) k_keyed_split_lookup(size_t n, const uint8_t* __restrict__ keyed130,
+                                                            const keyset_entry* __restrict__ lut, uint32_t n_lut,
+                                                            const uint64_t* __restrict__ ks_pk12,
+                                                            const uint8_t* __restrict__ ks_inf, uint8_t* __restrict__ pk96,
+                                                            uint8_t* __restrict__ pk_inf, uint8_t* __restrict__ ok,
+                                                            uint8_t* __restrict__ sigs81, uint32_t* __restrict__ key_idx,
+                                                            uint32_t* __restrict__ miss_count) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool miss = false;
+    if (i < n) {
+        const uint8_t* rec = keyed130 + 130 * i;
+        fp6 x;
+#pragma unroll
+        for (int k = 0; k < 6; k++) x.c[k] = load_u64_le(rec + 8 * k);
+        uint32_t k = keyset_lookup(lut, n_lut, x.c, rec[48]);
+        miss = k == KEYSET_MISS;
+        if (!miss) {
+            uint64_t* o = reinterpret_cast<uint64_t*>(pk96 + 96 * i);
+#pragma unroll
+            for (int c = 0; c < 12; c++) o[c] = ks_pk12[12 * (size_t)k + c];
+            pk_inf[i] = ks_inf[k];
+            ok[i] = 1;
+        } else {
+            fp6 ox, oy;
+            bool inf;
+            bool good = decompress_point(x, rec[48], ox, oy, inf);
+            store_point96(pk96 + 96 * i, ox, oy);
+            pk_inf[i] = inf ? 1 : 0;
+            ok[i] = good ? 1 : 0;
+        }
+        key_idx[i] = k;
+        for (int c = 0; c < 81; c++) sigs81[81 * i + c] = rec[49 + c];
+    }
+    unsigned m = __ballot_sync(0xffffffffu, miss);   // every launch is a whole number of warps
+    if ((threadIdx.x & 31) == 0 && m) atomicAdd(miss_count, (unsigned)__popc(m));
+}
 
 // Signature::verify against registered keys: the shape of k_verify_fast (block-agreed challenge hash, stand-in inputs
 // for threads without work, the same verdicts and hand-back list), with h*P from the key's table instead of the
 // doubling chain and no subgroup check (the key's status).  Items handed back are finished by k_verify, which reads
 // the key k_keyset_gather placed in the planes.
+// LOOKUP: the items of a keyed call (k_keyed_split_lookup), where key_idx[i] == KEYSET_MISS marks a record whose key
+// is not in the set: it is handed to k_verify, which reads the key decompressed into the planes.
+template <bool LOOKUP>
 __global__ void __launch_bounds__(VERIFY_THREADS) k_verify_reg(soa_batch in, const uint32_t* __restrict__ key_idx,
                                                                const uint8_t* __restrict__ key_status,
                                                                const uint64_t* __restrict__ ktab,
@@ -713,6 +785,11 @@ __global__ void __launch_bounds__(VERIFY_THREADS) k_verify_reg(soa_batch in, con
     // a record that is not malformed has an index inside the set (k_keyset_gather)
     bool keyed = !(fl & (FL_MALFORMED | FL_PK_INF));
     uint32_t k = keyed ? key_idx[i] : 0;
+    bool miss = LOOKUP && k == KEYSET_MISS;
+    if (miss) {
+        keyed = false;
+        k = 0;
+    }
     uint8_t st = keyed ? key_status[k] : KEY_OK;
     bool work = keyed && st == KEY_OK;
     uint64_t off = work ? msg_off[i] : 0, len = work ? msg_off[i + 1] - off : 0;
@@ -744,6 +821,7 @@ __global__ void __launch_bounds__(VERIFY_THREADS) k_verify_reg(soa_batch in, con
     uint8_t v;
     if (fl & FL_MALFORMED) v = VERDICT_MALFORMED;
     else if (fl & FL_PK_INF) v = VERDICT_NEEDS_EXACT;   // the identity key is the exact kernel's business
+    else if (miss) v = VERDICT_NEEDS_EXACT;
     else v = reg_verdict(st, x_ok, fr, r, sx);
     verdicts[i] = v;
     if (v == VERDICT_NEEDS_EXACT) work_list[atomicAdd(work_count, 1u)] = (uint32_t)i;
@@ -1396,21 +1474,25 @@ struct schnorr_b200_keyset {
     uint8_t* pk_inf = nullptr;  // [n_keys]
     uint8_t* status = nullptr;  // [n_keys] KEY_OK / KEY_NOT_TORSION_FREE / KEY_MALFORMED
     uint64_t* ktab = nullptr;   // [n_keys][KT_KEY_U64]; zeros for keys without a table
+    keyset_entry* lut = nullptr;  // [n_lut] the findable encodings, sorted (keyset.cuh: keyset_lookup)
+    uint32_t n_lut = 0;
     bool any_not_torsion_free = false;  // a key of status KEY_NOT_TORSION_FREE: batches use the per-signature points
     std::vector<schnorr_b200_keyset*> shards;
 };
 
 static void keyset_free(schnorr_b200_keyset* ks) {
     for (schnorr_b200_keyset* sh : ks->shards) keyset_free(sh);
-    if (ks->pk12 || ks->ktab) {
+    if (ks->pk12 || ks->ktab || ks->lut) {
         cudaSetDevice(ks->device);
         cudaFree(ks->pk12);   // pk_inf and status live in the same allocation
         cudaFree(ks->ktab);
+        cudaFree(ks->lut);
     }
     delete ks;
 }
 
-// registration on one device: copies the records, k_keyset_register, the tables of the keys with status 0
+// registration on one device: copies the records, k_keyset_register, the tables of the keys with status 0, and the
+// lookup table of the encodings (k_keyset_encode; sorted on the host while the key tables are built)
 static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const uint8_t* pk96, const uint8_t* pk_inf,
                         uint8_t* status) {
     const size_t n = ks->n_keys;
@@ -1426,6 +1508,16 @@ static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const ui
     CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk12, pk96, n * 96, cudaMemcpyHostToDevice, ctx->stream));
     if (pk_inf) CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk_inf, pk_inf, n, cudaMemcpyHostToDevice, ctx->stream));
     else CUDA_TRY(ctx, cudaMemsetAsync(ks->pk_inf, 0, n, ctx->stream));
+    void* enc;  // lookup entries, then the findable flags
+    if (int rc = ensure_scratch(ctx, SL_E, n * (sizeof(keyset_entry) + 1), &enc)) return rc;
+    std::vector<keyset_entry> entries(n);
+    std::vector<uint8_t> findable(n);
+    k_keyset_encode<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, ks->pk12, ks->pk_inf, (keyset_entry*)enc,
+                                                              (uint8_t*)enc + n * sizeof(keyset_entry));
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaMemcpyAsync(entries.data(), enc, n * sizeof(keyset_entry), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(findable.data(), (uint8_t*)enc + n * sizeof(keyset_entry), n, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_aux, ctx->stream));
     void* tmp;  // skip flags, then the table bases
     size_t skip_bytes = (n + 15) / 16 * 16;
     if (int rc = ensure_scratch(ctx, SL_D, skip_bytes + n * KT_WINDOWS * sizeof(jac_pt), &tmp)) return rc;
@@ -1434,6 +1526,14 @@ static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const ui
     ctx->launches += 1;
     if (int rc = build_tables(ctx, n, ks->pk12, skip, KT_W, KT_WINDOWS, (jac_pt*)((uint8_t*)tmp + skip_bytes), ks->ktab)) return rc;
     if (status) CUDA_TRY(ctx, cudaMemcpyAsync(status, ks->status, n, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev_aux));
+    size_t m = 0;
+    for (size_t k = 0; k < n; k++)
+        if (findable[k]) entries[m++] = entries[k];
+    m = keyset_sort_entries(entries.data(), m);
+    ks->n_lut = (uint32_t)m;
+    CUDA_TRY(ctx, cudaMalloc(&ks->lut, (m ? m : 1) * sizeof(keyset_entry)));
+    if (m) CUDA_TRY(ctx, cudaMemcpyAsync(ks->lut, entries.data(), m * sizeof(keyset_entry), cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
 }
@@ -1445,7 +1545,9 @@ static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const ui
 static constexpr size_t REG_SMALL_MAX = 384;
 
 // the fast kernel over an ingested batch of registered items, then the exact kernel over the items it handed back;
-// exact_only and small calls go through launch_verify (same verdicts: the planes hold each item's key record)
+// exact_only and small calls go through launch_verify (same verdicts: the planes hold each item's key record).
+// LOOKUP: key_idx may hold KEYSET_MISS (k_keyed_split_lookup); those items are finished by k_verify.
+template <bool LOOKUP>
 static int launch_verify_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, const soa_batch& soa,
                                     const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     cudaStream_t st = ctx->stream;
@@ -1457,7 +1559,7 @@ static int launch_verify_registered(schnorr_b200_ctx* ctx, const schnorr_b200_ke
     CUDA_TRY(ctx, cudaMemsetAsync(counter, 0, 4, st));
     ctx->exact_counters_used = 1;
     unsigned grid = grid_for(soa.n, VERIFY_THREADS);
-    k_verify_reg<<<grid, VERIFY_THREADS, 0, st>>>(soa, key_idx, ks->status, ks->ktab, msgs, msg_off, ctx->gtab, verdicts, list, counter);
+    k_verify_reg<LOOKUP><<<grid, VERIFY_THREADS, 0, st>>>(soa, key_idx, ks->status, ks->ktab, msgs, msg_off, ctx->gtab, verdicts, list, counter);
     k_verify<<<grid, VERIFY_THREADS, 0, st>>>(soa, msgs, msg_off, ctx->gtab, verdicts, list, counter);
     ctx->launches += 2;
     return 0;
@@ -1477,7 +1579,7 @@ static int verify_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyse
     k_ingest<<<grid_for(n, INGEST_THREADS), INGEST_THREADS, 0, ctx->stream>>>(n, sigs81, (uint8_t*)d_pk, (uint8_t*)d_inf, soa);
     ctx->launches += 2;
     cudaEventRecord(ctx->ev_k0, ctx->stream);
-    if (int rc = launch_verify_registered(ctx, ks, soa, key_idx, msgs, msg_off, verdicts)) return rc;
+    if (int rc = launch_verify_registered<false>(ctx, ks, soa, key_idx, msgs, msg_off, verdicts)) return rc;
     cudaEventRecord(ctx->ev_k1, ctx->stream);
     CUDA_TRY(ctx, cudaGetLastError());
     return 0;
@@ -1576,6 +1678,142 @@ int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx* ctx, const schnorr
     NOT_ON_MULTI(ctx);
     if (n == 0) return SCHNORR_B200_OK;
     return verify_registered_dev(ctx, ks, n, sigs81, key_idx, msgs, msg_off, verdicts);
+}
+
+}  // extern "C"
+
+// ---- KeyedSignature records against a registered key set ----------------------------------------------------------
+// A record whose key is in the set takes k_verify_reg with the registered record; every other record (a miss) is
+// decompressed and finished by k_verify, the exact kernel, at about 1.8x the cost of k_verify_fast per item.  Host
+// calls whose miss fraction is above this run verify_many on the decoded records instead (the verdicts are the same).
+// Measured on a B200 (1000 W, 1965 MHz; profiles/r5_keyed_registered.md), 2^20 records, for 1 to 16 384 keys: the
+// lookup path takes 21.6-22.0 / 32.2-32.6 / 88.9-89.1 ms at 0 / 1/16 / 1/2 misses against 76.6-76.9 ms for
+// verify_keyed_many; the line between the last two points crosses it at 0.41.
+static constexpr double KEYED_REG_MAX_MISS_FRACTION = 0.4;
+
+// device buffers, single-device context, arguments checked by the caller.  `select`: read the miss count of the front
+// end (synchronises) and take verify_many above KEYED_REG_MAX_MISS_FRACTION.
+// Scratch: J decoded keys, K identity / ok flags | key indices | miss counter, L signatures (the slots of
+// verify_keyed_many_dev, which small calls run); the kernels after them use A-C and M.
+static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
+                                       const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts, bool select) {
+    if (n <= REG_SMALL_MAX) return schnorr_b200_verify_keyed_many_dev(ctx, n, keyed130, msgs, msg_off, verdicts);
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const size_t sz_flags = (2 * n + 255) & ~(size_t)255, sz_idx = (4 * n + 255) & ~(size_t)255;
+    void *d_pk, *d_k, *d_sig;
+    if (int rc = ensure_scratch(ctx, SL_J, n * 96, &d_pk)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_K, sz_flags + sz_idx + 16, &d_k)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_L, n * 81 + 256, &d_sig)) return rc;
+    uint8_t* d_inf = (uint8_t*)d_k;
+    uint8_t* d_ok = d_inf + n;
+    uint32_t* d_idx = (uint32_t*)((uint8_t*)d_k + sz_flags);
+    uint32_t* d_miss = (uint32_t*)((uint8_t*)d_k + sz_flags + sz_idx);
+    CUDA_TRY(ctx, cudaMemsetAsync(d_miss, 0, 4, st));
+    k_keyed_split_lookup<<<grid_for(n, 128), 128, 0, st>>>(n, keyed130, ks->lut, ks->n_lut, ks->pk12, ks->pk_inf, (uint8_t*)d_pk,
+                                                          d_inf, d_ok, (uint8_t*)d_sig, d_idx, d_miss);
+    ctx->launches += 1;
+    bool lookup_path = true;
+    if (select) {
+        uint32_t misses = 0;
+        CUDA_TRY(ctx, cudaMemcpyAsync(&misses, d_miss, 4, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(ctx, cudaStreamSynchronize(st));
+        lookup_path = misses <= KEYED_REG_MAX_MISS_FRACTION * (double)n;
+    }
+    if (lookup_path) {
+        soa_batch soa;
+        if (int rc = alloc_soa(ctx, n, &soa)) return rc;
+        k_ingest<<<grid_for(n, INGEST_THREADS), INGEST_THREADS, 0, st>>>(n, (uint8_t*)d_sig, (uint8_t*)d_pk, d_inf, soa);
+        ctx->launches += 1;
+        cudaEventRecord(ctx->ev_k0, st);
+        if (int rc = launch_verify_registered<true>(ctx, ks, soa, d_idx, msgs, msg_off, verdicts)) return rc;
+        cudaEventRecord(ctx->ev_k1, st);
+    } else if (int rc = schnorr_b200_verify_many_dev(ctx, n, (uint8_t*)d_sig, (uint8_t*)d_pk, d_inf, msgs, msg_off, verdicts)) {
+        return rc;
+    }
+    k_mask_verdicts<<<grid_for(n, 256), 256, 0, st>>>(n, d_ok, verdicts);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return 0;
+}
+
+// host buffers, single-device context: staged in D, F, G, verdicts in H, synchronised
+static int verify_keyed_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
+                                        const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    size_t mb = msg_off[n];
+    void *d_rec, *d_m, *d_off, *d_out;
+    if (int rc = stage_in(ctx, SL_D, keyed130, n * 130, &d_rec)) return rc;
+    if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
+    if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
+    if (int rc = verify_keyed_registered_dev(ctx, ks, n, (uint8_t*)d_rec, (uint8_t*)d_m, (uint64_t*)d_off, (uint8_t*)d_out, true))
+        return rc;
+    CUDA_TRY(ctx, cudaMemcpyAsync(verdicts, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+extern "C" {
+
+int schnorr_b200_keyset_lookup(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keys49,
+                               uint32_t* key_idx) {
+    if (!ctx || !ks || (n && (!keys49 || !key_idx))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n == 0) return SCHNORR_B200_OK;
+    schnorr_b200_ctx* c = ctx->shards.empty() ? ctx : ctx->shards[0];
+    const schnorr_b200_keyset* kc = ks->shards.empty() ? ks : ks->shards[0];
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    void *d_in, *d_out;
+    if (int rc = stage_in(c, SL_D, keys49, n * 49, &d_in)) return rc;
+    if (int rc = ensure_scratch(c, SL_H, n * 4, &d_out)) return rc;
+    k_keyset_lookup<<<grid_for(n, 128), 128, 0, c->stream>>>(n, (uint8_t*)d_in, kc->lut, kc->n_lut, (uint32_t*)d_out);
+    c->launches += 1;
+    CUDA_TRY(c, cudaGetLastError());
+    CUDA_TRY(c, cudaMemcpyAsync(key_idx, d_out, n * 4, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    return SCHNORR_B200_OK;
+}
+
+int schnorr_b200_keyset_lookup_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keys49,
+                                   uint32_t* key_idx) {
+    if (!ctx || !ks || (n && (!keys49 || !key_idx))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    NOT_ON_MULTI(ctx);
+    if (n == 0) return SCHNORR_B200_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    k_keyset_lookup<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, keys49, ks->lut, ks->n_lut, key_idx);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return SCHNORR_B200_OK;
+}
+
+int schnorr_b200_verify_keyed_registered_many(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                              const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off,
+                                              uint8_t* verdicts) {
+    if (!ctx || !ks || (n && (!keyed130 || !msg_off || !verdicts))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n == 0) return SCHNORR_B200_OK;
+    CHECK_MSG_OFF(ctx, n, msg_off);
+    if (msg_off[n] && !msgs) return SCHNORR_B200_EARG;
+    if (ctx->shards.empty()) return verify_keyed_registered_host(ctx, ks, n, keyed130, msgs, msg_off, verdicts);
+    auto sl = multi_slices(ctx, n);
+    return multi_run(ctx, sl, [&](int k, shard_slice s) {
+        auto off = rebase_offsets(msg_off, s.lo, s.hi);
+        return verify_keyed_registered_host(ctx->shards[k], ks->shards[k], s.hi - s.lo, keyed130 + 130 * s.lo,
+                                            msgs ? msgs + msg_off[s.lo] : nullptr, off.data(), verdicts + s.lo);
+    });
+}
+
+int schnorr_b200_verify_keyed_registered_many_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                                  const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off,
+                                                  uint8_t* verdicts) {
+    // msgs is required too: the offset table lives on the device, so whether every message is empty is not known here
+    if (!ctx || !ks || (n && (!keyed130 || !msgs || !msg_off || !verdicts))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    NOT_ON_MULTI(ctx);
+    if (n == 0) return SCHNORR_B200_OK;
+    return verify_keyed_registered_dev(ctx, ks, n, keyed130, msgs, msg_off, verdicts, false);
 }
 
 }  // extern "C"

@@ -228,6 +228,37 @@ class Engine:
                                                                     _ptr(msgs), _ptr(off), _ptr(verdicts)),
                     "verify_registered_many_dev")
 
+    def keyset_lookup(self, keyset, keys49):
+        """49-byte compressed keys -> uint32 indices into `keyset`: the smallest index of a registered key whose encoding
+        is exactly those bytes and which decompresses to its registered record, else 0xFFFFFFFF."""
+        keys49 = _u8(keys49, 49)
+        n = keys49.shape[0]
+        out = np.full(n, 0xFFFFFFFF, dtype=np.uint32)
+        self._check(self._L.schnorr_b200_keyset_lookup(self._h, keyset.handle, n, _ptr(keys49), _ptr(out)), "keyset_lookup")
+        return out
+
+    def keyset_lookup_dev(self, keyset, n, keys49, key_idx):
+        """Device buffers (key_idx: n uint32), enqueued on the engine's stream, no synchronisation."""
+        self._check(self._L.schnorr_b200_keyset_lookup_dev(self._h, keyset.handle, n, _ptr(keys49), _ptr(key_idx)),
+                    "keyset_lookup_dev")
+
+    def verify_keyed_registered_many(self, keyset, keyed130, msgs, off):
+        """KeyedSignature wire records against a registered key set -> verdicts (those of verify_keyed_many)."""
+        keyed130, msgs = _u8(keyed130, 130), _u8(msgs)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = keyed130.shape[0]
+        self._check_offsets(n, n, off, msgs)
+        out = np.full(n, 255, dtype=np.uint8)
+        self._check(self._L.schnorr_b200_verify_keyed_registered_many(self._h, keyset.handle, n, _ptr(keyed130), _ptr(msgs),
+                                                                      _ptr(off), _ptr(out)), "verify_keyed_registered_many")
+        return out
+
+    def verify_keyed_registered_many_dev(self, keyset, n, keyed130, msgs, off, verdicts):
+        """Device buffers, enqueued on the engine's stream, no synchronisation (always the lookup path)."""
+        self._check(self._L.schnorr_b200_verify_keyed_registered_many_dev(self._h, keyset.handle, n, _ptr(keyed130),
+                                                                          _ptr(msgs), _ptr(off), _ptr(verdicts)),
+                    "verify_keyed_registered_many_dev")
+
     def verify_batch(self, sigs81, pk96, pk_inf, msgs, off, rand32):
         """-> (verdict, lhs97, rhs97)"""
         sigs81, pk96, msgs, rand32 = _u8(sigs81, 81), _u8(pk96, 96), _u8(msgs), _u8(rand32, 32)
@@ -422,6 +453,10 @@ class Engine:
     def verify_many_dev(self, n, sigs81, pk96, pk_inf, msgs, off, verdicts):
         self._check(self._L.schnorr_b200_verify_many_dev(self._h, n, _ptr(sigs81), _ptr(pk96), _ptr(pk_inf), _ptr(msgs),
                                                          _ptr(off), _ptr(verdicts)), "verify_many_dev")
+
+    def verify_keyed_many_dev(self, n, keyed130, msgs, off, verdicts):
+        self._check(self._L.schnorr_b200_verify_keyed_many_dev(self._h, n, _ptr(keyed130), _ptr(msgs), _ptr(off),
+                                                               _ptr(verdicts)), "verify_keyed_many_dev")
 
     def hash_messages_dev(self, n, rx48, pk96, msgs, off, digests):
         self._check(self._L.schnorr_b200_hash_messages_dev(self._h, n, _ptr(rx48), _ptr(pk96), _ptr(msgs), _ptr(off),
