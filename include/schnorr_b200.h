@@ -21,7 +21,9 @@
  *    signature is data (a verdict), never an error code.
  *  - `*_dev` variants take DEVICE pointers for every buffer, enqueue on the context stream and do
  *    not synchronise; the host variants copy in, run the same kernels, copy out and synchronise.
- *  - a context is single-owner: one in-flight call per context; create several for concurrency.
+ *  - a context is single-owner: one in-flight call per context; create several for concurrency.  The same holds for
+ *    a registered key set: an update (keyset_append / _replace / _remove) synchronises every device of the context,
+ *    so *_dev calls enqueued before it see the old set and calls made after it the new one.
  *  - there is NO CPU fallback: without a CUDA device `schnorr_b200_create` fails.
  */
 #ifndef SCHNORR_B200_H
@@ -156,6 +158,43 @@ int schnorr_b200_verify_registered_many(schnorr_b200_ctx *ctx, const schnorr_b20
 int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
                                             const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
                                             const uint64_t *msg_off, uint8_t *verdicts);
+
+/* Updating a registered key set in place (a validator or committee set: a key joins, rotates, leaves).  After every
+ * update the set is exactly, byte for byte on every device, what keyset_create builds from the current list of slot
+ * records: records, identity flags, status bytes, tables (zeros for slots without one) and the lookup table (smallest
+ * findable index per encoding), and whether batches may sum the key side per key.
+ *  - keyset_append registers n keys in the next slots (indices n_keys ... n_keys + n - 1); EARG when the set would
+ *    reach 2^32 slots.  Records, status bytes and tables grow geometrically, so repeated appends copy the tables only
+ *    O(log n) times; while a buffer grows, the device holds the old and the new one (old plus new slots' tables).
+ *  - keyset_replace registers pk96[j] / pk_inf[j] in slot key_idx[j]; the slot keeps its index.  EARG for an index at
+ *    or beyond n_keys and for an index repeated in one call.
+ *  - keyset_remove writes the record of an index outside the set (96 bytes of 0xFF, identity flag 0) into the listed
+ *    slots: status 3, no table, not findable, so a removed index behaves like an index outside the set everywhere
+ *    (verdict 3, a malformed batch, flag 3 in locate_invalid_registered, a miss in keyset_lookup).  Repeated and
+ *    already removed indices are accepted.  Removed slots keep their index and memory and still count in n_keys
+ *    (and in the batch rule of set_registered_batch_threshold); keyset_replace reuses them.
+ * pk_inf may be NULL; status (optional, n bytes) as in keyset_create; n == 0 returns OK.  Argument checks and every
+ * allocation come before the set is written: an update that returns EARG, or fails to allocate, leaves it unchanged.
+ * An update synchronises every device of the context before it returns: *_dev calls enqueued before it see the old
+ * set, calls made after it the new one, and grown buffers are freed only after the work that may read them.  Registrations
+ * of up to set_keyset_block_threshold keys run one thread block per key (lowest latency), larger ones one thread per key.
+ * (No reference counterpart: the reference verifies each signature from scratch, src/signature.rs:181-205.) */
+int schnorr_b200_keyset_append(schnorr_b200_ctx *ctx, schnorr_b200_keyset *ks, size_t n, const uint8_t *pk96,
+                               const uint8_t *pk_inf, uint8_t *status);
+int schnorr_b200_keyset_replace(schnorr_b200_ctx *ctx, schnorr_b200_keyset *ks, size_t n, const uint32_t *key_idx,
+                                const uint8_t *pk96, const uint8_t *pk_inf, uint8_t *status);
+int schnorr_b200_keyset_remove(schnorr_b200_ctx *ctx, schnorr_b200_keyset *ks, size_t n, const uint32_t *key_idx);
+/* Registrations (keyset_create, _append, _replace) of at most `max_keys` keys run one thread block per key, larger ones
+ * one thread per key; the results are identical.  0 = never, SIZE_MAX = always (tests).  Default 512 (measured: one
+ * key 0.64 against 3.5 ms per replace call, 512 keys 10.3 against 12.8 ms, 4096 keys 81.5 against 79.5 ms). */
+int schnorr_b200_set_keyset_block_threshold(schnorr_b200_ctx *ctx, size_t max_keys);
+/* Test hook (no reference counterpart): copies to the host, from device `device_index` of the context (0 for a
+ * single-device context), slots first ... first + count - 1 of the set -- pk96 (count x 96 B), pk_inf (count),
+ * status (count), tables (count x 32 x 129 x 12 u64) -- and the lookup table: lut64 (room for n_keys entries of 64 B:
+ * 6 x-limbs, flag u32, index u32, pad u64) and *n_lut.  Any output may be NULL.  Synchronises. */
+int schnorr_b200_keyset_debug_export(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, int device_index, size_t first,
+                                     size_t count, uint8_t *pk96, uint8_t *pk_inf, uint8_t *status, uint64_t *tables,
+                                     uint8_t *lut64, uint32_t *n_lut);
 
 /* Compressed keys against a registered key set.  Registration also builds a sorted table of the set's encodings
  * (PublicKey::to_bytes of key k, src/public.rs:49-51, exactly as schnorr_b200_compress writes it), searched on the device

@@ -181,6 +181,33 @@ public:
         return result_from_verdict(verdict);
     }
     Result verify_keyed(const KeyedSignature& keyed, const std::vector<uint8_t>& message) const;
+    // registers `keys` in the next slots (schnorr_b200_keyset_append) -> the index of the first; status() and size()
+    // follow
+    size_t append(const std::vector<PublicKey>& keys) {
+        size_t first = size();
+        std::vector<uint8_t> pks, inf, st(keys.size(), 255);
+        pack_keys(keys, pks, inf);
+        eng_.check(schnorr_b200_keyset_append(eng_.get(), ks_, keys.size(), pks.data(), inf.data(), st.data()), "keyset_append");
+        status_.insert(status_.end(), st.begin(), st.end());
+        return first;
+    }
+    // registers keys[j] in slot indices[j] (distinct, inside the set; schnorr_b200_keyset_replace)
+    void replace(const std::vector<size_t>& indices, const std::vector<PublicKey>& keys) {
+        if (indices.size() != keys.size()) throw std::logic_error("one index per key");
+        std::vector<uint32_t> idx = checked_indices(indices);
+        std::vector<uint8_t> pks, inf, st(keys.size(), 255);
+        pack_keys(keys, pks, inf);
+        eng_.check(schnorr_b200_keyset_replace(eng_.get(), ks_, keys.size(), idx.data(), pks.data(), inf.data(), st.data()),
+                   "keyset_replace");
+        for (size_t j = 0; j < idx.size(); j++) status_[idx[j]] = st[j];
+    }
+    // removes slots (schnorr_b200_keyset_remove): they keep their index, and using it throws as an index outside the
+    // set does (verdict 3); status 3
+    void remove(const std::vector<size_t>& indices) {
+        std::vector<uint32_t> idx = checked_indices(indices);
+        eng_.check(schnorr_b200_keyset_remove(eng_.get(), ks_, idx.size(), idx.data()), "keyset_remove");
+        for (uint32_t k : idx) status_[k] = 3;
+    }
     // verify_batch(signatures, [keys[i] for i in indices], messages, rng) with the key side summed per key of the set
     // (schnorr_b200_verify_batch_registered); an index outside the set makes the batch malformed, which throws
     Result verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
@@ -193,6 +220,22 @@ public:
                                        const std::function<void(uint8_t*, size_t)>& rng) const;
 
 private:
+    static void pack_keys(const std::vector<PublicKey>& keys, std::vector<uint8_t>& pks, std::vector<uint8_t>& inf) {
+        pks.resize(keys.size() * 96);
+        inf.resize(keys.size());
+        for (size_t i = 0; i < keys.size(); i++) {
+            std::memcpy(&pks[i * 96], keys[i].xy.data(), 96);
+            inf[i] = keys[i].infinity;
+        }
+    }
+    std::vector<uint32_t> checked_indices(const std::vector<size_t>& indices) const {
+        std::vector<uint32_t> idx(indices.size());
+        for (size_t j = 0; j < indices.size(); j++) {
+            if (indices[j] >= size()) throw std::logic_error("index out of bounds: the key set has fewer slots");
+            idx[j] = (uint32_t)indices[j];
+        }
+        return idx;
+    }
     struct BatchInputs {
         std::vector<uint8_t> sigs, rand, blob;
         std::vector<uint32_t> idx;

@@ -36,6 +36,11 @@ _SIGNATURES = {
     "schnorr_b200_verify_many_dev": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 6),
     "schnorr_b200_keyset_create": (C.c_int, [C.c_void_p, _sz, _u8p, _u8p, _u8p, C.POINTER(C.c_void_p)]),
     "schnorr_b200_keyset_destroy": (None, [C.c_void_p]),
+    "schnorr_b200_keyset_append": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _u8p, _u8p, _u8p]),
+    "schnorr_b200_keyset_replace": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _u8p, _u8p, _u8p, _u8p]),
+    "schnorr_b200_keyset_remove": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _u8p]),
+    "schnorr_b200_set_keyset_block_threshold": (C.c_int, [C.c_void_p, _sz]),
+    "schnorr_b200_keyset_debug_export": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, _sz, _sz] + [_u8p] * 6),
     "schnorr_b200_verify_registered_many": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 5),
     "schnorr_b200_verify_registered_many_dev": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 5),
     "schnorr_b200_keyset_lookup": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _u8p, _u8p]),

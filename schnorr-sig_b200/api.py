@@ -199,6 +199,44 @@ class KeySet:
     def __len__(self):
         return self._handle.n_keys
 
+    @staticmethod
+    def _pack_keys(public_keys):
+        keys = list(public_keys)
+        pks = np.frombuffer(b"".join(k.xy for k in keys), dtype=np.uint8).reshape(len(keys), 96)
+        inf = np.array([k.infinity for k in keys], dtype=np.uint8)
+        return pks, inf
+
+    def _indices(self, indices):
+        idx = [int(i) for i in indices]
+        for i in idx:
+            if not 0 <= i < len(self):
+                raise PanicError("index out of bounds: the len is %d but the index is %d" % (len(self), i))
+        return np.array(idx, dtype=np.uint32)
+
+    def append(self, public_keys) -> range:
+        """Registers keys in the next slots; returns their indices.  `status` grows with them."""
+        pks, inf = self._pack_keys(public_keys)
+        first = len(self)
+        st = default_engine().keyset_append(self._handle, pks, inf)
+        self.status = np.concatenate([self.status, st])
+        return range(first, len(self))
+
+    def replace(self, indices, public_keys):
+        """Registers public_keys[j] in slot indices[j] (distinct indices inside the set); the slots keep their index."""
+        idx = self._indices(indices)
+        pks, inf = self._pack_keys(public_keys)
+        assert len(idx) == len(pks), "one index per key"
+        st = default_engine().keyset_replace(self._handle, idx, pks, inf)
+        self.status = self.status.copy()
+        self.status[idx] = st
+
+    def remove(self, indices):
+        """Removes slots: they keep their index, which then panics as an index outside the set does (status 3)."""
+        idx = self._indices(indices)
+        default_engine().keyset_remove(self._handle, idx)
+        self.status = self.status.copy()
+        self.status[idx] = 3
+
     def verify_signature(self, index: int, signature: Signature, message: bytes) -> Result:
         """Signature::verify(message, &keys[index]); an index outside the set panics, as indexing a slice does."""
         index = int(index)

@@ -9,6 +9,7 @@
 // Written once and instantiated by the CUDA kernels (schnorr_b200.cu) and by the host test build (tests/hostsim).
 #pragma once
 #include <algorithm>
+#include <vector>
 
 #include "verify.cuh"
 
@@ -223,6 +224,30 @@ static inline size_t keyset_sort_entries(keyset_entry* entries, size_t n) {
     for (size_t i = 0; i < n; i++)
         if (m == 0 || keyset_cmp(entries[i].x, entries[i].flag, &entries[m - 1]) != 0) entries[m++] = entries[i];
     return m;
+}
+
+// Host side of an in-place update (schnorr_b200_keyset_append / _replace / _remove).  `all` holds the entry of every
+// findable slot, duplicate encodings included, sorted by (encoding, index).  The entries of the slots with
+// changed[index] != 0 are deleted, `added` (the new entries of the changed slots that are findable, any order) is
+// merged in, and `lut` receives the smallest index of every encoding: what keyset_sort_entries gives from scratch over
+// the findable slots, in O(K + m log m) for m added entries instead of a sort of the whole set.
+static inline void keyset_update_entries(std::vector<keyset_entry>& all, const uint8_t* changed, size_t n_slots,
+                                         std::vector<keyset_entry> added, std::vector<keyset_entry>& lut) {
+    auto less = [](const keyset_entry& a, const keyset_entry& b) {
+        int c = keyset_cmp(a.x, a.flag, &b);
+        return c != 0 ? c < 0 : a.index < b.index;
+    };
+    size_t m = 0;
+    for (size_t i = 0; i < all.size(); i++)
+        if (all[i].index >= n_slots || !changed[all[i].index]) all[m++] = all[i];
+    all.resize(m);
+    std::sort(added.begin(), added.end(), less);
+    std::vector<keyset_entry> merged(all.size() + added.size());
+    std::merge(all.begin(), all.end(), added.begin(), added.end(), merged.begin(), less);
+    all.swap(merged);
+    lut.clear();
+    for (const keyset_entry& e : all)
+        if (lut.empty() || keyset_cmp(e.x, e.flag, &lut.back()) != 0) lut.push_back(e);
 }
 
 // ---- batch verification against registered keys (src/batch.rs:84-130) -------------------------------------------

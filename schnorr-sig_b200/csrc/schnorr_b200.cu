@@ -8,6 +8,8 @@
 //   k_tab_*               signed-window tables of affine multiples: the fixed-base table of G at context creation,
 //                         the per-key tables of registered key sets
 //   k_keyset_register     registration of a key set (status + subgroup check per key)
+//   k_keyset_register_block  the same for a few keys, one thread block per key, with the table's window bases
+//   k_keyset_scatter      replaced slots of a key set: records, status and tables from a compact registration
 //   k_keyset_gather       key records of the items of a registered call (ahead of k_ingest)
 //   k_verify_reg          Signature::verify against registered keys (table additions, no doubling chain)
 //   k_keyset_encode       the lookup table of a key set's compressed encodings (sorted on the host)
@@ -47,6 +49,12 @@ static constexpr size_t GTAB_U64 = (size_t)GTAB_WINDOWS * GTAB_ENTRIES * 12;
 // 23.0 ms), 16 per key loses (2^10 / 64 keys 0.82 against 0.80 ms), 4 per key loses (2^16 / 16 384 keys 2.83
 // against 2.51 ms): the key terms of a warp per key cost more than the MSM points they remove.
 static constexpr size_t REG_BATCH_MIN_PER_KEY = 64;
+// Registrations (keyset_create / _append / _replace) of at most this many keys run one thread block per key
+// (k_keyset_register_block), larger ones one thread per key (k_keyset_register, k_tab_bases); the tables are then built
+// by k_tab_fill either way (schnorr_b200_set_keyset_block_threshold).  Measured on a B200 (1000 W, 1965 MHz;
+// profiles/r6_keyset_update.md), warm replace calls, block against thread kernels: 1 key 0.64 / 3.46 ms, 64 keys
+// 1.67 / 4.53 ms, 512 keys 10.3 / 12.8 ms, 4096 keys 81.5 / 79.5 ms (sets of 64 to 16 384 keys).
+static constexpr size_t KEYSET_BLOCK_MAX = 512;
 
 // N, O: batches against registered key sets (gathered key records; key-side accumulators and terms), which run
 // batch_partial_impl (A-G, I-L) on inputs staged in H or M
@@ -73,6 +81,7 @@ struct schnorr_b200_ctx {
     uint32_t last_msm_T = 0;
     uint64_t last_batch_points = 0;                 // MSM points of the last batch call (schnorr_b200_last_batch_points)
     size_t reg_batch_min_per_key = REG_BATCH_MIN_PER_KEY;
+    size_t keyset_block_max = KEYSET_BLOCK_MAX;     // registrations of up to this many keys: k_keyset_register_block
     size_t dist_max = 10240;                        // calls up to this many signatures use the six-lanes-per-signature kernel
     size_t one_max = 512;                           // ... and up to this many the block-per-signature kernel (one.cuh)
     size_t batch_dist_max = (size_t)1 << 18;        // batches up to this size hash their challenges on six lanes per signature
@@ -711,6 +720,32 @@ __global__ void __launch_bounds__(128) k_keyset_encode(size_t n_keys, const uint
     e.pad = 0;
     entries[k] = e;
 }
+// Replaced slots: the record, identity flag, status and table of compact key j go to slot idx[j] (a table of zeros for
+// keys registered without one).  One 16-byte word per thread.
+static constexpr size_t KT_KEY_U128 = KT_KEY_U64 / 2;
+__global__ void __launch_bounds__(256) k_keyset_scatter(size_t m, const uint32_t* __restrict__ idx,
+                                                        const uint64_t* __restrict__ src_pk12, const uint8_t* __restrict__ src_inf,
+                                                        const uint8_t* __restrict__ src_status,
+                                                        const ulonglong2* __restrict__ src_tab, uint64_t* __restrict__ pk12,
+                                                        uint8_t* __restrict__ pk_inf, uint8_t* __restrict__ status,
+                                                        ulonglong2* __restrict__ tab) {
+    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= m * (KT_KEY_U128 + 13)) return;
+    if (t < m * KT_KEY_U128) {
+        size_t j = t / KT_KEY_U128, w = t % KT_KEY_U128;
+        tab[(size_t)idx[j] * KT_KEY_U128 + w] = src_tab[t];
+        return;
+    }
+    t -= m * KT_KEY_U128;
+    size_t j = t / 13, c = t % 13;
+    size_t k = idx[j];
+    if (c < 12) {
+        pk12[12 * k + c] = src_pk12[12 * j + c];
+    } else {
+        pk_inf[k] = src_inf[j];
+        status[k] = src_status[j];
+    }
+}
 // 49-byte compressed keys -> index of the registered key with exactly that encoding, or KEYSET_MISS
 __global__ void __launch_bounds__(128) k_keyset_lookup(size_t n, const uint8_t* __restrict__ keys49,
                                                        const keyset_entry* __restrict__ lut, uint32_t n_lut,
@@ -965,6 +1000,8 @@ static int verify_many_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs
 // K2 for the smallest calls: one thread block per signature (uses the six-lane primitives of dist.cuh and the 24-lane
 // Jacobian toolkit of batch.cuh)
 #include "one.cuh"
+// registration of a few keys: one thread block per key (the phases of k_verify_one)
+#include "keyset_block.cuh"
 
 
 // Signature::verify over an ingested SoA batch: fast path (per-thread or warp-cooperative by call size), then the exact kernel over the handful of
@@ -1469,15 +1506,24 @@ int schnorr_b200_verify_keyed_many(schnorr_b200_ctx* ctx, size_t n, const uint8_
 struct schnorr_b200_keyset {
     schnorr_b200_ctx* ctx = nullptr;  // the context the set was created on
     int device = 0;
-    size_t n_keys = 0;
-    uint64_t* pk12 = nullptr;   // [n_keys][12] the registered records, gathered per item ahead of k_ingest
-    uint8_t* pk_inf = nullptr;  // [n_keys]
-    uint8_t* status = nullptr;  // [n_keys] KEY_OK / KEY_NOT_TORSION_FREE / KEY_MALFORMED
-    uint64_t* ktab = nullptr;   // [n_keys][KT_KEY_U64]; zeros for keys without a table
+    size_t n_keys = 0;          // slots, removed ones included
+    size_t cap = 0;             // slots allocated (append grows records, status and tables geometrically)
+    uint64_t* pk12 = nullptr;   // [cap][12] the registered records, gathered per item ahead of k_ingest
+    uint8_t* pk_inf = nullptr;  // [cap]
+    uint8_t* status = nullptr;  // [cap] KEY_OK / KEY_NOT_TORSION_FREE / KEY_MALFORMED
+    uint64_t* ktab = nullptr;   // [cap][KT_KEY_U64]; zeros for keys without a table and for unused slots
     keyset_entry* lut = nullptr;  // [n_lut] the findable encodings, sorted (keyset.cuh: keyset_lookup)
     uint32_t n_lut = 0;
+    size_t lut_cap = 0;
     bool any_not_torsion_free = false;  // a key of status KEY_NOT_TORSION_FREE: batches use the per-signature points
     std::vector<schnorr_b200_keyset*> shards;
+    // host model, on the set the caller holds (every device holds the same): the status of every slot, the lookup
+    // entry of every slot and whether it is findable, and every findable entry sorted with duplicates
+    // (keyset_update_entries)
+    std::vector<uint8_t> h_status;
+    std::vector<keyset_entry> h_entry;
+    std::vector<uint8_t> h_findable;
+    std::vector<keyset_entry> h_all;
 };
 
 static void keyset_free(schnorr_b200_keyset* ks) {
@@ -1491,50 +1537,113 @@ static void keyset_free(schnorr_b200_keyset* ks) {
     delete ks;
 }
 
-// registration on one device: copies the records, k_keyset_register, the tables of the keys with status 0, and the
-// lookup table of the encodings (k_keyset_encode; sorted on the host while the key tables are built)
+// the single-device sets of a set, with their contexts: the set itself on a single-device context
+static std::vector<std::pair<schnorr_b200_ctx*, schnorr_b200_keyset*>> keyset_devices(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks) {
+    std::vector<std::pair<schnorr_b200_ctx*, schnorr_b200_keyset*>> v;
+    if (ks->shards.empty()) v.emplace_back(ctx, ks);
+    for (size_t k = 0; k < ks->shards.size(); k++) v.emplace_back(ctx->shards[k], ks->shards[k]);
+    return v;
+}
+
+// records of `cap` slots: pk12 [cap][12] | pk_inf [cap] | status [cap]
+static int keyset_alloc_records(schnorr_b200_ctx* ctx, size_t cap, uint64_t** pk12, uint8_t** pk_inf, uint8_t** status) {
+    void* rec;
+    CUDA_TRY(ctx, cudaMalloc(&rec, cap * 96 + 2 * cap));
+    *pk12 = (uint64_t*)rec;
+    *pk_inf = (uint8_t*)rec + cap * 96;
+    *status = *pk_inf + cap;
+    return 0;
+}
+
+// Scratch of a registration of m keys (keyset_register): SL_D skip flags, then the table bases
+static size_t keyset_skip_bytes(size_t m) { return (m + 15) / 16 * 16; }
+static int keyset_register_scratch(schnorr_b200_ctx* ctx, size_t m, void** tmp) {
+    return ensure_scratch(ctx, SL_D, keyset_skip_bytes(m) + m * KT_WINDOWS * sizeof(jac_pt), tmp);
+}
+
+// Registration of m keys on one device, the one routine of create, append and replace: status[j] of record j
+// (keyset_key_status) and, for keys of status 0 other than the identity, the table at tab + j KT_KEY_U64 (left as it
+// is for the others).  Up to ctx->keyset_block_max keys run one block per key (k_keyset_register_block), more one
+// thread per key (k_keyset_register, k_tab_bases); k_tab_fill builds the tables.  Scratch: keyset_register_scratch.
+static int keyset_register(schnorr_b200_ctx* ctx, size_t m, const uint64_t* pk12, const uint8_t* pk_inf, uint8_t* status,
+                           uint64_t* tab) {
+    void* tmp;
+    if (int rc = keyset_register_scratch(ctx, m, &tmp)) return rc;
+    uint8_t* skip = (uint8_t*)tmp;
+    jac_pt* bases = (jac_pt*)((uint8_t*)tmp + keyset_skip_bytes(m));
+    if (m <= ctx->keyset_block_max) {
+        k_keyset_register_block<<<(unsigned)m, ONE_THREADS, 0, ctx->stream>>>(m, pk12, pk_inf, status, skip, bases);
+        size_t threads = m * (size_t)KT_WINDOWS * KT_ENTRIES;
+        k_tab_fill<<<grid_for(threads, 128), 128, 0, ctx->stream>>>(m, skip, KT_W, KT_WINDOWS, bases, tab);
+        ctx->launches += 2;
+        CUDA_TRY(ctx, cudaGetLastError());
+        return 0;
+    }
+    k_keyset_register<<<grid_for(m, 128), 128, 0, ctx->stream>>>(m, pk12, pk_inf, status, skip);
+    ctx->launches += 1;
+    return build_tables(ctx, m, pk12, skip, KT_W, KT_WINDOWS, bases, tab);
+}
+
+// Encodings of m records (k_keyset_encode), enqueued with their copies into `entries` / `findable` (host, m each);
+// the host may read them after ctx->ev_aux.  Scratch: SL_E.
+static int keyset_encode_async(schnorr_b200_ctx* ctx, size_t m, const uint64_t* pk12, const uint8_t* pk_inf,
+                               keyset_entry* entries, uint8_t* findable) {
+    void* enc;  // lookup entries, then the findable flags
+    if (int rc = ensure_scratch(ctx, SL_E, m * (sizeof(keyset_entry) + 1), &enc)) return rc;
+    k_keyset_encode<<<grid_for(m, 128), 128, 0, ctx->stream>>>(m, pk12, pk_inf, (keyset_entry*)enc,
+                                                              (uint8_t*)enc + m * sizeof(keyset_entry));
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaMemcpyAsync(entries, enc, m * sizeof(keyset_entry), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(findable, (uint8_t*)enc + m * sizeof(keyset_entry), m, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_aux, ctx->stream));
+    return 0;
+}
+
+// the lookup table `lut` uploaded to one device's set (the buffer was sized by the caller: lut_cap >= lut.size())
+static int keyset_upload_lut(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const std::vector<keyset_entry>& lut) {
+    ks->n_lut = (uint32_t)lut.size();
+    if (!lut.empty())
+        CUDA_TRY(ctx, cudaMemcpyAsync(ks->lut, lut.data(), lut.size() * sizeof(keyset_entry), cudaMemcpyHostToDevice, ctx->stream));
+    return 0;
+}
+
+// registration on one device: copies the records, registers them (keyset_register), and builds the lookup table of
+// the encodings (k_keyset_encode; sorted on the host while the key tables are built).  `model` (the first device):
+// also fills the host model of `top` and the status bytes.
 static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const uint8_t* pk96, const uint8_t* pk_inf,
-                        uint8_t* status) {
+                        schnorr_b200_keyset* top, bool model) {
     const size_t n = ks->n_keys;
     ks->device = ctx->device;
+    ks->cap = n;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    void* rec;
-    CUDA_TRY(ctx, cudaMalloc(&rec, n * 96 + 2 * n));
-    ks->pk12 = (uint64_t*)rec;
-    ks->pk_inf = (uint8_t*)rec + n * 96;
-    ks->status = ks->pk_inf + n;
+    if (int rc = keyset_alloc_records(ctx, n, &ks->pk12, &ks->pk_inf, &ks->status)) return rc;
     CUDA_TRY(ctx, cudaMalloc(&ks->ktab, n * KT_KEY_U64 * sizeof(uint64_t)));
     CUDA_TRY(ctx, cudaMemsetAsync(ks->ktab, 0, n * KT_KEY_U64 * sizeof(uint64_t), ctx->stream));
     CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk12, pk96, n * 96, cudaMemcpyHostToDevice, ctx->stream));
     if (pk_inf) CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk_inf, pk_inf, n, cudaMemcpyHostToDevice, ctx->stream));
     else CUDA_TRY(ctx, cudaMemsetAsync(ks->pk_inf, 0, n, ctx->stream));
-    void* enc;  // lookup entries, then the findable flags
-    if (int rc = ensure_scratch(ctx, SL_E, n * (sizeof(keyset_entry) + 1), &enc)) return rc;
     std::vector<keyset_entry> entries(n);
     std::vector<uint8_t> findable(n);
-    k_keyset_encode<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, ks->pk12, ks->pk_inf, (keyset_entry*)enc,
-                                                              (uint8_t*)enc + n * sizeof(keyset_entry));
-    ctx->launches += 1;
-    CUDA_TRY(ctx, cudaMemcpyAsync(entries.data(), enc, n * sizeof(keyset_entry), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(ctx, cudaMemcpyAsync(findable.data(), (uint8_t*)enc + n * sizeof(keyset_entry), n, cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_aux, ctx->stream));
-    void* tmp;  // skip flags, then the table bases
-    size_t skip_bytes = (n + 15) / 16 * 16;
-    if (int rc = ensure_scratch(ctx, SL_D, skip_bytes + n * KT_WINDOWS * sizeof(jac_pt), &tmp)) return rc;
-    uint8_t* skip = (uint8_t*)tmp;
-    k_keyset_register<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, ks->pk12, ks->pk_inf, ks->status, skip);
-    ctx->launches += 1;
-    if (int rc = build_tables(ctx, n, ks->pk12, skip, KT_W, KT_WINDOWS, (jac_pt*)((uint8_t*)tmp + skip_bytes), ks->ktab)) return rc;
-    if (status) CUDA_TRY(ctx, cudaMemcpyAsync(status, ks->status, n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (int rc = keyset_encode_async(ctx, n, ks->pk12, ks->pk_inf, entries.data(), findable.data())) return rc;
+    if (int rc = keyset_register(ctx, n, ks->pk12, ks->pk_inf, ks->status, ks->ktab)) return rc;
+    if (model) {
+        top->h_status.resize(n);
+        CUDA_TRY(ctx, cudaMemcpyAsync(top->h_status.data(), ks->status, n, cudaMemcpyDeviceToHost, ctx->stream));
+    }
     CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev_aux));
-    size_t m = 0;
+    std::vector<keyset_entry> added, all, lut;
     for (size_t k = 0; k < n; k++)
-        if (findable[k]) entries[m++] = entries[k];
-    m = keyset_sort_entries(entries.data(), m);
-    ks->n_lut = (uint32_t)m;
-    CUDA_TRY(ctx, cudaMalloc(&ks->lut, (m ? m : 1) * sizeof(keyset_entry)));
-    if (m) CUDA_TRY(ctx, cudaMemcpyAsync(ks->lut, entries.data(), m * sizeof(keyset_entry), cudaMemcpyHostToDevice, ctx->stream));
+        if (findable[k]) added.push_back(entries[k]);
+    keyset_update_entries(all, nullptr, 0, std::move(added), lut);
+    ks->lut_cap = lut.size() ? lut.size() : 1;
+    CUDA_TRY(ctx, cudaMalloc(&ks->lut, ks->lut_cap * sizeof(keyset_entry)));
+    if (int rc = keyset_upload_lut(ctx, ks, lut)) return rc;
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (model) {
+        top->h_entry.swap(entries);
+        top->h_findable.swap(findable);
+        top->h_all.swap(all);
+    }
     return 0;
 }
 
@@ -1612,6 +1721,183 @@ static int verify_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keys
         }                                                                       \
     } while (0)
 
+
+// any_not_torsion_free from the host model, and the slot count, on the set and its shards
+static void keyset_sync_flags(schnorr_b200_keyset* ks) {
+    bool off_subgroup = false;
+    for (uint8_t v : ks->h_status) off_subgroup |= v == KEY_NOT_TORSION_FREE;
+    ks->any_not_torsion_free = off_subgroup;
+    for (schnorr_b200_keyset* sh : ks->shards) {
+        sh->any_not_torsion_free = off_subgroup;
+        sh->n_keys = ks->n_keys;
+    }
+}
+
+// buffers of one device's set that an update allocates before it writes anything
+struct keyset_grow {
+    uint64_t* pk12 = nullptr;
+    uint8_t *pk_inf = nullptr, *status = nullptr;
+    uint64_t* ktab = nullptr;
+    size_t cap = 0;
+    keyset_entry* lut = nullptr;
+    size_t lut_cap = 0;
+    void *stage = nullptr, *ctab = nullptr;
+};
+static void keyset_grow_free(int device, keyset_grow& g) {
+    cudaSetDevice(device);
+    cudaFree(g.pk12);
+    cudaFree(g.ktab);
+    cudaFree(g.lut);
+    g.pk12 = nullptr;
+    g.ktab = nullptr;
+    g.lut = nullptr;
+}
+
+// append (key_idx == NULL: slots n_keys ... n_keys + m - 1) or replace (slots key_idx[j], distinct and inside the set)
+// of m keys, on every device; arguments checked by the caller.  The set ends exactly as keyset_create would build it
+// from the updated list of records.  Every allocation comes first, so a failure there leaves the set unchanged.  On
+// each device: the records are staged (SL_F); an append registers them into its new slots, a replace into a compact
+// table (SL_G) that k_keyset_scatter copies to the slots, zeros included.  The first device encodes them; the host
+// merges the new lookup entries into its model (keyset_update_entries) and uploads the table to every device.
+static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t m, const uint32_t* key_idx,
+                         const uint8_t* pk96, const uint8_t* pk_inf, uint8_t* status) {
+    auto devs = keyset_devices(ctx, ks);
+    const size_t n = ks->n_keys, new_n = key_idx ? n : n + m;
+    const size_t lut_need = ks->h_all.size() + m;  // distinct findable encodings after the update, at most
+    const size_t stage_bytes = m * 96 + (m + 15) / 16 * 16 + m * 4;
+    std::vector<keyset_grow> gr(devs.size());
+    auto fail = [&](int rc, size_t d) {
+        if (devs[d].first != ctx) ctx->err = "device " + std::to_string(devs[d].first->device) + ": " + devs[d].first->err;
+        for (size_t e = 0; e < devs.size(); e++) keyset_grow_free(devs[e].first->device, gr[e]);
+        return rc;
+    };
+    // ---- allocations
+    for (size_t d = 0; d < devs.size(); d++) {
+        schnorr_b200_ctx* c = devs[d].first;
+        schnorr_b200_keyset* s = devs[d].second;
+        keyset_grow& g = gr[d];
+        int rc = 0;
+        if (cudaSetDevice(c->device) != cudaSuccess) {
+            c->err = "cudaSetDevice failed";
+            return fail(SCHNORR_B200_ECUDA, d);
+        }
+        if (new_n > s->cap) {  // geometric growth: repeated appends copy the tables O(log n) times
+            g.cap = std::max(new_n, s->cap + s->cap / 2);
+            if ((rc = keyset_alloc_records(c, g.cap, &g.pk12, &g.pk_inf, &g.status))) return fail(rc, d);
+            if (cudaMalloc(&g.ktab, g.cap * KT_KEY_U64 * sizeof(uint64_t)) != cudaSuccess) {
+                c->err = "cudaMalloc of the grown key tables failed";
+                return fail(SCHNORR_B200_ECUDA, d);
+            }
+        }
+        if (lut_need > s->lut_cap) {
+            g.lut_cap = std::max(lut_need, s->lut_cap + s->lut_cap / 2);
+            if (cudaMalloc(&g.lut, g.lut_cap * sizeof(keyset_entry)) != cudaSuccess) {
+                c->err = "cudaMalloc of the lookup table failed";
+                return fail(SCHNORR_B200_ECUDA, d);
+            }
+        }
+        void* enc;
+        if ((rc = ensure_scratch(c, SL_F, stage_bytes, &g.stage))) return fail(rc, d);
+        if ((rc = keyset_register_scratch(c, m, &enc))) return fail(rc, d);
+        if (d == 0 && (rc = ensure_scratch(c, SL_E, m * (sizeof(keyset_entry) + 1), &enc))) return fail(rc, d);
+        if (key_idx && (rc = ensure_scratch(c, SL_G, m * KT_KEY_U64 * sizeof(uint64_t) + m, &g.ctab))) return fail(rc, d);
+    }
+    // ---- the set is written from here on
+    std::vector<keyset_entry> entries(m);
+    std::vector<uint8_t> findable(m), st(m);
+    std::vector<std::pair<int, void*>> old;  // replaced buffers, freed once every device has synchronised
+    for (size_t d = 0; d < devs.size(); d++) {
+        schnorr_b200_ctx* c = devs[d].first;
+        schnorr_b200_keyset* s = devs[d].second;
+        keyset_grow& g = gr[d];
+        cudaStream_t sm = c->stream;
+        int rc = 0;
+        CUDA_TRY(c, cudaSetDevice(c->device));
+        if (g.pk12) {  // one device-to-device copy per buffer; the new tail of the tables is zeros
+            CUDA_TRY(c, cudaMemcpyAsync(g.pk12, s->pk12, n * 96, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(g.pk_inf, s->pk_inf, n, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(g.status, s->status, n, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(g.ktab, s->ktab, n * KT_KEY_U64 * sizeof(uint64_t), cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemsetAsync(g.ktab + n * KT_KEY_U64, 0, (g.cap - n) * KT_KEY_U64 * sizeof(uint64_t), sm));
+            old.emplace_back(c->device, s->pk12);
+            old.emplace_back(c->device, s->ktab);
+            s->pk12 = g.pk12;
+            s->pk_inf = g.pk_inf;
+            s->status = g.status;
+            s->ktab = g.ktab;
+            s->cap = g.cap;
+            g.pk12 = nullptr;
+            g.ktab = nullptr;
+        }
+        if (g.lut) {
+            old.emplace_back(c->device, s->lut);
+            s->lut = g.lut;
+            s->lut_cap = g.lut_cap;
+            g.lut = nullptr;
+        }
+        uint64_t* spk = (uint64_t*)g.stage;
+        uint8_t* sinf = (uint8_t*)g.stage + m * 96;
+        uint32_t* sidx = (uint32_t*)(sinf + (m + 15) / 16 * 16);
+        CUDA_TRY(c, cudaMemcpyAsync(spk, pk96, m * 96, cudaMemcpyHostToDevice, sm));
+        if (pk_inf) CUDA_TRY(c, cudaMemcpyAsync(sinf, pk_inf, m, cudaMemcpyHostToDevice, sm));
+        else CUDA_TRY(c, cudaMemsetAsync(sinf, 0, m, sm));
+        if (d == 0 && (rc = keyset_encode_async(c, m, spk, sinf, entries.data(), findable.data()))) return rc;
+        uint8_t* new_status;
+        if (!key_idx) {
+            CUDA_TRY(c, cudaMemcpyAsync(s->pk12 + 12 * n, spk, m * 96, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(s->pk_inf + n, sinf, m, cudaMemcpyDeviceToDevice, sm));
+            new_status = s->status + n;
+            if ((rc = keyset_register(c, m, s->pk12 + 12 * n, s->pk_inf + n, new_status, s->ktab + n * KT_KEY_U64))) return rc;
+        } else {
+            uint64_t* ctab = (uint64_t*)g.ctab;
+            new_status = (uint8_t*)(ctab + m * KT_KEY_U64);
+            CUDA_TRY(c, cudaMemcpyAsync(sidx, key_idx, m * 4, cudaMemcpyHostToDevice, sm));
+            CUDA_TRY(c, cudaMemsetAsync(ctab, 0, m * KT_KEY_U64 * sizeof(uint64_t), sm));
+            if ((rc = keyset_register(c, m, spk, sinf, new_status, ctab))) return rc;
+            k_keyset_scatter<<<grid_for(m * (KT_KEY_U128 + 13), 256), 256, 0, sm>>>(
+                m, sidx, spk, sinf, new_status, (const ulonglong2*)ctab, s->pk12, s->pk_inf, s->status, (ulonglong2*)s->ktab);
+            c->launches += 1;
+            CUDA_TRY(c, cudaGetLastError());
+        }
+        if (d == 0) CUDA_TRY(c, cudaMemcpyAsync(st.data(), new_status, m, cudaMemcpyDeviceToHost, sm));
+    }
+    // ---- the host model and the lookup table
+    schnorr_b200_ctx* c0 = devs[0].first;
+    CUDA_TRY(c0, cudaSetDevice(c0->device));
+    CUDA_TRY(c0, cudaStreamSynchronize(c0->stream));
+    std::vector<uint8_t> changed(new_n, 0);
+    std::vector<keyset_entry> added, lut;
+    ks->h_status.resize(new_n);
+    ks->h_entry.resize(new_n);
+    ks->h_findable.resize(new_n);
+    for (size_t j = 0; j < m; j++) {
+        size_t k = key_idx ? key_idx[j] : n + j;
+        changed[k] = 1;
+        entries[j].index = (uint32_t)k;
+        ks->h_status[k] = st[j];
+        ks->h_entry[k] = entries[j];
+        ks->h_findable[k] = findable[j];
+        if (findable[j]) added.push_back(entries[j]);
+    }
+    keyset_update_entries(ks->h_all, changed.data(), new_n, std::move(added), lut);
+    for (auto& dv : devs) {
+        CUDA_TRY(dv.first, cudaSetDevice(dv.first->device));
+        if (int rc = keyset_upload_lut(dv.first, dv.second, lut)) return rc;
+    }
+    for (auto& dv : devs) {  // every device synchronised: work enqueued before the update has finished with the old buffers
+        CUDA_TRY(dv.first, cudaSetDevice(dv.first->device));
+        CUDA_TRY(dv.first, cudaStreamSynchronize(dv.first->stream));
+    }
+    for (auto& o : old) {
+        cudaSetDevice(o.first);
+        cudaFree(o.second);
+    }
+    ks->n_keys = new_n;
+    keyset_sync_flags(ks);
+    if (status) memcpy(status, st.data(), m);
+    return SCHNORR_B200_OK;
+}
+
 extern "C" {
 
 int schnorr_b200_keyset_create(schnorr_b200_ctx* ctx, size_t n_keys, const uint8_t* pk96, const uint8_t* pk_inf,
@@ -1622,17 +1908,16 @@ int schnorr_b200_keyset_create(schnorr_b200_ctx* ctx, size_t n_keys, const uint8
     schnorr_b200_keyset* ks = new schnorr_b200_keyset();
     ks->ctx = ctx;
     ks->n_keys = n_keys;
-    std::vector<uint8_t> st(n_keys);
     int rc = 0;
     if (ctx->shards.empty()) {
-        rc = keyset_build(ctx, ks, pk96, pk_inf, st.data());
+        rc = keyset_build(ctx, ks, pk96, pk_inf, ks, true);
     } else {  // one table per device; the status comes from the first (every shard computes the same)
         for (size_t k = 0; k < ctx->shards.size() && rc == 0; k++) {
             schnorr_b200_keyset* sh = new schnorr_b200_keyset();
             sh->ctx = ctx->shards[k];
             sh->n_keys = n_keys;
             ks->shards.push_back(sh);
-            rc = keyset_build(ctx->shards[k], sh, pk96, pk_inf, k == 0 ? st.data() : nullptr);
+            rc = keyset_build(ctx->shards[k], sh, pk96, pk_inf, ks, k == 0);
             if (rc) ctx->err = "device " + std::to_string(ctx->shards[k]->device) + ": " + ctx->shards[k]->err;
         }
     }
@@ -1640,17 +1925,91 @@ int schnorr_b200_keyset_create(schnorr_b200_ctx* ctx, size_t n_keys, const uint8
         keyset_free(ks);
         return rc;
     }
-    bool off_subgroup = false;
-    for (uint8_t v : st) off_subgroup |= v == KEY_NOT_TORSION_FREE;
-    ks->any_not_torsion_free = off_subgroup;
-    for (schnorr_b200_keyset* sh : ks->shards) sh->any_not_torsion_free = off_subgroup;
-    if (status) memcpy(status, st.data(), n_keys);
+    keyset_sync_flags(ks);
+    if (status) memcpy(status, ks->h_status.data(), n_keys);
     *out = ks;
     return SCHNORR_B200_OK;
 }
 
 void schnorr_b200_keyset_destroy(schnorr_b200_keyset* ks) {
     if (ks) keyset_free(ks);
+}
+
+int schnorr_b200_keyset_append(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t n, const uint8_t* pk96,
+                               const uint8_t* pk_inf, uint8_t* status) {
+    if (!ctx || !ks || (n && !pk96)) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n == 0) return SCHNORR_B200_OK;
+    if ((uint64_t)ks->n_keys + n >= ((uint64_t)1 << 32)) {
+        ctx->err = "a key set holds fewer than 2^32 slots";
+        return SCHNORR_B200_EARG;
+    }
+    return keyset_update(ctx, ks, n, nullptr, pk96, pk_inf, status);
+}
+
+int schnorr_b200_keyset_replace(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t n, const uint32_t* key_idx,
+                                const uint8_t* pk96, const uint8_t* pk_inf, uint8_t* status) {
+    if (!ctx || !ks || (n && (!key_idx || !pk96))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n == 0) return SCHNORR_B200_OK;
+    std::vector<uint32_t> sorted(key_idx, key_idx + n);
+    std::sort(sorted.begin(), sorted.end());
+    if (sorted.back() >= ks->n_keys) {
+        ctx->err = "a key index is outside the set";
+        return SCHNORR_B200_EARG;
+    }
+    if (std::adjacent_find(sorted.begin(), sorted.end()) != sorted.end()) {
+        ctx->err = "a key index is repeated in one replace call";
+        return SCHNORR_B200_EARG;
+    }
+    return keyset_update(ctx, ks, n, key_idx, pk96, pk_inf, status);
+}
+
+int schnorr_b200_keyset_remove(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t n, const uint32_t* key_idx) {
+    if (!ctx || !ks || (n && !key_idx)) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (n == 0) return SCHNORR_B200_OK;
+    std::vector<uint32_t> idx(key_idx, key_idx + n);
+    std::sort(idx.begin(), idx.end());
+    idx.erase(std::unique(idx.begin(), idx.end()), idx.end());
+    if (idx.back() >= ks->n_keys) {
+        ctx->err = "a key index is outside the set";
+        return SCHNORR_B200_EARG;
+    }
+    // the removed record: what k_keyset_gather writes for an index outside the set
+    std::vector<uint8_t> rec(idx.size() * 96, 0xFF), inf(idx.size(), 0);
+    return keyset_update(ctx, ks, idx.size(), idx.data(), rec.data(), inf.data(), nullptr);
+}
+
+int schnorr_b200_keyset_debug_export(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, int device_index, size_t first,
+                                     size_t count, uint8_t* pk96, uint8_t* pk_inf, uint8_t* status, uint64_t* tables,
+                                     uint8_t* lut64, uint32_t* n_lut) {
+    if (!ctx || !ks || device_index < 0 || first > ks->n_keys || count > ks->n_keys - first) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    if (device_index >= (int)(ctx->shards.empty() ? 1 : ctx->shards.size())) return SCHNORR_B200_EARG;
+    schnorr_b200_ctx* c = ctx->shards.empty() ? ctx : ctx->shards[device_index];
+    const schnorr_b200_keyset* s = ks->shards.empty() ? ks : ks->shards[device_index];
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    if (count) {
+        if (pk96) CUDA_TRY(c, cudaMemcpyAsync(pk96, s->pk12 + 12 * first, count * 96, cudaMemcpyDeviceToHost, c->stream));
+        if (pk_inf) CUDA_TRY(c, cudaMemcpyAsync(pk_inf, s->pk_inf + first, count, cudaMemcpyDeviceToHost, c->stream));
+        if (status) CUDA_TRY(c, cudaMemcpyAsync(status, s->status + first, count, cudaMemcpyDeviceToHost, c->stream));
+        if (tables)
+            CUDA_TRY(c, cudaMemcpyAsync(tables, s->ktab + first * KT_KEY_U64, count * KT_KEY_U64 * sizeof(uint64_t),
+                                        cudaMemcpyDeviceToHost, c->stream));
+    }
+    if (lut64 && s->n_lut)
+        CUDA_TRY(c, cudaMemcpyAsync(lut64, s->lut, s->n_lut * sizeof(keyset_entry), cudaMemcpyDeviceToHost, c->stream));
+    if (n_lut) *n_lut = s->n_lut;
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    return SCHNORR_B200_OK;
+}
+
+int schnorr_b200_set_keyset_block_threshold(schnorr_b200_ctx* ctx, size_t max_keys) {
+    if (!ctx) return SCHNORR_B200_EARG;
+    ctx->keyset_block_max = max_keys;
+    for (schnorr_b200_ctx* sh : ctx->shards) sh->keyset_block_max = max_keys;
+    return SCHNORR_B200_OK;
 }
 
 int schnorr_b200_verify_registered_many(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,

@@ -138,6 +138,10 @@ class Engine:
         self._check(self._L.schnorr_b200_set_registered_batch_threshold(self._h, int(min_signatures_per_key)),
                     "set_registered_batch_threshold")
 
+    def set_keyset_block_threshold(self, max_keys: int):
+        """Registrations of up to this many keys run one thread block per key (0 = never, 2**64 - 1 = always)."""
+        self._check(self._L.schnorr_b200_set_keyset_block_threshold(self._h, int(max_keys)), "set_keyset_block_threshold")
+
     def last_exact_count(self) -> int:
         """Items of the last verify_many* call that the fast path handed to the exact kernel."""
         c = C.c_uint64(0)
@@ -206,6 +210,53 @@ class Engine:
         self._check(self._L.schnorr_b200_keyset_create(self._h, n, _ptr(pk96), _ptr(inf), _ptr(status), C.byref(h)),
                     "keyset_create")
         return KeySetHandle(self, h, n), status
+
+    def keyset_append(self, keyset, pk96, pk_inf=None):
+        """Registers keys in the next slots of `keyset` (indices n_keys, n_keys + 1, ...) -> status uint8[n]."""
+        pk96 = _u8(pk96, 96)
+        n = pk96.shape[0]
+        inf = None if pk_inf is None else _u8(pk_inf)
+        self._check_inf(n, inf)
+        status = np.full(n, 255, dtype=np.uint8)
+        self._check(self._L.schnorr_b200_keyset_append(self._h, keyset.handle, n, _ptr(pk96), _ptr(inf), _ptr(status)),
+                    "keyset_append")
+        keyset.n_keys += n
+        return status
+
+    def keyset_replace(self, keyset, key_idx, pk96, pk_inf=None):
+        """Registers pk96[j] in slot key_idx[j] of `keyset` (distinct indices inside the set) -> status uint8[n]."""
+        pk96 = _u8(pk96, 96)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
+        n = pk96.shape[0]
+        if key_idx.ndim != 1 or key_idx.shape[0] != n:
+            raise ValueError("one key index per key")
+        inf = None if pk_inf is None else _u8(pk_inf)
+        self._check_inf(n, inf)
+        status = np.full(n, 255, dtype=np.uint8)
+        self._check(self._L.schnorr_b200_keyset_replace(self._h, keyset.handle, n, _ptr(key_idx), _ptr(pk96), _ptr(inf),
+                                                        _ptr(status)), "keyset_replace")
+        return status
+
+    def keyset_remove(self, keyset, key_idx):
+        """Removes slots of `keyset`: they keep their index and behave like an index outside the set (status 3)."""
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        self._check(self._L.schnorr_b200_keyset_remove(self._h, keyset.handle, key_idx.shape[0], _ptr(key_idx)),
+                    "keyset_remove")
+
+    def keyset_debug_export(self, keyset, device_index=0, first=0, count=None, tables=True):
+        """Test hook: one device's copy of the set -> dict(pk96, inf, status, tables [count, 32, 129, 12] uint64 or
+        None, lut [n_lut, 64] uint8)."""
+        count = keyset.n_keys - first if count is None else int(count)
+        pk = np.zeros((count, 96), dtype=np.uint8)
+        inf = np.zeros(count, dtype=np.uint8)
+        status = np.zeros(count, dtype=np.uint8)
+        tab = np.zeros((count, 32, 129, 12), dtype=np.uint64) if tables else None
+        lut = np.zeros((max(keyset.n_keys, 1), 64), dtype=np.uint8)
+        n_lut = C.c_uint32(0)
+        self._check(self._L.schnorr_b200_keyset_debug_export(self._h, keyset.handle, int(device_index), int(first), count,
+                                                             _ptr(pk), _ptr(inf), _ptr(status), _ptr(tab), _ptr(lut),
+                                                             C.byref(n_lut)), "keyset_debug_export")
+        return dict(pk96=pk, inf=inf, status=status, tables=tab, lut=lut[:n_lut.value].copy())
 
     def verify_registered_many(self, keyset, sigs81, key_idx, msgs, off):
         """Signature::verify of sigs81[i] over message i under key key_idx[i] of `keyset` -> verdicts (those of
