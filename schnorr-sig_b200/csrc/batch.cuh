@@ -1321,6 +1321,36 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     return SCHNORR_B200_OK;
 }
 
+// the partial of an empty batch: identity point, zero scalar
+static int batch_partial_empty(schnorr_b200_ctx* ctx, uint8_t* partial192) {
+    ctx->last_batch_points = 0;
+    uint64_t h[24] = {0};
+    h[0] = 1;
+    h[6] = 1;
+    CUDA_TRY(ctx, cudaMemcpyAsync(partial192, h, 192, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return SCHNORR_B200_OK;
+}
+
+// A whole batch on one device (its device selected): SL_L holds [64 B of batch_partial_impl | result | partial |
+// rhs_pre]; partial_fn(partial, rhs_pre) reduces the n > 0 signatures to the partial with (sum s e) G computed beside it
+// into rhs_pre (batch_partial_impl), and k_batch_finish writes the result to `result216`, or, when that is null, to the
+// result region of SL_L, which `result216` then points to (the host forms read it with read_result).
+template <typename F>
+static int batch_whole(schnorr_b200_ctx* ctx, size_t n, F partial_fn, uint8_t*& result216) {
+    void* d_res;
+    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
+    if (!result216) result216 = (uint8_t*)d_res + 64;
+    uint8_t* partial = (uint8_t*)d_res + 64 + RESULT_BYTES;
+    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;
+    if (int rc = n ? partial_fn(partial, rhs_pre) : batch_partial_empty(ctx, partial)) return rc;
+    if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
+    k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, result216, rhs_pre);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return SCHNORR_B200_OK;
+}
+
 // multi.cuh: a batch over every device of a multi-device context; partial(k, slice, rebased offsets, partial192) reduces
 // the non-empty slice of shard k to its partial on that shard's device
 template <typename F>
@@ -1335,15 +1365,7 @@ int schnorr_b200_batch_partial_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_
     if (!ctx || !partial192 || (n && (!sigs81 || !pk96 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
     NOT_ON_MULTI(ctx);
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    if (n == 0) {  // empty slice: identity point, zero scalar
-        ctx->last_batch_points = 0;
-        uint64_t h[24] = {0};
-        h[0] = 1;
-        h[6] = 1;
-        CUDA_TRY(ctx, cudaMemcpyAsync(partial192, h, 192, cudaMemcpyHostToDevice, ctx->stream));
-        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-        return SCHNORR_B200_OK;
-    }
+    if (n == 0) return batch_partial_empty(ctx, partial192);
     return batch_partial_impl(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, partial192);
 }
 
@@ -1365,20 +1387,9 @@ int schnorr_b200_verify_batch_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_t
     if (!ctx || !result216 || (n && (!sigs81 || !pk96 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
     NOT_ON_MULTI(ctx);
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    void* d_res;
-    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
-    uint8_t* partial = (uint8_t*)d_res + 64 + RESULT_BYTES;
-    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;
-    if (n == 0) {
-        if (int rc = schnorr_b200_batch_partial_dev(ctx, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, partial)) return rc;
-    } else {
-        if (int rc = batch_partial_impl(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, partial, rhs_pre)) return rc;
-        CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
-    }
-    k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, result216, rhs_pre);
-    ctx->launches += 1;
-    CUDA_TRY(ctx, cudaGetLastError());
-    return SCHNORR_B200_OK;
+    return batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+        return batch_partial_impl(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, partial, rhs_pre);
+    }, result216);
 }
 
 // Bisection over partial MSMs on DEVICE buffers.  A range whose own random linear combination
@@ -1464,47 +1475,41 @@ int schnorr_b200_locate_invalid_dev(schnorr_b200_ctx* ctx, size_t n, const uint8
     return locate_items(ctx, leaves, sigs81, pk96, pk_inf, msgs, msg_off, flags);
 }
 
+// the host forms of localisation, on inputs staged on the first device of ctx: the flags into d_flags, copied back to
+// `flags` and counted; the error text of a shard is copied up to ctx
+static int locate_invalid_staged(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
+                                 const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
+                                 uint8_t* d_flags, uint8_t* flags, uint64_t* n_bad) {
+    schnorr_b200_ctx* c = device_ctx(ctx, 0);
+    if (int rc = schnorr_b200_locate_invalid_dev(c, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, d_flags)) {
+        if (c != ctx) ctx->err = c->err;
+        return rc;
+    }
+    CUDA_TRY(c, cudaMemcpyAsync(flags, d_flags, n, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    if (n_bad)
+        for (size_t i = 0; i < n; i++) *n_bad += flags[i] != 0;
+    return SCHNORR_B200_OK;
+}
+
 int schnorr_b200_locate_invalid(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
                                 const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
                                 uint8_t* flags, uint64_t* n_bad) {
     if (!ctx || (n && (!sigs81 || !pk96 || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
     if (n_bad) *n_bad = 0;
     if (n == 0) return SCHNORR_B200_OK;
-    schnorr_b200_ctx* c = ctx->shards.empty() ? ctx : ctx->shards[0];   // localisation runs on the first device
+    schnorr_b200_ctx* c = device_ctx(ctx, 0);   // localisation runs on the first device
     CUDA_TRY(c, cudaSetDevice(c->device));
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
     // dedicated staging (slot M is only used by verify_many's work lists): inputs stay resident across the bisection
-    size_t sz_sig = (n * 81 + 255) & ~(size_t)255, sz_pk = (n * 96 + 255) & ~(size_t)255, sz_m = (mb + 255) & ~(size_t)255,
-           sz_off = ((n + 1) * 8 + 255) & ~(size_t)255, sz_rand = (n * 32 + 255) & ~(size_t)255, sz_inf = (n + 255) & ~(size_t)255;
-    void* blob;
-    if (int rc = ensure_scratch(c, SL_M, sz_sig + sz_pk + sz_m + sz_off + sz_rand + 2 * sz_inf, &blob)) return rc;
-    uint8_t* p = (uint8_t*)blob;
-    uint8_t *d_sig = p; p += sz_sig;
-    uint8_t *d_pk = p; p += sz_pk;
-    uint8_t *d_m = p; p += sz_m;
-    uint8_t *d_off = p; p += sz_off;
-    uint8_t *d_rand = p; p += sz_rand;
-    uint8_t *d_inf = p; p += sz_inf;
-    uint8_t *d_flags = p;
-    cudaStream_t st = c->stream;
-    CUDA_TRY(c, cudaMemcpyAsync(d_sig, sigs81, n * 81, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(d_pk, pk96, n * 96, cudaMemcpyHostToDevice, st));
-    if (mb) CUDA_TRY(c, cudaMemcpyAsync(d_m, msgs, mb, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(d_off, msg_off, (n + 1) * 8, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(d_rand, rand32, n * 32, cudaMemcpyHostToDevice, st));
-    if (pk_inf) CUDA_TRY(c, cudaMemcpyAsync(d_inf, pk_inf, n, cudaMemcpyHostToDevice, st));
-    int rc = schnorr_b200_locate_invalid_dev(c, n, d_sig, d_pk, pk_inf ? d_inf : nullptr, d_m, (const uint64_t*)d_off, d_rand, d_flags);
-    if (rc) {
-        if (c != ctx) ctx->err = c->err;
+    uint8_t *d_sig, *d_pk, *d_m, *d_off, *d_rand, *d_inf, *d_flags;
+    if (int rc = stage_in(c, SL_M, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                    {rand32, n * 32, &d_rand}, {pk_inf, n, &d_inf}, {nullptr, n, &d_flags}}))
         return rc;
-    }
-    CUDA_TRY(c, cudaMemcpyAsync(flags, d_flags, n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(c, cudaStreamSynchronize(st));
-    if (n_bad)
-        for (size_t i = 0; i < n; i++) *n_bad += flags[i] != 0;
-    return SCHNORR_B200_OK;
+    return locate_invalid_staged(ctx, n, d_sig, d_pk, pk_inf ? d_inf : nullptr, d_m, (const uint64_t*)d_off, d_rand, d_flags,
+                                 flags, n_bad);
 }
 
 static int read_result(schnorr_b200_ctx* ctx, const uint8_t* d_res, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
@@ -1530,37 +1535,19 @@ int schnorr_b200_batch_finish(schnorr_b200_ctx* ctx, size_t n_partials, const ui
     return read_result(ctx, res, verdict, lhs97, rhs97);
 }
 
-// host inputs -> staged on the device -> one 192-byte partial at `partial` (device memory of this context)
+// host inputs (n > 0) -> staged on the device -> one 192-byte partial at `partial` (device memory of this context)
 static int batch_partial_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
                               const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
                               uint8_t* partial, uint64_t* rhs_pre = nullptr) {
-    if (n == 0) return schnorr_b200_batch_partial_dev(ctx, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, partial);
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
     // staging slots distinct from those batch_partial_impl uses (A-G, J-L): one blob in slot H
-    void *d_sig, *d_pk, *d_inf = nullptr, *d_m, *d_off, *d_rand;
-    size_t sz_sig = (n * 81 + 255) & ~(size_t)255, sz_pk = (n * 96 + 255) & ~(size_t)255,
-           sz_m = (mb + 255) & ~(size_t)255, sz_off = ((n + 1) * 8 + 255) & ~(size_t)255,
-           sz_rand = (n * 32 + 255) & ~(size_t)255, sz_inf = (n + 255) & ~(size_t)255;
-    void* blob;
-    if (int rc = ensure_scratch(ctx, SL_H, sz_sig + sz_pk + sz_m + sz_off + sz_rand + sz_inf, &blob)) return rc;
-    uint8_t* p = (uint8_t*)blob;
-    d_sig = p; p += sz_sig;
-    d_pk = p; p += sz_pk;
-    d_m = p; p += sz_m;
-    d_off = p; p += sz_off;
-    d_rand = p; p += sz_rand;
-    if (pk_inf) d_inf = p;
-    cudaStream_t st = ctx->stream;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_sig, sigs81, n * 81, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_pk, pk96, n * 96, cudaMemcpyHostToDevice, st));
-    if (mb) CUDA_TRY(ctx, cudaMemcpyAsync(d_m, msgs, mb, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_off, msg_off, (n + 1) * 8, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_rand, rand32, n * 32, cudaMemcpyHostToDevice, st));
-    if (pk_inf) CUDA_TRY(ctx, cudaMemcpyAsync(d_inf, pk_inf, n, cudaMemcpyHostToDevice, st));
-    return batch_partial_impl(ctx, n, (uint8_t*)d_sig, (uint8_t*)d_pk, (uint8_t*)d_inf, (uint8_t*)d_m, (uint64_t*)d_off,
-                              (uint8_t*)d_rand, partial, rhs_pre);
+    uint8_t *d_sig, *d_pk, *d_m, *d_off, *d_rand, *d_inf;
+    if (int rc = stage_in(ctx, SL_H, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                      {rand32, n * 32, &d_rand}, {pk_inf, n, &d_inf}}))
+        return rc;
+    return batch_partial_impl(ctx, n, d_sig, d_pk, pk_inf ? d_inf : nullptr, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
 }
 
 int schnorr_b200_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
@@ -1574,16 +1561,11 @@ int schnorr_b200_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
                                       rand32 + 32 * s.lo, partial);
         });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    void* d_res;
-    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
-    uint8_t* res = (uint8_t*)d_res + 64;
-    uint8_t* partial = res + RESULT_BYTES;
-    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;   // (sum s e) G computed beside the MSM
-    if (int rc = batch_partial_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, partial, rhs_pre)) return rc;
-    if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
-    k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, res, rhs_pre);
-    ctx->launches += 1;
-    CUDA_TRY(ctx, cudaGetLastError());
+    uint8_t* res = nullptr;
+    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+            return batch_partial_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, partial, rhs_pre);
+        }, res))
+        return rc;
     return read_result(ctx, res, verdict, lhs97, rhs97);
 }
 

@@ -148,7 +148,7 @@ static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* m
         size_t cn = s.hi - s.lo;
         int r;
         if (cn == 0) {
-            r = batch_partial_host(sh, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, partial);
+            r = batch_partial_empty(sh, partial);
         } else {
             auto off = rebase_offsets(msg_off, s.lo, s.hi);
             r = partial_fn(k, s, off.data(), partial);

@@ -981,6 +981,31 @@ static int stage_in(schnorr_b200_ctx* ctx, int slot, const void* host, size_t by
     return 0;
 }
 
+// Several regions in one scratch slot, each starting on a 256-byte boundary: *dev receives the region's device
+// address, and `host` (when not null) is copied there.  A null `host` only reserves the region.
+struct stage_region {
+    const void* host;
+    size_t bytes;
+    uint8_t** dev;
+};
+static int stage_in(schnorr_b200_ctx* ctx, int slot, std::initializer_list<stage_region> regions) {
+    auto padded = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    size_t total = 0;
+    for (const stage_region& r : regions) total += padded(r.bytes);
+    void* blob;
+    if (int rc = ensure_scratch(ctx, slot, total, &blob)) return rc;
+    uint8_t* p = (uint8_t*)blob;
+    for (const stage_region& r : regions) {
+        *r.dev = p;
+        if (r.host && r.bytes) CUDA_TRY(ctx, cudaMemcpyAsync(p, r.host, r.bytes, cudaMemcpyHostToDevice, ctx->stream));
+        p += padded(r.bytes);
+    }
+    return 0;
+}
+
+// the single-device context of device k of a context: the context itself unless it has shards
+static schnorr_b200_ctx* device_ctx(schnorr_b200_ctx* ctx, size_t k) { return ctx->shards.empty() ? ctx : ctx->shards[k]; }
+
 #define MULTI_DISPATCH(ctx, call)                                  \
     do {                                                           \
         if ((ctx) && !(ctx)->shards.empty()) return call;          \
@@ -1502,11 +1527,9 @@ int schnorr_b200_verify_keyed_many(schnorr_b200_ctx* ctx, size_t n, const uint8_
 } // extern "C"
 
 // ---- registered key sets (keyset.cuh) ---------------------------------------------------------
-// On a multi-device context the set holds one single-device set per shard (`shards`), each with its own table.
-struct schnorr_b200_keyset {
-    schnorr_b200_ctx* ctx = nullptr;  // the context the set was created on
+// what one device of the context holds of a set (every device holds the same)
+struct keyset_dev {
     int device = 0;
-    size_t n_keys = 0;          // slots, removed ones included
     size_t cap = 0;             // slots allocated (append grows records, status and tables geometrically)
     uint64_t* pk12 = nullptr;   // [cap][12] the registered records, gathered per item ahead of k_ingest
     uint8_t* pk_inf = nullptr;  // [cap]
@@ -1515,34 +1538,30 @@ struct schnorr_b200_keyset {
     keyset_entry* lut = nullptr;  // [n_lut] the findable encodings, sorted (keyset.cuh: keyset_lookup)
     uint32_t n_lut = 0;
     size_t lut_cap = 0;
+};
+
+struct schnorr_b200_keyset {
+    schnorr_b200_ctx* ctx = nullptr;  // the context the set was created on
+    size_t n_keys = 0;                // slots, removed ones included
     bool any_not_torsion_free = false;  // a key of status KEY_NOT_TORSION_FREE: batches use the per-signature points
-    std::vector<schnorr_b200_keyset*> shards;
-    // host model, on the set the caller holds (every device holds the same): the status of every slot, the lookup
-    // entry of every slot and whether it is findable, and every findable entry sorted with duplicates
-    // (keyset_update_entries)
+    // host model: the status of every slot, the lookup entry of every slot and whether it is findable, and every
+    // findable entry sorted with duplicates (keyset_update_entries)
     std::vector<uint8_t> h_status;
     std::vector<keyset_entry> h_entry;
     std::vector<uint8_t> h_findable;
     std::vector<keyset_entry> h_all;
+    std::vector<keyset_dev> devs;     // devs[k] on device_ctx(ctx, k)
 };
 
 static void keyset_free(schnorr_b200_keyset* ks) {
-    for (schnorr_b200_keyset* sh : ks->shards) keyset_free(sh);
-    if (ks->pk12 || ks->ktab || ks->lut) {
-        cudaSetDevice(ks->device);
-        cudaFree(ks->pk12);   // pk_inf and status live in the same allocation
-        cudaFree(ks->ktab);
-        cudaFree(ks->lut);
-    }
+    for (keyset_dev& d : ks->devs)
+        if (d.pk12 || d.ktab || d.lut) {
+            cudaSetDevice(d.device);
+            cudaFree(d.pk12);   // pk_inf and status live in the same allocation
+            cudaFree(d.ktab);
+            cudaFree(d.lut);
+        }
     delete ks;
-}
-
-// the single-device sets of a set, with their contexts: the set itself on a single-device context
-static std::vector<std::pair<schnorr_b200_ctx*, schnorr_b200_keyset*>> keyset_devices(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks) {
-    std::vector<std::pair<schnorr_b200_ctx*, schnorr_b200_keyset*>> v;
-    if (ks->shards.empty()) v.emplace_back(ctx, ks);
-    for (size_t k = 0; k < ks->shards.size(); k++) v.emplace_back(ctx->shards[k], ks->shards[k]);
-    return v;
 }
 
 // records of `cap` slots: pk12 [cap][12] | pk_inf [cap] | status [cap]
@@ -1599,50 +1618,50 @@ static int keyset_encode_async(schnorr_b200_ctx* ctx, size_t m, const uint64_t* 
     return 0;
 }
 
-// the lookup table `lut` uploaded to one device's set (the buffer was sized by the caller: lut_cap >= lut.size())
-static int keyset_upload_lut(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const std::vector<keyset_entry>& lut) {
-    ks->n_lut = (uint32_t)lut.size();
+// the lookup table `lut` uploaded to one device (the buffer was sized by the caller: lut_cap >= lut.size())
+static int keyset_upload_lut(schnorr_b200_ctx* ctx, keyset_dev& kd, const std::vector<keyset_entry>& lut) {
+    kd.n_lut = (uint32_t)lut.size();
     if (!lut.empty())
-        CUDA_TRY(ctx, cudaMemcpyAsync(ks->lut, lut.data(), lut.size() * sizeof(keyset_entry), cudaMemcpyHostToDevice, ctx->stream));
+        CUDA_TRY(ctx, cudaMemcpyAsync(kd.lut, lut.data(), lut.size() * sizeof(keyset_entry), cudaMemcpyHostToDevice, ctx->stream));
     return 0;
 }
 
-// registration on one device: copies the records, registers them (keyset_register), and builds the lookup table of
-// the encodings (k_keyset_encode; sorted on the host while the key tables are built).  `model` (the first device):
-// also fills the host model of `top` and the status bytes.
-static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, const uint8_t* pk96, const uint8_t* pk_inf,
-                        schnorr_b200_keyset* top, bool model) {
+// registration of the set's n_keys records on device k (context ctx): copies the records, registers them
+// (keyset_register), and builds the lookup table of the encodings (k_keyset_encode; sorted on the host while the key
+// tables are built).  Device 0 also fills the host model.
+static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t k, const uint8_t* pk96, const uint8_t* pk_inf) {
     const size_t n = ks->n_keys;
-    ks->device = ctx->device;
-    ks->cap = n;
+    keyset_dev& kd = ks->devs[k];
+    kd.device = ctx->device;
+    kd.cap = n;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    if (int rc = keyset_alloc_records(ctx, n, &ks->pk12, &ks->pk_inf, &ks->status)) return rc;
-    CUDA_TRY(ctx, cudaMalloc(&ks->ktab, n * KT_KEY_U64 * sizeof(uint64_t)));
-    CUDA_TRY(ctx, cudaMemsetAsync(ks->ktab, 0, n * KT_KEY_U64 * sizeof(uint64_t), ctx->stream));
-    CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk12, pk96, n * 96, cudaMemcpyHostToDevice, ctx->stream));
-    if (pk_inf) CUDA_TRY(ctx, cudaMemcpyAsync(ks->pk_inf, pk_inf, n, cudaMemcpyHostToDevice, ctx->stream));
-    else CUDA_TRY(ctx, cudaMemsetAsync(ks->pk_inf, 0, n, ctx->stream));
+    if (int rc = keyset_alloc_records(ctx, n, &kd.pk12, &kd.pk_inf, &kd.status)) return rc;
+    CUDA_TRY(ctx, cudaMalloc(&kd.ktab, n * KT_KEY_U64 * sizeof(uint64_t)));
+    CUDA_TRY(ctx, cudaMemsetAsync(kd.ktab, 0, n * KT_KEY_U64 * sizeof(uint64_t), ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(kd.pk12, pk96, n * 96, cudaMemcpyHostToDevice, ctx->stream));
+    if (pk_inf) CUDA_TRY(ctx, cudaMemcpyAsync(kd.pk_inf, pk_inf, n, cudaMemcpyHostToDevice, ctx->stream));
+    else CUDA_TRY(ctx, cudaMemsetAsync(kd.pk_inf, 0, n, ctx->stream));
     std::vector<keyset_entry> entries(n);
     std::vector<uint8_t> findable(n);
-    if (int rc = keyset_encode_async(ctx, n, ks->pk12, ks->pk_inf, entries.data(), findable.data())) return rc;
-    if (int rc = keyset_register(ctx, n, ks->pk12, ks->pk_inf, ks->status, ks->ktab)) return rc;
-    if (model) {
-        top->h_status.resize(n);
-        CUDA_TRY(ctx, cudaMemcpyAsync(top->h_status.data(), ks->status, n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (int rc = keyset_encode_async(ctx, n, kd.pk12, kd.pk_inf, entries.data(), findable.data())) return rc;
+    if (int rc = keyset_register(ctx, n, kd.pk12, kd.pk_inf, kd.status, kd.ktab)) return rc;
+    if (k == 0) {
+        ks->h_status.resize(n);
+        CUDA_TRY(ctx, cudaMemcpyAsync(ks->h_status.data(), kd.status, n, cudaMemcpyDeviceToHost, ctx->stream));
     }
     CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev_aux));
     std::vector<keyset_entry> added, all, lut;
-    for (size_t k = 0; k < n; k++)
-        if (findable[k]) added.push_back(entries[k]);
+    for (size_t j = 0; j < n; j++)
+        if (findable[j]) added.push_back(entries[j]);
     keyset_update_entries(all, nullptr, 0, std::move(added), lut);
-    ks->lut_cap = lut.size() ? lut.size() : 1;
-    CUDA_TRY(ctx, cudaMalloc(&ks->lut, ks->lut_cap * sizeof(keyset_entry)));
-    if (int rc = keyset_upload_lut(ctx, ks, lut)) return rc;
+    kd.lut_cap = lut.size() ? lut.size() : 1;
+    CUDA_TRY(ctx, cudaMalloc(&kd.lut, kd.lut_cap * sizeof(keyset_entry)));
+    if (int rc = keyset_upload_lut(ctx, kd, lut)) return rc;
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    if (model) {
-        top->h_entry.swap(entries);
-        top->h_findable.swap(findable);
-        top->h_all.swap(all);
+    if (k == 0) {
+        ks->h_entry.swap(entries);
+        ks->h_findable.swap(findable);
+        ks->h_all.swap(all);
     }
     return 0;
 }
@@ -1657,7 +1676,7 @@ static constexpr size_t REG_SMALL_MAX = 384;
 // exact_only and small calls go through launch_verify (same verdicts: the planes hold each item's key record).
 // LOOKUP: key_idx may hold KEYSET_MISS (k_keyed_split_lookup); those items are finished by k_verify.
 template <bool LOOKUP>
-static int launch_verify_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, const soa_batch& soa,
+static int launch_verify_registered(schnorr_b200_ctx* ctx, const keyset_dev& kd, const soa_batch& soa,
                                     const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     cudaStream_t st = ctx->stream;
     if (ctx->exact_only || soa.n <= REG_SMALL_MAX) return launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, 0, soa.n, st);
@@ -1668,34 +1687,35 @@ static int launch_verify_registered(schnorr_b200_ctx* ctx, const schnorr_b200_ke
     CUDA_TRY(ctx, cudaMemsetAsync(counter, 0, 4, st));
     ctx->exact_counters_used = 1;
     unsigned grid = grid_for(soa.n, VERIFY_THREADS);
-    k_verify_reg<LOOKUP><<<grid, VERIFY_THREADS, 0, st>>>(soa, key_idx, ks->status, ks->ktab, msgs, msg_off, ctx->gtab, verdicts, list, counter);
+    k_verify_reg<LOOKUP><<<grid, VERIFY_THREADS, 0, st>>>(soa, key_idx, kd.status, kd.ktab, msgs, msg_off, ctx->gtab, verdicts, list, counter);
     k_verify<<<grid, VERIFY_THREADS, 0, st>>>(soa, msgs, msg_off, ctx->gtab, verdicts, list, counter);
     ctx->launches += 2;
     return 0;
 }
 
-// device buffers, single-device context, arguments checked by the caller
-static int verify_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+// device buffers on device k of the set (context ctx), arguments checked by the caller
+static int verify_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* sigs81,
                                  const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
+    const keyset_dev& kd = ks->devs[k];
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     void *d_pk, *d_inf;
     if (int rc = ensure_scratch(ctx, SL_E, n * 96, &d_pk)) return rc;
     if (int rc = ensure_scratch(ctx, SL_I, n, &d_inf)) return rc;
     soa_batch soa;
     if (int rc = alloc_soa(ctx, n, &soa)) return rc;
-    k_keyset_gather<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, key_idx, ks->n_keys, ks->pk12, ks->pk_inf, (uint64_t*)d_pk,
+    k_keyset_gather<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, key_idx, ks->n_keys, kd.pk12, kd.pk_inf, (uint64_t*)d_pk,
                                                               (uint8_t*)d_inf);
     k_ingest<<<grid_for(n, INGEST_THREADS), INGEST_THREADS, 0, ctx->stream>>>(n, sigs81, (uint8_t*)d_pk, (uint8_t*)d_inf, soa);
     ctx->launches += 2;
     cudaEventRecord(ctx->ev_k0, ctx->stream);
-    if (int rc = launch_verify_registered<false>(ctx, ks, soa, key_idx, msgs, msg_off, verdicts)) return rc;
+    if (int rc = launch_verify_registered<false>(ctx, kd, soa, key_idx, msgs, msg_off, verdicts)) return rc;
     cudaEventRecord(ctx->ev_k1, ctx->stream);
     CUDA_TRY(ctx, cudaGetLastError());
     return 0;
 }
 
-// host buffers, single-device context: staged with cudaMemcpyAsync, verdicts copied back, synchronised
-static int verify_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+// host buffers on device k of the set: staged with cudaMemcpyAsync, verdicts copied back, synchronised
+static int verify_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* sigs81,
                                   const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     size_t mb = msg_off[n];
@@ -1705,7 +1725,7 @@ static int verify_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keys
     if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
     if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
     if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
-    if (int rc = verify_registered_dev(ctx, ks, n, (uint8_t*)d_sig, (uint32_t*)d_idx, (uint8_t*)d_m, (uint64_t*)d_off,
+    if (int rc = verify_registered_dev(ctx, ks, k, n, (uint8_t*)d_sig, (uint32_t*)d_idx, (uint8_t*)d_m, (uint64_t*)d_off,
                                        (uint8_t*)d_out))
         return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(verdicts, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1721,16 +1741,9 @@ static int verify_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keys
         }                                                                       \
     } while (0)
 
-
-// any_not_torsion_free from the host model, and the slot count, on the set and its shards
-static void keyset_sync_flags(schnorr_b200_keyset* ks) {
-    bool off_subgroup = false;
-    for (uint8_t v : ks->h_status) off_subgroup |= v == KEY_NOT_TORSION_FREE;
-    ks->any_not_torsion_free = off_subgroup;
-    for (schnorr_b200_keyset* sh : ks->shards) {
-        sh->any_not_torsion_free = off_subgroup;
-        sh->n_keys = ks->n_keys;
-    }
+// whether the host model holds a key of status KEY_NOT_TORSION_FREE
+static bool keyset_any_not_torsion_free(const schnorr_b200_keyset* ks) {
+    return std::find(ks->h_status.begin(), ks->h_status.end(), KEY_NOT_TORSION_FREE) != ks->h_status.end();
 }
 
 // buffers of one device's set that an update allocates before it writes anything
@@ -1761,36 +1774,36 @@ static void keyset_grow_free(int device, keyset_grow& g) {
 // merges the new lookup entries into its model (keyset_update_entries) and uploads the table to every device.
 static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t m, const uint32_t* key_idx,
                          const uint8_t* pk96, const uint8_t* pk_inf, uint8_t* status) {
-    auto devs = keyset_devices(ctx, ks);
     const size_t n = ks->n_keys, new_n = key_idx ? n : n + m;
     const size_t lut_need = ks->h_all.size() + m;  // distinct findable encodings after the update, at most
     const size_t stage_bytes = m * 96 + (m + 15) / 16 * 16 + m * 4;
-    std::vector<keyset_grow> gr(devs.size());
+    std::vector<keyset_grow> gr(ks->devs.size());
     auto fail = [&](int rc, size_t d) {
-        if (devs[d].first != ctx) ctx->err = "device " + std::to_string(devs[d].first->device) + ": " + devs[d].first->err;
-        for (size_t e = 0; e < devs.size(); e++) keyset_grow_free(devs[e].first->device, gr[e]);
+        schnorr_b200_ctx* c = device_ctx(ctx, d);
+        if (c != ctx) ctx->err = "device " + std::to_string(c->device) + ": " + c->err;
+        for (size_t e = 0; e < gr.size(); e++) keyset_grow_free(ks->devs[e].device, gr[e]);
         return rc;
     };
     // ---- allocations
-    for (size_t d = 0; d < devs.size(); d++) {
-        schnorr_b200_ctx* c = devs[d].first;
-        schnorr_b200_keyset* s = devs[d].second;
+    for (size_t d = 0; d < ks->devs.size(); d++) {
+        schnorr_b200_ctx* c = device_ctx(ctx, d);
+        const keyset_dev& s = ks->devs[d];
         keyset_grow& g = gr[d];
         int rc = 0;
         if (cudaSetDevice(c->device) != cudaSuccess) {
             c->err = "cudaSetDevice failed";
             return fail(SCHNORR_B200_ECUDA, d);
         }
-        if (new_n > s->cap) {  // geometric growth: repeated appends copy the tables O(log n) times
-            g.cap = std::max(new_n, s->cap + s->cap / 2);
+        if (new_n > s.cap) {  // geometric growth: repeated appends copy the tables O(log n) times
+            g.cap = std::max(new_n, s.cap + s.cap / 2);
             if ((rc = keyset_alloc_records(c, g.cap, &g.pk12, &g.pk_inf, &g.status))) return fail(rc, d);
             if (cudaMalloc(&g.ktab, g.cap * KT_KEY_U64 * sizeof(uint64_t)) != cudaSuccess) {
                 c->err = "cudaMalloc of the grown key tables failed";
                 return fail(SCHNORR_B200_ECUDA, d);
             }
         }
-        if (lut_need > s->lut_cap) {
-            g.lut_cap = std::max(lut_need, s->lut_cap + s->lut_cap / 2);
+        if (lut_need > s.lut_cap) {
+            g.lut_cap = std::max(lut_need, s.lut_cap + s.lut_cap / 2);
             if (cudaMalloc(&g.lut, g.lut_cap * sizeof(keyset_entry)) != cudaSuccess) {
                 c->err = "cudaMalloc of the lookup table failed";
                 return fail(SCHNORR_B200_ECUDA, d);
@@ -1806,33 +1819,33 @@ static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t 
     std::vector<keyset_entry> entries(m);
     std::vector<uint8_t> findable(m), st(m);
     std::vector<std::pair<int, void*>> old;  // replaced buffers, freed once every device has synchronised
-    for (size_t d = 0; d < devs.size(); d++) {
-        schnorr_b200_ctx* c = devs[d].first;
-        schnorr_b200_keyset* s = devs[d].second;
+    for (size_t d = 0; d < ks->devs.size(); d++) {
+        schnorr_b200_ctx* c = device_ctx(ctx, d);
+        keyset_dev& s = ks->devs[d];
         keyset_grow& g = gr[d];
         cudaStream_t sm = c->stream;
         int rc = 0;
         CUDA_TRY(c, cudaSetDevice(c->device));
         if (g.pk12) {  // one device-to-device copy per buffer; the new tail of the tables is zeros
-            CUDA_TRY(c, cudaMemcpyAsync(g.pk12, s->pk12, n * 96, cudaMemcpyDeviceToDevice, sm));
-            CUDA_TRY(c, cudaMemcpyAsync(g.pk_inf, s->pk_inf, n, cudaMemcpyDeviceToDevice, sm));
-            CUDA_TRY(c, cudaMemcpyAsync(g.status, s->status, n, cudaMemcpyDeviceToDevice, sm));
-            CUDA_TRY(c, cudaMemcpyAsync(g.ktab, s->ktab, n * KT_KEY_U64 * sizeof(uint64_t), cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(g.pk12, s.pk12, n * 96, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(g.pk_inf, s.pk_inf, n, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(g.status, s.status, n, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(g.ktab, s.ktab, n * KT_KEY_U64 * sizeof(uint64_t), cudaMemcpyDeviceToDevice, sm));
             CUDA_TRY(c, cudaMemsetAsync(g.ktab + n * KT_KEY_U64, 0, (g.cap - n) * KT_KEY_U64 * sizeof(uint64_t), sm));
-            old.emplace_back(c->device, s->pk12);
-            old.emplace_back(c->device, s->ktab);
-            s->pk12 = g.pk12;
-            s->pk_inf = g.pk_inf;
-            s->status = g.status;
-            s->ktab = g.ktab;
-            s->cap = g.cap;
+            old.emplace_back(c->device, s.pk12);
+            old.emplace_back(c->device, s.ktab);
+            s.pk12 = g.pk12;
+            s.pk_inf = g.pk_inf;
+            s.status = g.status;
+            s.ktab = g.ktab;
+            s.cap = g.cap;
             g.pk12 = nullptr;
             g.ktab = nullptr;
         }
         if (g.lut) {
-            old.emplace_back(c->device, s->lut);
-            s->lut = g.lut;
-            s->lut_cap = g.lut_cap;
+            old.emplace_back(c->device, s.lut);
+            s.lut = g.lut;
+            s.lut_cap = g.lut_cap;
             g.lut = nullptr;
         }
         uint64_t* spk = (uint64_t*)g.stage;
@@ -1844,10 +1857,10 @@ static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t 
         if (d == 0 && (rc = keyset_encode_async(c, m, spk, sinf, entries.data(), findable.data()))) return rc;
         uint8_t* new_status;
         if (!key_idx) {
-            CUDA_TRY(c, cudaMemcpyAsync(s->pk12 + 12 * n, spk, m * 96, cudaMemcpyDeviceToDevice, sm));
-            CUDA_TRY(c, cudaMemcpyAsync(s->pk_inf + n, sinf, m, cudaMemcpyDeviceToDevice, sm));
-            new_status = s->status + n;
-            if ((rc = keyset_register(c, m, s->pk12 + 12 * n, s->pk_inf + n, new_status, s->ktab + n * KT_KEY_U64))) return rc;
+            CUDA_TRY(c, cudaMemcpyAsync(s.pk12 + 12 * n, spk, m * 96, cudaMemcpyDeviceToDevice, sm));
+            CUDA_TRY(c, cudaMemcpyAsync(s.pk_inf + n, sinf, m, cudaMemcpyDeviceToDevice, sm));
+            new_status = s.status + n;
+            if ((rc = keyset_register(c, m, s.pk12 + 12 * n, s.pk_inf + n, new_status, s.ktab + n * KT_KEY_U64))) return rc;
         } else {
             uint64_t* ctab = (uint64_t*)g.ctab;
             new_status = (uint8_t*)(ctab + m * KT_KEY_U64);
@@ -1855,14 +1868,14 @@ static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t 
             CUDA_TRY(c, cudaMemsetAsync(ctab, 0, m * KT_KEY_U64 * sizeof(uint64_t), sm));
             if ((rc = keyset_register(c, m, spk, sinf, new_status, ctab))) return rc;
             k_keyset_scatter<<<grid_for(m * (KT_KEY_U128 + 13), 256), 256, 0, sm>>>(
-                m, sidx, spk, sinf, new_status, (const ulonglong2*)ctab, s->pk12, s->pk_inf, s->status, (ulonglong2*)s->ktab);
+                m, sidx, spk, sinf, new_status, (const ulonglong2*)ctab, s.pk12, s.pk_inf, s.status, (ulonglong2*)s.ktab);
             c->launches += 1;
             CUDA_TRY(c, cudaGetLastError());
         }
         if (d == 0) CUDA_TRY(c, cudaMemcpyAsync(st.data(), new_status, m, cudaMemcpyDeviceToHost, sm));
     }
     // ---- the host model and the lookup table
-    schnorr_b200_ctx* c0 = devs[0].first;
+    schnorr_b200_ctx* c0 = device_ctx(ctx, 0);
     CUDA_TRY(c0, cudaSetDevice(c0->device));
     CUDA_TRY(c0, cudaStreamSynchronize(c0->stream));
     std::vector<uint8_t> changed(new_n, 0);
@@ -1880,20 +1893,23 @@ static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t 
         if (findable[j]) added.push_back(entries[j]);
     }
     keyset_update_entries(ks->h_all, changed.data(), new_n, std::move(added), lut);
-    for (auto& dv : devs) {
-        CUDA_TRY(dv.first, cudaSetDevice(dv.first->device));
-        if (int rc = keyset_upload_lut(dv.first, dv.second, lut)) return rc;
+    for (size_t d = 0; d < ks->devs.size(); d++) {
+        schnorr_b200_ctx* c = device_ctx(ctx, d);
+        CUDA_TRY(c, cudaSetDevice(c->device));
+        if (int rc = keyset_upload_lut(c, ks->devs[d], lut)) return rc;
     }
-    for (auto& dv : devs) {  // every device synchronised: work enqueued before the update has finished with the old buffers
-        CUDA_TRY(dv.first, cudaSetDevice(dv.first->device));
-        CUDA_TRY(dv.first, cudaStreamSynchronize(dv.first->stream));
+    // every device synchronised: work enqueued before the update has finished with the old buffers
+    for (size_t d = 0; d < ks->devs.size(); d++) {
+        schnorr_b200_ctx* c = device_ctx(ctx, d);
+        CUDA_TRY(c, cudaSetDevice(c->device));
+        CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     }
     for (auto& o : old) {
         cudaSetDevice(o.first);
         cudaFree(o.second);
     }
+    ks->any_not_torsion_free = keyset_any_not_torsion_free(ks);
     ks->n_keys = new_n;
-    keyset_sync_flags(ks);
     if (status) memcpy(status, st.data(), m);
     return SCHNORR_B200_OK;
 }
@@ -1908,24 +1924,17 @@ int schnorr_b200_keyset_create(schnorr_b200_ctx* ctx, size_t n_keys, const uint8
     schnorr_b200_keyset* ks = new schnorr_b200_keyset();
     ks->ctx = ctx;
     ks->n_keys = n_keys;
-    int rc = 0;
-    if (ctx->shards.empty()) {
-        rc = keyset_build(ctx, ks, pk96, pk_inf, ks, true);
-    } else {  // one table per device; the status comes from the first (every shard computes the same)
-        for (size_t k = 0; k < ctx->shards.size() && rc == 0; k++) {
-            schnorr_b200_keyset* sh = new schnorr_b200_keyset();
-            sh->ctx = ctx->shards[k];
-            sh->n_keys = n_keys;
-            ks->shards.push_back(sh);
-            rc = keyset_build(ctx->shards[k], sh, pk96, pk_inf, ks, k == 0);
-            if (rc) ctx->err = "device " + std::to_string(ctx->shards[k]->device) + ": " + ctx->shards[k]->err;
+    ks->devs.resize(schnorr_b200_device_count(ctx));
+    // one table per device; the host model and the status come from the first (every device computes the same)
+    for (size_t k = 0; k < ks->devs.size(); k++) {
+        schnorr_b200_ctx* c = device_ctx(ctx, k);
+        if (int rc = keyset_build(c, ks, k, pk96, pk_inf)) {
+            if (c != ctx) ctx->err = "device " + std::to_string(c->device) + ": " + c->err;
+            keyset_free(ks);
+            return rc;
         }
     }
-    if (rc) {
-        keyset_free(ks);
-        return rc;
-    }
-    keyset_sync_flags(ks);
+    ks->any_not_torsion_free = keyset_any_not_torsion_free(ks);
     if (status) memcpy(status, ks->h_status.data(), n_keys);
     *out = ks;
     return SCHNORR_B200_OK;
@@ -1986,21 +1995,21 @@ int schnorr_b200_keyset_debug_export(schnorr_b200_ctx* ctx, const schnorr_b200_k
                                      uint8_t* lut64, uint32_t* n_lut) {
     if (!ctx || !ks || device_index < 0 || first > ks->n_keys || count > ks->n_keys - first) return SCHNORR_B200_EARG;
     CHECK_KEYSET(ctx, ks);
-    if (device_index >= (int)(ctx->shards.empty() ? 1 : ctx->shards.size())) return SCHNORR_B200_EARG;
-    schnorr_b200_ctx* c = ctx->shards.empty() ? ctx : ctx->shards[device_index];
-    const schnorr_b200_keyset* s = ks->shards.empty() ? ks : ks->shards[device_index];
+    if (device_index >= (int)ks->devs.size()) return SCHNORR_B200_EARG;
+    schnorr_b200_ctx* c = device_ctx(ctx, device_index);
+    const keyset_dev& s = ks->devs[device_index];
     CUDA_TRY(c, cudaSetDevice(c->device));
     if (count) {
-        if (pk96) CUDA_TRY(c, cudaMemcpyAsync(pk96, s->pk12 + 12 * first, count * 96, cudaMemcpyDeviceToHost, c->stream));
-        if (pk_inf) CUDA_TRY(c, cudaMemcpyAsync(pk_inf, s->pk_inf + first, count, cudaMemcpyDeviceToHost, c->stream));
-        if (status) CUDA_TRY(c, cudaMemcpyAsync(status, s->status + first, count, cudaMemcpyDeviceToHost, c->stream));
+        if (pk96) CUDA_TRY(c, cudaMemcpyAsync(pk96, s.pk12 + 12 * first, count * 96, cudaMemcpyDeviceToHost, c->stream));
+        if (pk_inf) CUDA_TRY(c, cudaMemcpyAsync(pk_inf, s.pk_inf + first, count, cudaMemcpyDeviceToHost, c->stream));
+        if (status) CUDA_TRY(c, cudaMemcpyAsync(status, s.status + first, count, cudaMemcpyDeviceToHost, c->stream));
         if (tables)
-            CUDA_TRY(c, cudaMemcpyAsync(tables, s->ktab + first * KT_KEY_U64, count * KT_KEY_U64 * sizeof(uint64_t),
+            CUDA_TRY(c, cudaMemcpyAsync(tables, s.ktab + first * KT_KEY_U64, count * KT_KEY_U64 * sizeof(uint64_t),
                                         cudaMemcpyDeviceToHost, c->stream));
     }
-    if (lut64 && s->n_lut)
-        CUDA_TRY(c, cudaMemcpyAsync(lut64, s->lut, s->n_lut * sizeof(keyset_entry), cudaMemcpyDeviceToHost, c->stream));
-    if (n_lut) *n_lut = s->n_lut;
+    if (lut64 && s.n_lut)
+        CUDA_TRY(c, cudaMemcpyAsync(lut64, s.lut, s.n_lut * sizeof(keyset_entry), cudaMemcpyDeviceToHost, c->stream));
+    if (n_lut) *n_lut = s.n_lut;
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     return SCHNORR_B200_OK;
 }
@@ -2019,11 +2028,11 @@ int schnorr_b200_verify_registered_many(schnorr_b200_ctx* ctx, const schnorr_b20
     if (n == 0) return SCHNORR_B200_OK;
     CHECK_MSG_OFF(ctx, n, msg_off);
     if (msg_off[n] && !msgs) return SCHNORR_B200_EARG;
-    if (ctx->shards.empty()) return verify_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, verdicts);
+    if (ctx->shards.empty()) return verify_registered_host(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, verdicts);
     auto sl = multi_slices(ctx, n);
     return multi_run(ctx, sl, [&](int k, shard_slice s) {
         auto off = rebase_offsets(msg_off, s.lo, s.hi);
-        return verify_registered_host(ctx->shards[k], ks->shards[k], s.hi - s.lo, sigs81 + 81 * s.lo, key_idx + s.lo,
+        return verify_registered_host(ctx->shards[k], ks, k, s.hi - s.lo, sigs81 + 81 * s.lo, key_idx + s.lo,
                                       msgs ? msgs + msg_off[s.lo] : nullptr, off.data(), verdicts + s.lo);
     });
 }
@@ -2036,7 +2045,7 @@ int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx* ctx, const schnorr
     CHECK_KEYSET(ctx, ks);
     NOT_ON_MULTI(ctx);
     if (n == 0) return SCHNORR_B200_OK;
-    return verify_registered_dev(ctx, ks, n, sigs81, key_idx, msgs, msg_off, verdicts);
+    return verify_registered_dev(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, verdicts);
 }
 
 }  // extern "C"
@@ -2054,23 +2063,22 @@ static constexpr double KEYED_REG_MAX_MISS_FRACTION = 0.4;
 // end (synchronises) and take verify_many above KEYED_REG_MAX_MISS_FRACTION.
 // Scratch: J decoded keys, K identity / ok flags | key indices | miss counter, L signatures (the slots of
 // verify_keyed_many_dev, which small calls run); the kernels after them use A-C and M.
-static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
-                                       const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts, bool select) {
+static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
+                                       const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts,
+                                       bool select) {
     if (n <= REG_SMALL_MAX) return schnorr_b200_verify_keyed_many_dev(ctx, n, keyed130, msgs, msg_off, verdicts);
+    const keyset_dev& kd = ks->devs[k];
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const size_t sz_flags = (2 * n + 255) & ~(size_t)255, sz_idx = (4 * n + 255) & ~(size_t)255;
-    void *d_pk, *d_k, *d_sig;
+    void *d_pk, *d_sig;
+    uint8_t *d_inf, *d_idx, *d_miss;
     if (int rc = ensure_scratch(ctx, SL_J, n * 96, &d_pk)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_K, sz_flags + sz_idx + 16, &d_k)) return rc;
+    if (int rc = stage_in(ctx, SL_K, {{nullptr, 2 * n, &d_inf}, {nullptr, 4 * n, &d_idx}, {nullptr, 4, &d_miss}})) return rc;
     if (int rc = ensure_scratch(ctx, SL_L, n * 81 + 256, &d_sig)) return rc;
-    uint8_t* d_inf = (uint8_t*)d_k;
     uint8_t* d_ok = d_inf + n;
-    uint32_t* d_idx = (uint32_t*)((uint8_t*)d_k + sz_flags);
-    uint32_t* d_miss = (uint32_t*)((uint8_t*)d_k + sz_flags + sz_idx);
     CUDA_TRY(ctx, cudaMemsetAsync(d_miss, 0, 4, st));
-    k_keyed_split_lookup<<<grid_for(n, 128), 128, 0, st>>>(n, keyed130, ks->lut, ks->n_lut, ks->pk12, ks->pk_inf, (uint8_t*)d_pk,
-                                                          d_inf, d_ok, (uint8_t*)d_sig, d_idx, d_miss);
+    k_keyed_split_lookup<<<grid_for(n, 128), 128, 0, st>>>(n, keyed130, kd.lut, kd.n_lut, kd.pk12, kd.pk_inf, (uint8_t*)d_pk,
+                                                          d_inf, d_ok, (uint8_t*)d_sig, (uint32_t*)d_idx, (uint32_t*)d_miss);
     ctx->launches += 1;
     bool lookup_path = true;
     if (select) {
@@ -2085,7 +2093,7 @@ static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200
         k_ingest<<<grid_for(n, INGEST_THREADS), INGEST_THREADS, 0, st>>>(n, (uint8_t*)d_sig, (uint8_t*)d_pk, d_inf, soa);
         ctx->launches += 1;
         cudaEventRecord(ctx->ev_k0, st);
-        if (int rc = launch_verify_registered<true>(ctx, ks, soa, d_idx, msgs, msg_off, verdicts)) return rc;
+        if (int rc = launch_verify_registered<true>(ctx, kd, soa, (uint32_t*)d_idx, msgs, msg_off, verdicts)) return rc;
         cudaEventRecord(ctx->ev_k1, st);
     } else if (int rc = schnorr_b200_verify_many_dev(ctx, n, (uint8_t*)d_sig, (uint8_t*)d_pk, d_inf, msgs, msg_off, verdicts)) {
         return rc;
@@ -2096,9 +2104,9 @@ static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200
     return 0;
 }
 
-// host buffers, single-device context: staged in D, F, G, verdicts in H, synchronised
-static int verify_keyed_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
-                                        const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
+// host buffers on device k of the set: staged in D, F, G, verdicts in H, synchronised
+static int verify_keyed_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
+                                        const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     size_t mb = msg_off[n];
     void *d_rec, *d_m, *d_off, *d_out;
@@ -2106,7 +2114,7 @@ static int verify_keyed_registered_host(schnorr_b200_ctx* ctx, const schnorr_b20
     if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
     if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
     if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
-    if (int rc = verify_keyed_registered_dev(ctx, ks, n, (uint8_t*)d_rec, (uint8_t*)d_m, (uint64_t*)d_off, (uint8_t*)d_out, true))
+    if (int rc = verify_keyed_registered_dev(ctx, ks, k, n, (uint8_t*)d_rec, (uint8_t*)d_m, (uint64_t*)d_off, (uint8_t*)d_out, true))
         return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(verdicts, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -2120,13 +2128,13 @@ int schnorr_b200_keyset_lookup(schnorr_b200_ctx* ctx, const schnorr_b200_keyset*
     if (!ctx || !ks || (n && (!keys49 || !key_idx))) return SCHNORR_B200_EARG;
     CHECK_KEYSET(ctx, ks);
     if (n == 0) return SCHNORR_B200_OK;
-    schnorr_b200_ctx* c = ctx->shards.empty() ? ctx : ctx->shards[0];
-    const schnorr_b200_keyset* kc = ks->shards.empty() ? ks : ks->shards[0];
+    schnorr_b200_ctx* c = device_ctx(ctx, 0);
+    const keyset_dev& kd = ks->devs[0];
     CUDA_TRY(c, cudaSetDevice(c->device));
     void *d_in, *d_out;
     if (int rc = stage_in(c, SL_D, keys49, n * 49, &d_in)) return rc;
     if (int rc = ensure_scratch(c, SL_H, n * 4, &d_out)) return rc;
-    k_keyset_lookup<<<grid_for(n, 128), 128, 0, c->stream>>>(n, (uint8_t*)d_in, kc->lut, kc->n_lut, (uint32_t*)d_out);
+    k_keyset_lookup<<<grid_for(n, 128), 128, 0, c->stream>>>(n, (uint8_t*)d_in, kd.lut, kd.n_lut, (uint32_t*)d_out);
     c->launches += 1;
     CUDA_TRY(c, cudaGetLastError());
     CUDA_TRY(c, cudaMemcpyAsync(key_idx, d_out, n * 4, cudaMemcpyDeviceToHost, c->stream));
@@ -2141,7 +2149,7 @@ int schnorr_b200_keyset_lookup_dev(schnorr_b200_ctx* ctx, const schnorr_b200_key
     NOT_ON_MULTI(ctx);
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    k_keyset_lookup<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, keys49, ks->lut, ks->n_lut, key_idx);
+    k_keyset_lookup<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, keys49, ks->devs[0].lut, ks->devs[0].n_lut, key_idx);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
     return SCHNORR_B200_OK;
@@ -2155,11 +2163,11 @@ int schnorr_b200_verify_keyed_registered_many(schnorr_b200_ctx* ctx, const schno
     if (n == 0) return SCHNORR_B200_OK;
     CHECK_MSG_OFF(ctx, n, msg_off);
     if (msg_off[n] && !msgs) return SCHNORR_B200_EARG;
-    if (ctx->shards.empty()) return verify_keyed_registered_host(ctx, ks, n, keyed130, msgs, msg_off, verdicts);
+    if (ctx->shards.empty()) return verify_keyed_registered_host(ctx, ks, 0, n, keyed130, msgs, msg_off, verdicts);
     auto sl = multi_slices(ctx, n);
     return multi_run(ctx, sl, [&](int k, shard_slice s) {
         auto off = rebase_offsets(msg_off, s.lo, s.hi);
-        return verify_keyed_registered_host(ctx->shards[k], ks->shards[k], s.hi - s.lo, keyed130 + 130 * s.lo,
+        return verify_keyed_registered_host(ctx->shards[k], ks, k, s.hi - s.lo, keyed130 + 130 * s.lo,
                                             msgs ? msgs + msg_off[s.lo] : nullptr, off.data(), verdicts + s.lo);
     });
 }
@@ -2172,7 +2180,7 @@ int schnorr_b200_verify_keyed_registered_many_dev(schnorr_b200_ctx* ctx, const s
     CHECK_KEYSET(ctx, ks);
     NOT_ON_MULTI(ctx);
     if (n == 0) return SCHNORR_B200_OK;
-    return verify_keyed_registered_dev(ctx, ks, n, keyed130, msgs, msg_off, verdicts, false);
+    return verify_keyed_registered_dev(ctx, ks, 0, n, keyed130, msgs, msg_off, verdicts, false);
 }
 
 }  // extern "C"
@@ -2186,64 +2194,49 @@ static bool reg_batch_aggregates(const schnorr_b200_ctx* ctx, const schnorr_b200
     return n > ctx->batch_small_max && !ks->any_not_torsion_free && n / ks->n_keys >= ctx->reg_batch_min_per_key;
 }
 
-// one 192-byte partial of a registered batch on device buffers (single-device context, arguments checked)
-static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+// one 192-byte partial of a registered batch of n > 0 signatures on device buffers of device k of the set (arguments
+// checked)
+static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* sigs81,
                                     const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
                                     uint8_t* partial192, uint64_t* rhs_pre) {
-    if (n == 0) return schnorr_b200_batch_partial_dev(ctx, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, partial192);
+    const keyset_dev& kd = ks->devs[k];
     cudaStream_t st = ctx->stream;
-    const size_t sz_pk = (n * 96 + 255) & ~(size_t)255;
-    void* d_pk;
-    if (int rc = ensure_scratch(ctx, SL_N, sz_pk + n, &d_pk)) return rc;
-    uint8_t* d_inf = (uint8_t*)d_pk + sz_pk;
-    k_keyset_gather<<<grid_for(n, 128), 128, 0, st>>>(n, key_idx, ks->n_keys, ks->pk12, ks->pk_inf, (uint64_t*)d_pk, d_inf);
+    uint8_t *d_pk, *d_inf;
+    if (int rc = stage_in(ctx, SL_N, {{nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}})) return rc;
+    k_keyset_gather<<<grid_for(n, 128), 128, 0, st>>>(n, key_idx, ks->n_keys, kd.pk12, kd.pk_inf, (uint64_t*)d_pk, d_inf);
     ctx->launches += 1;
     if (!reg_batch_aggregates(ctx, ks, n))
-        return batch_partial_impl(ctx, n, sigs81, (uint8_t*)d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre);
-    // key side: column sums | per-block key terms | key partial | MSM partial | 64 zero bytes
+        return batch_partial_impl(ctx, n, sigs81, d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre);
+    // key side: per-block key terms | column sums, key partial, MSM partial, 64 zero bytes
     size_t max_blocks = (size_t)2 * ctx->sm_count, want = (ks->n_keys + KEYTERM_THREADS / 32 - 1) / (KEYTERM_THREADS / 32);
     unsigned blocks = (unsigned)(want < max_blocks ? want : max_blocks);
-    const size_t sz_cols = ks->n_keys * 8 * sizeof(unsigned long long), sz_terms = ((size_t)blocks * sizeof(jac_pt) + 255) & ~(size_t)255;
-    void* d_key;
-    if (int rc = ensure_scratch(ctx, SL_O, sz_cols + sz_terms + 192 + 192 + 64, &d_key)) return rc;
-    uint8_t* p = (uint8_t*)d_key;
+    const size_t sz_cols = ks->n_keys * 8 * sizeof(unsigned long long);
+    uint8_t *d_terms, *d_cols;
+    if (int rc = stage_in(ctx, SL_O, {{nullptr, (size_t)blocks * sizeof(jac_pt), &d_terms}, {nullptr, sz_cols + 192 + 192 + 64, &d_cols}}))
+        return rc;
     reg_batch rb;
     rb.key_idx = key_idx;
     rb.n_keys = ks->n_keys;
-    rb.ktab = ks->ktab;
-    rb.cols = (unsigned long long*)p;
-    rb.terms = (uint64_t*)(p + sz_cols);
+    rb.ktab = kd.ktab;
+    rb.cols = (unsigned long long*)d_cols;
+    rb.terms = (uint64_t*)d_terms;
     rb.term_blocks = blocks;
-    rb.key_partial = (uint64_t*)(p + sz_cols + sz_terms);
+    rb.key_partial = (uint64_t*)(d_cols + sz_cols);
     rb.msm_partial = rb.key_partial + 24;
     rb.zero = (const uint32_t*)(rb.msm_partial + 24);
     CUDA_TRY(ctx, cudaMemsetAsync((void*)rb.zero, 0, 64, st));
-    return batch_partial_impl(ctx, n, sigs81, (uint8_t*)d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre, &rb);
+    return batch_partial_impl(ctx, n, sigs81, d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre, &rb);
 }
 
-// host inputs (offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
-static int batch_partial_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
-                                         const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
-                                         const uint8_t* rand32, uint8_t* partial, uint64_t* rhs_pre) {
-    if (n == 0) return batch_partial_registered(ctx, ks, 0, nullptr, nullptr, nullptr, nullptr, nullptr, partial, nullptr);
-    size_t mb = msg_off[n];
-    size_t sz_sig = (n * 81 + 255) & ~(size_t)255, sz_idx = (n * 4 + 255) & ~(size_t)255, sz_m = (mb + 255) & ~(size_t)255,
-           sz_off = ((n + 1) * 8 + 255) & ~(size_t)255;
-    void* blob;
-    if (int rc = ensure_scratch(ctx, SL_H, sz_sig + sz_idx + sz_m + sz_off + n * 32, &blob)) return rc;
-    uint8_t* p = (uint8_t*)blob;
-    uint8_t* d_sig = p; p += sz_sig;
-    uint8_t* d_idx = p; p += sz_idx;
-    uint8_t* d_m = p; p += sz_m;
-    uint8_t* d_off = p; p += sz_off;
-    uint8_t* d_rand = p;
-    cudaStream_t st = ctx->stream;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_sig, sigs81, n * 81, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_idx, key_idx, n * 4, cudaMemcpyHostToDevice, st));
-    if (mb) CUDA_TRY(ctx, cudaMemcpyAsync(d_m, msgs, mb, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_off, msg_off, (n + 1) * 8, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_rand, rand32, n * 32, cudaMemcpyHostToDevice, st));
-    return batch_partial_registered(ctx, ks, n, d_sig, (uint32_t*)d_idx, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
+// host inputs (n > 0, offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
+static int batch_partial_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
+                                         const uint8_t* sigs81, const uint32_t* key_idx, const uint8_t* msgs,
+                                         const uint64_t* msg_off, const uint8_t* rand32, uint8_t* partial, uint64_t* rhs_pre) {
+    uint8_t *d_sig, *d_idx, *d_m, *d_off, *d_rand;
+    if (int rc = stage_in(ctx, SL_H, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, msg_off[n], &d_m},
+                                      {msg_off, (n + 1) * 8, &d_off}, {rand32, n * 32, &d_rand}}))
+        return rc;
+    return batch_partial_registered(ctx, ks, k, n, d_sig, (uint32_t*)d_idx, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
 }
 
 extern "C" {
@@ -2259,20 +2252,15 @@ int schnorr_b200_verify_batch_registered(schnorr_b200_ctx* ctx, const schnorr_b2
     }
     if (!ctx->shards.empty())
         return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
-            return batch_partial_registered_host(ctx->shards[k], ks->shards[k], s.hi - s.lo, sigs81 + 81 * s.lo, key_idx + s.lo,
+            return batch_partial_registered_host(ctx->shards[k], ks, k, s.hi - s.lo, sigs81 + 81 * s.lo, key_idx + s.lo,
                                                  msgs ? msgs + msg_off[s.lo] : nullptr, off, rand32 + 32 * s.lo, partial, nullptr);
         });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    void* d_res;
-    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
-    uint8_t* res = (uint8_t*)d_res + 64;
-    uint8_t* partial = res + RESULT_BYTES;
-    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;   // (sum s e) G computed beside the MSM
-    if (int rc = batch_partial_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand32, partial, rhs_pre)) return rc;
-    if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
-    k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, res, rhs_pre);
-    ctx->launches += 1;
-    CUDA_TRY(ctx, cudaGetLastError());
+    uint8_t* res = nullptr;
+    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+            return batch_partial_registered_host(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, rand32, partial, rhs_pre);
+        }, res))
+        return rc;
     return read_result(ctx, res, verdict, lhs97, rhs97);
 }
 
@@ -2283,16 +2271,9 @@ int schnorr_b200_verify_batch_registered_dev(schnorr_b200_ctx* ctx, const schnor
     CHECK_KEYSET(ctx, ks);
     NOT_ON_MULTI(ctx);
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    void* d_res;
-    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
-    uint8_t* partial = (uint8_t*)d_res + 64 + RESULT_BYTES;
-    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;
-    if (int rc = batch_partial_registered(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand32, partial, rhs_pre)) return rc;
-    if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
-    k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, result216, rhs_pre);
-    ctx->launches += 1;
-    CUDA_TRY(ctx, cudaGetLastError());
-    return SCHNORR_B200_OK;
+    return batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+        return batch_partial_registered(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, rand32, partial, rhs_pre);
+    }, result216);
 }
 
 // localisation on the first device: the inputs staged in slot M, the items' key records gathered into slot N, then the
@@ -2307,42 +2288,18 @@ int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx* ctx, const schnorr_
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
-    schnorr_b200_ctx* c = ctx->shards.empty() ? ctx : ctx->shards[0];
-    const schnorr_b200_keyset* kc = ks->shards.empty() ? ks : ks->shards[0];
+    schnorr_b200_ctx* c = device_ctx(ctx, 0);
+    const keyset_dev& kd = ks->devs[0];
     CUDA_TRY(c, cudaSetDevice(c->device));
-    size_t sz_sig = (n * 81 + 255) & ~(size_t)255, sz_idx = (n * 4 + 255) & ~(size_t)255, sz_m = (mb + 255) & ~(size_t)255,
-           sz_off = ((n + 1) * 8 + 255) & ~(size_t)255, sz_rand = (n * 32 + 255) & ~(size_t)255;
-    void *blob, *recs;
-    const size_t sz_pk = (n * 96 + 255) & ~(size_t)255;
-    if (int rc = ensure_scratch(c, SL_M, sz_sig + sz_idx + sz_m + sz_off + sz_rand + n, &blob)) return rc;
-    if (int rc = ensure_scratch(c, SL_N, sz_pk + n, &recs)) return rc;
-    uint8_t* p = (uint8_t*)blob;
-    uint8_t* d_sig = p; p += sz_sig;
-    uint8_t* d_idx = p; p += sz_idx;
-    uint8_t* d_m = p; p += sz_m;
-    uint8_t* d_off = p; p += sz_off;
-    uint8_t* d_rand = p; p += sz_rand;
-    uint8_t* d_flags = p;
-    uint8_t* d_pk = (uint8_t*)recs;
-    uint8_t* d_inf = d_pk + sz_pk;
-    cudaStream_t st = c->stream;
-    CUDA_TRY(c, cudaMemcpyAsync(d_sig, sigs81, n * 81, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(d_idx, key_idx, n * 4, cudaMemcpyHostToDevice, st));
-    if (mb) CUDA_TRY(c, cudaMemcpyAsync(d_m, msgs, mb, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(d_off, msg_off, (n + 1) * 8, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(d_rand, rand32, n * 32, cudaMemcpyHostToDevice, st));
-    k_keyset_gather<<<grid_for(n, 128), 128, 0, st>>>(n, (uint32_t*)d_idx, kc->n_keys, kc->pk12, kc->pk_inf, (uint64_t*)d_pk, d_inf);
-    c->launches += 1;
-    int rc = schnorr_b200_locate_invalid_dev(c, n, d_sig, d_pk, d_inf, d_m, (const uint64_t*)d_off, d_rand, d_flags);
-    if (rc) {
-        if (c != ctx) ctx->err = c->err;
+    uint8_t *d_sig, *d_idx, *d_m, *d_off, *d_rand, *d_flags, *d_pk, *d_inf;
+    if (int rc = stage_in(c, SL_M, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                    {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}}))
         return rc;
-    }
-    CUDA_TRY(c, cudaMemcpyAsync(flags, d_flags, n, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(c, cudaStreamSynchronize(st));
-    if (n_bad)
-        for (size_t i = 0; i < n; i++) *n_bad += flags[i] != 0;
-    return SCHNORR_B200_OK;
+    if (int rc = stage_in(c, SL_N, {{nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}})) return rc;
+    k_keyset_gather<<<grid_for(n, 128), 128, 0, c->stream>>>(n, (uint32_t*)d_idx, ks->n_keys, kd.pk12, kd.pk_inf, (uint64_t*)d_pk,
+                                                            d_inf);
+    c->launches += 1;
+    return locate_invalid_staged(ctx, n, d_sig, d_pk, d_inf, d_m, (const uint64_t*)d_off, d_rand, d_flags, flags, n_bad);
 }
 
 // ---- keygen / sign ---------------------------------------------------------------------------
