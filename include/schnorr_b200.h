@@ -261,11 +261,14 @@ int schnorr_b200_batch_finish(schnorr_b200_ctx *ctx, size_t n_partials, const ui
 
 /* Failed-batch localisation (SURVEY.md 8(f) f3).  The reference answers a bad batch with ONE Err for the lot
  * (src/batch.rs:125-129); this names the culprits, in BATCH semantics: item i is bad when its own term of the batch
- * equation, R_i - h_i P_i - e_i G with R_i = from_compressed(sig_i.x) INCLUDING the flag byte and no subgroup check on
- * P_i (src/batch.rs:102-106), is not the identity -- e.g. a signature whose y-sign flag is flipped fails the batch although
- * Signature::verify (x-only, src/signature.rs:186,200) accepts it.  Bisection over partial MSMs (a range whose own random
- * linear combination holds is clean), exact per-item check on the failing slices.  flags[i] = 0 clean, 2 bad, 3 malformed
- * (the reference panics on it); *n_bad (optional) = number of non-zero flags.  rand32 as in verify_batch. */
+ * equation, s_i D_i with D_i = R_i - h_i P_i - e_i G, R_i = from_compressed(sig_i.x) INCLUDING the flag byte and no
+ * subgroup check on P_i (src/batch.rs:102-106), is not the identity -- e.g. a signature whose y-sign flag is flipped fails
+ * the batch although Signature::verify (x-only, src/signature.rs:186,200) accepts it, while an item with s_i = 0, or with
+ * a D_i of small order that its randomiser kills, cannot fail the batch and is not flagged, whichever items surround it.
+ * Bisection over partial MSMs (a range whose own random linear combination holds is clean), exact per-item check on the
+ * failing slices: only items inside a failing slice can be flagged, so items whose non-identity terms cancel within a
+ * slice (two torsion-shifted R with odd randomisers: T2 + T2 = O) are not.  flags[i] = 0 clean, 2 bad, 3 malformed (the reference panics on it); *n_bad (optional) = number of
+ * non-zero flags.  rand32 as in verify_batch. */
 int schnorr_b200_locate_invalid(schnorr_b200_ctx *ctx, size_t n, const uint8_t *sigs81, const uint8_t *pk96,
                                 const uint8_t *pk_inf, const uint8_t *msgs, const uint64_t *msg_off,
                                 const uint8_t *rand32, uint8_t *flags, uint64_t *n_bad);

@@ -748,13 +748,31 @@ __global__ void __launch_bounds__(32) k_batch_finish(size_t np, const uint64_t* 
 // ---- f3: failed-batch localisation --------------------------------------------------------------
 // The reference returns ONE Err for the whole batch (src/batch.rs:125-129).  What the batch equation sums per item is
 //     D_i = R_i - h_i P_i - e_i G          with R_i = from_compressed(sig_i.x) INCLUDING its flag byte (src/batch.rs:104)
-// and no subgroup check on P_i (src/batch.rs:102-106) -- so "item i is what makes the batch fail" means D_i != O, which is
-// NOT the verdict of Signature::verify (x-only comparison, flag byte ignored, subgroup check first).  k_batch_item_check
-// evaluates exactly that for the items of a work list (exact Jacobian arithmetic: adversarial inputs welcome):
-//     out[i] = 0  D_i == O      2  D_i != O      3  malformed (the reference panics: src/batch.rs:67,104)
+// and no subgroup check on P_i (src/batch.rs:102-106).  The batch sums s_i D_i (the scalars reduced mod q), so "item i is
+// what makes the batch fail" means its own term s_i D_i != O: a property of the item and its randomiser alone, whatever
+// slice the bisection puts it in.  That is NOT the verdict of Signature::verify (x-only comparison, flag byte ignored,
+// subgroup check first).  k_batch_item_check evaluates exactly that for the items of a work list (exact Jacobian
+// arithmetic: adversarial inputs welcome).  Only items inside failing slices reach it: a slice whose non-O terms sum to
+// O (two torsion-shifted items T2 + T2, say) passes the bisection and its items stay unflagged.
+//     out[i] = 0  s_i D_i == O      2  s_i D_i != O      3  malformed (the reference panics: src/batch.rs:67,104)
+// s R + (s h mod q)(-P) - (s e mod q) G == O: one item's term of the batch equation, exactly as k_batch_prepare forms
+// its scalars.  Out of line: the rare path of k_batch_item_check, kept from adding to the kernel's register pressure.
+SB_DEV_NOINLINE bool batch_term_is_identity(fp6 rx, fp6 ry, bool r_inf, fp6 px, fp6 py, bool pk_inf, scalar s, scalar h,
+                                            scalar e, const uint64_t* __restrict__ gtab) {
+    scalar t = pk_inf ? sc_zero() : sc_mul(h, s);
+    jac_pt pr = jac_from_affine(rx, ry, r_inf), pp = jac_from_affine(px, fp6_neg(py), pk_inf), term = jac_identity();
+#pragma unroll 1
+    for (int b = 255; b >= 0; b--) {
+        jac_dbl_mem(&term);
+        if (sc_bits(s, b, 1)) jac_add_mem(&term, &pr, false);
+        if (sc_bits(t, b, 1)) jac_add_mem(&term, &pp, false);
+    }
+    fixed_base_accumulate(&term, sc_neg(sc_mul(s, e)), gtab);
+    return jac_is_identity(term);
+}
 __global__ void __launch_bounds__(VERIFY_THREADS, VERIFY_MIN_BLOCKS) k_batch_item_check(
-    soa_batch in, const uint8_t* __restrict__ msgs, const uint64_t* __restrict__ msg_off, const uint64_t* __restrict__ gtab,
-    uint8_t* __restrict__ out) {
+    soa_batch in, const uint8_t* __restrict__ msgs, const uint64_t* __restrict__ msg_off, const uint8_t* __restrict__ rand32,
+    const uint64_t* __restrict__ gtab, uint8_t* __restrict__ out) {
     struct d_slot {
         jac_pt p;
         uint64_t pad;
@@ -778,8 +796,8 @@ __global__ void __launch_bounds__(VERIFY_THREADS, VERIFY_MIN_BLOCKS) k_batch_ite
     uint64_t off = msg_off[i];
     scalar h = challenge_scalar(sx, px, py, pk_inf, msgs + off, msg_off[i + 1] - off);
     jac_pt r;
-    (void)torsion_check_and_mul(jac_from_affine(px, py, pk_inf), h, &r, &s_d[threadIdx.x].p);   // h P (subgroup verdict unused)
-    fixed_base_accumulate(&r, e, gtab);                                                          // + e G
+    bool torsion_free = torsion_check_and_mul(jac_from_affine(px, py, pk_inf), h, &r, &s_d[threadIdx.x].p);   // h P
+    fixed_base_accumulate(&r, e, gtab);                                                                       // + e G
     bool same;
     if (jac_is_identity(r)) {
         same = r_inf;
@@ -789,6 +807,12 @@ __global__ void __launch_bounds__(VERIFY_THREADS, VERIFY_MIN_BLOCKS) k_batch_ite
         fp6 zz = fp6_sqr(r.Z);
         same = fp6_eq(r.X, fp6_mul(rx, zz)) && fp6_eq(r.Y, fp6_mul(ry, fp6_mul(zz, r.Z)));
     }
+    // D_i == O and [q]P_i == O: the item's term s_i D_i is O.  Otherwise (rare) evaluate the term exactly as the batch
+    // sums it, s R_i + (s h mod q)(-P_i) - (s e mod q) G: an item with s_i D_i == O (s_i = 0, or D_i of small order
+    // and a randomiser that kills it) cannot make the batch fail, and flagging it would make its flag depend on whether
+    // its neighbours put it into a failing slice
+    if (!same || !torsion_free)
+        same = batch_term_is_identity(rx, ry, r_inf, px, py, pk_inf, sc_from_u256(sc_load_le(rand32 + 32 * i)), h, e, gtab);
     out[i] = same ? VERDICT_OK : VERDICT_INVALID_SIGNATURE;
 }
 
@@ -1405,7 +1429,7 @@ struct locate_range {
 };
 static int locate_items(schnorr_b200_ctx* ctx, const std::vector<locate_range>& ranges, const uint8_t* sigs81,
                         const uint8_t* pk96, const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off,
-                        uint8_t* flags) {
+                        const uint8_t* rand32, uint8_t* flags) {
     for (const locate_range& r : ranges) {
         size_t cn = r.hi - r.lo;
         if (cn == 0) continue;
@@ -1413,7 +1437,8 @@ static int locate_items(schnorr_b200_ctx* ctx, const std::vector<locate_range>& 
         if (int rc = alloc_soa(ctx, cn, &soa)) return rc;
         k_ingest<<<grid_for(cn, INGEST_THREADS), INGEST_THREADS, 0, ctx->stream>>>(cn, sigs81 + 81 * r.lo, pk96 + 96 * r.lo,
                                                                                    pk_inf ? pk_inf + r.lo : nullptr, soa);
-        k_batch_item_check<<<grid_for(cn, VERIFY_THREADS), VERIFY_THREADS, 0, ctx->stream>>>(soa, msgs, msg_off + r.lo, ctx->gtab,
+        k_batch_item_check<<<grid_for(cn, VERIFY_THREADS), VERIFY_THREADS, 0, ctx->stream>>>(soa, msgs, msg_off + r.lo,
+                                                                                           rand32 + 32 * r.lo, ctx->gtab,
                                                                                            flags + r.lo);
         ctx->launches += 2;
         CUDA_TRY(ctx, cudaGetLastError());
@@ -1472,7 +1497,7 @@ int schnorr_b200_locate_invalid_dev(schnorr_b200_ctx* ctx, size_t n, const uint8
         for (size_t k = 0; k < parts.size(); k++)
             if (host[k * slot] != VERDICT_OK) suspects.push_back(parts[k]);   // Err or malformed: look inside
     }
-    return locate_items(ctx, leaves, sigs81, pk96, pk_inf, msgs, msg_off, flags);
+    return locate_items(ctx, leaves, sigs81, pk96, pk_inf, msgs, msg_off, rand32, flags);
 }
 
 // the host forms of localisation, on inputs staged on the first device of ctx: the flags into d_flags, copied back to
