@@ -302,8 +302,45 @@ int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx *ctx, const schnorr_
                                            const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
                                            const uint64_t *msg_off, const uint8_t *rand32, uint8_t *flags,
                                            uint64_t *n_bad);
+/* verify_batch (src/batch.rs:31-130) over n 130-byte KeyedSignature wire records (49-byte compressed public key ||
+ * 81-byte signature, src/signature.rs:237-271), message i and randomiser i.  *verdict, lhs97 and rhs97 are, byte for
+ * byte, those of verify_batch on the FRONT-END records: for a record whose key decodes, its signature bytes and the
+ * decoded key; for a record whose key does not decode, the record of an index outside a set (96 bytes of 0xFF,
+ * identity flag 0), so the batch is malformed (verdict 3), as unwrapping KeyedSignature::from_bytes panics.  A scalar
+ * e >= q is malformed as in verify_batch.  The host form shards a multi-device context in contiguous slices (one
+ * partial per shard, finished on the first device); the _dev form (device buffers, no synchronisation, result216 as in
+ * verify_batch_dev) needs a single-device context and a non-NULL msgs. */
+int schnorr_b200_verify_batch_keyed(schnorr_b200_ctx *ctx, size_t n, const uint8_t *keyed130, const uint8_t *msgs,
+                                    const uint64_t *msg_off, const uint8_t *rand32, int *verdict, uint8_t *lhs97,
+                                    uint8_t *rhs97);
+int schnorr_b200_verify_batch_keyed_dev(schnorr_b200_ctx *ctx, size_t n, const uint8_t *keyed130, const uint8_t *msgs,
+                                        const uint64_t *msg_off, const uint8_t *rand32, uint8_t *result216);
+/* verify_batch_keyed against a registered key set: the same bytes as verify_batch_keyed on the same records, whatever
+ * the set holds (src/signature.rs:237-271, src/batch.rs:31-130).  A record whose key bytes are the encoding of a
+ * findable key k (keyset_lookup) takes key k's registered record; every other record (a miss) is decoded as in
+ * verify_batch_keyed.  When the rules of verify_batch_registered select the key side summed per key (more than
+ * batch_small_max records, no key of status 1 in the set, at least set_registered_batch_threshold records per key),
+ * the hits' terms are summed per key and the MSM runs over the n points R_i and the m misses' keys: one path for any
+ * mix of hits and misses, since a miss costs one MSM point.  The host form reads m (one synchronisation) and plans the
+ * MSM for n + m points; the _dev form does not synchronise and plans for 2n.  Sharding and the _dev form's
+ * requirements as in verify_batch_keyed. */
+int schnorr_b200_verify_batch_keyed_registered(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                               const uint8_t *keyed130, const uint8_t *msgs, const uint64_t *msg_off,
+                                               const uint8_t *rand32, int *verdict, uint8_t *lhs97, uint8_t *rhs97);
+int schnorr_b200_verify_batch_keyed_registered_dev(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                                   const uint8_t *keyed130, const uint8_t *msgs, const uint64_t *msg_off,
+                                                   const uint8_t *rand32, uint8_t *result216);
+/* locate_invalid (above) over keyed records, without and with a registered key set: the flags and *n_bad of
+ * locate_invalid on the front-end records of verify_batch_keyed; a record whose key does not decode gets flag 3.  Run on
+ * the first device.                                  src/signature.rs:237-271, src/batch.rs:31-130 */
+int schnorr_b200_locate_invalid_keyed(schnorr_b200_ctx *ctx, size_t n, const uint8_t *keyed130, const uint8_t *msgs,
+                                      const uint64_t *msg_off, const uint8_t *rand32, uint8_t *flags, uint64_t *n_bad);
+int schnorr_b200_locate_invalid_keyed_registered(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                                 const uint8_t *keyed130, const uint8_t *msgs, const uint64_t *msg_off,
+                                                 const uint8_t *rand32, uint8_t *flags, uint64_t *n_bad);
 /* MSM points of the last batch verification on this context (all devices of a multi-device context): 2n for
- * verify_batch, n for a registered batch summed per key, 0 for the block-per-signature form of small batches. */
+ * verify_batch, n for a registered batch summed per key, 0 for the block-per-signature form of small batches; for
+ * keyed records summed per key, n + m (host forms, m misses) or 2n (the _dev form). */
 int schnorr_b200_last_batch_points(const schnorr_b200_ctx *ctx, uint64_t *points);
 /* Registered batches sum the key side per key when they hold at least `min_signatures_per_key` signatures per key of
  * the set (0: whenever the other rules allow it).  Default 64 (measured crossover, profiles/r4_registered_batch.md). */

@@ -218,6 +218,14 @@ public:
     std::vector<size_t> locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                                        const std::vector<std::vector<uint8_t>>& messages,
                                        const std::function<void(uint8_t*, size_t)>& rng) const;
+    // verify_batch_keyed (below) with the records whose key is in the set taking its registered record and the key side
+    // summed per key (schnorr_b200_verify_batch_keyed_registered): the same result
+    Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const std::vector<std::vector<uint8_t>>& messages,
+                              const std::function<void(uint8_t*, size_t)>& rng) const;
+    // locate_invalid_keyed (below) against the set (schnorr_b200_locate_invalid_keyed_registered)
+    std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
+                                             const std::vector<std::vector<uint8_t>>& messages,
+                                             const std::function<void(uint8_t*, size_t)>& rng) const;
 
 private:
     static void pack_keys(const std::vector<PublicKey>& keys, std::vector<uint8_t>& pks, std::vector<uint8_t>& inf) {
@@ -348,6 +356,85 @@ inline std::vector<size_t> KeySet::locate_invalid(const std::vector<size_t>& ind
         if (flags[i]) bad.push_back(i);
     }
     return bad;
+}
+
+// the 130-byte records, messages and randomisers of a batch over keyed signatures
+struct KeyedBatchInputs {
+    std::vector<uint8_t> recs, rand, blob;
+    std::vector<uint64_t> off;
+    size_t n() const { return off.size() - 1; }
+};
+inline KeyedBatchInputs keyed_batch_inputs(const std::vector<KeyedSignature>& keyed,
+                                           const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
+    if (messages.size() != keyed.size()) throw std::logic_error("We should have the same number of messages than signatures");
+    size_t n = keyed.size();
+    KeyedBatchInputs in;
+    in.recs.resize(n * KEYED_SIGNATURE_LENGTH);
+    in.rand.resize(n * 32);
+    in.off.assign(n + 1, 0);
+    for (size_t i = 0; i < n; i++) {
+        auto b = keyed[i].to_bytes();
+        std::memcpy(&in.recs[i * KEYED_SIGNATURE_LENGTH], b.data(), KEYED_SIGNATURE_LENGTH);
+        in.blob.insert(in.blob.end(), messages[i].begin(), messages[i].end());
+        in.off[i + 1] = in.blob.size();
+    }
+    rng(in.rand.data(), in.rand.size());
+    for (size_t i = 0; i < n; i++) in.rand[i * 32 + 31] &= 0x3f;
+    return in;
+}
+inline std::vector<size_t> located(const std::vector<uint8_t>& flags) {
+    std::vector<size_t> bad;
+    for (size_t i = 0; i < flags.size(); i++) {
+        if (flags[i] == 3) throw std::logic_error("called `Option::unwrap()` on a `None` value (non-canonical encoding)");
+        if (flags[i]) bad.push_back(i);
+    }
+    return bad;
+}
+
+// verify_batch([k.signature ...], [k.public_key ...], messages, rng) over KeyedSignature wire records, the keys decoded on
+// the device (schnorr_b200_verify_batch_keyed); a key that does not decode makes the batch malformed, which throws
+inline Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const std::vector<std::vector<uint8_t>>& messages,
+                                 const Rng& rng) {
+    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
+    int verdict = -1;
+    Engine& eng = Engine::instance();
+    eng.check(schnorr_b200_verify_batch_keyed(eng.get(), in.n(), in.recs.data(), in.blob.empty() ? nullptr : in.blob.data(),
+                                              in.off.data(), in.rand.data(), &verdict, nullptr, nullptr),
+              "verify_batch_keyed");
+    return result_from_verdict(verdict);
+}
+// indices of the records whose own term of the batch equation fails (schnorr_b200_locate_invalid_keyed); a record whose
+// key or signature does not decode throws
+inline std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
+                                                const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
+    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
+    std::vector<uint8_t> flags(in.n(), 0);
+    Engine& eng = Engine::instance();
+    eng.check(schnorr_b200_locate_invalid_keyed(eng.get(), in.n(), in.recs.data(), in.blob.empty() ? nullptr : in.blob.data(),
+                                                in.off.data(), in.rand.data(), flags.data(), nullptr),
+              "locate_invalid_keyed");
+    return located(flags);
+}
+inline Result KeySet::verify_batch_keyed(const std::vector<KeyedSignature>& keyed,
+                                         const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
+    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
+    int verdict = -1;
+    eng_.check(schnorr_b200_verify_batch_keyed_registered(eng_.get(), ks_, in.n(), in.recs.data(),
+                                                          in.blob.empty() ? nullptr : in.blob.data(), in.off.data(),
+                                                          in.rand.data(), &verdict, nullptr, nullptr),
+               "verify_batch_keyed_registered");
+    return result_from_verdict(verdict);
+}
+inline std::vector<size_t> KeySet::locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
+                                                        const std::vector<std::vector<uint8_t>>& messages,
+                                                        const Rng& rng) const {
+    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
+    std::vector<uint8_t> flags(in.n(), 0);
+    eng_.check(schnorr_b200_locate_invalid_keyed_registered(eng_.get(), ks_, in.n(), in.recs.data(),
+                                                            in.blob.empty() ? nullptr : in.blob.data(), in.off.data(),
+                                                            in.rand.data(), flags.data(), nullptr),
+               "locate_invalid_keyed_registered");
+    return located(flags);
 }
 
 }  // namespace schnorr_sig

@@ -7,11 +7,13 @@ there is no CPU fallback.
 """
 from .api import (KEYED_SIGNATURE_LENGTH, PUBLIC_KEY_LENGTH, SCALAR_LENGTH, SIGNATURE_LENGTH, KeyedSignature,
                   KeyPair, KeySet, OsRng, PanicError, PrivateKey, PublicKey, Result, Signature, SignatureError,
-                  verify_batch, verify_prepared_batch, locate_invalid, ChainCode, ExtendedPrivateKey, ExtendedPublicKey)
+                  verify_batch, verify_prepared_batch, locate_invalid, verify_batch_keyed, locate_invalid_keyed,
+                  ChainCode, ExtendedPrivateKey, ExtendedPublicKey)
 from .engine import Engine, EngineError, default_engine, OK, INVALID_PUBLIC_KEY, INVALID_SIGNATURE, MALFORMED
 from . import synth, distributed  # noqa: F401
 from .distributed import ShardedVerifier, shard_bounds
 
 __all__ = ["Engine", "EngineError", "default_engine", "KeyPair", "KeySet", "PrivateKey", "PublicKey", "Signature",
            "KeyedSignature", "SignatureError", "PanicError", "Result", "OsRng", "verify_batch",
-           "verify_prepared_batch", "locate_invalid", "ChainCode", "ExtendedPrivateKey", "ExtendedPublicKey", "synth", "distributed", "ShardedVerifier", "shard_bounds"]
+           "verify_prepared_batch", "locate_invalid", "verify_batch_keyed", "locate_invalid_keyed",
+           "ChainCode", "ExtendedPrivateKey", "ExtendedPublicKey", "synth", "distributed", "ShardedVerifier", "shard_bounds"]

@@ -9,6 +9,7 @@ field or curve elements.
   PrivateKey::new / sign / to_bytes / from_bytes       src/private.rs:49-82, src/signature.rs:65-80
   KeyPair::new / sign / verify_signature               src/keypair.rs:57-65, src/signature.rs:114-165
   verify_batch                                         src/batch.rs:31-50
+  verify_batch_keyed / locate_invalid_keyed            src/signature.rs:237-271, src/batch.rs:31-130
   SignatureError                                       src/error.rs:13-31
 """
 import os
@@ -299,6 +300,21 @@ class KeySet:
             out.append((int(i), SignatureError(SignatureError.InvalidSignature)))
         return out
 
+    def verify_batch_keyed(self, keyed_signatures, messages, rng=None) -> Result:
+        """verify_batch_keyed (below) with the records whose key is in the set taking its registered record and the
+        key side summed per key: the same result."""
+        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
+        v, _lhs, _rhs = default_engine().verify_batch_keyed_registered(self._handle, recs, blob, off, rand)
+        return _result_from_verdict(v)
+
+    def locate_invalid_keyed(self, keyed_signatures, messages, rng=None):
+        """locate_invalid_keyed (below) with the records whose key is in the set taking its registered record."""
+        if len(keyed_signatures) == 0:
+            assert len(messages) == 0
+            return []
+        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
+        return _keyed_located(default_engine().locate_invalid_keyed_registered(self._handle, recs, blob, off, rand))
+
 
 class KeyedSignature:
     def __init__(self, public_key: PublicKey, signature: Signature):
@@ -535,6 +551,48 @@ def locate_invalid(signatures, public_keys, messages, rng=None):
             raise PanicError("signature %d has a non-canonical or undecodable encoding" % i)
         out.append((int(i), SignatureError(SignatureError.InvalidSignature)))
     return out
+
+
+def _keyed_batch_inputs(keyed_signatures, messages, rng):
+    n = len(keyed_signatures)
+    assert len(messages) == n, "We should have the same number of messages than signatures"
+    recs = [k.to_bytes() if isinstance(k, KeyedSignature) else bytes(k) for k in keyed_signatures]
+    assert all(len(b) == KEYED_SIGNATURE_LENGTH for b in recs)
+    recs = np.frombuffer(b"".join(recs), dtype=np.uint8).reshape(n, KEYED_SIGNATURE_LENGTH)
+    blob, off = _pack(messages)
+    rng = rng or OsRng()
+    rand = np.zeros((n, 32), dtype=np.uint8)
+    for i in range(n):
+        rand[i] = np.frombuffer(_random_scalar(rng).to_bytes(32, "little"), dtype=np.uint8)
+    return recs, blob, off, rand
+
+
+def _keyed_located(flags):
+    out = []
+    for i in np.nonzero(flags)[0]:
+        if flags[i] == MALFORMED:
+            raise PanicError("record %d has an undecodable key or a non-canonical or undecodable signature" % i)
+        out.append((int(i), SignatureError(SignatureError.InvalidSignature)))
+    return out
+
+
+def verify_batch_keyed(keyed_signatures, messages, rng=None) -> Result:
+    """verify_batch over KeyedSignature objects or their 130-byte records (src/signature.rs:237-271,
+    src/batch.rs:31-130): verify_batch([k.signature ...], [k.public_key ...], messages, rng) with the keys decoded on
+    the device.  A record whose key does not decode panics, as unwrapping KeyedSignature::from_bytes does."""
+    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
+    v, _lhs, _rhs = default_engine().verify_batch_keyed(recs, blob, off, rand)
+    return _result_from_verdict(v)
+
+
+def locate_invalid_keyed(keyed_signatures, messages, rng=None):
+    """locate_invalid over KeyedSignature objects or their 130-byte records: [(index, SignatureError), ...] in batch
+    semantics; a record whose key or signature does not decode panics."""
+    if len(keyed_signatures) == 0:
+        assert len(messages) == 0
+        return []
+    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
+    return _keyed_located(default_engine().locate_invalid_keyed(recs, blob, off, rand))
 
 
 def verify_prepared_batch(randomizers32, signatures, public_keys, messages) -> Result:

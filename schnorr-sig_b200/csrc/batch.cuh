@@ -1072,7 +1072,10 @@ __global__ void __launch_bounds__(SMALL_REDUCE_THREADS) k_batch_small_reduce(siz
 // of a warp with the same key add their limbs first (16-bit halves: 32 of them fit a 32-bit reduction), then one atomic
 // per group and limb.  Integer addition commutes: the sums do not depend on the order of the atomics.  A malformed item
 // (an index outside the set among them) never addresses the accumulator; its t_i is zero anyway.
+// LOOKUP: the items of keyed records (k_keyed_split_lookup), after k_keyed_route: key_idx[i] == KEYSET_MISS marks a miss,
+// whose t_i stays in the MSM and is skipped here, and `scalars` is the key-side copy, t_i at [i] instead of [n + i].
 static constexpr int KEYSUM_THREADS = 256;
+template <bool LOOKUP>
 __global__ void __launch_bounds__(KEYSUM_THREADS) k_keyset_scalar_sum(soa_batch in, const uint32_t* __restrict__ key_idx,
                                                                       const uint32_t* __restrict__ scalars,
                                                                       unsigned long long* __restrict__ cols) {
@@ -1081,9 +1084,10 @@ __global__ void __launch_bounds__(KEYSUM_THREADS) k_keyset_scalar_sum(soa_batch 
     int lane = threadIdx.x & 31;
     bool live = i < n && !(in.flags[i] & FL_MALFORMED);   // every lane stays for the warp-wide match below
     uint32_t k = live ? key_idx[i] : 0xffffffffu;           // a live index is inside the set (k_keyset_gather)
+    if (LOOKUP && k == KEYSET_MISS) live = false;          // a miss groups with the dead lanes (the same k)
     uint4 a = make_uint4(0, 0, 0, 0), b = a;
     if (live) {
-        const uint4* t = reinterpret_cast<const uint4*>(scalars + (n + i) * 8);
+        const uint4* t = reinterpret_cast<const uint4*>(scalars + (LOOKUP ? i : n + i) * 8);
         a = t[0];
         b = t[1];
     }
@@ -1169,6 +1173,58 @@ __global__ void __launch_bounds__(32) k_partial_add(const uint64_t* __restrict__
     out[23] = 0;
 }
 
+// Keyed records against a registered set (k_keyed_split_lookup, reg_batch::miss_count): every item's key-side term goes
+// to exactly one side.  k_batch_prepare has written (-P_i, t_i) into points and scalars [n, 2n).  A hit
+// (key_idx[i] != KEYSET_MISS) is summed with its key: k_keyset_scalar_sum<true> reads t_i from the copy tk[i].  A miss
+// stays in the MSM, compacted into [n, n + m) in record order (the exclusive scan of the miss flags, k_scan_local /
+// k_scan_offsets); scalars [n + m, 2n) become zero, which gives no bucket entry (msm_digit 0).  A malformed item's t_i
+// is zero: it adds nothing on either side.
+// Two hazards are ruled out by construction:
+//   - the key side never reads [n, 2n) while it is rewritten: it reads tk, and these kernels run on the main stream
+//     ahead of the fork to the second stream;
+//   - the compaction never overwrites a slot it has not read yet: k_keyed_route copies the misses out to mpts / msc,
+//     and k_keyed_compact, a later launch, copies them back into [n, n + m).
+__global__ void __launch_bounds__(256) k_keyed_miss_flags(size_t n, const uint32_t* __restrict__ key_idx,
+                                                          uint32_t* __restrict__ miss) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) miss[i] = key_idx[i] == KEYSET_MISS;
+}
+__global__ void __launch_bounds__(256) k_keyed_route(size_t n, const uint32_t* __restrict__ key_idx,
+                                                     const uint32_t* __restrict__ pos, const uint64_t* __restrict__ pts,
+                                                     const uint32_t* __restrict__ scalars, uint32_t* __restrict__ tk,
+                                                     uint64_t* __restrict__ mpts, uint32_t* __restrict__ msc) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint4* t = reinterpret_cast<const uint4*>(scalars + (n + i) * 8);
+    uint4 a = t[0], b = t[1];
+    uint4* o = reinterpret_cast<uint4*>(tk + i * 8);
+    o[0] = a;
+    o[1] = b;
+    if (key_idx[i] != KEYSET_MISS) return;
+    size_t p = pos[i];
+    o = reinterpret_cast<uint4*>(msc + p * 8);
+    o[0] = a;
+    o[1] = b;
+#pragma unroll
+    for (int c = 0; c < 12; c++) mpts[p * 12 + c] = pts[(n + i) * 12 + c];
+}
+__global__ void __launch_bounds__(256) k_keyed_compact(size_t n, const uint32_t* __restrict__ miss_count,
+                                                       const uint64_t* __restrict__ mpts, const uint32_t* __restrict__ msc,
+                                                       uint64_t* __restrict__ pts, uint32_t* __restrict__ scalars) {
+    size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    uint4* o = reinterpret_cast<uint4*>(scalars + (n + j) * 8);
+    if (j >= *miss_count) {
+        o[0] = o[1] = make_uint4(0, 0, 0, 0);
+        return;
+    }
+    const uint4* t = reinterpret_cast<const uint4*>(msc + j * 8);
+    o[0] = t[0];
+    o[1] = t[1];
+#pragma unroll
+    for (int c = 0; c < 12; c++) pts[(n + j) * 12 + c] = mpts[j * 12 + c];
+}
+
 // key side of a registered batch (batch_partial_impl): the device buffers and the geometry of its launches
 struct reg_batch {
     const uint32_t* key_idx;   // [n] device
@@ -1180,13 +1236,20 @@ struct reg_batch {
     uint64_t* key_partial;     // 192 B
     uint64_t* msm_partial;     // 192 B
     const uint32_t* zero;      // 64 zero bytes: the key partial's scalar sum and bad flag
+    size_t msm_points;         // n; keyed records: n + m (m read on the host) or 2n (m not known when planning)
+    // keyed records only (null otherwise): key_idx holds KEYSET_MISS for the m misses, *miss_count = m (device); the
+    // route buffers of k_keyed_route: miss flags and their scan [n], scan tile totals, tk [n][8], mpts [n][12], msc [n][8]
+    const uint32_t* miss_count;
+    uint32_t *miss, *pos, *tile_total, *tk, *msc;
+    uint64_t* mpts;
 };
 
 // ---- host orchestration ----------------------------------------------------------------------
 // rhs_pre (optional, device, 13 x u64): single-device batches get (sum s_i e_i) G computed on the second stream beside the
 // MSM; the caller's finish kernel must wait on ctx->ev_aux
 // reg (optional): a batch against a registered key set (pk96 = the gathered records of its items): the MSM runs over the
-// n points R_i, the key terms c_k (-P_k) are computed on the second stream beside it and added to the MSM's partial
+// n points R_i, the key terms c_k (-P_k) are computed on the second stream beside it and added to the MSM's partial;
+// with reg->miss_count (keyed records) the MSM also keeps the misses' -P_i (k_keyed_route)
 static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
                               const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off,
                               const uint8_t* rand32, uint8_t* partial192, uint64_t* rhs_pre = nullptr,
@@ -1227,7 +1290,7 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
         CUDA_TRY(ctx, cudaGetLastError());
         return SCHNORR_B200_OK;
     }
-    size_t npts = reg ? n : 2 * n;   // k_batch_prepare writes 2n points and scalars either way
+    size_t npts = reg ? reg->msm_points : 2 * n;   // k_batch_prepare writes 2n points and scalars either way
     if (2 * n >= 0x7fffffffu) {
         ctx->err = "batch too large for 31-bit point indices";
         return SCHNORR_B200_EARG;
@@ -1297,6 +1360,17 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     if (sum_blocks > 256) sum_blocks = 256;
     k_scalar_sum<<<sum_blocks, 256, 0, st>>>(lin, n, lin_part);
     k_scalar_sum<<<1, 256, 0, st>>>(lin_part, (size_t)sum_blocks, lin_total);
+    if (reg && reg->miss_count) {   // keyed records: hits to the key side, misses compacted into [n, n + m) (k_keyed_route)
+        unsigned tiles = (unsigned)((n + SCAN_TILE - 1) / SCAN_TILE);
+        k_keyed_miss_flags<<<grid_for(n, 256), 256, 0, st>>>(n, reg->key_idx, reg->miss);
+        k_scan_local<<<tiles, SCAN_THREADS, 0, st>>>(reg->miss, n, reg->pos, reg->tile_total);
+        k_scan_offsets<<<tiles, SCAN_THREADS, 0, st>>>(n, reg->pos, reg->tile_total);
+        k_keyed_route<<<grid_for(n, 256), 256, 0, st>>>(n, reg->key_idx, reg->pos, (uint64_t*)d_pts, (uint32_t*)d_sc, reg->tk,
+                                                        reg->mpts, reg->msc);
+        k_keyed_compact<<<grid_for(n, 256), 256, 0, st>>>(n, reg->miss_count, reg->mpts, reg->msc, (uint64_t*)d_pts,
+                                                          (uint32_t*)d_sc);
+        ctx->launches += 5;
+    }
     if (rhs_pre || reg) {
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_chunk[1], st));
         CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_chunk[1], 0));
@@ -1305,8 +1379,12 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
             ctx->launches += 1;
         }
         if (reg) {   // the key side: per-key scalar sums, key terms, their sum as a partial
-            k_keyset_scalar_sum<<<grid_for(n, KEYSUM_THREADS), KEYSUM_THREADS, 0, ctx->aux_stream>>>(soa, reg->key_idx,
-                                                                                                  (uint32_t*)d_sc, reg->cols);
+            if (reg->miss_count)
+                k_keyset_scalar_sum<true><<<grid_for(n, KEYSUM_THREADS), KEYSUM_THREADS, 0, ctx->aux_stream>>>(
+                    soa, reg->key_idx, reg->tk, reg->cols);
+            else
+                k_keyset_scalar_sum<false><<<grid_for(n, KEYSUM_THREADS), KEYSUM_THREADS, 0, ctx->aux_stream>>>(
+                    soa, reg->key_idx, (uint32_t*)d_sc, reg->cols);
             k_keyset_batch_term<<<reg->term_blocks, KEYTERM_THREADS, 0, ctx->aux_stream>>>(reg->n_keys, reg->cols, reg->ktab,
                                                                                             reg->terms);
             k_batch_small_reduce<<<1, SMALL_REDUCE_THREADS, 0, ctx->aux_stream>>>(reg->term_blocks, reg->terms, reg->zero,

@@ -16,6 +16,7 @@
 //   k_keyset_lookup       compressed keys -> indices into a registered key set (binary search)
 //   k_keyed_split_lookup  KeyedSignature records against a registered key set: registered record on a hit, decompressed
 //                         key on a miss, ahead of k_ingest
+//   k_keyed_bad_records   batches over KeyedSignature records: an undecodable key -> the record of an index outside a set
 //   k_imad_peak       K6  integer-multiply roofline calibration
 //   batch kernels     K3/K4  in batch.cuh (Pippenger MSM)
 // No CPU fallback exists: every entry point needs a live CUDA context.
@@ -593,6 +594,17 @@ __global__ void __launch_bounds__(128) k_split_keyed(size_t n, const uint8_t* __
 __global__ void k_mask_verdicts(size_t n, const uint8_t* __restrict__ ok, uint8_t* __restrict__ verdicts) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n && !ok[i]) verdicts[i] = VERDICT_MALFORMED;
+}
+// Batches over keyed records: a record whose key does not decode gets the record of an index outside a set
+// (k_keyset_gather), all-ones limbs and identity flag 0, which k_ingest flags as malformed: the batch is malformed, as
+// unwrapping KeyedSignature::from_bytes on such a record panics.
+__global__ void __launch_bounds__(128) k_keyed_bad_records(size_t n, const uint8_t* __restrict__ ok, uint64_t* __restrict__ pk12,
+                                                           uint8_t* __restrict__ pk_inf) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || ok[i]) return;
+#pragma unroll
+    for (int c = 0; c < 12; c++) pk12[12 * i + c] = ~0ULL;
+    pk_inf[i] = 0;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2194,6 +2206,46 @@ static bool reg_batch_aggregates(const schnorr_b200_ctx* ctx, const schnorr_b200
     return n > ctx->batch_small_max && !ks->any_not_torsion_free && n / ks->n_keys >= ctx->reg_batch_min_per_key;
 }
 
+// The key side of an aggregated batch on device k of the set, in slot O: per-block key terms | column sums, key partial,
+// MSM partial, 64 zero bytes | for keyed records (miss_count != null) the route buffers of k_keyed_route.  The MSM is
+// planned for msm_points points.
+static int reg_batch_setup(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint32_t* key_idx,
+                           const uint32_t* miss_count, size_t msm_points, reg_batch* rb) {
+    size_t max_blocks = (size_t)2 * ctx->sm_count, want = (ks->n_keys + KEYTERM_THREADS / 32 - 1) / (KEYTERM_THREADS / 32);
+    unsigned blocks = (unsigned)(want < max_blocks ? want : max_blocks);
+    const size_t sz_cols = ks->n_keys * 8 * sizeof(unsigned long long);
+    size_t r = miss_count ? n : 0;   // route buffers
+    uint8_t *d_terms, *d_cols, *d_miss, *d_pos, *d_tiles, *d_tk, *d_mpts, *d_msc;
+    if (int rc = stage_in(ctx, SL_O, {{nullptr, (size_t)blocks * sizeof(jac_pt), &d_terms},
+                                      {nullptr, sz_cols + 192 + 192 + 64, &d_cols},
+                                      {nullptr, r * 4, &d_miss},
+                                      {nullptr, r * 4, &d_pos},
+                                      {nullptr, (r + SCAN_TILE - 1) / SCAN_TILE * 4, &d_tiles},
+                                      {nullptr, r * 32, &d_tk},
+                                      {nullptr, r * 96, &d_mpts},
+                                      {nullptr, r * 32, &d_msc}}))
+        return rc;
+    rb->key_idx = key_idx;
+    rb->n_keys = ks->n_keys;
+    rb->ktab = ks->devs[k].ktab;
+    rb->cols = (unsigned long long*)d_cols;
+    rb->terms = (uint64_t*)d_terms;
+    rb->term_blocks = blocks;
+    rb->key_partial = (uint64_t*)(d_cols + sz_cols);
+    rb->msm_partial = rb->key_partial + 24;
+    rb->zero = (const uint32_t*)(rb->msm_partial + 24);
+    rb->msm_points = msm_points;
+    rb->miss_count = miss_count;
+    rb->miss = (uint32_t*)d_miss;
+    rb->pos = (uint32_t*)d_pos;
+    rb->tile_total = (uint32_t*)d_tiles;
+    rb->tk = (uint32_t*)d_tk;
+    rb->mpts = (uint64_t*)d_mpts;
+    rb->msc = (uint32_t*)d_msc;
+    CUDA_TRY(ctx, cudaMemsetAsync((void*)rb->zero, 0, 64, ctx->stream));
+    return SCHNORR_B200_OK;
+}
+
 // one 192-byte partial of a registered batch of n > 0 signatures on device buffers of device k of the set (arguments
 // checked)
 static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* sigs81,
@@ -2207,24 +2259,8 @@ static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_ke
     ctx->launches += 1;
     if (!reg_batch_aggregates(ctx, ks, n))
         return batch_partial_impl(ctx, n, sigs81, d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre);
-    // key side: per-block key terms | column sums, key partial, MSM partial, 64 zero bytes
-    size_t max_blocks = (size_t)2 * ctx->sm_count, want = (ks->n_keys + KEYTERM_THREADS / 32 - 1) / (KEYTERM_THREADS / 32);
-    unsigned blocks = (unsigned)(want < max_blocks ? want : max_blocks);
-    const size_t sz_cols = ks->n_keys * 8 * sizeof(unsigned long long);
-    uint8_t *d_terms, *d_cols;
-    if (int rc = stage_in(ctx, SL_O, {{nullptr, (size_t)blocks * sizeof(jac_pt), &d_terms}, {nullptr, sz_cols + 192 + 192 + 64, &d_cols}}))
-        return rc;
     reg_batch rb;
-    rb.key_idx = key_idx;
-    rb.n_keys = ks->n_keys;
-    rb.ktab = kd.ktab;
-    rb.cols = (unsigned long long*)d_cols;
-    rb.terms = (uint64_t*)d_terms;
-    rb.term_blocks = blocks;
-    rb.key_partial = (uint64_t*)(d_cols + sz_cols);
-    rb.msm_partial = rb.key_partial + 24;
-    rb.zero = (const uint32_t*)(rb.msm_partial + 24);
-    CUDA_TRY(ctx, cudaMemsetAsync((void*)rb.zero, 0, 64, st));
+    if (int rc = reg_batch_setup(ctx, ks, k, n, key_idx, nullptr, n, &rb)) return rc;
     return batch_partial_impl(ctx, n, sigs81, d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre, &rb);
 }
 
@@ -2300,6 +2336,170 @@ int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx* ctx, const schnorr_
                                                             d_inf);
     c->launches += 1;
     return locate_invalid_staged(ctx, n, d_sig, d_pk, d_inf, d_m, (const uint64_t*)d_off, d_rand, d_flags, flags, n_bad);
+}
+
+}  // extern "C"
+
+// ---- batch verification over KeyedSignature records (src/signature.rs:237-271, src/batch.rs:31-130) -----------------
+// The front end writes, in slot N, the records verify_batch sees: the signature bytes and the decoded key -- key k's
+// registered record where the key bytes are the encoding of a findable key k of `ks` (the same bytes decompression
+// gives) -- or, where the key does not decode, the record of an index outside a set, which makes the batch malformed.
+// With a set, idx holds each record's key index or KEYSET_MISS, and *miss the number of misses.
+struct keyed_front {
+    uint8_t *pk, *inf, *sig, *idx, *miss;
+};
+static int keyed_front_end(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* keyed130,
+                           keyed_front* f) {
+    cudaStream_t st = ctx->stream;
+    uint8_t* ok;
+    if (int rc = stage_in(ctx, SL_N, {{nullptr, n * 96, &f->pk}, {nullptr, n, &f->inf}, {nullptr, n, &ok}, {nullptr, n * 81, &f->sig},
+                                      {nullptr, ks ? n * 4 : 0, &f->idx}, {nullptr, 4, &f->miss}}))
+        return rc;
+    if (ks) {
+        const keyset_dev& kd = ks->devs[k];
+        CUDA_TRY(ctx, cudaMemsetAsync(f->miss, 0, 4, st));
+        k_keyed_split_lookup<<<grid_for(n, 128), 128, 0, st>>>(n, keyed130, kd.lut, kd.n_lut, kd.pk12, kd.pk_inf, f->pk, f->inf,
+                                                              ok, f->sig, (uint32_t*)f->idx, (uint32_t*)f->miss);
+    } else {
+        k_split_keyed<<<grid_for(n, 128), 128, 0, st>>>(n, keyed130, f->pk, f->inf, ok, f->sig);
+    }
+    k_keyed_bad_records<<<grid_for(n, 128), 128, 0, st>>>(n, ok, (uint64_t*)f->pk, f->inf);
+    ctx->launches += 2;
+    return SCHNORR_B200_OK;
+}
+
+// One 192-byte partial of a batch over n > 0 keyed records on device buffers (arguments checked), against device k's
+// copy of `ks` when a set is given.  Under the rules of reg_batch_aggregates the hits' key side is summed per key and
+// the MSM runs over the n points R_i and the misses' -P_i (k_keyed_route); otherwise the front-end records take the
+// per-signature pipeline.  read_misses (host forms): read the miss count, which synchronises, and plan the MSM for
+// n + m points; the _dev forms plan for 2n.
+static int batch_partial_keyed(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* keyed130,
+                               const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32, uint8_t* partial192,
+                               uint64_t* rhs_pre, bool read_misses) {
+    keyed_front f;
+    if (int rc = keyed_front_end(ctx, ks, k, n, keyed130, &f)) return rc;
+    if (!ks || !reg_batch_aggregates(ctx, ks, n))
+        return batch_partial_impl(ctx, n, f.sig, f.pk, f.inf, msgs, msg_off, rand32, partial192, rhs_pre);
+    size_t points = 2 * n;
+    if (read_misses) {
+        uint32_t m = 0;
+        CUDA_TRY(ctx, cudaMemcpyAsync(&m, f.miss, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        points = n + m;
+    }
+    reg_batch rb;
+    if (int rc = reg_batch_setup(ctx, ks, k, n, (const uint32_t*)f.idx, (const uint32_t*)f.miss, points, &rb)) return rc;
+    return batch_partial_impl(ctx, n, f.sig, f.pk, f.inf, msgs, msg_off, rand32, partial192, rhs_pre, &rb);
+}
+
+// host inputs (n > 0, offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
+static int batch_partial_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
+                                    const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
+                                    uint8_t* partial, uint64_t* rhs_pre) {
+    uint8_t *d_rec, *d_m, *d_off, *d_rand;
+    if (int rc = stage_in(ctx, SL_H, {{keyed130, n * 130, &d_rec}, {msgs, msg_off[n], &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                      {rand32, n * 32, &d_rand}}))
+        return rc;
+    return batch_partial_keyed(ctx, ks, k, n, d_rec, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre, true);
+}
+
+// the host forms, with or without a set (ks checked by the caller)
+static int verify_batch_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
+                                   const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32, int* verdict,
+                                   uint8_t* lhs97, uint8_t* rhs97) {
+    if (n) {
+        CHECK_MSG_OFF(ctx, n, msg_off);
+        if (msg_off[n] && !msgs) return SCHNORR_B200_EARG;
+    }
+    if (!ctx->shards.empty())
+        return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
+            return batch_partial_keyed_host(ctx->shards[k], ks, k, s.hi - s.lo, keyed130 + 130 * s.lo,
+                                            msgs ? msgs + msg_off[s.lo] : nullptr, off, rand32 + 32 * s.lo, partial, nullptr);
+        });
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    uint8_t* res = nullptr;
+    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+            return batch_partial_keyed_host(ctx, ks, 0, n, keyed130, msgs, msg_off, rand32, partial, rhs_pre);
+        }, res))
+        return rc;
+    return read_result(ctx, res, verdict, lhs97, rhs97);
+}
+
+// localisation on the first device: the inputs staged in slot M, the front-end records in slot N, then the bisection of
+// schnorr_b200_locate_invalid_dev (which uses neither slot)
+static int locate_invalid_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
+                                     const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32, uint8_t* flags,
+                                     uint64_t* n_bad) {
+    if (n_bad) *n_bad = 0;
+    if (n == 0) return SCHNORR_B200_OK;
+    CHECK_MSG_OFF(ctx, n, msg_off);
+    size_t mb = msg_off[n];
+    if (mb && !msgs) return SCHNORR_B200_EARG;
+    schnorr_b200_ctx* c = device_ctx(ctx, 0);
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    uint8_t *d_rec, *d_m, *d_off, *d_rand, *d_flags;
+    if (int rc = stage_in(c, SL_M, {{keyed130, n * 130, &d_rec}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                    {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}}))
+        return rc;
+    keyed_front f;
+    if (int rc = keyed_front_end(c, ks, 0, n, d_rec, &f)) {
+        if (c != ctx) ctx->err = c->err;
+        return rc;
+    }
+    return locate_invalid_staged(ctx, n, f.sig, f.pk, f.inf, d_m, (const uint64_t*)d_off, d_rand, d_flags, flags, n_bad);
+}
+
+extern "C" {
+
+int schnorr_b200_verify_batch_keyed(schnorr_b200_ctx* ctx, size_t n, const uint8_t* keyed130, const uint8_t* msgs,
+                                    const uint64_t* msg_off, const uint8_t* rand32, int* verdict, uint8_t* lhs97,
+                                    uint8_t* rhs97) {
+    if (!ctx || !verdict || (n && (!keyed130 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+    return verify_batch_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand32, verdict, lhs97, rhs97);
+}
+
+int schnorr_b200_verify_batch_keyed_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_t* keyed130, const uint8_t* msgs,
+                                        const uint64_t* msg_off, const uint8_t* rand32, uint8_t* result216) {
+    if (!ctx || !result216 || (n && (!keyed130 || !msgs || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+    NOT_ON_MULTI(ctx);
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+        return batch_partial_keyed(ctx, nullptr, 0, n, keyed130, msgs, msg_off, rand32, partial, rhs_pre, false);
+    }, result216);
+}
+
+int schnorr_b200_verify_batch_keyed_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                               const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off,
+                                               const uint8_t* rand32, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    if (!ctx || !ks || !verdict || (n && (!keyed130 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    return verify_batch_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand32, verdict, lhs97, rhs97);
+}
+
+int schnorr_b200_verify_batch_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                                   const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off,
+                                                   const uint8_t* rand32, uint8_t* result216) {
+    if (!ctx || !ks || !result216 || (n && (!keyed130 || !msgs || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    NOT_ON_MULTI(ctx);
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+        return batch_partial_keyed(ctx, ks, 0, n, keyed130, msgs, msg_off, rand32, partial, rhs_pre, false);
+    }, result216);
+}
+
+int schnorr_b200_locate_invalid_keyed(schnorr_b200_ctx* ctx, size_t n, const uint8_t* keyed130, const uint8_t* msgs,
+                                      const uint64_t* msg_off, const uint8_t* rand32, uint8_t* flags, uint64_t* n_bad) {
+    if (!ctx || (n && (!keyed130 || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
+    return locate_invalid_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand32, flags, n_bad);
+}
+
+int schnorr_b200_locate_invalid_keyed_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                                 const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off,
+                                                 const uint8_t* rand32, uint8_t* flags, uint64_t* n_bad) {
+    if (!ctx || !ks || (n && (!keyed130 || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    return locate_invalid_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand32, flags, n_bad);
 }
 
 // ---- keygen / sign ---------------------------------------------------------------------------

@@ -128,7 +128,8 @@ class Engine:
 
     def last_batch_points(self) -> int:
         """MSM points of the last batch call: 2n for verify_batch, n for a registered batch summed per key, 0 for the
-        block-per-signature form of small batches."""
+        block-per-signature form of small batches; keyed records summed per key: n + m (host form, m misses) or 2n
+        (_dev form)."""
         c = C.c_uint64(0)
         self._check(self._L.schnorr_b200_last_batch_points(self._h, C.byref(c)), "last_batch_points")
         return int(c.value)
@@ -362,6 +363,61 @@ class Engine:
         assert int(nb.value) == int(np.count_nonzero(flags))
         return flags
 
+    def _keyed_batch_args(self, keyed130, msgs, off, rand32):
+        keyed130, msgs, rand32 = _u8(keyed130, 130), _u8(msgs), _u8(rand32, 32)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = keyed130.shape[0]
+        self._check_offsets(n, n, off, msgs)
+        if rand32.shape[0] != n:
+            raise AssertionError("one randomiser per signature")
+        return n, keyed130, msgs, off, rand32
+
+    def verify_batch_keyed(self, keyed130, msgs, off, rand32):
+        """verify_batch over 130-byte KeyedSignature records -> (verdict, lhs97, rhs97), those of verify_batch on the
+        decoded keys (3 when a key does not decode)."""
+        return self._batch_keyed(None, keyed130, msgs, off, rand32)
+
+    def verify_batch_keyed_registered(self, keyset, keyed130, msgs, off, rand32):
+        """verify_batch_keyed against a registered key set -> (verdict, lhs97, rhs97), those of verify_batch_keyed."""
+        return self._batch_keyed(keyset, keyed130, msgs, off, rand32)
+
+    def _batch_keyed(self, keyset, keyed130, msgs, off, rand32):
+        n, keyed130, msgs, off, rand32 = self._keyed_batch_args(keyed130, msgs, off, rand32)
+        verdict = C.c_int(-1)
+        lhs = np.zeros(97, dtype=np.uint8)
+        rhs = np.zeros(97, dtype=np.uint8)
+        if keyset is None:
+            rc = self._L.schnorr_b200_verify_batch_keyed(self._h, n, _ptr(keyed130), _ptr(msgs), _ptr(off), _ptr(rand32),
+                                                         C.byref(verdict), _ptr(lhs), _ptr(rhs))
+        else:
+            rc = self._L.schnorr_b200_verify_batch_keyed_registered(self._h, keyset.handle, n, _ptr(keyed130), _ptr(msgs),
+                                                                    _ptr(off), _ptr(rand32), C.byref(verdict), _ptr(lhs),
+                                                                    _ptr(rhs))
+        self._check(rc, "verify_batch_keyed" if keyset is None else "verify_batch_keyed_registered")
+        return verdict.value, lhs, rhs
+
+    def locate_invalid_keyed(self, keyed130, msgs, off, rand32):
+        """locate_invalid over KeyedSignature records -> uint8[n] (3 where a key does not decode)."""
+        return self._locate_keyed(None, keyed130, msgs, off, rand32)
+
+    def locate_invalid_keyed_registered(self, keyset, keyed130, msgs, off, rand32):
+        """locate_invalid_keyed against a registered key set -> the flags of locate_invalid_keyed."""
+        return self._locate_keyed(keyset, keyed130, msgs, off, rand32)
+
+    def _locate_keyed(self, keyset, keyed130, msgs, off, rand32):
+        n, keyed130, msgs, off, rand32 = self._keyed_batch_args(keyed130, msgs, off, rand32)
+        flags = np.zeros(n, dtype=np.uint8)
+        nb = C.c_uint64(0)
+        if keyset is None:
+            rc = self._L.schnorr_b200_locate_invalid_keyed(self._h, n, _ptr(keyed130), _ptr(msgs), _ptr(off), _ptr(rand32),
+                                                           _ptr(flags), C.byref(nb))
+        else:
+            rc = self._L.schnorr_b200_locate_invalid_keyed_registered(self._h, keyset.handle, n, _ptr(keyed130), _ptr(msgs),
+                                                                      _ptr(off), _ptr(rand32), _ptr(flags), C.byref(nb))
+        self._check(rc, "locate_invalid_keyed" if keyset is None else "locate_invalid_keyed_registered")
+        assert int(nb.value) == int(np.count_nonzero(flags))
+        return flags
+
     def locate_invalid(self, sigs81, pk96, pk_inf, msgs, off, rand32):
         """Failed-batch localisation in batch semantics -> uint8[n]: 0 clean, 2 bad, 3 malformed (see the header)."""
         sigs81, pk96, msgs, rand32 = _u8(sigs81, 81), _u8(pk96, 96), _u8(msgs), _u8(rand32, 32)
@@ -531,6 +587,19 @@ class Engine:
         self._check(self._L.schnorr_b200_verify_batch_registered_dev(self._h, keyset.handle, n, _ptr(sigs81), _ptr(key_idx),
                                                                      _ptr(msgs), _ptr(off), _ptr(rand32), _ptr(result216)),
                     "verify_batch_registered_dev")
+
+    def verify_batch_keyed_dev(self, n, keyed130, msgs, off, rand32, result216):
+        """Batch over KeyedSignature records on device buffers, enqueued on the engine's stream, no synchronisation;
+        result216 as in verify_batch_dev."""
+        self._check(self._L.schnorr_b200_verify_batch_keyed_dev(self._h, n, _ptr(keyed130), _ptr(msgs), _ptr(off),
+                                                                _ptr(rand32), _ptr(result216)), "verify_batch_keyed_dev")
+
+    def verify_batch_keyed_registered_dev(self, keyset, n, keyed130, msgs, off, rand32, result216):
+        """verify_batch_keyed_dev against a registered key set (MSM planned for 2n points)."""
+        self._check(self._L.schnorr_b200_verify_batch_keyed_registered_dev(self._h, keyset.handle, n, _ptr(keyed130),
+                                                                           _ptr(msgs), _ptr(off), _ptr(rand32),
+                                                                           _ptr(result216)),
+                    "verify_batch_keyed_registered_dev")
 
     def batch_partial_dev(self, n, sigs81, pk96, pk_inf, msgs, off, rand32, partial192):
         self._check(self._L.schnorr_b200_batch_partial_dev(self._h, n, _ptr(sigs81), _ptr(pk96), _ptr(pk_inf),
