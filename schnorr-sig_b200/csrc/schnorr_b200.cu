@@ -646,7 +646,6 @@ __global__ void __launch_bounds__(SIGN_THREADS) k_derive_public(size_t n, const 
     if (i >= n) return;
     uint32_t index = indices[i];
     uint8_t* o = children81 + 81 * i;
-    scalar t = derive_public_tweak(parent_xpk81, parent_xpk81 + 49, index, o + 49);
     const uint64_t* p = reinterpret_cast<const uint64_t*>(parent96);
     fp6 px, py;
 #pragma unroll
@@ -654,6 +653,13 @@ __global__ void __launch_bounds__(SIGN_THREADS) k_derive_public(size_t n, const 
         px.c[k] = p[k];
         py.c[k] = p[6 + k];
     }
+    // the tweak hashes PublicKey::to_bytes of the decoded parent (:255), not the bytes it was given: a 2-torsion parent
+    // (y = 0) decodes under either sign bit and re-encodes with the bit clear.  The x limbs of a decodable record are
+    // already its canonical encoding.
+    uint8_t pk49[49];
+    for (int k = 0; k < 48; k++) pk49[k] = parent_xpk81[k];
+    pk49[48] = compress_flags(py, parent_inf[0] != 0);
+    scalar t = derive_public_tweak(pk49, parent_xpk81 + 49, index, o + 49);
     jac_pt acc = fixed_base_mul(t, gtab);                       // I_L G   (src/derivation.rs:263)
     bool tweak_inf = jac_is_identity(acc);
     acc = jac_madd(acc, px, py, parent_inf[0] != 0);            // + parent key (:264)
