@@ -82,10 +82,10 @@ SB_DEV fp_t fp_reduce96_nc(uint32_t x0, uint32_t x1, uint32_t x2) {
         ".reg .u32 c;\n\t"
         "mad.lo.cc.u32 %0, %4, 0xffffffff, %2;\n\t"   // (x1:x0) + x2 * (2^32 - 1)
         "madc.hi.cc.u32 %1, %4, 0xffffffff, %3;\n\t"
-        "addc.u32 c, 0, 0;\n\t"                       // wrapped 2^64 == EPS
-        "sub.u32 c, 0, c;\n\t"
-        "add.cc.u32 %0, %0, c;\n\t"
-        "addc.u32 %1, %1, 0;\n\t"
+        "addc.u32 c, 0, 0;\n\t"                       // wrapped 2^64 == EPS: + c EPS = - (0 : c) + (c : 0)
+        "sub.cc.u32 %0, %0, c;\n\t"
+        "subc.u32 %1, %1, 0;\n\t"
+        "add.u32 %1, %1, c;\n\t"
         "}"
         : "=&r"(t0), "=&r"(t1)
         : "r"(x0), "r"(x1), "r"(x2));
@@ -136,23 +136,24 @@ SB_DEV fp_t fp_reduce96(uint32_t x0, uint32_t x1, uint32_t x2) { return fp_canon
 template <bool CANON>
 SB_DEV fp_t fp_reduce160_t(uint32_t x0, uint32_t x1, uint32_t x2, uint32_t x3, uint32_t x4) {
 #if defined(__CUDA_ARCH__) && SB_FOLD_WIDE
-    // V = (x1:x0) + x2 (2^32 - 1) - (x4:x3) lies in (-2^40, 2^65 - 2^33): the fold may carry (c = 1), the subtraction
-    // may borrow (m = -1); the net multiple k = c + m of 2^64 = EPS (mod p) is applied once -- (t + k EPS) cannot wrap
-    // again (k = 1: t <= 2^64 - 2^33; k = -1: t >= 2^64 - 2^40).
+    // V = (x1:x0) + x2 (2^32 - 1) - (x4:x3) lies in (-2^40, 2^65 - 2^33): the subtraction may borrow (m = -1), the fold
+    // may carry (c = 1); the net multiple k = c + m of 2^64 = EPS (mod p) is applied once -- (t + k EPS) cannot wrap
+    // again (k = 1: t <= 2^64 - 2^33; k = -1: t >= 2^64 - 2^40).  Subtracting first lets the fold's carry-out land
+    // directly in k (one addc instead of an addc, an add and a predicated copy), and k EPS = (k : 0) - (k >> 31 : k) is
+    // applied as a subtraction, which needs no negated copy of k.  t and k are those of the fold-first order.
     uint32_t t0, t1;
     asm("{\n\t"
-        ".reg .u32 c, m, k;\n\t"
-        "mad.lo.cc.u32 %0, %4, 0xffffffff, %2;\n\t"
-        "madc.hi.cc.u32 %1, %4, 0xffffffff, %3;\n\t"
-        "addc.u32 c, 0, 0;\n\t"
-        "sub.cc.u32 %0, %0, %5;\n\t"
-        "subc.cc.u32 %1, %1, %6;\n\t"
+        ".reg .u32 m, k;\n\t"
+        "sub.cc.u32 %0, %2, %5;\n\t"
+        "subc.cc.u32 %1, %3, %6;\n\t"
         "subc.u32 m, 0, 0;\n\t"
-        "add.u32 k, c, m;\n\t"
-        "sub.u32 m, 0, k;\n\t"            // k EPS = (k >> 31 : -k) in two's complement
-        "shr.s32 c, k, 31;\n\t"
-        "add.cc.u32 %0, %0, m;\n\t"
-        "addc.u32 %1, %1, c;\n\t"
+        "mad.lo.cc.u32 %0, %4, 0xffffffff, %0;\n\t"
+        "madc.hi.cc.u32 %1, %4, 0xffffffff, %1;\n\t"
+        "addc.u32 k, m, 0;\n\t"
+        "shr.s32 m, k, 31;\n\t"           // + k EPS = - (k >> 31 : k) + (k : 0)
+        "sub.cc.u32 %0, %0, k;\n\t"
+        "subc.u32 %1, %1, m;\n\t"
+        "add.u32 %1, %1, k;\n\t"
         "}"
         : "=&r"(t0), "=&r"(t1)
         : "r"(x0), "r"(x1), "r"(x2), "r"(x3), "r"(x4));
@@ -311,7 +312,7 @@ SB_DEV void wide_add64(wide_acc& w, uint64_t v) {
 
 // ---- single products -----------------------------------------------------------------------------
 // Dedicated 64x64 multiply / square for the long exponentiation chains (Rescue S-boxes, inversions,
-// square roots): 4 (3) IMAD.WIDE, two carry adds and a 13-instruction reduction.  The *_nc forms
+// square roots): 4 (3) IMAD.WIDE, two carry adds and the reduction of fp_reduce160_t.  The *_nc forms
 // accept ANY 64-bit representatives and return a value < 2^64 that may be >= p ("not canonical"):
 // chains stay in that form and canonicalise once at the end (fp_canon).
 SB_DEV fp_t fp_canon(fp_t x) { return x >= FP_P ? x - FP_P : x; }
@@ -332,17 +333,16 @@ SB_DEV fp_t fp_mul_nc(fp_t a, fp_t b) {
         "madc.hi.cc.u32 p2, %3, %4, p2;\n\t"
         "addc.u32 p3, p3, 0;\n\t"
 #if SB_FOLD_WIDE
-        "mad.lo.cc.u32 %0, p2, 0xffffffff, p0;\n\t"   // (p1:p0) + p2 * (2^32 - 1)   [2^64 == 2^32 - 1]
-        "madc.hi.cc.u32 %1, p2, 0xffffffff, p1;\n\t"
-        "addc.u32 c, 0, 0;\n\t"
-        "sub.cc.u32 %0, %0, p3;\n\t"                  // - p3                        [2^96 == -1]
-        "subc.cc.u32 %1, %1, 0;\n\t"
+        "sub.cc.u32 %0, p0, p3;\n\t"                  // (p1:p0) - p3                [2^96 == -1]
+        "subc.cc.u32 %1, p1, 0;\n\t"
         "subc.u32 m, 0, 0;\n\t"
-        "add.u32 m0, c, m;\n\t"                       // net multiple of 2^64 == EPS: -1, 0, 1 (fp_reduce160_t)
-        "sub.u32 m, 0, m0;\n\t"
+        "mad.lo.cc.u32 %0, p2, 0xffffffff, %0;\n\t"   // + p2 * (2^32 - 1)           [2^64 == 2^32 - 1]
+        "madc.hi.cc.u32 %1, p2, 0xffffffff, %1;\n\t"
+        "addc.u32 m0, m, 0;\n\t"                      // net multiple of 2^64 == EPS: -1, 0, 1 (fp_reduce160_t)
         "shr.s32 c, m0, 31;\n\t"
-        "add.cc.u32 %0, %0, m;\n\t"
-        "addc.u32 %1, %1, c;\n\t"
+        "sub.cc.u32 %0, %0, m0;\n\t"
+        "subc.u32 %1, %1, c;\n\t"
+        "add.u32 %1, %1, m0;\n\t"
 #else
         "sub.cc.u32 %0, p0, p3;\n\t"      // (p1:p0) - p3          [2^96 == -1]
         "subc.cc.u32 %1, p1, 0;\n\t"
@@ -385,17 +385,16 @@ SB_DEV fp_t fp_sqr_nc(fp_t a) {
         "addc.cc.u32 p2, p2, c1;\n\t"
         "addc.u32 p3, p3, c2;\n\t"
 #if SB_FOLD_WIDE
-        "mad.lo.cc.u32 %0, p2, 0xffffffff, p0;\n\t"
-        "madc.hi.cc.u32 %1, p2, 0xffffffff, p1;\n\t"
-        "addc.u32 c, 0, 0;\n\t"
-        "sub.cc.u32 %0, %0, p3;\n\t"
-        "subc.cc.u32 %1, %1, 0;\n\t"
+        "sub.cc.u32 %0, p0, p3;\n\t"
+        "subc.cc.u32 %1, p1, 0;\n\t"
         "subc.u32 m, 0, 0;\n\t"
-        "add.u32 m0, c, m;\n\t"
-        "sub.u32 m, 0, m0;\n\t"
+        "mad.lo.cc.u32 %0, p2, 0xffffffff, %0;\n\t"
+        "madc.hi.cc.u32 %1, p2, 0xffffffff, %1;\n\t"
+        "addc.u32 m0, m, 0;\n\t"
         "shr.s32 c, m0, 31;\n\t"
-        "add.cc.u32 %0, %0, m;\n\t"
-        "addc.u32 %1, %1, c;\n\t"
+        "sub.cc.u32 %0, %0, m0;\n\t"
+        "subc.u32 %1, %1, c;\n\t"
+        "add.u32 %1, %1, m0;\n\t"
 #else
         "sub.cc.u32 %0, p0, p3;\n\t"
         "subc.cc.u32 %1, p1, 0;\n\t"
@@ -447,9 +446,9 @@ SB_DEV fp_t fp_mul7_nc(fp_t a) {
         "mad.lo.cc.u32 %0, x2, 0xffffffff, %0;\n\t"   // + x2 * (2^32 - 1)
         "madc.hi.cc.u32 %1, x2, 0xffffffff, %1;\n\t"
         "addc.u32 c, 0, 0;\n\t"
-        "sub.u32 c, 0, c;\n\t"
-        "add.cc.u32 %0, %0, c;\n\t"
-        "addc.u32 %1, %1, 0;\n\t"
+        "sub.cc.u32 %0, %0, c;\n\t"
+        "subc.u32 %1, %1, 0;\n\t"
+        "add.u32 %1, %1, c;\n\t"
 #else
         "sub.cc.u32 m0, 0, x2;\n\t"       // + x2 * (2^32 - 1)
         "subc.u32 m1, x2, 0;\n\t"
