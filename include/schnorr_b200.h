@@ -338,6 +338,43 @@ int schnorr_b200_locate_invalid_keyed(schnorr_b200_ctx *ctx, size_t n, const uin
 int schnorr_b200_locate_invalid_keyed_registered(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
                                                  const uint8_t *keyed130, const uint8_t *msgs, const uint64_t *msg_off,
                                                  const uint8_t *rand32, uint8_t *flags, uint64_t *n_bad);
+
+/* Batch randomisers from a 32-byte seed: Scalar::random / generate_batch_coefficients (src/batch.rs:56-81, :75-78)
+ * computed on the device.  Randomiser i of a seed is
+ *     s_i = int_le(SHA-512("schnorr-sig_b200/batch-randomizer/v1" || seed32 || le64(i))) mod q
+ * (32 canonical LE bytes): one SHA-512 compression, reduced wide like Scalar::random's 64 random bytes.  The batch
+ * equation is sound only while the randomisers are unpredictable to whoever produced the signatures, so the seed must
+ * be drawn fresh from a CSPRNG for every batch and kept from the signers until the verdict: a signer who knows the seed
+ * in advance can build a batch whose invalid terms cancel.
+ *
+ * batch_randomizers writes randomisers first_index ... first_index + n - 1 to rand32 (n x 32 B).  EARG for a NULL seed
+ * and when the last index, first_index + n - 1, does not fit in a u64.  The host form's bytes do not depend on the
+ * device count of the context; the _dev form (seed32 and rand32 on the device, no synchronisation) needs a single-device
+ * context.  The randomisers of a failed seeded batch, batch_randomizers(seed32, 0, n), feed locate_invalid*. */
+int schnorr_b200_batch_randomizers(schnorr_b200_ctx *ctx, size_t n, const uint8_t *seed32, uint64_t first_index,
+                                   uint8_t *rand32);
+int schnorr_b200_batch_randomizers_dev(schnorr_b200_ctx *ctx, size_t n, const uint8_t *seed32, uint64_t first_index,
+                                       uint8_t *rand32);
+/* Seeded host forms of the four batch verifications (src/batch.rs:31-50 with generate_batch_coefficients, :56-81): the
+ * arguments of the parent entry point with a 32-byte seed in place of rand32.  *verdict, lhs97 and rhs97 are, byte for
+ * byte, the parent's given rand32 = batch_randomizers(seed32, 0, n).  The randomisers are generated on the device where
+ * the batch runs (shard k of a multi-device context generates its own slice), so a call sends 32 bytes of randomness
+ * instead of 32 per signature.  Path selection and sharding as in the parent.  EARG for a NULL seed. */
+int schnorr_b200_verify_batch_seeded(schnorr_b200_ctx *ctx, size_t n, const uint8_t *sigs81, const uint8_t *pk96,
+                                     const uint8_t *pk_inf, const uint8_t *msgs, const uint64_t *msg_off,
+                                     const uint8_t *seed32, int *verdict, uint8_t *lhs97, uint8_t *rhs97);
+int schnorr_b200_verify_batch_registered_seeded(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                                const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
+                                                const uint64_t *msg_off, const uint8_t *seed32, int *verdict,
+                                                uint8_t *lhs97, uint8_t *rhs97);
+int schnorr_b200_verify_batch_keyed_seeded(schnorr_b200_ctx *ctx, size_t n, const uint8_t *keyed130, const uint8_t *msgs,
+                                           const uint64_t *msg_off, const uint8_t *seed32, int *verdict, uint8_t *lhs97,
+                                           uint8_t *rhs97);
+int schnorr_b200_verify_batch_keyed_registered_seeded(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                                      const uint8_t *keyed130, const uint8_t *msgs,
+                                                      const uint64_t *msg_off, const uint8_t *seed32, int *verdict,
+                                                      uint8_t *lhs97, uint8_t *rhs97);
+
 /* MSM points of the last batch verification on this context (all devices of a multi-device context): 2n for
  * verify_batch, n for a registered batch summed per key, 0 for the block-per-signature form of small batches; for
  * keyed records summed per key, n + m (host forms, m misses) or 2n (the _dev form). */

@@ -226,6 +226,18 @@ public:
     std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                              const std::vector<std::vector<uint8_t>>& messages,
                                              const std::function<void(uint8_t*, size_t)>& rng) const;
+    // the same four with the randomisers generated on the device from a 32-byte seed (schnorr_b200_batch_randomizers):
+    // the seed must be fresh from a CSPRNG for every batch and unknown to the signers until the verdict
+    Result verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                        const std::vector<std::vector<uint8_t>>& messages, const std::array<uint8_t, 32>& seed) const;
+    std::vector<size_t> locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                       const std::vector<std::vector<uint8_t>>& messages,
+                                       const std::array<uint8_t, 32>& seed) const;
+    Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const std::vector<std::vector<uint8_t>>& messages,
+                              const std::array<uint8_t, 32>& seed) const;
+    std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
+                                             const std::vector<std::vector<uint8_t>>& messages,
+                                             const std::array<uint8_t, 32>& seed) const;
 
 private:
     static void pack_keys(const std::vector<PublicKey>& keys, std::vector<uint8_t>& pks, std::vector<uint8_t>& inf) {
@@ -252,6 +264,11 @@ private:
     BatchInputs batch_inputs(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                              const std::vector<std::vector<uint8_t>>& messages,
                              const std::function<void(uint8_t*, size_t)>& rng) const;
+    // batch_inputs without the randomisers
+    BatchInputs batch_records(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                              const std::vector<std::vector<uint8_t>>& messages) const;
+    Result registered_verdict(const BatchInputs& in, const uint8_t* seed) const;
+    std::vector<size_t> registered_located(const BatchInputs& in) const;
     Engine& eng_;
     schnorr_b200_keyset* ks_ = nullptr;
     std::vector<uint8_t> status_;
@@ -279,35 +296,74 @@ inline Result KeySet::verify_keyed(const KeyedSignature& keyed, const std::vecto
 // per signature (src/batch.rs:75-78); 32 bytes with the top two bits cleared are uniform below 2^254 < q.
 using Rng = std::function<void(uint8_t*, size_t)>;
 
-inline Result verify_batch(const std::vector<Signature>& signatures, const std::vector<PublicKey>& public_keys,
-                           const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
+// the signature and key records and the messages of a batch
+struct BatchArrays {
+    std::vector<uint8_t> sigs, pks, inf, blob;
+    std::vector<uint64_t> off;
+    size_t n() const { return off.size() - 1; }
+    const uint8_t* msgs() const { return blob.empty() ? nullptr : blob.data(); }
+};
+inline BatchArrays batch_arrays(const std::vector<Signature>& signatures, const std::vector<PublicKey>& public_keys,
+                                const std::vector<std::vector<uint8_t>>& messages) {
     if (signatures.size() != public_keys.size())
         throw std::logic_error("We should have the same number of signatures than public keys");
     if (messages.size() != public_keys.size())
         throw std::logic_error("We should have the same number of messages than public keys");
     size_t n = signatures.size();
-    std::vector<uint8_t> sigs(n * 81), pks(n * 96), inf(n), rand(n * 32), blob;
-    std::vector<uint64_t> off(n + 1, 0);
+    BatchArrays a;
+    a.sigs.resize(n * 81);
+    a.pks.resize(n * 96);
+    a.inf.resize(n);
+    a.off.assign(n + 1, 0);
     for (size_t i = 0; i < n; i++) {
         auto b = signatures[i].to_bytes();
-        std::memcpy(&sigs[i * 81], b.data(), 81);
-        std::memcpy(&pks[i * 96], public_keys[i].xy.data(), 96);
-        inf[i] = public_keys[i].infinity;
-        blob.insert(blob.end(), messages[i].begin(), messages[i].end());
-        off[i + 1] = blob.size();
+        std::memcpy(&a.sigs[i * 81], b.data(), 81);
+        std::memcpy(&a.pks[i * 96], public_keys[i].xy.data(), 96);
+        a.inf[i] = public_keys[i].infinity;
+        a.blob.insert(a.blob.end(), messages[i].begin(), messages[i].end());
+        a.off[i + 1] = a.blob.size();
     }
+    return a;
+}
+
+inline Result verify_batch(const std::vector<Signature>& signatures, const std::vector<PublicKey>& public_keys,
+                           const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
+    BatchArrays a = batch_arrays(signatures, public_keys, messages);
+    size_t n = a.n();
+    std::vector<uint8_t> rand(n * 32);
     rng(rand.data(), rand.size());
     for (size_t i = 0; i < n; i++) rand[i * 32 + 31] &= 0x3f;
     int verdict = -1;
     Engine& eng = Engine::instance();
-    eng.check(schnorr_b200_verify_batch(eng.get(), n, sigs.data(), pks.data(), inf.data(), blob.empty() ? nullptr : blob.data(),
-                                        off.data(), rand.data(), &verdict, nullptr, nullptr),
+    eng.check(schnorr_b200_verify_batch(eng.get(), n, a.sigs.data(), a.pks.data(), a.inf.data(), a.msgs(), a.off.data(),
+                                        rand.data(), &verdict, nullptr, nullptr),
               "verify_batch");
     return result_from_verdict(verdict);
 }
 
-inline KeySet::BatchInputs KeySet::batch_inputs(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
-                                                const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
+// verify_batch with the randomisers generated on the device from a 32-byte seed (schnorr_b200_verify_batch_seeded): the
+// seed must be fresh from a CSPRNG for every batch and unknown to the signers until the verdict
+inline Result verify_batch(const std::vector<Signature>& signatures, const std::vector<PublicKey>& public_keys,
+                           const std::vector<std::vector<uint8_t>>& messages, const std::array<uint8_t, 32>& seed) {
+    BatchArrays a = batch_arrays(signatures, public_keys, messages);
+    int verdict = -1;
+    Engine& eng = Engine::instance();
+    eng.check(schnorr_b200_verify_batch_seeded(eng.get(), a.n(), a.sigs.data(), a.pks.data(), a.inf.data(), a.msgs(),
+                                               a.off.data(), seed.data(), &verdict, nullptr, nullptr),
+              "verify_batch_seeded");
+    return result_from_verdict(verdict);
+}
+
+// the randomisers 0 ... n - 1 of a seed, as the seeded entry points generate them (schnorr_b200_batch_randomizers): the
+// rand32 that localises a failed seeded batch
+inline std::vector<uint8_t> batch_randomizers(Engine& eng, size_t n, const std::array<uint8_t, 32>& seed) {
+    std::vector<uint8_t> rand(n * 32);
+    eng.check(schnorr_b200_batch_randomizers(eng.get(), n, seed.data(), 0, rand.data()), "batch_randomizers");
+    return rand;
+}
+
+inline KeySet::BatchInputs KeySet::batch_records(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                                 const std::vector<std::vector<uint8_t>>& messages) const {
     if (signatures.size() != indices.size())
         throw std::logic_error("We should have the same number of signatures than public keys");
     if (messages.size() != indices.size())
@@ -315,7 +371,6 @@ inline KeySet::BatchInputs KeySet::batch_inputs(const std::vector<size_t>& indic
     size_t n = signatures.size();
     BatchInputs in;
     in.sigs.resize(n * 81);
-    in.rand.resize(n * 32);
     in.idx.resize(n);
     in.off.assign(n + 1, 0);
     for (size_t i = 0; i < n; i++) {
@@ -325,25 +380,58 @@ inline KeySet::BatchInputs KeySet::batch_inputs(const std::vector<size_t>& indic
         in.blob.insert(in.blob.end(), messages[i].begin(), messages[i].end());
         in.off[i + 1] = in.blob.size();
     }
+    return in;
+}
+
+inline KeySet::BatchInputs KeySet::batch_inputs(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                                const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
+    BatchInputs in = batch_records(indices, signatures, messages);
+    size_t n = in.idx.size();
+    in.rand.resize(n * 32);
     rng(in.rand.data(), in.rand.size());
     for (size_t i = 0; i < n; i++) in.rand[i * 32 + 31] &= 0x3f;
     return in;
 }
 
+// the verdict of a registered batch: randomisers from in.rand, or generated on the device from `seed` when it is not null
+inline Result KeySet::registered_verdict(const BatchInputs& in, const uint8_t* seed) const {
+    int verdict = -1;
+    const uint8_t* msgs = in.blob.empty() ? nullptr : in.blob.data();
+    if (seed)
+        eng_.check(schnorr_b200_verify_batch_registered_seeded(eng_.get(), ks_, in.idx.size(), in.sigs.data(), in.idx.data(),
+                                                               msgs, in.off.data(), seed, &verdict, nullptr, nullptr),
+                   "verify_batch_registered_seeded");
+    else
+        eng_.check(schnorr_b200_verify_batch_registered(eng_.get(), ks_, in.idx.size(), in.sigs.data(), in.idx.data(), msgs,
+                                                        in.off.data(), in.rand.data(), &verdict, nullptr, nullptr),
+                   "verify_batch_registered");
+    return result_from_verdict(verdict);
+}
+
 inline Result KeySet::verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                                    const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
-    BatchInputs in = batch_inputs(indices, signatures, messages, rng);
-    int verdict = -1;
-    eng_.check(schnorr_b200_verify_batch_registered(eng_.get(), ks_, in.idx.size(), in.sigs.data(), in.idx.data(),
-                                                    in.blob.empty() ? nullptr : in.blob.data(), in.off.data(), in.rand.data(),
-                                                    &verdict, nullptr, nullptr),
-               "verify_batch_registered");
-    return result_from_verdict(verdict);
+    return registered_verdict(batch_inputs(indices, signatures, messages, rng), nullptr);
+}
+
+inline Result KeySet::verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                   const std::vector<std::vector<uint8_t>>& messages, const std::array<uint8_t, 32>& seed) const {
+    return registered_verdict(batch_records(indices, signatures, messages), seed.data());
 }
 
 inline std::vector<size_t> KeySet::locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                                                   const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
-    BatchInputs in = batch_inputs(indices, signatures, messages, rng);
+    return registered_located(batch_inputs(indices, signatures, messages, rng));
+}
+
+inline std::vector<size_t> KeySet::locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
+                                                  const std::vector<std::vector<uint8_t>>& messages,
+                                                  const std::array<uint8_t, 32>& seed) const {
+    BatchInputs in = batch_records(indices, signatures, messages);
+    in.rand = batch_randomizers(eng_, in.idx.size(), seed);
+    return registered_located(in);
+}
+
+inline std::vector<size_t> KeySet::registered_located(const BatchInputs& in) const {
     size_t n = in.idx.size();
     std::vector<uint8_t> flags(n, 0);
     eng_.check(schnorr_b200_locate_invalid_registered(eng_.get(), ks_, n, in.sigs.data(), in.idx.data(),
@@ -364,13 +452,13 @@ struct KeyedBatchInputs {
     std::vector<uint64_t> off;
     size_t n() const { return off.size() - 1; }
 };
-inline KeyedBatchInputs keyed_batch_inputs(const std::vector<KeyedSignature>& keyed,
-                                           const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
+// keyed_batch_inputs without the randomisers
+inline KeyedBatchInputs keyed_batch_records(const std::vector<KeyedSignature>& keyed,
+                                            const std::vector<std::vector<uint8_t>>& messages) {
     if (messages.size() != keyed.size()) throw std::logic_error("We should have the same number of messages than signatures");
     size_t n = keyed.size();
     KeyedBatchInputs in;
     in.recs.resize(n * KEYED_SIGNATURE_LENGTH);
-    in.rand.resize(n * 32);
     in.off.assign(n + 1, 0);
     for (size_t i = 0; i < n; i++) {
         auto b = keyed[i].to_bytes();
@@ -378,6 +466,13 @@ inline KeyedBatchInputs keyed_batch_inputs(const std::vector<KeyedSignature>& ke
         in.blob.insert(in.blob.end(), messages[i].begin(), messages[i].end());
         in.off[i + 1] = in.blob.size();
     }
+    return in;
+}
+inline KeyedBatchInputs keyed_batch_inputs(const std::vector<KeyedSignature>& keyed,
+                                           const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
+    KeyedBatchInputs in = keyed_batch_records(keyed, messages);
+    size_t n = in.n();
+    in.rand.resize(n * 32);
     rng(in.rand.data(), in.rand.size());
     for (size_t i = 0; i < n; i++) in.rand[i * 32 + 31] &= 0x3f;
     return in;
@@ -391,50 +486,95 @@ inline std::vector<size_t> located(const std::vector<uint8_t>& flags) {
     return bad;
 }
 
+// the verdict of verify_batch_keyed (ks null) or of verify_batch_keyed_registered on prepared records: randomisers from
+// in.rand, or generated on the device from `seed` when it is not null
+inline Result keyed_verdict(Engine& eng, const schnorr_b200_keyset* ks, const KeyedBatchInputs& in, const uint8_t* seed) {
+    int verdict = -1;
+    const uint8_t* msgs = in.blob.empty() ? nullptr : in.blob.data();
+    if (ks && seed)
+        eng.check(schnorr_b200_verify_batch_keyed_registered_seeded(eng.get(), ks, in.n(), in.recs.data(), msgs, in.off.data(),
+                                                                    seed, &verdict, nullptr, nullptr),
+                  "verify_batch_keyed_registered_seeded");
+    else if (ks)
+        eng.check(schnorr_b200_verify_batch_keyed_registered(eng.get(), ks, in.n(), in.recs.data(), msgs, in.off.data(),
+                                                             in.rand.data(), &verdict, nullptr, nullptr),
+                  "verify_batch_keyed_registered");
+    else if (seed)
+        eng.check(schnorr_b200_verify_batch_keyed_seeded(eng.get(), in.n(), in.recs.data(), msgs, in.off.data(), seed, &verdict,
+                                                         nullptr, nullptr),
+                  "verify_batch_keyed_seeded");
+    else
+        eng.check(schnorr_b200_verify_batch_keyed(eng.get(), in.n(), in.recs.data(), msgs, in.off.data(), in.rand.data(),
+                                                  &verdict, nullptr, nullptr),
+                  "verify_batch_keyed");
+    return result_from_verdict(verdict);
+}
+// the culprits of locate_invalid_keyed (ks null) or of locate_invalid_keyed_registered on prepared records
+inline std::vector<size_t> keyed_culprits(Engine& eng, const schnorr_b200_keyset* ks, const KeyedBatchInputs& in) {
+    std::vector<uint8_t> flags(in.n(), 0);
+    const uint8_t* msgs = in.blob.empty() ? nullptr : in.blob.data();
+    if (ks)
+        eng.check(schnorr_b200_locate_invalid_keyed_registered(eng.get(), ks, in.n(), in.recs.data(), msgs, in.off.data(),
+                                                               in.rand.data(), flags.data(), nullptr),
+                  "locate_invalid_keyed_registered");
+    else
+        eng.check(schnorr_b200_locate_invalid_keyed(eng.get(), in.n(), in.recs.data(), msgs, in.off.data(), in.rand.data(),
+                                                    flags.data(), nullptr),
+                  "locate_invalid_keyed");
+    return located(flags);
+}
+// keyed records with the randomisers 0 ... n - 1 of a seed: the inputs that localise a failed seeded batch
+inline KeyedBatchInputs keyed_seeded_inputs(Engine& eng, const std::vector<KeyedSignature>& keyed,
+                                            const std::vector<std::vector<uint8_t>>& messages,
+                                            const std::array<uint8_t, 32>& seed) {
+    KeyedBatchInputs in = keyed_batch_records(keyed, messages);
+    in.rand = batch_randomizers(eng, in.n(), seed);
+    return in;
+}
+
 // verify_batch([k.signature ...], [k.public_key ...], messages, rng) over KeyedSignature wire records, the keys decoded on
 // the device (schnorr_b200_verify_batch_keyed); a key that does not decode makes the batch malformed, which throws
 inline Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const std::vector<std::vector<uint8_t>>& messages,
                                  const Rng& rng) {
-    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
-    int verdict = -1;
-    Engine& eng = Engine::instance();
-    eng.check(schnorr_b200_verify_batch_keyed(eng.get(), in.n(), in.recs.data(), in.blob.empty() ? nullptr : in.blob.data(),
-                                              in.off.data(), in.rand.data(), &verdict, nullptr, nullptr),
-              "verify_batch_keyed");
-    return result_from_verdict(verdict);
+    return keyed_verdict(Engine::instance(), nullptr, keyed_batch_inputs(keyed, messages, rng), nullptr);
 }
 // indices of the records whose own term of the batch equation fails (schnorr_b200_locate_invalid_keyed); a record whose
 // key or signature does not decode throws
 inline std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                                 const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
-    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
-    std::vector<uint8_t> flags(in.n(), 0);
+    return keyed_culprits(Engine::instance(), nullptr, keyed_batch_inputs(keyed, messages, rng));
+}
+// the same two with the randomisers generated on the device from a 32-byte seed (schnorr_b200_verify_batch_keyed_seeded,
+// schnorr_b200_batch_randomizers): the seed must be fresh from a CSPRNG for every batch and unknown to the signers until
+// the verdict
+inline Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const std::vector<std::vector<uint8_t>>& messages,
+                                 const std::array<uint8_t, 32>& seed) {
+    return keyed_verdict(Engine::instance(), nullptr, keyed_batch_records(keyed, messages), seed.data());
+}
+inline std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
+                                                const std::vector<std::vector<uint8_t>>& messages,
+                                                const std::array<uint8_t, 32>& seed) {
     Engine& eng = Engine::instance();
-    eng.check(schnorr_b200_locate_invalid_keyed(eng.get(), in.n(), in.recs.data(), in.blob.empty() ? nullptr : in.blob.data(),
-                                                in.off.data(), in.rand.data(), flags.data(), nullptr),
-              "locate_invalid_keyed");
-    return located(flags);
+    return keyed_culprits(eng, nullptr, keyed_seeded_inputs(eng, keyed, messages, seed));
 }
 inline Result KeySet::verify_batch_keyed(const std::vector<KeyedSignature>& keyed,
                                          const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
-    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
-    int verdict = -1;
-    eng_.check(schnorr_b200_verify_batch_keyed_registered(eng_.get(), ks_, in.n(), in.recs.data(),
-                                                          in.blob.empty() ? nullptr : in.blob.data(), in.off.data(),
-                                                          in.rand.data(), &verdict, nullptr, nullptr),
-               "verify_batch_keyed_registered");
-    return result_from_verdict(verdict);
+    return keyed_verdict(eng_, ks_, keyed_batch_inputs(keyed, messages, rng), nullptr);
 }
 inline std::vector<size_t> KeySet::locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                                         const std::vector<std::vector<uint8_t>>& messages,
                                                         const Rng& rng) const {
-    KeyedBatchInputs in = keyed_batch_inputs(keyed, messages, rng);
-    std::vector<uint8_t> flags(in.n(), 0);
-    eng_.check(schnorr_b200_locate_invalid_keyed_registered(eng_.get(), ks_, in.n(), in.recs.data(),
-                                                            in.blob.empty() ? nullptr : in.blob.data(), in.off.data(),
-                                                            in.rand.data(), flags.data(), nullptr),
-               "locate_invalid_keyed_registered");
-    return located(flags);
+    return keyed_culprits(eng_, ks_, keyed_batch_inputs(keyed, messages, rng));
+}
+inline Result KeySet::verify_batch_keyed(const std::vector<KeyedSignature>& keyed,
+                                         const std::vector<std::vector<uint8_t>>& messages,
+                                         const std::array<uint8_t, 32>& seed) const {
+    return keyed_verdict(eng_, ks_, keyed_batch_records(keyed, messages), seed.data());
+}
+inline std::vector<size_t> KeySet::locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
+                                                        const std::vector<std::vector<uint8_t>>& messages,
+                                                        const std::array<uint8_t, 32>& seed) const {
+    return keyed_culprits(eng_, ks_, keyed_seeded_inputs(eng_, keyed, messages, seed));
 }
 
 }  // namespace schnorr_sig

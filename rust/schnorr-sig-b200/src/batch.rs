@@ -42,3 +42,31 @@ pub fn locate_invalid(signatures: &[Signature], public_keys: &[PublicKey], messa
     assert!(flags.iter().all(|&f| f != 3), "called `Option::unwrap()` on a `None` value");
     flags.iter().enumerate().filter(|(_, &f)| f != 0).map(|(i, _)| i).collect()
 }
+
+/// `verify_batch` with the randomisers generated on the device from a 32-byte seed instead of drawn from an RNG on the
+/// host (`Scalar::random` per signature, src/batch.rs:75-78): the host sends 32 bytes instead of 32 per signature.  The
+/// seed must come fresh from a CSPRNG for every batch and stay unknown to the signers until the verdict; a signer who
+/// knows it in advance can build a batch whose invalid terms cancel.
+pub fn verify_batch_seeded(signatures: &[Signature], public_keys: &[PublicKey], messages: &[&[u8]],
+                           seed: &[u8; 32]) -> Result<(), SignatureError> {
+    assert!(signatures.len() == public_keys.len(), "We should have the same number of signatures than public keys");
+    assert!(messages.len() == public_keys.len(), "We should have the same number of messages than public keys");
+    let (sigs, pks, infs) = records(signatures, public_keys);
+    match ENGINE.with(|e| e.verify_batch_seeded(&sigs, &pks, &infs, messages, seed)) {
+        0 => Ok(()),
+        2 => Err(SignatureError::InvalidSignature),
+        _ => panic!("called `Option::unwrap()` on a `None` value"),
+    }
+}
+
+/// `locate_invalid` with the randomisers of `verify_batch_seeded(.., seed)`: the culprits of that failed batch.
+pub fn locate_invalid_seeded(signatures: &[Signature], public_keys: &[PublicKey], messages: &[&[u8]],
+                             seed: &[u8; 32]) -> Vec<usize> {
+    let (sigs, pks, infs) = records(signatures, public_keys);
+    let flags = ENGINE.with(|e| {
+        let rand = e.batch_randomizers(sigs.len(), seed, 0);
+        e.locate_invalid(&sigs, &pks, &infs, messages, &rand)
+    });
+    assert!(flags.iter().all(|&f| f != 3), "called `Option::unwrap()` on a `None` value");
+    flags.iter().enumerate().filter(|(_, &f)| f != 0).map(|(i, _)| i).collect()
+}

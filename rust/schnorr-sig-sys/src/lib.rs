@@ -12,6 +12,10 @@ use core::ffi::{c_char, c_int, c_uint, c_void};
 pub struct schnorr_b200_ctx {
     _private: [u8; 0],
 }
+#[repr(C)]
+pub struct schnorr_b200_keyset {
+    _private: [u8; 0],
+}
 
 pub const SCHNORR_B200_OK: c_int = 0;
 pub const SCHNORR_B200_EARG: c_int = -1;
@@ -41,6 +45,22 @@ extern "C" {
     pub fn schnorr_b200_locate_invalid(ctx: *mut schnorr_b200_ctx, n: usize, sigs81: *const u8, pk96: *const u8,
         pk_inf: *const u8, msgs: *const u8, msg_off: *const u64, rand32: *const u8, flags: *mut u8,
         n_bad: *mut u64) -> c_int;
+    pub fn schnorr_b200_batch_randomizers(ctx: *mut schnorr_b200_ctx, n: usize, seed32: *const u8, first_index: u64,
+        rand32: *mut u8) -> c_int;
+    pub fn schnorr_b200_batch_randomizers_dev(ctx: *mut schnorr_b200_ctx, n: usize, seed32: *const u8, first_index: u64,
+        rand32: *mut u8) -> c_int;
+    pub fn schnorr_b200_verify_batch_seeded(ctx: *mut schnorr_b200_ctx, n: usize, sigs81: *const u8, pk96: *const u8,
+        pk_inf: *const u8, msgs: *const u8, msg_off: *const u64, seed32: *const u8, verdict: *mut c_int,
+        lhs97: *mut u8, rhs97: *mut u8) -> c_int;
+    pub fn schnorr_b200_verify_batch_registered_seeded(ctx: *mut schnorr_b200_ctx, ks: *const schnorr_b200_keyset,
+        n: usize, sigs81: *const u8, key_idx: *const u32, msgs: *const u8, msg_off: *const u64, seed32: *const u8,
+        verdict: *mut c_int, lhs97: *mut u8, rhs97: *mut u8) -> c_int;
+    pub fn schnorr_b200_verify_batch_keyed_seeded(ctx: *mut schnorr_b200_ctx, n: usize, keyed130: *const u8,
+        msgs: *const u8, msg_off: *const u64, seed32: *const u8, verdict: *mut c_int, lhs97: *mut u8,
+        rhs97: *mut u8) -> c_int;
+    pub fn schnorr_b200_verify_batch_keyed_registered_seeded(ctx: *mut schnorr_b200_ctx, ks: *const schnorr_b200_keyset,
+        n: usize, keyed130: *const u8, msgs: *const u8, msg_off: *const u64, seed32: *const u8, verdict: *mut c_int,
+        lhs97: *mut u8, rhs97: *mut u8) -> c_int;
     pub fn schnorr_b200_keygen(ctx: *mut schnorr_b200_ctx, n: usize, sk32: *const u8, pk96: *mut u8, pk_inf: *mut u8) -> c_int;
     pub fn schnorr_b200_sign_many(ctx: *mut schnorr_b200_ctx, n: usize, sk32: *const u8, pk96: *const u8,
         pk_inf: *const u8, msgs: *const u8, msg_off: *const u64, nonce32: *const u8, sigs81: *mut u8) -> c_int;
@@ -120,6 +140,29 @@ impl Engine {
         };
         self.check(rc, "schnorr_b200_verify_batch");
         verdict as u8
+    }
+
+    /// `verify_batch` with randomisers `0 .. n` generated on the device from a 32-byte seed; returns the verdict.
+    pub fn verify_batch_seeded(&self, sigs: &[[u8; 81]], pks: &[[u8; 96]], pk_inf: &[u8], messages: &[&[u8]],
+                               seed: &[u8; 32]) -> u8 {
+        assert!(sigs.len() == pks.len() && messages.len() == sigs.len());
+        let (blob, off) = pack_messages(messages);
+        let mut verdict: c_int = -1;
+        let rc = unsafe {
+            schnorr_b200_verify_batch_seeded(self.0, sigs.len(), sigs.as_ptr().cast(), pks.as_ptr().cast(), pk_inf.as_ptr(),
+                                             blob.as_ptr(), off.as_ptr(), seed.as_ptr(), &mut verdict,
+                                             core::ptr::null_mut(), core::ptr::null_mut())
+        };
+        self.check(rc, "schnorr_b200_verify_batch_seeded");
+        verdict as u8
+    }
+
+    /// Randomisers `first .. first + n` of a seed: the `rand` that `verify_batch_seeded` used for `first = 0`.
+    pub fn batch_randomizers(&self, n: usize, seed: &[u8; 32], first: u64) -> Vec<[u8; 32]> {
+        let mut rand = vec![[0u8; 32]; n];
+        let rc = unsafe { schnorr_b200_batch_randomizers(self.0, n, seed.as_ptr(), first, rand.as_mut_ptr().cast()) };
+        self.check(rc, "schnorr_b200_batch_randomizers");
+        rand
     }
 
     /// Per-item flags of a failed batch, batch semantics (0 clean, 2 culprit, 3 malformed).

@@ -106,6 +106,22 @@ def _random_scalar(rng) -> int:
     return int.from_bytes(rng.fill_bytes(64), "little") % _Q
 
 
+def _randomizers(n, rng, seed, materialise):
+    """The n x 32 randomiser bytes of a batch: one Scalar::random per signature from rng (OsRng by default); given a
+    32-byte seed instead, None -- the seeded entry points generate them on the device -- or, with materialise, the same
+    randomisers read back (Engine.batch_randomizers(n, seed)), which localise a failed seeded batch.  The seed must be
+    fresh from a CSPRNG for every batch and unknown to the signers until the verdict (include/schnorr_b200.h)."""
+    if seed is not None:
+        if rng is not None:
+            raise ValueError("a batch takes its randomisers from an rng or from a seed, not both")
+        return default_engine().batch_randomizers(n, seed) if materialise else None
+    rng = rng or OsRng()
+    rand = np.zeros((n, 32), dtype=np.uint8)
+    for i in range(n):
+        rand[i] = np.frombuffer(_random_scalar(rng).to_bytes(32, "little"), dtype=np.uint8)
+    return rand
+
+
 def _pack(msgs):
     off = np.zeros(len(msgs) + 1, dtype=np.uint64)
     off[1:] = np.cumsum([len(m) for m in msgs])
@@ -265,33 +281,33 @@ class KeySet:
                                                            blob, off)
         return _result_from_verdict(int(v[0]))
 
-    def _batch_inputs(self, indices, signatures, messages, rng):
+    def _batch_inputs(self, indices, signatures, messages, rng, seed=None, materialise=True):
         n = len(signatures)
         assert len(indices) == n, "We should have the same number of signatures than public keys"
         assert len(messages) == n, "We should have the same number of messages than public keys"
         idx = np.array([int(i) if 0 <= int(i) < 2**32 else 2**32 - 1 for i in indices], dtype=np.uint32)
         sigs = np.frombuffer(b"".join(s.to_bytes() for s in signatures), dtype=np.uint8).reshape(n, 81)
         blob, off = _pack(messages)
-        rng = rng or OsRng()
-        rand = np.zeros((n, 32), dtype=np.uint8)
-        for i in range(n):
-            rand[i] = np.frombuffer(_random_scalar(rng).to_bytes(32, "little"), dtype=np.uint8)
-        return sigs, idx, blob, off, rand
+        return sigs, idx, blob, off, _randomizers(n, rng, seed, materialise)
 
-    def verify_batch(self, indices, signatures, messages, rng=None) -> Result:
+    def verify_batch(self, indices, signatures, messages, rng=None, *, seed=None) -> Result:
         """verify_batch(signatures, [keys[i] for i in indices], messages, rng) (src/batch.rs:31-130) with the key side of
-        the batch equation summed per key of the set; an index outside the set gives the malformed-batch error."""
-        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng)
-        v, _lhs, _rhs = default_engine().verify_batch_registered(self._handle, sigs, idx, blob, off, rand)
+        the batch equation summed per key of the set; an index outside the set gives the malformed-batch error.  seed
+        (32 bytes, instead of rng): the randomisers are generated on the device from it."""
+        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng, seed, materialise=False)
+        if rand is None:
+            v, _lhs, _rhs = default_engine().verify_batch_registered_seeded(self._handle, sigs, idx, blob, off, seed)
+        else:
+            v, _lhs, _rhs = default_engine().verify_batch_registered(self._handle, sigs, idx, blob, off, rand)
         return _result_from_verdict(v)
 
-    def locate_invalid(self, indices, signatures, messages, rng=None):
+    def locate_invalid(self, indices, signatures, messages, rng=None, *, seed=None):
         """locate_invalid(signatures, [keys[i] for i in indices], messages, rng): [(index, SignatureError), ...] in batch
         semantics; a malformed item or an index outside the set panics."""
         if len(signatures) == 0:
             assert len(indices) == 0 and len(messages) == 0
             return []
-        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng)
+        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng, seed)
         flags = default_engine().locate_invalid_registered(self._handle, sigs, idx, blob, off, rand)
         out = []
         for i in np.nonzero(flags)[0]:
@@ -300,19 +316,22 @@ class KeySet:
             out.append((int(i), SignatureError(SignatureError.InvalidSignature)))
         return out
 
-    def verify_batch_keyed(self, keyed_signatures, messages, rng=None) -> Result:
+    def verify_batch_keyed(self, keyed_signatures, messages, rng=None, *, seed=None) -> Result:
         """verify_batch_keyed (below) with the records whose key is in the set taking its registered record and the
         key side summed per key: the same result."""
-        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
-        v, _lhs, _rhs = default_engine().verify_batch_keyed_registered(self._handle, recs, blob, off, rand)
+        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed, materialise=False)
+        if rand is None:
+            v, _lhs, _rhs = default_engine().verify_batch_keyed_registered_seeded(self._handle, recs, blob, off, seed)
+        else:
+            v, _lhs, _rhs = default_engine().verify_batch_keyed_registered(self._handle, recs, blob, off, rand)
         return _result_from_verdict(v)
 
-    def locate_invalid_keyed(self, keyed_signatures, messages, rng=None):
+    def locate_invalid_keyed(self, keyed_signatures, messages, rng=None, *, seed=None):
         """locate_invalid_keyed (below) with the records whose key is in the set taking its registered record."""
         if len(keyed_signatures) == 0:
             assert len(messages) == 0
             return []
-        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
+        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed)
         return _keyed_located(default_engine().locate_invalid_keyed_registered(self._handle, recs, blob, off, rand))
 
 
@@ -511,39 +530,37 @@ class ExtendedPublicKey:
         return isinstance(other, ExtendedPublicKey) and (self.key, self.chaincode) == (other.key, other.chaincode)
 
 
-def verify_batch(signatures, public_keys, messages, rng=None) -> Result:
+def verify_batch(signatures, public_keys, messages, rng=None, *, seed=None) -> Result:
     """src/batch.rs:31-50: asserts equal lengths, draws one full-width random scalar per signature,
-    checks  sum s_i R_i - sum s_i h_i P_i == (sum s_i e_i) G  on the GPU."""
+    checks  sum s_i R_i - sum s_i h_i P_i == (sum s_i e_i) G  on the GPU.  seed (32 bytes, instead of rng): the
+    randomisers are generated on the device from it (Engine.batch_randomizers); it must be fresh from a CSPRNG for every
+    batch and unknown to the signers until the verdict."""
     assert len(signatures) == len(public_keys), "We should have the same number of signatures than public keys"
     assert len(messages) == len(public_keys), "We should have the same number of messages than public keys"
-    rng = rng or OsRng()
-    n = len(signatures)
-    rand = np.zeros((n, 32), dtype=np.uint8)
-    for i in range(n):
-        rand[i] = np.frombuffer(_random_scalar(rng).to_bytes(32, "little"), dtype=np.uint8)
+    rand = _randomizers(len(signatures), rng, seed, materialise=False)
+    if rand is None:
+        v, _lhs, _rhs = default_engine().verify_batch_seeded(*_batch_arrays(signatures, public_keys, messages), seed)
+        return _result_from_verdict(v)
     return verify_prepared_batch(rand, signatures, public_keys, messages)
 
 
-def locate_invalid(signatures, public_keys, messages, rng=None):
+def locate_invalid(signatures, public_keys, messages, rng=None, *, seed=None):
     """Failed-batch localisation (SURVEY.md 8 f3).  The reference returns one Err for the whole batch
     (src/batch.rs:125-129); this returns [(index, SignatureError), ...] for every item whose own term of the batch
     equation fails -- BATCH semantics (src/batch.rs:102-106): the signature's point is decompressed with its flag byte,
     public keys are not subgroup-checked.  A signature with a flipped y-sign flag is therefore reported here (it makes
     verify_batch fail) although Signature::verify accepts it.  Runs on the device: bisection over partial MSMs, then an
     exact per-item check of the failing slices (schnorr_b200_locate_invalid).  Malformed encodings panic as in
-    verify_batch."""
+    verify_batch.  seed: the randomisers of verify_batch(..., seed=seed), to localise that failed batch."""
     n = len(signatures)
     assert len(public_keys) == n and len(messages) == n
     if n == 0:
         return []
-    rng = rng or OsRng()
     sigs = np.frombuffer(b"".join(s.to_bytes() for s in signatures), dtype=np.uint8).reshape(n, 81)
     pks = np.frombuffer(b"".join(k.xy for k in public_keys), dtype=np.uint8).reshape(n, 96)
     inf = np.array([k.infinity for k in public_keys], dtype=np.uint8)
     blob, off = _pack(messages)
-    rand = np.zeros((n, 32), dtype=np.uint8)
-    for i in range(n):
-        rand[i] = np.frombuffer(_random_scalar(rng).to_bytes(32, "little"), dtype=np.uint8)
+    rand = _randomizers(n, rng, seed, materialise=True)
     flags = default_engine().locate_invalid(sigs, pks, inf, blob, off, rand)
     out = []
     for i in np.nonzero(flags)[0]:
@@ -553,18 +570,14 @@ def locate_invalid(signatures, public_keys, messages, rng=None):
     return out
 
 
-def _keyed_batch_inputs(keyed_signatures, messages, rng):
+def _keyed_batch_inputs(keyed_signatures, messages, rng, seed=None, materialise=True):
     n = len(keyed_signatures)
     assert len(messages) == n, "We should have the same number of messages than signatures"
     recs = [k.to_bytes() if isinstance(k, KeyedSignature) else bytes(k) for k in keyed_signatures]
     assert all(len(b) == KEYED_SIGNATURE_LENGTH for b in recs)
     recs = np.frombuffer(b"".join(recs), dtype=np.uint8).reshape(n, KEYED_SIGNATURE_LENGTH)
     blob, off = _pack(messages)
-    rng = rng or OsRng()
-    rand = np.zeros((n, 32), dtype=np.uint8)
-    for i in range(n):
-        rand[i] = np.frombuffer(_random_scalar(rng).to_bytes(32, "little"), dtype=np.uint8)
-    return recs, blob, off, rand
+    return recs, blob, off, _randomizers(n, rng, seed, materialise)
 
 
 def _keyed_located(flags):
@@ -576,31 +589,38 @@ def _keyed_located(flags):
     return out
 
 
-def verify_batch_keyed(keyed_signatures, messages, rng=None) -> Result:
+def verify_batch_keyed(keyed_signatures, messages, rng=None, *, seed=None) -> Result:
     """verify_batch over KeyedSignature objects or their 130-byte records (src/signature.rs:237-271,
     src/batch.rs:31-130): verify_batch([k.signature ...], [k.public_key ...], messages, rng) with the keys decoded on
     the device.  A record whose key does not decode panics, as unwrapping KeyedSignature::from_bytes does."""
-    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
-    v, _lhs, _rhs = default_engine().verify_batch_keyed(recs, blob, off, rand)
+    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed, materialise=False)
+    if rand is None:
+        v, _lhs, _rhs = default_engine().verify_batch_keyed_seeded(recs, blob, off, seed)
+    else:
+        v, _lhs, _rhs = default_engine().verify_batch_keyed(recs, blob, off, rand)
     return _result_from_verdict(v)
 
 
-def locate_invalid_keyed(keyed_signatures, messages, rng=None):
+def locate_invalid_keyed(keyed_signatures, messages, rng=None, *, seed=None):
     """locate_invalid over KeyedSignature objects or their 130-byte records: [(index, SignatureError), ...] in batch
     semantics; a record whose key or signature does not decode panics."""
     if len(keyed_signatures) == 0:
         assert len(messages) == 0
         return []
-    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng)
+    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed)
     return _keyed_located(default_engine().locate_invalid_keyed(recs, blob, off, rand))
 
 
-def verify_prepared_batch(randomizers32, signatures, public_keys, messages) -> Result:
-    """The reference's seam for caller-supplied randomisers (src/batch.rs:84-130)."""
+def _batch_arrays(signatures, public_keys, messages):
     n = len(signatures)
     sigs = np.frombuffer(b"".join(s.to_bytes() for s in signatures), dtype=np.uint8).reshape(n, 81)
     pks = np.frombuffer(b"".join(k.xy for k in public_keys), dtype=np.uint8).reshape(n, 96)
     inf = np.array([k.infinity for k in public_keys], dtype=np.uint8)
     blob, off = _pack(messages)
-    v, _lhs, _rhs = default_engine().verify_batch(sigs, pks, inf, blob, off, randomizers32)
+    return sigs, pks, inf, blob, off
+
+
+def verify_prepared_batch(randomizers32, signatures, public_keys, messages) -> Result:
+    """The reference's seam for caller-supplied randomisers (src/batch.rs:84-130)."""
+    v, _lhs, _rhs = default_engine().verify_batch(*_batch_arrays(signatures, public_keys, messages), randomizers32)
     return _result_from_verdict(v)

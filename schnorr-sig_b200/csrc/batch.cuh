@@ -1225,6 +1225,20 @@ __global__ void __launch_bounds__(256) k_keyed_compact(size_t n, const uint32_t*
     for (int c = 0; c < 12; c++) pts[(n + j) * 12 + c] = mpts[j * 12 + c];
 }
 
+// the randomisers first ... first + n - 1 of a 32-byte seed (device) as n x 32 canonical LE bytes, one per thread
+// (derive.cuh batch_randomizer): they fill the buffer the batch kernels read as rand32
+__global__ void __launch_bounds__(128) k_batch_randomizers(size_t n, const uint8_t* __restrict__ seed32, uint64_t first,
+                                                           uint8_t* __restrict__ out32) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    scalar s = batch_randomizer(seed32, first + i);
+    uint8_t* o = out32 + 32 * i;
+#pragma unroll
+    for (int k = 0; k < 8; k++)
+#pragma unroll
+        for (int b = 0; b < 4; b++) o[4 * k + b] = (uint8_t)(s.l[k] >> (8 * b));
+}
+
 // key side of a registered batch (batch_partial_impl): the device buffers and the geometry of its launches
 struct reg_batch {
     const uint32_t* key_idx;   // [n] device
@@ -1638,38 +1652,77 @@ int schnorr_b200_batch_finish(schnorr_b200_ctx* ctx, size_t n_partials, const ui
     return read_result(ctx, res, verdict, lhs97, rhs97);
 }
 
+// Where the randomisers of a host-form batch come from: the caller's n x 32 bytes (`host`), or, when `host` is null, the
+// generator run on the device from the 32-byte `seed` for the indices first, first + 1, ...  Staging copies `host` into
+// the randomiser region, or copies only the seed and reserves the region for rand_generate.
+struct rand_source {
+    const uint8_t* host;
+    const uint8_t* seed;
+    uint64_t first;
+    // the source of the items from `lo` on (a shard's slice)
+    rand_source from(size_t lo) const { return host ? rand_source{host + 32 * lo, nullptr, 0} : rand_source{nullptr, seed, first + lo}; }
+    stage_region rand_region(size_t n, uint8_t** d_rand) const { return {host, n * 32, d_rand}; }
+    stage_region seed_region(uint8_t** d_seed) const { return {seed, host ? (size_t)0 : (size_t)32, d_seed}; }
+};
+static rand_source rand_from_host(const uint8_t* rand32) { return {rand32, nullptr, 0}; }
+static rand_source rand_from_seed(const uint8_t* seed32) { return {nullptr, seed32, 0}; }
+
+// n randomisers of a seeded source into d_rand (device), enqueued on the context stream; nothing for host bytes
+static int rand_generate(schnorr_b200_ctx* ctx, size_t n, const rand_source& rs, const uint8_t* d_seed, uint8_t* d_rand) {
+    if (rs.host || n == 0) return SCHNORR_B200_OK;
+    k_batch_randomizers<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, d_seed, rs.first, d_rand);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    return SCHNORR_B200_OK;
+}
+
 // host inputs (n > 0) -> staged on the device -> one 192-byte partial at `partial` (device memory of this context)
 static int batch_partial_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
-                              const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
+                              const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const rand_source& rs,
                               uint8_t* partial, uint64_t* rhs_pre = nullptr) {
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
     // staging slots distinct from those batch_partial_impl uses (A-G, J-L): one blob in slot H
-    uint8_t *d_sig, *d_pk, *d_m, *d_off, *d_rand, *d_inf;
+    uint8_t *d_sig, *d_pk, *d_m, *d_off, *d_rand, *d_inf, *d_seed;
     if (int rc = stage_in(ctx, SL_H, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                                      {rand32, n * 32, &d_rand}, {pk_inf, n, &d_inf}}))
+                                      rs.rand_region(n, &d_rand), {pk_inf, n, &d_inf}, rs.seed_region(&d_seed)}))
         return rc;
+    if (int rc = rand_generate(ctx, n, rs, d_seed, d_rand)) return rc;
     return batch_partial_impl(ctx, n, d_sig, d_pk, pk_inf ? d_inf : nullptr, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
+}
+
+// the host forms of verify_batch (arguments checked)
+static int verify_batch_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
+                             const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const rand_source& rs,
+                             int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    if (!ctx->shards.empty())
+        return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
+            return batch_partial_host(ctx->shards[k], s.hi - s.lo, sigs81 + 81 * s.lo, pk96 + 96 * s.lo,
+                                      pk_inf ? pk_inf + s.lo : nullptr, msgs ? msgs + msg_off[s.lo] : nullptr, off,
+                                      rs.from(s.lo), partial);
+        });
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    uint8_t* res = nullptr;
+    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+            return batch_partial_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rs, partial, rhs_pre);
+        }, res))
+        return rc;
+    return read_result(ctx, res, verdict, lhs97, rhs97);
 }
 
 int schnorr_b200_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
                               const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
                               int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
     if (!ctx || !verdict || (n && (!sigs81 || !pk96 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
-    if (!ctx->shards.empty())
-        return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
-            return batch_partial_host(ctx->shards[k], s.hi - s.lo, sigs81 + 81 * s.lo, pk96 + 96 * s.lo,
-                                      pk_inf ? pk_inf + s.lo : nullptr, msgs ? msgs + msg_off[s.lo] : nullptr, off,
-                                      rand32 + 32 * s.lo, partial);
-        });
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    uint8_t* res = nullptr;
-    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
-            return batch_partial_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, partial, rhs_pre);
-        }, res))
-        return rc;
-    return read_result(ctx, res, verdict, lhs97, rhs97);
+    return verify_batch_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand_from_host(rand32), verdict, lhs97, rhs97);
+}
+
+int schnorr_b200_verify_batch_seeded(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
+                                     const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* seed32,
+                                     int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    if (!ctx || !verdict || !seed32 || (n && (!sigs81 || !pk96 || !msg_off))) return SCHNORR_B200_EARG;
+    return verify_batch_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rand_from_seed(seed32), verdict, lhs97, rhs97);
 }
 
 }  // extern "C"

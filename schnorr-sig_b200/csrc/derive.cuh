@@ -107,6 +107,21 @@ SB_DEV void hmac_sha512_short(const uint8_t* key, int key_len, const uint8_t* da
     sha512_finish_short(outer, 1, digest, 64, out64);
 }
 
+// ---- batch randomisers (include/schnorr_b200.h, schnorr_b200_batch_randomizers) -------------------------------------
+// s_i = int_le(SHA-512(TAG || seed || le64(i))) mod q: one compression of 76 bytes per signature index, reduced wide as
+// Scalar::random reduces 64 random bytes
+SB_DEV scalar batch_randomizer(const uint8_t* seed32, uint64_t index) {
+    const char tag[] = "schnorr-sig_b200/batch-randomizer/v1";
+    uint8_t msg[76], d[64];
+    for (int i = 0; i < 36; i++) msg[i] = (uint8_t)tag[i];
+    for (int i = 0; i < 32; i++) msg[36 + i] = seed32[i];
+    for (int b = 0; b < 8; b++) msg[68 + b] = (uint8_t)(index >> (8 * b));
+    sha512_state s;
+    sha512_init(s);
+    sha512_finish_short(s, 0, msg, 76, d);
+    return sc_from_u512(sc_load_le(d), sc_load_le(d + 32));
+}
+
 // ---- derivation steps (byte layouts: include/schnorr_b200.h) ---------------------------------------------------------
 // master: seed32 -> (sk32 || chain32); returns false for a zero key
 SB_DEV bool derive_master(const uint8_t* seed32, uint8_t* xsk64) {

@@ -131,6 +131,15 @@ SB_DEV scalar sc_mul(const scalar& a, const scalar& b) {
     for (int i = 0; i < 8; i++) r2.l[i] = SB_CONST_R2(i);
     return sc_montmul(sc_montmul(a, b), r2);
 }
+// lo + hi 2^256 mod q for a 512-bit little-endian integer given as its two 256-bit halves (the wide reduction of
+// Scalar::random): both halves are reduced first, because sc_montmul needs operands below q, and
+// montmul(hi, 2^512 mod q) = hi 2^256 mod q
+SB_DEV scalar sc_from_u512(const scalar& lo, const scalar& hi) {
+    scalar r2;
+#pragma unroll
+    for (int i = 0; i < 8; i++) r2.l[i] = SB_CONST_R2(i);
+    return sc_add(sc_from_u256(lo), sc_montmul(sc_from_u256(hi), r2));
+}
 
 SB_DEV scalar sc_load_le(const uint8_t* p) {
     scalar r;

@@ -2252,6 +2252,41 @@ static int reg_batch_setup(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks,
     return SCHNORR_B200_OK;
 }
 
+// ---- batch randomisers from a seed (rand_source, k_batch_randomizers) -------------------------------------------
+// the randomisers first_index ... first_index + n - 1 of a seed: EARG when the last index does not fit in a u64
+static bool rand_args_ok(const schnorr_b200_ctx* ctx, size_t n, const uint8_t* seed32, uint64_t first_index, const uint8_t* rand32) {
+    return ctx && seed32 && (n == 0 || (rand32 && first_index <= UINT64_MAX - ((uint64_t)n - 1)));
+}
+
+extern "C" {
+
+int schnorr_b200_batch_randomizers_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_t* seed32, uint64_t first_index,
+                                       uint8_t* rand32) {
+    if (!rand_args_ok(ctx, n, seed32, first_index, rand32)) return SCHNORR_B200_EARG;
+    NOT_ON_MULTI(ctx);
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    return rand_generate(ctx, n, rand_source{nullptr, seed32, first_index}, seed32, rand32);
+}
+
+int schnorr_b200_batch_randomizers(schnorr_b200_ctx* ctx, size_t n, const uint8_t* seed32, uint64_t first_index,
+                                   uint8_t* rand32) {
+    if (!rand_args_ok(ctx, n, seed32, first_index, rand32)) return SCHNORR_B200_EARG;
+    if (!ctx->shards.empty())
+        return multi_run(ctx, multi_slices(ctx, n), [&](int k, shard_slice s) {
+            return schnorr_b200_batch_randomizers(ctx->shards[k], s.hi - s.lo, seed32, first_index + s.lo, rand32 + 32 * s.lo);
+        });
+    if (n == 0) return SCHNORR_B200_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    uint8_t *d_seed, *d_rand;
+    if (int rc = stage_in(ctx, SL_H, {{seed32, 32, &d_seed}, {nullptr, n * 32, &d_rand}})) return rc;
+    if (int rc = rand_generate(ctx, n, rand_source{nullptr, seed32, first_index}, d_seed, d_rand)) return rc;
+    CUDA_TRY(ctx, cudaMemcpyAsync(rand32, d_rand, n * 32, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return SCHNORR_B200_OK;
+}
+
+}  // extern "C"
+
 // one 192-byte partial of a registered batch of n > 0 signatures on device buffers of device k of the set (arguments
 // checked)
 static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* sigs81,
@@ -2273,20 +2308,19 @@ static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_ke
 // host inputs (n > 0, offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
 static int batch_partial_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
                                          const uint8_t* sigs81, const uint32_t* key_idx, const uint8_t* msgs,
-                                         const uint64_t* msg_off, const uint8_t* rand32, uint8_t* partial, uint64_t* rhs_pre) {
-    uint8_t *d_sig, *d_idx, *d_m, *d_off, *d_rand;
+                                         const uint64_t* msg_off, const rand_source& rs, uint8_t* partial, uint64_t* rhs_pre) {
+    uint8_t *d_sig, *d_idx, *d_m, *d_off, *d_rand, *d_seed;
     if (int rc = stage_in(ctx, SL_H, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, msg_off[n], &d_m},
-                                      {msg_off, (n + 1) * 8, &d_off}, {rand32, n * 32, &d_rand}}))
+                                      {msg_off, (n + 1) * 8, &d_off}, rs.rand_region(n, &d_rand), rs.seed_region(&d_seed)}))
         return rc;
+    if (int rc = rand_generate(ctx, n, rs, d_seed, d_rand)) return rc;
     return batch_partial_registered(ctx, ks, k, n, d_sig, (uint32_t*)d_idx, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
 }
 
-extern "C" {
-
-int schnorr_b200_verify_batch_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
-                                         const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
-                                         const uint8_t* rand32, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
-    if (!ctx || !ks || !verdict || (n && (!sigs81 || !key_idx || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+// the host forms of verify_batch_registered (pointer arguments checked)
+static int verify_batch_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                        const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
+                                        const rand_source& rs, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
     CHECK_KEYSET(ctx, ks);
     if (n) {
         CHECK_MSG_OFF(ctx, n, msg_off);
@@ -2295,15 +2329,34 @@ int schnorr_b200_verify_batch_registered(schnorr_b200_ctx* ctx, const schnorr_b2
     if (!ctx->shards.empty())
         return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
             return batch_partial_registered_host(ctx->shards[k], ks, k, s.hi - s.lo, sigs81 + 81 * s.lo, key_idx + s.lo,
-                                                 msgs ? msgs + msg_off[s.lo] : nullptr, off, rand32 + 32 * s.lo, partial, nullptr);
+                                                 msgs ? msgs + msg_off[s.lo] : nullptr, off, rs.from(s.lo), partial, nullptr);
         });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     uint8_t* res = nullptr;
     if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
-            return batch_partial_registered_host(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, rand32, partial, rhs_pre);
+            return batch_partial_registered_host(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, rs, partial, rhs_pre);
         }, res))
         return rc;
     return read_result(ctx, res, verdict, lhs97, rhs97);
+}
+
+extern "C" {
+
+int schnorr_b200_verify_batch_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                         const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
+                                         const uint8_t* rand32, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    if (!ctx || !ks || !verdict || (n && (!sigs81 || !key_idx || !msg_off || !rand32))) return SCHNORR_B200_EARG;
+    return verify_batch_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand_from_host(rand32), verdict, lhs97,
+                                        rhs97);
+}
+
+int schnorr_b200_verify_batch_registered_seeded(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                                const uint8_t* sigs81, const uint32_t* key_idx, const uint8_t* msgs,
+                                                const uint64_t* msg_off, const uint8_t* seed32, int* verdict, uint8_t* lhs97,
+                                                uint8_t* rhs97) {
+    if (!ctx || !ks || !verdict || !seed32 || (n && (!sigs81 || !key_idx || !msg_off))) return SCHNORR_B200_EARG;
+    return verify_batch_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand_from_seed(seed32), verdict, lhs97,
+                                        rhs97);
 }
 
 int schnorr_b200_verify_batch_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
@@ -2400,18 +2453,19 @@ static int batch_partial_keyed(schnorr_b200_ctx* ctx, const schnorr_b200_keyset*
 
 // host inputs (n > 0, offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
 static int batch_partial_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
-                                    const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
+                                    const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, const rand_source& rs,
                                     uint8_t* partial, uint64_t* rhs_pre) {
-    uint8_t *d_rec, *d_m, *d_off, *d_rand;
+    uint8_t *d_rec, *d_m, *d_off, *d_rand, *d_seed;
     if (int rc = stage_in(ctx, SL_H, {{keyed130, n * 130, &d_rec}, {msgs, msg_off[n], &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                                      {rand32, n * 32, &d_rand}}))
+                                      rs.rand_region(n, &d_rand), rs.seed_region(&d_seed)}))
         return rc;
+    if (int rc = rand_generate(ctx, n, rs, d_seed, d_rand)) return rc;
     return batch_partial_keyed(ctx, ks, k, n, d_rec, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre, true);
 }
 
 // the host forms, with or without a set (ks checked by the caller)
 static int verify_batch_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
-                                   const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32, int* verdict,
+                                   const uint8_t* msgs, const uint64_t* msg_off, const rand_source& rs, int* verdict,
                                    uint8_t* lhs97, uint8_t* rhs97) {
     if (n) {
         CHECK_MSG_OFF(ctx, n, msg_off);
@@ -2420,12 +2474,12 @@ static int verify_batch_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_key
     if (!ctx->shards.empty())
         return multi_verify_batch(ctx, n, msg_off, verdict, lhs97, rhs97, [&](int k, auto s, const uint64_t* off, uint8_t* partial) {
             return batch_partial_keyed_host(ctx->shards[k], ks, k, s.hi - s.lo, keyed130 + 130 * s.lo,
-                                            msgs ? msgs + msg_off[s.lo] : nullptr, off, rand32 + 32 * s.lo, partial, nullptr);
+                                            msgs ? msgs + msg_off[s.lo] : nullptr, off, rs.from(s.lo), partial, nullptr);
         });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     uint8_t* res = nullptr;
     if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
-            return batch_partial_keyed_host(ctx, ks, 0, n, keyed130, msgs, msg_off, rand32, partial, rhs_pre);
+            return batch_partial_keyed_host(ctx, ks, 0, n, keyed130, msgs, msg_off, rs, partial, rhs_pre);
         }, res))
         return rc;
     return read_result(ctx, res, verdict, lhs97, rhs97);
@@ -2461,7 +2515,14 @@ int schnorr_b200_verify_batch_keyed(schnorr_b200_ctx* ctx, size_t n, const uint8
                                     const uint64_t* msg_off, const uint8_t* rand32, int* verdict, uint8_t* lhs97,
                                     uint8_t* rhs97) {
     if (!ctx || !verdict || (n && (!keyed130 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
-    return verify_batch_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand32, verdict, lhs97, rhs97);
+    return verify_batch_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand_from_host(rand32), verdict, lhs97, rhs97);
+}
+
+int schnorr_b200_verify_batch_keyed_seeded(schnorr_b200_ctx* ctx, size_t n, const uint8_t* keyed130, const uint8_t* msgs,
+                                           const uint64_t* msg_off, const uint8_t* seed32, int* verdict, uint8_t* lhs97,
+                                           uint8_t* rhs97) {
+    if (!ctx || !verdict || !seed32 || (n && (!keyed130 || !msg_off))) return SCHNORR_B200_EARG;
+    return verify_batch_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand_from_seed(seed32), verdict, lhs97, rhs97);
 }
 
 int schnorr_b200_verify_batch_keyed_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_t* keyed130, const uint8_t* msgs,
@@ -2479,7 +2540,15 @@ int schnorr_b200_verify_batch_keyed_registered(schnorr_b200_ctx* ctx, const schn
                                                const uint8_t* rand32, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
     if (!ctx || !ks || !verdict || (n && (!keyed130 || !msg_off || !rand32))) return SCHNORR_B200_EARG;
     CHECK_KEYSET(ctx, ks);
-    return verify_batch_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand32, verdict, lhs97, rhs97);
+    return verify_batch_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand_from_host(rand32), verdict, lhs97, rhs97);
+}
+
+int schnorr_b200_verify_batch_keyed_registered_seeded(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                                      const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off,
+                                                      const uint8_t* seed32, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    if (!ctx || !ks || !verdict || !seed32 || (n && (!keyed130 || !msg_off))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    return verify_batch_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand_from_seed(seed32), verdict, lhs97, rhs97);
 }
 
 int schnorr_b200_verify_batch_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,

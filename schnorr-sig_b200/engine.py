@@ -42,6 +42,13 @@ def _u8(a, cols=None):
     return a
 
 
+def _seed32(seed):
+    s = np.frombuffer(bytes(seed), dtype=np.uint8).copy() if isinstance(seed, (bytes, bytearray)) else _u8(seed).reshape(-1)
+    if s.shape != (32,):
+        raise ValueError("a batch seed is 32 bytes")
+    return s
+
+
 class Engine:
     def __init__(self, device=0):
         """device: a CUDA device index, or a list of indices for a multi-device context (a device may repeat)."""
@@ -328,17 +335,88 @@ class Engine:
                     "verify_batch")
         return verdict.value, lhs, rhs
 
+    def batch_randomizers(self, n, seed, first=0):
+        """Randomisers first ... first + n - 1 of a 32-byte seed -> uint8[n, 32] (schnorr_b200_batch_randomizers): the
+        rand32 that the seeded batch forms use for seed and first = 0."""
+        seed = _seed32(seed)
+        out = np.zeros((int(n), 32), dtype=np.uint8)
+        self._check(self._L.schnorr_b200_batch_randomizers(self._h, int(n), _ptr(seed), int(first), _ptr(out)),
+                    "batch_randomizers")
+        return out
+
+    def batch_randomizers_dev(self, n, seed32, first, rand32):
+        """Device buffers (seed32: 32 B, rand32: n x 32 B), enqueued on the engine's stream, no synchronisation."""
+        self._check(self._L.schnorr_b200_batch_randomizers_dev(self._h, int(n), _ptr(seed32), int(first), _ptr(rand32)),
+                    "batch_randomizers_dev")
+
+    def verify_batch_seeded(self, sigs81, pk96, pk_inf, msgs, off, seed):
+        """verify_batch with rand32 = batch_randomizers(n, seed), generated on the device -> (verdict, lhs97, rhs97)"""
+        sigs81, pk96, msgs, seed = _u8(sigs81, 81), _u8(pk96, 96), _u8(msgs), _seed32(seed)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = sigs81.shape[0]
+        self._check_offsets(n, pk96.shape[0], off, msgs)
+        inf = None if pk_inf is None else _u8(pk_inf)
+        verdict = C.c_int(-1)
+        lhs = np.zeros(97, dtype=np.uint8)
+        rhs = np.zeros(97, dtype=np.uint8)
+        self._check(self._L.schnorr_b200_verify_batch_seeded(self._h, n, _ptr(sigs81), _ptr(pk96), _ptr(inf), _ptr(msgs),
+                                                             _ptr(off), _ptr(seed), C.byref(verdict), _ptr(lhs), _ptr(rhs)),
+                    "verify_batch_seeded")
+        return verdict.value, lhs, rhs
+
+    def verify_batch_registered_seeded(self, keyset, sigs81, key_idx, msgs, off, seed):
+        """verify_batch_registered with rand32 = batch_randomizers(n, seed), generated on the device."""
+        n, sigs81, key_idx, msgs, off = self._registered_inputs(sigs81, key_idx, msgs, off)
+        seed = _seed32(seed)
+        verdict = C.c_int(-1)
+        lhs = np.zeros(97, dtype=np.uint8)
+        rhs = np.zeros(97, dtype=np.uint8)
+        self._check(self._L.schnorr_b200_verify_batch_registered_seeded(self._h, keyset.handle, n, _ptr(sigs81),
+                                                                        _ptr(key_idx), _ptr(msgs), _ptr(off), _ptr(seed),
+                                                                        C.byref(verdict), _ptr(lhs), _ptr(rhs)),
+                    "verify_batch_registered_seeded")
+        return verdict.value, lhs, rhs
+
+    def verify_batch_keyed_seeded(self, keyed130, msgs, off, seed):
+        """verify_batch_keyed with rand32 = batch_randomizers(n, seed), generated on the device."""
+        return self._batch_keyed_seeded(None, keyed130, msgs, off, seed)
+
+    def verify_batch_keyed_registered_seeded(self, keyset, keyed130, msgs, off, seed):
+        """verify_batch_keyed_registered with rand32 = batch_randomizers(n, seed), generated on the device."""
+        return self._batch_keyed_seeded(keyset, keyed130, msgs, off, seed)
+
+    def _batch_keyed_seeded(self, keyset, keyed130, msgs, off, seed):
+        n, keyed130, msgs, off = self._keyed_inputs(keyed130, msgs, off)
+        seed = _seed32(seed)
+        verdict = C.c_int(-1)
+        lhs = np.zeros(97, dtype=np.uint8)
+        rhs = np.zeros(97, dtype=np.uint8)
+        if keyset is None:
+            rc = self._L.schnorr_b200_verify_batch_keyed_seeded(self._h, n, _ptr(keyed130), _ptr(msgs), _ptr(off), _ptr(seed),
+                                                                C.byref(verdict), _ptr(lhs), _ptr(rhs))
+        else:
+            rc = self._L.schnorr_b200_verify_batch_keyed_registered_seeded(self._h, keyset.handle, n, _ptr(keyed130),
+                                                                           _ptr(msgs), _ptr(off), _ptr(seed),
+                                                                           C.byref(verdict), _ptr(lhs), _ptr(rhs))
+        self._check(rc, "verify_batch_keyed_seeded" if keyset is None else "verify_batch_keyed_registered_seeded")
+        return verdict.value, lhs, rhs
+
     def _registered_batch_args(self, sigs81, key_idx, msgs, off, rand32):
-        sigs81, msgs, rand32 = _u8(sigs81, 81), _u8(msgs), _u8(rand32, 32)
+        rand32 = _u8(rand32, 32)
+        n, sigs81, key_idx, msgs, off = self._registered_inputs(sigs81, key_idx, msgs, off)
+        if rand32.shape[0] != n:
+            raise AssertionError("one randomiser per signature")
+        return n, sigs81, key_idx, msgs, off, rand32
+
+    def _registered_inputs(self, sigs81, key_idx, msgs, off):
+        sigs81, msgs = _u8(sigs81, 81), _u8(msgs)
         key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32)
         off = np.ascontiguousarray(off, dtype=np.uint64)
         n = sigs81.shape[0]
         if key_idx.ndim != 1:
             raise ValueError("key_idx must be one-dimensional")
         self._check_offsets(n, key_idx.shape[0], off, msgs)
-        if rand32.shape[0] != n:
-            raise AssertionError("one randomiser per signature")
-        return n, sigs81, key_idx, msgs, off, rand32
+        return n, sigs81, key_idx, msgs, off
 
     def verify_batch_registered(self, keyset, sigs81, key_idx, msgs, off, rand32):
         """verify_batch of sigs81[i] over message i under key key_idx[i] of `keyset` -> (verdict, lhs97, rhs97), those of
@@ -364,13 +442,18 @@ class Engine:
         return flags
 
     def _keyed_batch_args(self, keyed130, msgs, off, rand32):
-        keyed130, msgs, rand32 = _u8(keyed130, 130), _u8(msgs), _u8(rand32, 32)
-        off = np.ascontiguousarray(off, dtype=np.uint64)
-        n = keyed130.shape[0]
-        self._check_offsets(n, n, off, msgs)
+        rand32 = _u8(rand32, 32)
+        n, keyed130, msgs, off = self._keyed_inputs(keyed130, msgs, off)
         if rand32.shape[0] != n:
             raise AssertionError("one randomiser per signature")
         return n, keyed130, msgs, off, rand32
+
+    def _keyed_inputs(self, keyed130, msgs, off):
+        keyed130, msgs = _u8(keyed130, 130), _u8(msgs)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = keyed130.shape[0]
+        self._check_offsets(n, n, off, msgs)
+        return n, keyed130, msgs, off
 
     def verify_batch_keyed(self, keyed130, msgs, off, rand32):
         """verify_batch over 130-byte KeyedSignature records -> (verdict, lhs97, rhs97), those of verify_batch on the
