@@ -431,6 +431,42 @@ int schnorr_b200_debug_field_ops(schnorr_b200_ctx *ctx, size_t n, const uint64_t
 int schnorr_b200_debug_lazy_ops(schnorr_b200_ctx *ctx, size_t n, const uint64_t *a6, const uint64_t *b6,
                                 uint64_t *out48);
 
+/* Test hook (no reference counterpart): one operation of the device field core (csrc/fp.cuh) on n items of raw
+ * 32-bit words, so that its carry and borrow paths can be driven word by word.  in16, out16: n x 16 u32 (host).
+ * Scalar ops: a = in[0:2], b = in[2:4] (little-endian words of a 64-bit value, any value, canonical or not); the
+ * reductions take x0..x4 = in[0:5]; FP_MUL_SMALL takes k and FP_SQR_N the count n from in[2]; the raw 64-bit result
+ * (not reduced further) goes to out[0:2].  Accumulator ops: the state e0..e4, o1..o3 = in[0:8], a = in[8:10],
+ * b = in[10:12], the repeat count of FP_WIDE_MAC_LOOP = in[12]; out[0:8] = the new state, out[8:10] =
+ * wide_reduce_nc, out[10:12] = wide_reduce of it.  Unused output words are 0.  A bad op returns SCHNORR_B200_EARG. */
+enum {
+    SCHNORR_B200_FP_SUB = 0,
+    SCHNORR_B200_FP_ADD,
+    SCHNORR_B200_FP_NEG,
+    SCHNORR_B200_FP_DBL,
+    SCHNORR_B200_FP_REDUCE96_NC,
+    SCHNORR_B200_FP_REDUCE96,
+    SCHNORR_B200_FP_REDUCE160_NC,
+    SCHNORR_B200_FP_REDUCE160,
+    SCHNORR_B200_FP_CANON_SEL,
+    SCHNORR_B200_FP_CANON,
+    SCHNORR_B200_FP_MUL_NC,
+    SCHNORR_B200_FP_SQR_NC,
+    SCHNORR_B200_FP_MUL,
+    SCHNORR_B200_FP_SQR,
+    SCHNORR_B200_FP_MUL7_NC,
+    SCHNORR_B200_FP_MUL_SMALL,
+    SCHNORR_B200_FP_SQR_N,
+    SCHNORR_B200_FP_INV,
+    SCHNORR_B200_FP_WIDE_MAC, /* first accumulator op */
+    SCHNORR_B200_FP_WIDE_MAC_SQR,
+    SCHNORR_B200_FP_WIDE_ADD64,
+    SCHNORR_B200_FP_WIDE_DOUBLE,
+    SCHNORR_B200_FP_WIDE_REDUCE,
+    SCHNORR_B200_FP_WIDE_MAC_LOOP,
+    SCHNORR_B200_FP_OP_COUNT
+};
+int schnorr_b200_debug_fp_core(schnorr_b200_ctx *ctx, int op, size_t n, const uint32_t *in16, uint32_t *out16);
+
 /* Integer-multiply roofline calibration: runs a register-resident chain of `iters` dependent-free
  * 32x32->64 multiply-adds per thread on a full grid and returns wide multiplies per second. */
 int schnorr_b200_imad_peak(schnorr_b200_ctx *ctx, int iters, double *wide_mul_per_s, double *elapsed_ms);

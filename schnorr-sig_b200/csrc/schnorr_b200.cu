@@ -926,6 +926,63 @@ __global__ void __launch_bounds__(128) k_debug_lazy(size_t n, const uint64_t* __
         for (int k = 0; k < 6; k++) out48[i * 48 + 6 * j + k] = r[j].c[k];
 }
 
+// test hook for the field core itself (fp.cuh), on raw 32-bit words: every item holds 16 input and 16 output words,
+// and one op runs for the whole launch (numbering in include/schnorr_b200.h, SCHNORR_B200_FP_*).  Scalar ops read
+// a = in[0:2], b = in[2:4] (the reductions read x0..x4 = in[0:5]; fp_mul_small and fp_sqr_n read their count from
+// in[2]) and write the result to out[0:2].  Accumulator ops read the state e0..e4, o1..o3 = in[0:8] and their operands
+// from in[8:12] (the loop count from in[12]), and write the new state to out[0:8], wide_reduce_nc to out[8:10] and
+// wide_reduce to out[10:12].
+__global__ void __launch_bounds__(128) k_debug_fp_core(int op, size_t n, const uint32_t* __restrict__ in16,
+                                                       uint32_t* __restrict__ out16) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t x[16], y[16] = {};
+    for (int k = 0; k < 16; k++) x[k] = in16[i * 16 + k];
+    fp_t a = ((uint64_t)x[1] << 32) | x[0], b = ((uint64_t)x[3] << 32) | x[2], r = 0;
+    if (op >= SCHNORR_B200_FP_WIDE_MAC) {
+        wide_acc w{x[0], x[1], x[2], x[3], x[4], x[5], x[6], x[7]};
+        fp_t u = ((uint64_t)x[9] << 32) | x[8], v = ((uint64_t)x[11] << 32) | x[10];
+        switch (op) {
+            case SCHNORR_B200_FP_WIDE_MAC: wide_mac(w, u, v); break;
+            case SCHNORR_B200_FP_WIDE_MAC_SQR: wide_mac_sqr(w, u); break;
+            case SCHNORR_B200_FP_WIDE_ADD64: wide_add64(w, u); break;
+            case SCHNORR_B200_FP_WIDE_DOUBLE: wide_double(w); break;
+            case SCHNORR_B200_FP_WIDE_MAC_LOOP:
+#pragma unroll 1
+                for (uint32_t k = 0; k < x[12]; k++) wide_mac(w, u, v);
+                break;
+            default: break;  // SCHNORR_B200_FP_WIDE_REDUCE: the state as given
+        }
+        y[0] = w.e0, y[1] = w.e1, y[2] = w.e2, y[3] = w.e3, y[4] = w.e4, y[5] = w.o1, y[6] = w.o2, y[7] = w.o3;
+        fp_t nc = wide_reduce_t<false>(w), cn = wide_reduce_t<true>(w);
+        y[8] = (uint32_t)nc, y[9] = (uint32_t)(nc >> 32), y[10] = (uint32_t)cn, y[11] = (uint32_t)(cn >> 32);
+    } else {
+        switch (op) {
+            case SCHNORR_B200_FP_SUB: r = fp_sub(a, b); break;
+            case SCHNORR_B200_FP_ADD: r = fp_add(a, b); break;
+            case SCHNORR_B200_FP_NEG: r = fp_neg(a); break;
+            case SCHNORR_B200_FP_DBL: r = fp_dbl(a); break;
+            case SCHNORR_B200_FP_REDUCE96_NC: r = fp_reduce96_nc(x[0], x[1], x[2]); break;
+            case SCHNORR_B200_FP_REDUCE96: r = fp_reduce96(x[0], x[1], x[2]); break;
+            case SCHNORR_B200_FP_REDUCE160_NC: r = fp_reduce160_t<false>(x[0], x[1], x[2], x[3], x[4]); break;
+            case SCHNORR_B200_FP_REDUCE160: r = fp_reduce160_t<true>(x[0], x[1], x[2], x[3], x[4]); break;
+            case SCHNORR_B200_FP_CANON_SEL: r = fp_canon_sel(a); break;
+            case SCHNORR_B200_FP_CANON: r = fp_canon(a); break;
+            case SCHNORR_B200_FP_MUL_NC: r = fp_mul_nc(a, b); break;
+            case SCHNORR_B200_FP_SQR_NC: r = fp_sqr_nc(a); break;
+            case SCHNORR_B200_FP_MUL: r = fp_mul(a, b); break;
+            case SCHNORR_B200_FP_SQR: r = fp_sqr(a); break;
+            case SCHNORR_B200_FP_MUL7_NC: r = fp_mul7_nc(a); break;
+            case SCHNORR_B200_FP_MUL_SMALL: r = fp_mul_small(a, x[2]); break;
+            case SCHNORR_B200_FP_SQR_N: r = fp_sqr_n(a, (int)x[2]); break;
+            case SCHNORR_B200_FP_INV: r = fp_inv(a); break;
+            default: break;
+        }
+        y[0] = (uint32_t)r, y[1] = (uint32_t)(r >> 32);
+    }
+    for (int k = 0; k < 16; k++) out16[i * 16 + k] = y[k];
+}
+
 // ------------------------------------------------------------------------------------------------
 // K6: integer-multiply roofline calibration.  8 independent accumulator chains per thread of
 // 32x32+64 -> 64 multiply-adds (IMAD.WIDE.U32), no memory traffic.
@@ -2793,6 +2850,22 @@ int schnorr_b200_debug_lazy_ops(schnorr_b200_ctx* ctx, size_t n, const uint64_t*
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaMemcpyAsync(out48, d_o, n * 48 * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return SCHNORR_B200_OK;
+}
+
+int schnorr_b200_debug_fp_core(schnorr_b200_ctx* ctx, int op, size_t n, const uint32_t* in16, uint32_t* out16) {
+    MULTI_DISPATCH(ctx, schnorr_b200_debug_fp_core(ctx->shards[0], op, n, in16, out16));
+    if (!ctx || op < 0 || op >= SCHNORR_B200_FP_OP_COUNT || (n && (!in16 || !out16))) return SCHNORR_B200_EARG;
+    if (n == 0) return SCHNORR_B200_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    void *d_in, *d_o;
+    if (int rc = stage_in(ctx, SL_D, in16, n * 64, &d_in)) return rc;
+    if (int rc = ensure_scratch(ctx, SL_H, n * 64, &d_o)) return rc;
+    k_debug_fp_core<<<grid_for(n, 128), 128, 0, ctx->stream>>>(op, n, (uint32_t*)d_in, (uint32_t*)d_o);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    CUDA_TRY(ctx, cudaMemcpyAsync(out16, d_o, n * 64, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return SCHNORR_B200_OK;
 }

@@ -628,6 +628,20 @@ class Engine:
         self._check(self._L.schnorr_b200_debug_lazy_ops(self._h, a6.shape[0], _ptr(a6), _ptr(b6), _ptr(out)), "debug_lazy_ops")
         return out
 
+    # op numbers of debug_fp_core (enum SCHNORR_B200_FP_* of include/schnorr_b200.h)
+    FP_CORE_OPS = ("sub", "add", "neg", "dbl", "reduce96_nc", "reduce96", "reduce160_nc", "reduce160", "canon_sel",
+                   "canon", "mul_nc", "sqr_nc", "mul", "sqr", "mul7_nc", "mul_small", "sqr_n", "inv",
+                   "wide_mac", "wide_mac_sqr", "wide_add64", "wide_double", "wide_reduce", "wide_mac_loop")
+
+    def debug_fp_core(self, op, in16):
+        """Test hook: one device field-core op (a name of FP_CORE_OPS or its number) on n items of 16 raw u32 words
+        -> [n, 16] uint32 (layout in include/schnorr_b200.h)."""
+        code = self.FP_CORE_OPS.index(op) if isinstance(op, str) else int(op)
+        in16 = np.ascontiguousarray(in16, dtype=np.uint32).reshape(-1, 16)
+        out = np.zeros((in16.shape[0], 16), dtype=np.uint32)
+        self._check(self._L.schnorr_b200_debug_fp_core(self._h, code, in16.shape[0], _ptr(in16), _ptr(out)), "debug_fp_core")
+        return out
+
     def imad_peak(self, iters=1 << 16):
         w = C.c_double(0)
         ms = C.c_double(0)
