@@ -1260,7 +1260,8 @@ struct reg_batch {
 
 // ---- host orchestration ----------------------------------------------------------------------
 // rhs_pre (optional, device, 13 x u64): single-device batches get (sum s_i e_i) G computed on the second stream beside the
-// MSM; the caller's finish kernel must wait on ctx->ev_aux
+// MSM.  Whatever runs on the second stream is joined into the context stream before this returns, so the regions it
+// reads may be released then.
 // reg (optional): a batch against a registered key set (pk96 = the gathered records of its items): the MSM runs over the
 // n points R_i, the key terms c_k (-P_k) are computed on the second stream beside it and added to the MSM's partial;
 // with reg->miss_count (keyed records) the MSM also keeps the misses' -P_i (k_keyed_route)
@@ -1268,13 +1269,13 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
                               const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off,
                               const uint8_t* rand32, uint8_t* partial192, uint64_t* rhs_pre = nullptr,
                               const reg_batch* reg = nullptr) {
+    scratch_scope scope(ctx->scratch, ctx->stream);
     soa_batch soa;
     if (int rc = alloc_soa(ctx, n, &soa)) return rc;
     if (n <= ctx->batch_small_max && !reg) {   // one thread block per signature (latency), see k_batch_small
         void *d_terms, *d_lin, *d_small;
-        if (int rc = ensure_scratch(ctx, SL_D, n * 18 * 8, &d_terms)) return rc;
-        if (int rc = ensure_scratch(ctx, SL_F, n * 32 + 512 * 32, &d_lin)) return rc;
-        if (int rc = ensure_scratch(ctx, SL_L, 64, &d_small)) return rc;
+        if (int rc = stage_in(ctx, {{nullptr, n * 18 * 8, &d_terms}, {nullptr, n * 32 + 512 * 32, &d_lin}, {nullptr, 64, &d_small}}))
+            return rc;
         uint32_t* lin = (uint32_t*)d_lin;
         uint32_t* lin_part = lin + n * 8;
         uint32_t* lin_total = lin_part + 256 * 8;
@@ -1296,6 +1297,7 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
             ctx->launches += 1;
         }
         k_batch_small_reduce<<<1, SMALL_REDUCE_THREADS, 0, st>>>(n, (uint64_t*)d_terms, lin_total, bad, (uint64_t*)partial192);
+        if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_aux, 0));
         ctx->last_msm_c = 4;
         ctx->last_msm_K = SMALL_WINDOWS;
         ctx->last_msm_T = 0;
@@ -1316,15 +1318,15 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     }
     size_t nslots = (size_t)pl.K * (pl.B + 1);
     void *d_pts, *d_sc, *d_lin, *d_cnt, *d_sorted, *d_buckets, *d_small;
-    if (int rc = ensure_scratch(ctx, SL_D, 2 * n * 96, &d_pts)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, 2 * n * 32, &d_sc)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_F, n * 32 + 512 * 32, &d_lin)) return rc;
     size_t scan_tiles_max = (nslots + SCAN_TILE - 1) / SCAN_TILE;
-    if (int rc = ensure_scratch(ctx, SL_G, nslots * 4 * 3 + 4 * scan_tiles_max + 64, &d_cnt)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_J, npts * pl.K * 4, &d_sorted)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_K, sizeof(jac_pt) * ((size_t)pl.K * pl.B + (size_t)pl.K * pl.chunks + pl.K), &d_buckets))
+    if (int rc = stage_in(ctx, {{nullptr, 2 * n * 96, &d_pts},
+                                {nullptr, 2 * n * 32, &d_sc},
+                                {nullptr, n * 32 + 512 * 32, &d_lin},
+                                {nullptr, nslots * 4 * 3 + 4 * scan_tiles_max + 64, &d_cnt},
+                                {nullptr, npts * pl.K * 4, &d_sorted},
+                                {nullptr, sizeof(jac_pt) * ((size_t)pl.K * pl.B + (size_t)pl.K * pl.chunks + pl.K), &d_buckets},
+                                {nullptr, 64, &d_small}}))
         return rc;
-    if (int rc = ensure_scratch(ctx, SL_L, 64, &d_small)) return rc;
     // segment length: 8..32 entries per thread, longer for very large batches (bounds the partial arrays)
     size_t max_entries = npts * (size_t)pl.K;
     // 8 (small batches: more, shorter chains -- the accumulation is latency-bound there) .. 32 entries per thread
@@ -1339,7 +1341,7 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     size_t nseg = ((max_entries + T - 1) / T + 127) / 128 * 128;
     void* d_parts;
     size_t max_long = nseg / MSM_LONG_SPAN + 1;  // buckets that can span >= MSM_LONG_SPAN segments
-    if (int rc = ensure_scratch(ctx, SL_I, nseg * 2 * sizeof(seg_partial) + 4 * max_long, &d_parts)) return rc;
+    if (int rc = stage_in(ctx, {{nullptr, nseg * 2 * sizeof(seg_partial) + 4 * max_long, &d_parts}})) return rc;
     uint32_t* long_list = (uint32_t*)((uint8_t*)d_parts + nseg * 2 * sizeof(seg_partial));
     uint32_t* long_count = (uint32_t*)d_small + 1;  // zeroed with the `bad` flag below
     uint32_t* counts = (uint32_t*)d_cnt;
@@ -1428,8 +1430,8 @@ static int batch_partial_impl(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     k_msm_window_fold<<<pl.K, FOLD_THREADS, 0, st>>>(pl, chunk_out, windows);
     k_msm_horner<<<1, 32, 0, st>>>(pl, windows, lin_total, bad, reg ? reg->msm_partial : (uint64_t*)partial192);
     ctx->launches += 14;
+    if (rhs_pre || reg) CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_aux, 0));
     if (reg) {
-        CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_aux, 0));
         k_partial_add<<<1, 32, 0, st>>>(reg->msm_partial, reg->key_partial, (uint64_t*)partial192);
         ctx->launches += 1;
     }
@@ -1448,23 +1450,40 @@ static int batch_partial_empty(schnorr_b200_ctx* ctx, uint8_t* partial192) {
     return SCHNORR_B200_OK;
 }
 
-// A whole batch on one device (its device selected): SL_L holds [64 B of batch_partial_impl | result | partial |
-// rhs_pre]; partial_fn(partial, rhs_pre) reduces the n > 0 signatures to the partial with (sum s e) G computed beside it
-// into rhs_pre (batch_partial_impl), and k_batch_finish writes the result to `result216`, or, when that is null, to the
-// result region of SL_L, which `result216` then points to (the host forms read it with read_result).
+// A whole batch on one device (its device selected): partial_fn(partial, rhs_pre) reduces the n > 0 signatures to the
+// partial with (sum s e) G computed beside it into rhs_pre (batch_partial_impl), and k_batch_finish writes the result
+// to `result216` (device).
 template <typename F>
-static int batch_whole(schnorr_b200_ctx* ctx, size_t n, F partial_fn, uint8_t*& result216) {
-    void* d_res;
-    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192 + 128, &d_res)) return rc;
-    if (!result216) result216 = (uint8_t*)d_res + 64;
-    uint8_t* partial = (uint8_t*)d_res + 64 + RESULT_BYTES;
-    uint64_t* rhs_pre = n ? (uint64_t*)(partial + 192) : nullptr;
+static int batch_whole(schnorr_b200_ctx* ctx, size_t n, F partial_fn, uint8_t* result216) {
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    uint8_t* partial;
+    uint64_t* rhs_pre;
+    if (int rc = stage_in(ctx, {{nullptr, 192, &partial}, {nullptr, 128, &rhs_pre}})) return rc;
+    if (!n) rhs_pre = nullptr;
     if (int rc = n ? partial_fn(partial, rhs_pre) : batch_partial_empty(ctx, partial)) return rc;
-    if (rhs_pre) CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_aux, 0));
     k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, result216, rhs_pre);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
     return SCHNORR_B200_OK;
+}
+
+static int read_result(schnorr_b200_ctx* ctx, const uint8_t* d_res, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    uint8_t h[RESULT_BYTES];
+    CUDA_TRY(ctx, cudaMemcpyAsync(h, d_res, RESULT_BYTES, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    *verdict = h[0];
+    if (lhs97) memcpy(lhs97, h + 8, 97);
+    if (rhs97) memcpy(rhs97, h + 112, 97);
+    return SCHNORR_B200_OK;
+}
+// batch_whole into a result region of this call, read back into the host outputs
+template <typename F>
+static int batch_whole_host(schnorr_b200_ctx* ctx, size_t n, F partial_fn, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    uint8_t* res;
+    if (int rc = stage_in(ctx, {{nullptr, RESULT_BYTES, &res}})) return rc;
+    if (int rc = batch_whole(ctx, n, partial_fn, res)) return rc;
+    return read_result(ctx, res, verdict, lhs97, rhs97);
 }
 
 // multi.cuh: a batch over every device of a multi-device context; partial(k, slice, rebased offsets, partial192) reduces
@@ -1525,6 +1544,7 @@ static int locate_items(schnorr_b200_ctx* ctx, const std::vector<locate_range>& 
     for (const locate_range& r : ranges) {
         size_t cn = r.hi - r.lo;
         if (cn == 0) continue;
+        scratch_scope scope(ctx->scratch, ctx->stream);
         soa_batch soa;
         if (int rc = alloc_soa(ctx, cn, &soa)) return rc;
         k_ingest<<<grid_for(cn, INGEST_THREADS), INGEST_THREADS, 0, ctx->stream>>>(cn, sigs81 + 81 * r.lo, pk96 + 96 * r.lo,
@@ -1534,7 +1554,7 @@ static int locate_items(schnorr_b200_ctx* ctx, const std::vector<locate_range>& 
                                                                                            flags + r.lo);
         ctx->launches += 2;
         CUDA_TRY(ctx, cudaGetLastError());
-        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));   // the SoA scratch is reused by the next range
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     }
     return SCHNORR_B200_OK;
 }
@@ -1548,10 +1568,10 @@ int schnorr_b200_locate_invalid_dev(schnorr_b200_ctx* ctx, size_t n, const uint8
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     CUDA_TRY(ctx, cudaMemsetAsync(flags, 0, n, ctx->stream));
     std::vector<locate_range> suspects{{0, n}}, leaves;
-    void* d_res;
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    uint8_t* base;
     const size_t slot = RESULT_BYTES + 192 + 40;   // result | partial, per sub-range
-    if (int rc = ensure_scratch(ctx, SL_L, 64 + slot * LOCATE_FANOUT * 64, &d_res)) return rc;
-    uint8_t* base = (uint8_t*)d_res + 64;
+    if (int rc = stage_in(ctx, {{nullptr, slot * LOCATE_FANOUT * 64, &base}})) return rc;
     bool first = true;
     while (!suspects.empty()) {
         // cut every suspect range (the whole batch is first checked as it is: a batch that verifies has no culprit)
@@ -1620,35 +1640,26 @@ int schnorr_b200_locate_invalid(schnorr_b200_ctx* ctx, size_t n, const uint8_t* 
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
-    // dedicated staging (slot M is only used by verify_many's work lists): inputs stay resident across the bisection
+    // the inputs stay resident across the bisection
+    scratch_scope scope(c->scratch, c->stream);
     uint8_t *d_sig, *d_pk, *d_m, *d_off, *d_rand, *d_inf, *d_flags;
-    if (int rc = stage_in(c, SL_M, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                                    {rand32, n * 32, &d_rand}, {pk_inf, n, &d_inf}, {nullptr, n, &d_flags}}))
+    if (int rc = stage_in(c, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                              {rand32, n * 32, &d_rand}, {pk_inf, n, &d_inf}, {nullptr, n, &d_flags}}))
         return rc;
     return locate_invalid_staged(ctx, n, d_sig, d_pk, pk_inf ? d_inf : nullptr, d_m, (const uint64_t*)d_off, d_rand, d_flags,
                                  flags, n_bad);
 }
 
-static int read_result(schnorr_b200_ctx* ctx, const uint8_t* d_res, int* verdict, uint8_t* lhs97, uint8_t* rhs97) {
-    uint8_t h[RESULT_BYTES];
-    CUDA_TRY(ctx, cudaMemcpyAsync(h, d_res, RESULT_BYTES, cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    *verdict = h[0];
-    if (lhs97) memcpy(lhs97, h + 8, 97);
-    if (rhs97) memcpy(rhs97, h + 112, 97);
-    return SCHNORR_B200_OK;
-}
 
 int schnorr_b200_batch_finish(schnorr_b200_ctx* ctx, size_t n_partials, const uint8_t* partials192_host, int* verdict,
                               uint8_t* lhs97, uint8_t* rhs97) {
     if (!ctx || !partials192_host || !verdict || n_partials == 0) return SCHNORR_B200_EARG;
     MULTI_DISPATCH(ctx, schnorr_b200_batch_finish(ctx->shards[0], n_partials, partials192_host, verdict, lhs97, rhs97));
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    void *d_p, *d_res;
-    if (int rc = stage_in(ctx, SL_H, partials192_host, n_partials * 192, &d_p)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_L, 64 + RESULT_BYTES + 192, &d_res)) return rc;
-    uint8_t* res = (uint8_t*)d_res + 64;
-    if (int rc = schnorr_b200_batch_finish_dev(ctx, n_partials, (uint8_t*)d_p, res)) return rc;
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    uint8_t *d_p, *res;
+    if (int rc = stage_in(ctx, {{partials192_host, n_partials * 192, &d_p}, {nullptr, RESULT_BYTES, &res}})) return rc;
+    if (int rc = schnorr_b200_batch_finish_dev(ctx, n_partials, d_p, res)) return rc;
     return read_result(ctx, res, verdict, lhs97, rhs97);
 }
 
@@ -1683,10 +1694,10 @@ static int batch_partial_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* si
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
-    // staging slots distinct from those batch_partial_impl uses (A-G, J-L): one blob in slot H
+    scratch_scope scope(ctx->scratch, ctx->stream);
     uint8_t *d_sig, *d_pk, *d_m, *d_off, *d_rand, *d_inf, *d_seed;
-    if (int rc = stage_in(ctx, SL_H, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                                      rs.rand_region(n, &d_rand), {pk_inf, n, &d_inf}, rs.seed_region(&d_seed)}))
+    if (int rc = stage_in(ctx, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                rs.rand_region(n, &d_rand), {pk_inf, n, &d_inf}, rs.seed_region(&d_seed)}))
         return rc;
     if (int rc = rand_generate(ctx, n, rs, d_seed, d_rand)) return rc;
     return batch_partial_impl(ctx, n, d_sig, d_pk, pk_inf ? d_inf : nullptr, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
@@ -1703,12 +1714,9 @@ static int verify_batch_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sig
                                       rs.from(s.lo), partial);
         });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    uint8_t* res = nullptr;
-    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
-            return batch_partial_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rs, partial, rhs_pre);
-        }, res))
-        return rc;
-    return read_result(ctx, res, verdict, lhs97, rhs97);
+    return batch_whole_host(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+        return batch_partial_host(ctx, n, sigs81, pk96, pk_inf, msgs, msg_off, rs, partial, rhs_pre);
+    }, verdict, lhs97, rhs97);
 }
 
 int schnorr_b200_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,

@@ -126,25 +126,20 @@ static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* m
     size_t g = sl.size();
     schnorr_b200_ctx* root = ctx->shards[0];
     CUDA_TRY(root, cudaSetDevice(root->device));
-    // root buffer: [64 B flags of batch_partial_impl | result | g partials]
-    void* d_res;
-    if (int rc = ensure_scratch(root, SL_L, 64 + RESULT_BYTES + 192 * (g + 1), &d_res)) {
+    // the shard-0 worker below nests its scope inside this one while this thread waits for it
+    scratch_scope scope(root->scratch, root->stream);
+    uint8_t *res, *gathered;   // gathered: g x 192 B on the root device
+    if (int rc = stage_in(root, {{nullptr, RESULT_BYTES, &res}, {nullptr, 192 * g, &gathered}})) {
         ctx->err = root->err;
         return rc;
     }
-    uint8_t* res = (uint8_t*)d_res + 64;
-    uint8_t* gathered = res + RESULT_BYTES;  // g x 192 B on the root device
     int rc = multi_run(ctx, sl, [&](int k, shard_slice s) {
         schnorr_b200_ctx* sh = ctx->shards[k];
         if (cudaSetDevice(sh->device) != cudaSuccess) return (int)SCHNORR_B200_ECUDA;
-        uint8_t* partial;
-        if (k == 0) {
-            partial = gathered;  // the root writes its partial in place
-        } else {
-            void* d_loc;
-            if (int r2 = ensure_scratch(sh, SL_L, 64 + RESULT_BYTES + 192, &d_loc)) return r2;
-            partial = (uint8_t*)d_loc + 64 + RESULT_BYTES;
-        }
+        scratch_scope shard_scope(sh->scratch, sh->stream);
+        uint8_t* partial = gathered;  // the root writes its partial in place
+        if (k != 0)
+            if (int r2 = stage_in(sh, {{nullptr, 192, &partial}})) return r2;
         size_t cn = s.hi - s.lo;
         int r;
         if (cn == 0) {

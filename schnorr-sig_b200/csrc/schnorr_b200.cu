@@ -25,6 +25,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <deque>
 #include <string>
 #include <vector>
 
@@ -35,6 +36,7 @@
 #include "dist.cuh"
 #include "debug_ops.cuh"
 #include "derive.cuh"
+#include "scratch.cuh"
 
 using namespace sb;
 
@@ -57,17 +59,12 @@ static constexpr size_t REG_BATCH_MIN_PER_KEY = 64;
 // 1.67 / 4.53 ms, 512 keys 10.3 / 12.8 ms, 4096 keys 81.5 / 79.5 ms (sets of 64 to 16 384 keys).
 static constexpr size_t KEYSET_BLOCK_MAX = 512;
 
-// N, O: batches against registered key sets (gathered key records; key-side accumulators and terms), which run
-// batch_partial_impl (A-G, I-L) on inputs staged in H or M
-enum scratch_slot { SL_A = 0, SL_B, SL_C, SL_D, SL_E, SL_F, SL_G, SL_H, SL_I, SL_J, SL_K, SL_L, SL_M, SL_N, SL_O, SL_COUNT };
-
 struct schnorr_b200_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
     cudaStream_t own_stream = nullptr;
     uint64_t* gtab = nullptr;
-    void* scratch[SL_COUNT] = {};
-    size_t scratch_cap[SL_COUNT] = {};
+    scratch_arena scratch;                          // every temporary device buffer of a call (scratch.cuh)
     uint64_t launches = 0;
     int sm_count = 148;
     cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr;  // bracket the dominant kernel of the last call
@@ -87,8 +84,9 @@ struct schnorr_b200_ctx {
     size_t one_max = 512;                           // ... and up to this many the block-per-signature kernel (one.cuh)
     size_t batch_dist_max = (size_t)1 << 18;        // batches up to this size hash their challenges on six lanes per signature
     size_t batch_small_max = 256;                   // batches up to this size run one thread block per signature (k_batch_small)
-    int exact_counters_used = 0;                    // work-list counters written by the last verify call
     static constexpr int MAX_CHUNKS = 16;
+    uint32_t* exact_counters = nullptr;             // [MAX_CHUNKS] items handed to the exact kernel, per pipeline chunk
+    int exact_counters_used = 0;                    // counters written by the last verify call
     cudaEvent_t ev_chunk[MAX_CHUNKS] = {};
     std::string err;
     // multi-device context (schnorr_b200_create_multi): one single-device context per listed device; empty otherwise
@@ -104,20 +102,20 @@ struct schnorr_b200_ctx {
         }                                                                                        \
     } while (0)
 
-static int ensure_scratch(schnorr_b200_ctx* ctx, int slot, size_t bytes, void** out) {
-    if (bytes == 0) bytes = 16;
-    if (ctx->scratch_cap[slot] < bytes) {
-        if (ctx->scratch[slot]) {
-            CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-            CUDA_TRY(ctx, cudaFree(ctx->scratch[slot]));
-            ctx->scratch[slot] = nullptr;
-            ctx->scratch_cap[slot] = 0;
-        }
-        size_t cap = bytes + bytes / 8;
-        CUDA_TRY(ctx, cudaMalloc(&ctx->scratch[slot], cap));
-        ctx->scratch_cap[slot] = cap;
+// Regions of the context's scratch arena, taken in the innermost open scope: *dev receives each region's device
+// address, and `host` (when not null) is copied there on the context stream.  A null `host` only reserves the region.
+struct stage_region {
+    const void* host;
+    size_t bytes;
+    void** dev;
+    template <typename T>
+    stage_region(const void* h, size_t b, T** d) : host(h), bytes(b), dev(reinterpret_cast<void**>(d)) {}
+};
+static int stage_in(schnorr_b200_ctx* ctx, std::initializer_list<stage_region> regions) {
+    for (const stage_region& r : regions) {
+        CUDA_TRY(ctx, ctx->scratch.take(r.bytes, r.dev));
+        if (r.host && r.bytes) CUDA_TRY(ctx, cudaMemcpyAsync(*r.dev, r.host, r.bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
-    *out = ctx->scratch[slot];
     return 0;
 }
 
@@ -1021,16 +1019,10 @@ static int build_tables(schnorr_b200_ctx* ctx, size_t n_pts, const uint64_t* pts
     return 0;
 }
 
+// the SoA planes of n items, in the caller's scope
 static int alloc_soa(schnorr_b200_ctx* ctx, size_t n, soa_batch* b) {
-    void *p, *f, *sf;
-    if (int rc = ensure_scratch(ctx, SL_A, sizeof(ulonglong2) * SOA_PLANES * n, &p)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_B, n, &f)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_C, n, &sf)) return rc;
-    b->planes = (ulonglong2*)p;
-    b->flags = (uint8_t*)f;
-    b->sig_flag = (uint8_t*)sf;
     b->n = n;
-    return 0;
+    return stage_in(ctx, {{nullptr, sizeof(ulonglong2) * SOA_PLANES * n, &b->planes}, {nullptr, n, &b->flags}, {nullptr, n, &b->sig_flag}});
 }
 
 // The offset table of a HOST call must start at 0 and be non-decreasing (the reference's `&[&[u8]]` cannot express
@@ -1048,35 +1040,6 @@ static bool msg_off_valid(size_t n, const uint64_t* msg_off) {
             return SCHNORR_B200_EARG;                                                             \
         }                                                                                         \
     } while (0)
-
-// host -> device staging helper
-static int stage_in(schnorr_b200_ctx* ctx, int slot, const void* host, size_t bytes, void** dev) {
-    if (int rc = ensure_scratch(ctx, slot, bytes, dev)) return rc;
-    if (host && bytes) CUDA_TRY(ctx, cudaMemcpyAsync(*dev, host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    return 0;
-}
-
-// Several regions in one scratch slot, each starting on a 256-byte boundary: *dev receives the region's device
-// address, and `host` (when not null) is copied there.  A null `host` only reserves the region.
-struct stage_region {
-    const void* host;
-    size_t bytes;
-    uint8_t** dev;
-};
-static int stage_in(schnorr_b200_ctx* ctx, int slot, std::initializer_list<stage_region> regions) {
-    auto padded = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    size_t total = 0;
-    for (const stage_region& r : regions) total += padded(r.bytes);
-    void* blob;
-    if (int rc = ensure_scratch(ctx, slot, total, &blob)) return rc;
-    uint8_t* p = (uint8_t*)blob;
-    for (const stage_region& r : regions) {
-        *r.dev = p;
-        if (r.host && r.bytes) CUDA_TRY(ctx, cudaMemcpyAsync(p, r.host, r.bytes, cudaMemcpyHostToDevice, ctx->stream));
-        p += padded(r.bytes);
-    }
-    return 0;
-}
 
 // the single-device context of device k of a context: the context itself unless it has shards
 static schnorr_b200_ctx* device_ctx(schnorr_b200_ctx* ctx, size_t k) { return ctx->shards.empty() ? ctx : ctx->shards[k]; }
@@ -1105,10 +1068,10 @@ static int verify_many_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs
 
 
 // Signature::verify over an ingested SoA batch: fast path (per-thread or warp-cooperative by call size), then the exact kernel over the handful of
-// items it handed back.  `list_base` = first element of this batch in the per-call work list (pipelined chunks
-// use disjoint regions), `counter` = index of its counter.
+// items it handed back.  `counter` = index of this batch's exact-path counter (pipelined chunks use one each); its
+// work list is taken in the caller's scope, which must outlive the kernels on `st`.
 static int launch_verify(schnorr_b200_ctx* ctx, const soa_batch& soa, const uint8_t* msgs, const uint64_t* msg_off,
-                         uint8_t* verdicts, size_t list_base, int counter, size_t list_total, cudaStream_t st) {
+                         uint8_t* verdicts, int counter, cudaStream_t st) {
     unsigned grid = grid_for(soa.n, VERIFY_THREADS);
     if (counter == 0) ctx->exact_counters_used = 0;
     if (ctx->exact_only) {
@@ -1116,10 +1079,9 @@ static int launch_verify(schnorr_b200_ctx* ctx, const soa_batch& soa, const uint
         ctx->launches += 1;
         return 0;
     }
-    void* wl;
-    if (int rc = ensure_scratch(ctx, SL_M, 4 * (list_total + schnorr_b200_ctx::MAX_CHUNKS), &wl)) return rc;
-    uint32_t* counters = (uint32_t*)wl;
-    uint32_t* list = counters + schnorr_b200_ctx::MAX_CHUNKS + list_base;
+    uint32_t* list;
+    if (int rc = stage_in(ctx, {{nullptr, 4 * soa.n, &list}})) return rc;
+    uint32_t* counters = ctx->exact_counters;
     CUDA_TRY(ctx, cudaMemsetAsync(counters + counter, 0, 4, st));
     if (counter + 1 > ctx->exact_counters_used) ctx->exact_counters_used = counter + 1;
     if (soa.n <= ctx->one_max)
@@ -1202,6 +1164,7 @@ int schnorr_b200_create(int device, schnorr_b200_ctx** out) {
     CREATE_TRY(cudaMemcpyToSymbol(c_q_wnaf5, CHEETAH_Q_WNAF5, sizeof(CHEETAH_Q_WNAF5)));  // the tail of the symbol stays zero
     CREATE_TRY(cudaMemcpyToSymbol(c_q_wnaf4, CHEETAH_Q_WNAF4, 256));
     CREATE_TRY(cudaMalloc(&ctx->gtab, GTAB_U64 * sizeof(uint64_t)));
+    CREATE_TRY(cudaMalloc(&ctx->exact_counters, schnorr_b200_ctx::MAX_CHUNKS * sizeof(uint32_t)));
     jac_pt* bases = nullptr;  // the GTAB_WINDOWS bases, then G itself (12 limbs)
     CREATE_TRY(cudaMalloc(&bases, sizeof(jac_pt) * GTAB_WINDOWS + 96));
     uint64_t* g12 = reinterpret_cast<uint64_t*>(bases + GTAB_WINDOWS);
@@ -1250,9 +1213,8 @@ void schnorr_b200_destroy(schnorr_b200_ctx* ctx) {
     }
     cudaSetDevice(ctx->device);
     if (ctx->own_stream) cudaStreamSynchronize(ctx->own_stream);
-    for (int s = 0; s < SL_COUNT; s++)
-        if (ctx->scratch[s]) cudaFree(ctx->scratch[s]);
     if (ctx->gtab) cudaFree(ctx->gtab);
+    if (ctx->exact_counters) cudaFree(ctx->exact_counters);
     for (int c = 0; c < schnorr_b200_ctx::MAX_CHUNKS; c++)
         if (ctx->ev_chunk[c]) cudaEventDestroy(ctx->ev_chunk[c]);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -1373,11 +1335,11 @@ int schnorr_b200_last_exact_count(schnorr_b200_ctx* ctx, uint64_t* count) {
         }
         return SCHNORR_B200_OK;
     }
-    if (ctx->exact_counters_used == 0 || !ctx->scratch[SL_M]) return SCHNORR_B200_OK;
+    if (ctx->exact_counters_used == 0) return SCHNORR_B200_OK;
     uint32_t c[schnorr_b200_ctx::MAX_CHUNKS] = {};
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    CUDA_TRY(ctx, cudaMemcpy(c, ctx->scratch[SL_M], 4 * ctx->exact_counters_used, cudaMemcpyDeviceToHost));
+    CUDA_TRY(ctx, cudaMemcpy(c, ctx->exact_counters, 4 * ctx->exact_counters_used, cudaMemcpyDeviceToHost));
     for (int i = 0; i < ctx->exact_counters_used; i++) *count += c[i];
     return SCHNORR_B200_OK;
 }
@@ -1409,12 +1371,11 @@ int schnorr_b200_hash_messages(schnorr_b200_ctx* ctx, size_t n, const uint8_t* r
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_rx, *d_pk, *d_m, *d_off, *d_out;
-    if (int rc = stage_in(ctx, SL_D, rx48, n * 48, &d_rx)) return rc;
-    if (int rc = stage_in(ctx, SL_E, pk96, n * 96, &d_pk)) return rc;
-    if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
-    if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n * 32, &d_out)) return rc;
+    if (int rc = stage_in(ctx, {{rx48, n * 48, &d_rx}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                {nullptr, n * 32, &d_out}}))
+        return rc;
     if (int rc = schnorr_b200_hash_messages_dev(ctx, n, (uint8_t*)d_rx, (uint8_t*)d_pk, (uint8_t*)d_m, (uint64_t*)d_off,
                                                 (uint8_t*)d_out))
         return rc;
@@ -1431,11 +1392,12 @@ int schnorr_b200_verify_many_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_t*
     if (!ctx || (n && (!sigs81 || !pk96 || !msg_off || !verdicts))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     soa_batch soa;
     if (int rc = alloc_soa(ctx, n, &soa)) return rc;
     k_ingest<<<grid_for(n, INGEST_THREADS), INGEST_THREADS, 0, ctx->stream>>>(n, sigs81, pk96, pk_inf, soa);
     cudaEventRecord(ctx->ev_k0, ctx->stream);
-    if (int rc = launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, 0, n, ctx->stream)) return rc;
+    if (int rc = launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, ctx->stream)) return rc;
     cudaEventRecord(ctx->ev_k1, ctx->stream);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
@@ -1473,14 +1435,12 @@ static int verify_many_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs
     const uint64_t base = msg_off[0];
     size_t mb = msg_off[n] - base;
     if (mb && !msgs) return SCHNORR_B200_EARG;
-    void *d_sig, *d_pk, *d_inf = nullptr, *d_m, *d_off, *d_out;
-    if (int rc = ensure_scratch(ctx, SL_D, n * 81, &d_sig)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, n * 96, &d_pk)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_F, mb, &d_m)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_G, (n + 1) * 8, &d_off)) return rc;
-    if (pk_inf)
-        if (int rc = ensure_scratch(ctx, SL_I, n, &d_inf)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
+    // the copy stream and the second compute stream are joined into the context stream before this scope closes
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    void *d_sig, *d_pk, *d_inf, *d_m, *d_off, *d_out;
+    if (int rc = stage_in(ctx, {{nullptr, n * 81, &d_sig}, {nullptr, n * 96, &d_pk}, {nullptr, mb, &d_m}, {nullptr, (n + 1) * 8, &d_off},
+                                {nullptr, pk_inf ? n : 0, &d_inf}, {nullptr, n, &d_out}}))
+        return rc;
     soa_batch soa;
     if (int rc = alloc_soa(ctx, n, &soa)) return rc;
     // chunk plan in whole kernel waves (no partial-wave tail between chunks): 1, 3, 8 waves, then the rest.
@@ -1501,7 +1461,7 @@ static int verify_many_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs
     }
     cudaStream_t cs = ctx->copy_stream, ks = ctx->stream, ks2 = ctx->aux_stream;
     // neither the copy stream nor the second compute stream may overtake work of a previous call that still reads the
-    // scratch buffers
+    // scratch regions
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev_chunk[0], ks));
     CUDA_TRY(ctx, cudaStreamWaitEvent(cs, ctx->ev_chunk[0], 0));
     CUDA_TRY(ctx, cudaStreamWaitEvent(ks2, ctx->ev_chunk[0], 0));
@@ -1538,7 +1498,7 @@ static int verify_many_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs
                                                                          pk_inf ? (uint8_t*)d_inf + lo : nullptr, sc);
         if (st == ks) cudaEventRecord(ctx->ev_k0, ks);
         // the kernels index the message blob with the caller's absolute offsets: shift the device base accordingly
-        if (int rc = launch_verify(ctx, sc, (uint8_t*)d_m - base, (uint64_t*)d_off + lo, (uint8_t*)d_out + lo, lo, c, n, st)) return rc;
+        if (int rc = launch_verify(ctx, sc, (uint8_t*)d_m - base, (uint64_t*)d_off + lo, (uint8_t*)d_out + lo, c, st)) return rc;
         if (st == ks) cudaEventRecord(ctx->ev_k1, ks);
         ctx->launches += 1;
     }
@@ -1563,10 +1523,9 @@ int schnorr_b200_verify_keyed_many_dev(schnorr_b200_ctx* ctx, size_t n, const ui
     if (!ctx || (n && (!keyed130 || !msg_off || !verdicts))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_pk, *d_inf, *d_ok, *d_sig;
-    if (int rc = ensure_scratch(ctx, SL_J, n * 96, &d_pk)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_K, n * 2, &d_inf)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_L, n * 81 + 256, &d_sig)) return rc;
+    if (int rc = stage_in(ctx, {{nullptr, n * 96, &d_pk}, {nullptr, n * 2, &d_inf}, {nullptr, n * 81 + 256, &d_sig}})) return rc;
     d_ok = (uint8_t*)d_inf + n;
     k_split_keyed<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, keyed130, (uint8_t*)d_pk, (uint8_t*)d_inf, (uint8_t*)d_ok,
                                                            (uint8_t*)d_sig);
@@ -1587,11 +1546,10 @@ int schnorr_b200_verify_keyed_many(schnorr_b200_ctx* ctx, size_t n, const uint8_
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_rec, *d_m, *d_off, *d_out;
-    if (int rc = stage_in(ctx, SL_D, keyed130, n * 130, &d_rec)) return rc;
-    if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
-    if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
+    if (int rc = stage_in(ctx, {{keyed130, n * 130, &d_rec}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off}, {nullptr, n, &d_out}}))
+        return rc;
     if (int rc = schnorr_b200_verify_keyed_many_dev(ctx, n, (uint8_t*)d_rec, (uint8_t*)d_m, (uint64_t*)d_off, (uint8_t*)d_out))
         return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(verdicts, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1649,22 +1607,27 @@ static int keyset_alloc_records(schnorr_b200_ctx* ctx, size_t cap, uint64_t** pk
     return 0;
 }
 
-// Scratch of a registration of m keys (keyset_register): SL_D skip flags, then the table bases
-static size_t keyset_skip_bytes(size_t m) { return (m + 15) / 16 * 16; }
-static int keyset_register_scratch(schnorr_b200_ctx* ctx, size_t m, void** tmp) {
-    return ensure_scratch(ctx, SL_D, keyset_skip_bytes(m) + m * KT_WINDOWS * sizeof(jac_pt), tmp);
+// device memory of a registration of m keys (keyset_register) and of their encodings (keyset_encode_async), taken by
+// the caller so that an update can take all of it before it writes anything
+struct keyset_reg_mem {
+    uint8_t* skip;          // [m]
+    jac_pt* bases;          // [m][KT_WINDOWS]
+    keyset_entry* entries;  // [m] (encodings only)
+    uint8_t* findable;      // [m] (encodings only)
+};
+static int keyset_take_reg_mem(schnorr_b200_ctx* ctx, size_t m, bool encode, keyset_reg_mem* r) {
+    return stage_in(ctx, {{nullptr, m, &r->skip}, {nullptr, m * KT_WINDOWS * sizeof(jac_pt), &r->bases},
+                          {nullptr, encode ? m * sizeof(keyset_entry) : 0, &r->entries}, {nullptr, encode ? m : 0, &r->findable}});
 }
 
 // Registration of m keys on one device, the one routine of create, append and replace: status[j] of record j
 // (keyset_key_status) and, for keys of status 0 other than the identity, the table at tab + j KT_KEY_U64 (left as it
 // is for the others).  Up to ctx->keyset_block_max keys run one block per key (k_keyset_register_block), more one
-// thread per key (k_keyset_register, k_tab_bases); k_tab_fill builds the tables.  Scratch: keyset_register_scratch.
+// thread per key (k_keyset_register, k_tab_bases); k_tab_fill builds the tables.
 static int keyset_register(schnorr_b200_ctx* ctx, size_t m, const uint64_t* pk12, const uint8_t* pk_inf, uint8_t* status,
-                           uint64_t* tab) {
-    void* tmp;
-    if (int rc = keyset_register_scratch(ctx, m, &tmp)) return rc;
-    uint8_t* skip = (uint8_t*)tmp;
-    jac_pt* bases = (jac_pt*)((uint8_t*)tmp + keyset_skip_bytes(m));
+                           uint64_t* tab, const keyset_reg_mem& mem) {
+    uint8_t* skip = mem.skip;
+    jac_pt* bases = mem.bases;
     if (m <= ctx->keyset_block_max) {
         k_keyset_register_block<<<(unsigned)m, ONE_THREADS, 0, ctx->stream>>>(m, pk12, pk_inf, status, skip, bases);
         size_t threads = m * (size_t)KT_WINDOWS * KT_ENTRIES;
@@ -1679,16 +1642,13 @@ static int keyset_register(schnorr_b200_ctx* ctx, size_t m, const uint64_t* pk12
 }
 
 // Encodings of m records (k_keyset_encode), enqueued with their copies into `entries` / `findable` (host, m each);
-// the host may read them after ctx->ev_aux.  Scratch: SL_E.
+// the host may read them after ctx->ev_aux.
 static int keyset_encode_async(schnorr_b200_ctx* ctx, size_t m, const uint64_t* pk12, const uint8_t* pk_inf,
-                               keyset_entry* entries, uint8_t* findable) {
-    void* enc;  // lookup entries, then the findable flags
-    if (int rc = ensure_scratch(ctx, SL_E, m * (sizeof(keyset_entry) + 1), &enc)) return rc;
-    k_keyset_encode<<<grid_for(m, 128), 128, 0, ctx->stream>>>(m, pk12, pk_inf, (keyset_entry*)enc,
-                                                              (uint8_t*)enc + m * sizeof(keyset_entry));
+                               keyset_entry* entries, uint8_t* findable, const keyset_reg_mem& mem) {
+    k_keyset_encode<<<grid_for(m, 128), 128, 0, ctx->stream>>>(m, pk12, pk_inf, mem.entries, mem.findable);
     ctx->launches += 1;
-    CUDA_TRY(ctx, cudaMemcpyAsync(entries, enc, m * sizeof(keyset_entry), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(ctx, cudaMemcpyAsync(findable, (uint8_t*)enc + m * sizeof(keyset_entry), m, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(entries, mem.entries, m * sizeof(keyset_entry), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(findable, mem.findable, m, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev_aux, ctx->stream));
     return 0;
 }
@@ -1710,6 +1670,9 @@ static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t k
     kd.device = ctx->device;
     kd.cap = n;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    keyset_reg_mem mem;
+    if (int rc = keyset_take_reg_mem(ctx, n, true, &mem)) return rc;
     if (int rc = keyset_alloc_records(ctx, n, &kd.pk12, &kd.pk_inf, &kd.status)) return rc;
     CUDA_TRY(ctx, cudaMalloc(&kd.ktab, n * KT_KEY_U64 * sizeof(uint64_t)));
     CUDA_TRY(ctx, cudaMemsetAsync(kd.ktab, 0, n * KT_KEY_U64 * sizeof(uint64_t), ctx->stream));
@@ -1718,8 +1681,8 @@ static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t k
     else CUDA_TRY(ctx, cudaMemsetAsync(kd.pk_inf, 0, n, ctx->stream));
     std::vector<keyset_entry> entries(n);
     std::vector<uint8_t> findable(n);
-    if (int rc = keyset_encode_async(ctx, n, kd.pk12, kd.pk_inf, entries.data(), findable.data())) return rc;
-    if (int rc = keyset_register(ctx, n, kd.pk12, kd.pk_inf, kd.status, kd.ktab)) return rc;
+    if (int rc = keyset_encode_async(ctx, n, kd.pk12, kd.pk_inf, entries.data(), findable.data(), mem)) return rc;
+    if (int rc = keyset_register(ctx, n, kd.pk12, kd.pk_inf, kd.status, kd.ktab, mem)) return rc;
     if (k == 0) {
         ks->h_status.resize(n);
         CUDA_TRY(ctx, cudaMemcpyAsync(ks->h_status.data(), kd.status, n, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1749,16 +1712,16 @@ static constexpr size_t REG_SMALL_MAX = 384;
 
 // the fast kernel over an ingested batch of registered items, then the exact kernel over the items it handed back;
 // exact_only and small calls go through launch_verify (same verdicts: the planes hold each item's key record).
-// LOOKUP: key_idx may hold KEYSET_MISS (k_keyed_split_lookup); those items are finished by k_verify.
+// LOOKUP: key_idx may hold KEYSET_MISS (k_keyed_split_lookup); those items are finished by k_verify.  The work list is
+// taken in the caller's scope.
 template <bool LOOKUP>
 static int launch_verify_registered(schnorr_b200_ctx* ctx, const keyset_dev& kd, const soa_batch& soa,
                                     const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     cudaStream_t st = ctx->stream;
-    if (ctx->exact_only || soa.n <= REG_SMALL_MAX) return launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, 0, soa.n, st);
-    void* wl;
-    if (int rc = ensure_scratch(ctx, SL_M, 4 * (soa.n + schnorr_b200_ctx::MAX_CHUNKS), &wl)) return rc;
-    uint32_t* counter = (uint32_t*)wl;
-    uint32_t* list = counter + schnorr_b200_ctx::MAX_CHUNKS;
+    if (ctx->exact_only || soa.n <= REG_SMALL_MAX) return launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, st);
+    uint32_t* list;
+    if (int rc = stage_in(ctx, {{nullptr, 4 * soa.n, &list}})) return rc;
+    uint32_t* counter = ctx->exact_counters;
     CUDA_TRY(ctx, cudaMemsetAsync(counter, 0, 4, st));
     ctx->exact_counters_used = 1;
     unsigned grid = grid_for(soa.n, VERIFY_THREADS);
@@ -1773,9 +1736,9 @@ static int verify_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyse
                                  const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     const keyset_dev& kd = ks->devs[k];
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_pk, *d_inf;
-    if (int rc = ensure_scratch(ctx, SL_E, n * 96, &d_pk)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_I, n, &d_inf)) return rc;
+    if (int rc = stage_in(ctx, {{nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}})) return rc;
     soa_batch soa;
     if (int rc = alloc_soa(ctx, n, &soa)) return rc;
     k_keyset_gather<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, key_idx, ks->n_keys, kd.pk12, kd.pk_inf, (uint64_t*)d_pk,
@@ -1794,12 +1757,11 @@ static int verify_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keys
                                   const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     size_t mb = msg_off[n];
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_sig, *d_idx, *d_m, *d_off, *d_out;
-    if (int rc = stage_in(ctx, SL_D, sigs81, n * 81, &d_sig)) return rc;
-    if (int rc = stage_in(ctx, SL_J, key_idx, n * 4, &d_idx)) return rc;
-    if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
-    if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
+    if (int rc = stage_in(ctx, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                {nullptr, n, &d_out}}))
+        return rc;
     if (int rc = verify_registered_dev(ctx, ks, k, n, (uint8_t*)d_sig, (uint32_t*)d_idx, (uint8_t*)d_m, (uint64_t*)d_off,
                                        (uint8_t*)d_out))
         return rc;
@@ -1821,7 +1783,8 @@ static bool keyset_any_not_torsion_free(const schnorr_b200_keyset* ks) {
     return std::find(ks->h_status.begin(), ks->h_status.end(), KEY_NOT_TORSION_FREE) != ks->h_status.end();
 }
 
-// buffers of one device's set that an update allocates before it writes anything
+// buffers of one device's set that an update allocates before it writes anything: grown ones, and the scratch
+// regions of the update (staged records, the compact table of a replace, registration and encodings)
 struct keyset_grow {
     uint64_t* pk12 = nullptr;
     uint8_t *pk_inf = nullptr, *status = nullptr;
@@ -1829,7 +1792,12 @@ struct keyset_grow {
     size_t cap = 0;
     keyset_entry* lut = nullptr;
     size_t lut_cap = 0;
-    void *stage = nullptr, *ctab = nullptr;
+    uint64_t* spk = nullptr;
+    uint8_t* sinf = nullptr;
+    uint32_t* sidx = nullptr;
+    uint64_t* ctab = nullptr;
+    uint8_t* cstatus = nullptr;
+    keyset_reg_mem reg{};
 };
 static void keyset_grow_free(int device, keyset_grow& g) {
     cudaSetDevice(device);
@@ -1843,16 +1811,17 @@ static void keyset_grow_free(int device, keyset_grow& g) {
 
 // append (key_idx == NULL: slots n_keys ... n_keys + m - 1) or replace (slots key_idx[j], distinct and inside the set)
 // of m keys, on every device; arguments checked by the caller.  The set ends exactly as keyset_create would build it
-// from the updated list of records.  Every allocation comes first, so a failure there leaves the set unchanged.  On
-// each device: the records are staged (SL_F); an append registers them into its new slots, a replace into a compact
-// table (SL_G) that k_keyset_scatter copies to the slots, zeros included.  The first device encodes them; the host
-// merges the new lookup entries into its model (keyset_update_entries) and uploads the table to every device.
+// from the updated list of records.  Every allocation comes first, scratch regions included (one scope per device, open
+// for the whole update), so a failure there leaves the set unchanged.  On each device: the records are staged; an
+// append registers them into its new slots, a replace into a compact table that k_keyset_scatter copies to the slots,
+// zeros included.  The first device encodes them; the host merges the new lookup entries into its model
+// (keyset_update_entries) and uploads the table to every device.
 static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t m, const uint32_t* key_idx,
                          const uint8_t* pk96, const uint8_t* pk_inf, uint8_t* status) {
     const size_t n = ks->n_keys, new_n = key_idx ? n : n + m;
     const size_t lut_need = ks->h_all.size() + m;  // distinct findable encodings after the update, at most
-    const size_t stage_bytes = m * 96 + (m + 15) / 16 * 16 + m * 4;
     std::vector<keyset_grow> gr(ks->devs.size());
+    std::deque<scratch_scope> scopes;
     auto fail = [&](int rc, size_t d) {
         schnorr_b200_ctx* c = device_ctx(ctx, d);
         if (c != ctx) ctx->err = "device " + std::to_string(c->device) + ": " + c->err;
@@ -1884,11 +1853,12 @@ static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t 
                 return fail(SCHNORR_B200_ECUDA, d);
             }
         }
-        void* enc;
-        if ((rc = ensure_scratch(c, SL_F, stage_bytes, &g.stage))) return fail(rc, d);
-        if ((rc = keyset_register_scratch(c, m, &enc))) return fail(rc, d);
-        if (d == 0 && (rc = ensure_scratch(c, SL_E, m * (sizeof(keyset_entry) + 1), &enc))) return fail(rc, d);
-        if (key_idx && (rc = ensure_scratch(c, SL_G, m * KT_KEY_U64 * sizeof(uint64_t) + m, &g.ctab))) return fail(rc, d);
+        scopes.emplace_back(c->scratch, c->stream);
+        const size_t r = key_idx ? m : 0;   // a replace: key indices and the compact table
+        if ((rc = stage_in(c, {{nullptr, m * 96, &g.spk}, {nullptr, m, &g.sinf}, {nullptr, r * 4, &g.sidx},
+                               {nullptr, r * KT_KEY_U64 * sizeof(uint64_t), &g.ctab}, {nullptr, r, &g.cstatus}})))
+            return fail(rc, d);
+        if ((rc = keyset_take_reg_mem(c, m, d == 0, &g.reg))) return fail(rc, d);
     }
     // ---- the set is written from here on
     std::vector<keyset_entry> entries(m);
@@ -1923,27 +1893,25 @@ static int keyset_update(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t 
             s.lut_cap = g.lut_cap;
             g.lut = nullptr;
         }
-        uint64_t* spk = (uint64_t*)g.stage;
-        uint8_t* sinf = (uint8_t*)g.stage + m * 96;
-        uint32_t* sidx = (uint32_t*)(sinf + (m + 15) / 16 * 16);
+        uint64_t* spk = g.spk;
+        uint8_t* sinf = g.sinf;
         CUDA_TRY(c, cudaMemcpyAsync(spk, pk96, m * 96, cudaMemcpyHostToDevice, sm));
         if (pk_inf) CUDA_TRY(c, cudaMemcpyAsync(sinf, pk_inf, m, cudaMemcpyHostToDevice, sm));
         else CUDA_TRY(c, cudaMemsetAsync(sinf, 0, m, sm));
-        if (d == 0 && (rc = keyset_encode_async(c, m, spk, sinf, entries.data(), findable.data()))) return rc;
+        if (d == 0 && (rc = keyset_encode_async(c, m, spk, sinf, entries.data(), findable.data(), g.reg))) return rc;
         uint8_t* new_status;
         if (!key_idx) {
             CUDA_TRY(c, cudaMemcpyAsync(s.pk12 + 12 * n, spk, m * 96, cudaMemcpyDeviceToDevice, sm));
             CUDA_TRY(c, cudaMemcpyAsync(s.pk_inf + n, sinf, m, cudaMemcpyDeviceToDevice, sm));
             new_status = s.status + n;
-            if ((rc = keyset_register(c, m, s.pk12 + 12 * n, s.pk_inf + n, new_status, s.ktab + n * KT_KEY_U64))) return rc;
+            if ((rc = keyset_register(c, m, s.pk12 + 12 * n, s.pk_inf + n, new_status, s.ktab + n * KT_KEY_U64, g.reg))) return rc;
         } else {
-            uint64_t* ctab = (uint64_t*)g.ctab;
-            new_status = (uint8_t*)(ctab + m * KT_KEY_U64);
-            CUDA_TRY(c, cudaMemcpyAsync(sidx, key_idx, m * 4, cudaMemcpyHostToDevice, sm));
-            CUDA_TRY(c, cudaMemsetAsync(ctab, 0, m * KT_KEY_U64 * sizeof(uint64_t), sm));
-            if ((rc = keyset_register(c, m, spk, sinf, new_status, ctab))) return rc;
+            new_status = g.cstatus;
+            CUDA_TRY(c, cudaMemcpyAsync(g.sidx, key_idx, m * 4, cudaMemcpyHostToDevice, sm));
+            CUDA_TRY(c, cudaMemsetAsync(g.ctab, 0, m * KT_KEY_U64 * sizeof(uint64_t), sm));
+            if ((rc = keyset_register(c, m, spk, sinf, new_status, g.ctab, g.reg))) return rc;
             k_keyset_scatter<<<grid_for(m * (KT_KEY_U128 + 13), 256), 256, 0, sm>>>(
-                m, sidx, spk, sinf, new_status, (const ulonglong2*)ctab, s.pk12, s.pk_inf, s.status, (ulonglong2*)s.ktab);
+                m, g.sidx, spk, sinf, new_status, (const ulonglong2*)g.ctab, s.pk12, s.pk_inf, s.status, (ulonglong2*)s.ktab);
             c->launches += 1;
             CUDA_TRY(c, cudaGetLastError());
         }
@@ -2136,8 +2104,6 @@ static constexpr double KEYED_REG_MAX_MISS_FRACTION = 0.4;
 
 // device buffers, single-device context, arguments checked by the caller.  `select`: read the miss count of the front
 // end (synchronises) and take verify_many above KEYED_REG_MAX_MISS_FRACTION.
-// Scratch: J decoded keys, K identity / ok flags | key indices | miss counter, L signatures (the slots of
-// verify_keyed_many_dev, which small calls run); the kernels after them use A-C and M.
 static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
                                        const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts,
                                        bool select) {
@@ -2145,11 +2111,12 @@ static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200
     const keyset_dev& kd = ks->devs[k];
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
+    scratch_scope scope(ctx->scratch, st);
     void *d_pk, *d_sig;
     uint8_t *d_inf, *d_idx, *d_miss;
-    if (int rc = ensure_scratch(ctx, SL_J, n * 96, &d_pk)) return rc;
-    if (int rc = stage_in(ctx, SL_K, {{nullptr, 2 * n, &d_inf}, {nullptr, 4 * n, &d_idx}, {nullptr, 4, &d_miss}})) return rc;
-    if (int rc = ensure_scratch(ctx, SL_L, n * 81 + 256, &d_sig)) return rc;
+    if (int rc = stage_in(ctx, {{nullptr, n * 96, &d_pk}, {nullptr, 2 * n, &d_inf}, {nullptr, 4 * n, &d_idx}, {nullptr, 4, &d_miss},
+                                {nullptr, n * 81 + 256, &d_sig}}))
+        return rc;
     uint8_t* d_ok = d_inf + n;
     CUDA_TRY(ctx, cudaMemsetAsync(d_miss, 0, 4, st));
     k_keyed_split_lookup<<<grid_for(n, 128), 128, 0, st>>>(n, keyed130, kd.lut, kd.n_lut, kd.pk12, kd.pk_inf, (uint8_t*)d_pk,
@@ -2179,16 +2146,15 @@ static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200
     return 0;
 }
 
-// host buffers on device k of the set: staged in D, F, G, verdicts in H, synchronised
+// host buffers on device k of the set: staged with cudaMemcpyAsync, verdicts copied back, synchronised
 static int verify_keyed_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
                                         const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     size_t mb = msg_off[n];
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_rec, *d_m, *d_off, *d_out;
-    if (int rc = stage_in(ctx, SL_D, keyed130, n * 130, &d_rec)) return rc;
-    if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
-    if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n, &d_out)) return rc;
+    if (int rc = stage_in(ctx, {{keyed130, n * 130, &d_rec}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off}, {nullptr, n, &d_out}}))
+        return rc;
     if (int rc = verify_keyed_registered_dev(ctx, ks, k, n, (uint8_t*)d_rec, (uint8_t*)d_m, (uint64_t*)d_off, (uint8_t*)d_out, true))
         return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(verdicts, d_out, n, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2206,9 +2172,9 @@ int schnorr_b200_keyset_lookup(schnorr_b200_ctx* ctx, const schnorr_b200_keyset*
     schnorr_b200_ctx* c = device_ctx(ctx, 0);
     const keyset_dev& kd = ks->devs[0];
     CUDA_TRY(c, cudaSetDevice(c->device));
+    scratch_scope scope(c->scratch, c->stream);
     void *d_in, *d_out;
-    if (int rc = stage_in(c, SL_D, keys49, n * 49, &d_in)) return rc;
-    if (int rc = ensure_scratch(c, SL_H, n * 4, &d_out)) return rc;
+    if (int rc = stage_in(c, {{keys49, n * 49, &d_in}, {nullptr, n * 4, &d_out}})) return rc;
     k_keyset_lookup<<<grid_for(n, 128), 128, 0, c->stream>>>(n, (uint8_t*)d_in, kd.lut, kd.n_lut, (uint32_t*)d_out);
     c->launches += 1;
     CUDA_TRY(c, cudaGetLastError());
@@ -2269,9 +2235,9 @@ static bool reg_batch_aggregates(const schnorr_b200_ctx* ctx, const schnorr_b200
     return n > ctx->batch_small_max && !ks->any_not_torsion_free && n / ks->n_keys >= ctx->reg_batch_min_per_key;
 }
 
-// The key side of an aggregated batch on device k of the set, in slot O: per-block key terms | column sums, key partial,
-// MSM partial, 64 zero bytes | for keyed records (miss_count != null) the route buffers of k_keyed_route.  The MSM is
-// planned for msm_points points.
+// The key side of an aggregated batch on device k of the set, in the caller's scope: per-block key terms | column sums,
+// key partial, MSM partial, 64 zero bytes | for keyed records (miss_count != null) the route buffers of k_keyed_route.
+// The MSM is planned for msm_points points.
 static int reg_batch_setup(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint32_t* key_idx,
                            const uint32_t* miss_count, size_t msm_points, reg_batch* rb) {
     size_t max_blocks = (size_t)2 * ctx->sm_count, want = (ks->n_keys + KEYTERM_THREADS / 32 - 1) / (KEYTERM_THREADS / 32);
@@ -2279,14 +2245,14 @@ static int reg_batch_setup(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks,
     const size_t sz_cols = ks->n_keys * 8 * sizeof(unsigned long long);
     size_t r = miss_count ? n : 0;   // route buffers
     uint8_t *d_terms, *d_cols, *d_miss, *d_pos, *d_tiles, *d_tk, *d_mpts, *d_msc;
-    if (int rc = stage_in(ctx, SL_O, {{nullptr, (size_t)blocks * sizeof(jac_pt), &d_terms},
-                                      {nullptr, sz_cols + 192 + 192 + 64, &d_cols},
-                                      {nullptr, r * 4, &d_miss},
-                                      {nullptr, r * 4, &d_pos},
-                                      {nullptr, (r + SCAN_TILE - 1) / SCAN_TILE * 4, &d_tiles},
-                                      {nullptr, r * 32, &d_tk},
-                                      {nullptr, r * 96, &d_mpts},
-                                      {nullptr, r * 32, &d_msc}}))
+    if (int rc = stage_in(ctx, {{nullptr, (size_t)blocks * sizeof(jac_pt), &d_terms},
+                                {nullptr, sz_cols + 192 + 192 + 64, &d_cols},
+                                {nullptr, r * 4, &d_miss},
+                                {nullptr, r * 4, &d_pos},
+                                {nullptr, (r + SCAN_TILE - 1) / SCAN_TILE * 4, &d_tiles},
+                                {nullptr, r * 32, &d_tk},
+                                {nullptr, r * 96, &d_mpts},
+                                {nullptr, r * 32, &d_msc}}))
         return rc;
     rb->key_idx = key_idx;
     rb->n_keys = ks->n_keys;
@@ -2334,8 +2300,9 @@ int schnorr_b200_batch_randomizers(schnorr_b200_ctx* ctx, size_t n, const uint8_
         });
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     uint8_t *d_seed, *d_rand;
-    if (int rc = stage_in(ctx, SL_H, {{seed32, 32, &d_seed}, {nullptr, n * 32, &d_rand}})) return rc;
+    if (int rc = stage_in(ctx, {{seed32, 32, &d_seed}, {nullptr, n * 32, &d_rand}})) return rc;
     if (int rc = rand_generate(ctx, n, rand_source{nullptr, seed32, first_index}, d_seed, d_rand)) return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(rand32, d_rand, n * 32, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -2351,8 +2318,9 @@ static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_ke
                                     uint8_t* partial192, uint64_t* rhs_pre) {
     const keyset_dev& kd = ks->devs[k];
     cudaStream_t st = ctx->stream;
+    scratch_scope scope(ctx->scratch, st);
     uint8_t *d_pk, *d_inf;
-    if (int rc = stage_in(ctx, SL_N, {{nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}})) return rc;
+    if (int rc = stage_in(ctx, {{nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}})) return rc;
     k_keyset_gather<<<grid_for(n, 128), 128, 0, st>>>(n, key_idx, ks->n_keys, kd.pk12, kd.pk_inf, (uint64_t*)d_pk, d_inf);
     ctx->launches += 1;
     if (!reg_batch_aggregates(ctx, ks, n))
@@ -2362,13 +2330,14 @@ static int batch_partial_registered(schnorr_b200_ctx* ctx, const schnorr_b200_ke
     return batch_partial_impl(ctx, n, sigs81, d_pk, d_inf, msgs, msg_off, rand32, partial192, rhs_pre, &rb);
 }
 
-// host inputs (n > 0, offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
+// host inputs (n > 0, offsets checked) -> staged on the device -> one partial at `partial` (device memory of this context)
 static int batch_partial_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
                                          const uint8_t* sigs81, const uint32_t* key_idx, const uint8_t* msgs,
                                          const uint64_t* msg_off, const rand_source& rs, uint8_t* partial, uint64_t* rhs_pre) {
+    scratch_scope scope(ctx->scratch, ctx->stream);
     uint8_t *d_sig, *d_idx, *d_m, *d_off, *d_rand, *d_seed;
-    if (int rc = stage_in(ctx, SL_H, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, msg_off[n], &d_m},
-                                      {msg_off, (n + 1) * 8, &d_off}, rs.rand_region(n, &d_rand), rs.seed_region(&d_seed)}))
+    if (int rc = stage_in(ctx, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, msg_off[n], &d_m},
+                                {msg_off, (n + 1) * 8, &d_off}, rs.rand_region(n, &d_rand), rs.seed_region(&d_seed)}))
         return rc;
     if (int rc = rand_generate(ctx, n, rs, d_seed, d_rand)) return rc;
     return batch_partial_registered(ctx, ks, k, n, d_sig, (uint32_t*)d_idx, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre);
@@ -2389,12 +2358,9 @@ static int verify_batch_registered_host(schnorr_b200_ctx* ctx, const schnorr_b20
                                                  msgs ? msgs + msg_off[s.lo] : nullptr, off, rs.from(s.lo), partial, nullptr);
         });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    uint8_t* res = nullptr;
-    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
-            return batch_partial_registered_host(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, rs, partial, rhs_pre);
-        }, res))
-        return rc;
-    return read_result(ctx, res, verdict, lhs97, rhs97);
+    return batch_whole_host(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+        return batch_partial_registered_host(ctx, ks, 0, n, sigs81, key_idx, msgs, msg_off, rs, partial, rhs_pre);
+    }, verdict, lhs97, rhs97);
 }
 
 extern "C" {
@@ -2428,8 +2394,8 @@ int schnorr_b200_verify_batch_registered_dev(schnorr_b200_ctx* ctx, const schnor
     }, result216);
 }
 
-// localisation on the first device: the inputs staged in slot M, the items' key records gathered into slot N, then the
-// per-signature bisection of schnorr_b200_locate_invalid_dev (which uses neither slot)
+// localisation on the first device: the inputs staged, the items' key records gathered, then the per-signature bisection
+// of schnorr_b200_locate_invalid_dev
 int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
                                            const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
                                            const uint8_t* rand32, uint8_t* flags, uint64_t* n_bad) {
@@ -2443,11 +2409,11 @@ int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx* ctx, const schnorr_
     schnorr_b200_ctx* c = device_ctx(ctx, 0);
     const keyset_dev& kd = ks->devs[0];
     CUDA_TRY(c, cudaSetDevice(c->device));
+    scratch_scope scope(c->scratch, c->stream);
     uint8_t *d_sig, *d_idx, *d_m, *d_off, *d_rand, *d_flags, *d_pk, *d_inf;
-    if (int rc = stage_in(c, SL_M, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                                    {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}}))
+    if (int rc = stage_in(c, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                              {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}, {nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}}))
         return rc;
-    if (int rc = stage_in(c, SL_N, {{nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}})) return rc;
     k_keyset_gather<<<grid_for(n, 128), 128, 0, c->stream>>>(n, (uint32_t*)d_idx, ks->n_keys, kd.pk12, kd.pk_inf, (uint64_t*)d_pk,
                                                             d_inf);
     c->launches += 1;
@@ -2457,7 +2423,7 @@ int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx* ctx, const schnorr_
 }  // extern "C"
 
 // ---- batch verification over KeyedSignature records (src/signature.rs:237-271, src/batch.rs:31-130) -----------------
-// The front end writes, in slot N, the records verify_batch sees: the signature bytes and the decoded key -- key k's
+// The front end writes, in regions of the caller's scope, the records verify_batch sees: the signature bytes and the decoded key -- key k's
 // registered record where the key bytes are the encoding of a findable key k of `ks` (the same bytes decompression
 // gives) -- or, where the key does not decode, the record of an index outside a set, which makes the batch malformed.
 // With a set, idx holds each record's key index or KEYSET_MISS, and *miss the number of misses.
@@ -2468,8 +2434,8 @@ static int keyed_front_end(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks,
                            keyed_front* f) {
     cudaStream_t st = ctx->stream;
     uint8_t* ok;
-    if (int rc = stage_in(ctx, SL_N, {{nullptr, n * 96, &f->pk}, {nullptr, n, &f->inf}, {nullptr, n, &ok}, {nullptr, n * 81, &f->sig},
-                                      {nullptr, ks ? n * 4 : 0, &f->idx}, {nullptr, 4, &f->miss}}))
+    if (int rc = stage_in(ctx, {{nullptr, n * 96, &f->pk}, {nullptr, n, &f->inf}, {nullptr, n, &ok}, {nullptr, n * 81, &f->sig},
+                                {nullptr, ks ? n * 4 : 0, &f->idx}, {nullptr, 4, &f->miss}}))
         return rc;
     if (ks) {
         const keyset_dev& kd = ks->devs[k];
@@ -2492,6 +2458,7 @@ static int keyed_front_end(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks,
 static int batch_partial_keyed(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n, const uint8_t* keyed130,
                                const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32, uint8_t* partial192,
                                uint64_t* rhs_pre, bool read_misses) {
+    scratch_scope scope(ctx->scratch, ctx->stream);
     keyed_front f;
     if (int rc = keyed_front_end(ctx, ks, k, n, keyed130, &f)) return rc;
     if (!ks || !reg_batch_aggregates(ctx, ks, n))
@@ -2508,13 +2475,14 @@ static int batch_partial_keyed(schnorr_b200_ctx* ctx, const schnorr_b200_keyset*
     return batch_partial_impl(ctx, n, f.sig, f.pk, f.inf, msgs, msg_off, rand32, partial192, rhs_pre, &rb);
 }
 
-// host inputs (n > 0, offsets checked) -> staged in slot H -> one partial at `partial` (device memory of this context)
+// host inputs (n > 0, offsets checked) -> staged on the device -> one partial at `partial` (device memory of this context)
 static int batch_partial_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
                                     const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, const rand_source& rs,
                                     uint8_t* partial, uint64_t* rhs_pre) {
+    scratch_scope scope(ctx->scratch, ctx->stream);
     uint8_t *d_rec, *d_m, *d_off, *d_rand, *d_seed;
-    if (int rc = stage_in(ctx, SL_H, {{keyed130, n * 130, &d_rec}, {msgs, msg_off[n], &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                                      rs.rand_region(n, &d_rand), rs.seed_region(&d_seed)}))
+    if (int rc = stage_in(ctx, {{keyed130, n * 130, &d_rec}, {msgs, msg_off[n], &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                rs.rand_region(n, &d_rand), rs.seed_region(&d_seed)}))
         return rc;
     if (int rc = rand_generate(ctx, n, rs, d_seed, d_rand)) return rc;
     return batch_partial_keyed(ctx, ks, k, n, d_rec, d_m, (uint64_t*)d_off, d_rand, partial, rhs_pre, true);
@@ -2534,16 +2502,13 @@ static int verify_batch_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_key
                                             msgs ? msgs + msg_off[s.lo] : nullptr, off, rs.from(s.lo), partial, nullptr);
         });
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    uint8_t* res = nullptr;
-    if (int rc = batch_whole(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
-            return batch_partial_keyed_host(ctx, ks, 0, n, keyed130, msgs, msg_off, rs, partial, rhs_pre);
-        }, res))
-        return rc;
-    return read_result(ctx, res, verdict, lhs97, rhs97);
+    return batch_whole_host(ctx, n, [&](uint8_t* partial, uint64_t* rhs_pre) {
+        return batch_partial_keyed_host(ctx, ks, 0, n, keyed130, msgs, msg_off, rs, partial, rhs_pre);
+    }, verdict, lhs97, rhs97);
 }
 
-// localisation on the first device: the inputs staged in slot M, the front-end records in slot N, then the bisection of
-// schnorr_b200_locate_invalid_dev (which uses neither slot)
+// localisation on the first device: the inputs staged, the front-end records, then the bisection of
+// schnorr_b200_locate_invalid_dev
 static int locate_invalid_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
                                      const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32, uint8_t* flags,
                                      uint64_t* n_bad) {
@@ -2554,9 +2519,10 @@ static int locate_invalid_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_k
     if (mb && !msgs) return SCHNORR_B200_EARG;
     schnorr_b200_ctx* c = device_ctx(ctx, 0);
     CUDA_TRY(c, cudaSetDevice(c->device));
+    scratch_scope scope(c->scratch, c->stream);
     uint8_t *d_rec, *d_m, *d_off, *d_rand, *d_flags;
-    if (int rc = stage_in(c, SL_M, {{keyed130, n * 130, &d_rec}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                                    {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}}))
+    if (int rc = stage_in(c, {{keyed130, n * 130, &d_rec}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                              {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}}))
         return rc;
     keyed_front f;
     if (int rc = keyed_front_end(c, ks, 0, n, d_rec, &f)) {
@@ -2650,10 +2616,9 @@ int schnorr_b200_keygen(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sk32, ui
     if (!ctx || (n && (!sk32 || !pk96))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_sk, *d_pk, *d_inf;
-    if (int rc = stage_in(ctx, SL_D, sk32, n * 32, &d_sk)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, n * 96, &d_pk)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_I, n, &d_inf)) return rc;
+    if (int rc = stage_in(ctx, {{sk32, n * 32, &d_sk}, {nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}})) return rc;
     if (int rc = schnorr_b200_keygen_dev(ctx, n, (uint8_t*)d_sk, (uint8_t*)d_pk, (uint8_t*)d_inf)) return rc;
     CUDA_TRY(ctx, cudaMemsetAsync(d_sk, 0, n * 32, ctx->stream));  // the staging arena is reused: do not keep secret keys in it
     CUDA_TRY(ctx, cudaMemcpyAsync(pk96, d_pk, n * 96, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2684,16 +2649,12 @@ int schnorr_b200_sign_many(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sk32,
     CHECK_MSG_OFF(ctx, n, msg_off);
     size_t mb = msg_off[n];
     if (mb && !msgs) return SCHNORR_B200_EARG;
-    void *d_sk, *d_pk, *d_inf = nullptr, *d_m, *d_off, *d_nonce, *d_out;
-    if (int rc = stage_in(ctx, SL_D, sk32, n * 32, &d_sk)) return rc;
-    if (int rc = stage_in(ctx, SL_E, pk96, n * 96, &d_pk)) return rc;
-    if (int rc = stage_in(ctx, SL_F, msgs, mb, &d_m)) return rc;
-    if (int rc = stage_in(ctx, SL_G, msg_off, (n + 1) * 8, &d_off)) return rc;
-    if (pk_inf)
-        if (int rc = stage_in(ctx, SL_I, pk_inf, n, &d_inf)) return rc;
-    if (int rc = stage_in(ctx, SL_J, nonce32, n * 32, &d_nonce)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n * 81, &d_out)) return rc;
-    if (int rc = schnorr_b200_sign_many_dev(ctx, n, (uint8_t*)d_sk, (uint8_t*)d_pk, (uint8_t*)d_inf, (uint8_t*)d_m,
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    void *d_sk, *d_pk, *d_inf, *d_m, *d_off, *d_nonce, *d_out;
+    if (int rc = stage_in(ctx, {{sk32, n * 32, &d_sk}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
+                                {pk_inf, pk_inf ? n : 0, &d_inf}, {nonce32, n * 32, &d_nonce}, {nullptr, n * 81, &d_out}}))
+        return rc;
+    if (int rc = schnorr_b200_sign_many_dev(ctx, n, (uint8_t*)d_sk, (uint8_t*)d_pk, pk_inf ? (uint8_t*)d_inf : nullptr, (uint8_t*)d_m,
                                             (uint64_t*)d_off, (uint8_t*)d_nonce, (uint8_t*)d_out))
         return rc;
     CUDA_TRY(ctx, cudaMemsetAsync(d_sk, 0, n * 32, ctx->stream));      // secret keys and nonces do not stay in the
@@ -2709,10 +2670,9 @@ int schnorr_b200_derive_master_keys(schnorr_b200_ctx* ctx, size_t n, const uint8
     MULTI_DISPATCH(ctx, schnorr_b200_derive_master_keys(ctx->shards[0], n, seeds32, xsk64, ok));
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_in, *d_out, *d_ok;
-    if (int rc = stage_in(ctx, SL_D, seeds32, n * 32, &d_in)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, n * 64, &d_out)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_I, n, &d_ok)) return rc;
+    if (int rc = stage_in(ctx, {{seeds32, n * 32, &d_in}, {nullptr, n * 64, &d_out}, {nullptr, n, &d_ok}})) return rc;
     k_derive_master<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, (uint8_t*)d_in, (uint8_t*)d_out, (uint8_t*)d_ok);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
@@ -2729,12 +2689,12 @@ int schnorr_b200_derive_private_children(schnorr_b200_ctx* ctx, size_t n, const 
     MULTI_DISPATCH(ctx, schnorr_b200_derive_private_children(ctx->shards[0], n, parent_xsk64, indices, children_xsk64, ok));
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_par, *d_idx, *d_out, *d_ok;
-    if (int rc = ensure_scratch(ctx, SL_D, 128, &d_par)) return rc;          // [0,64) parent, [64,128) its public key bytes
+    // [0,64) parent, [64,128) its public key bytes
+    if (int rc = stage_in(ctx, {{nullptr, 128, &d_par}, {indices, n * 4, &d_idx}, {nullptr, n * 64, &d_out}, {nullptr, n, &d_ok}}))
+        return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(d_par, parent_xsk64, 64, cudaMemcpyHostToDevice, ctx->stream));
-    if (int rc = stage_in(ctx, SL_F, indices, n * 4, &d_idx)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, n * 64, &d_out)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_I, n, &d_ok)) return rc;
     uint8_t* d_pk49 = (uint8_t*)d_par + 64;
     k_parent_public<<<1, 32, 0, ctx->stream>>>((uint8_t*)d_par, ctx->gtab, d_pk49);
     k_derive_private<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, (uint8_t*)d_par, d_pk49, (uint32_t*)d_idx, (uint8_t*)d_out,
@@ -2754,13 +2714,13 @@ int schnorr_b200_derive_public_children(schnorr_b200_ctx* ctx, size_t n, const u
     MULTI_DISPATCH(ctx, schnorr_b200_derive_public_children(ctx->shards[0], n, parent_xpk81, indices, children_xpk81, ok));
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_par, *d_idx, *d_out, *d_ok;
     // parent record (81) | decompressed key (96) | identity flag (1) | decode flag (1), 16-byte aligned pieces
-    if (int rc = ensure_scratch(ctx, SL_D, 96 + 96 + 16 + 16, &d_par)) return rc;
+    if (int rc = stage_in(ctx, {{nullptr, 96 + 96 + 16 + 16, &d_par}, {indices, n * 4, &d_idx}, {nullptr, n * 81, &d_out},
+                                {nullptr, n, &d_ok}}))
+        return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync(d_par, parent_xpk81, 81, cudaMemcpyHostToDevice, ctx->stream));
-    if (int rc = stage_in(ctx, SL_F, indices, n * 4, &d_idx)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, n * 81, &d_out)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_I, n, &d_ok)) return rc;
     uint8_t *d_pk96 = (uint8_t*)d_par + 96, *d_inf = d_pk96 + 96, *d_dec = d_inf + 16;
     k_decompress<<<1, 128, 0, ctx->stream>>>(1, (uint8_t*)d_par, d_pk96, d_inf, d_dec);   // ExtendedPublicKey::from_bytes (:295-311)
     k_derive_public<<<grid_for(n, SIGN_THREADS), SIGN_THREADS, 0, ctx->stream>>>(n, (uint8_t*)d_par, d_pk96, d_inf, (uint32_t*)d_idx,
@@ -2786,11 +2746,9 @@ int schnorr_b200_decompress(schnorr_b200_ctx* ctx, size_t n, const uint8_t* in49
     if (!ctx || (n && (!in49 || !pk96 || !pk_inf || !ok))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_in, *d_pk, *d_inf, *d_ok;
-    if (int rc = stage_in(ctx, SL_D, in49, n * 49, &d_in)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_E, n * 96, &d_pk)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_I, n, &d_inf)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n, &d_ok)) return rc;
+    if (int rc = stage_in(ctx, {{in49, n * 49, &d_in}, {nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}, {nullptr, n, &d_ok}})) return rc;
     k_decompress<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, (uint8_t*)d_in, (uint8_t*)d_pk, (uint8_t*)d_inf,
                                                             (uint8_t*)d_ok);
     ctx->launches += 1;
@@ -2806,12 +2764,10 @@ int schnorr_b200_compress(schnorr_b200_ctx* ctx, size_t n, const uint8_t* pk96, 
     if (!ctx || (n && (!pk96 || !out49))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    void *d_pk, *d_inf = nullptr, *d_out;
-    if (int rc = stage_in(ctx, SL_E, pk96, n * 96, &d_pk)) return rc;
-    if (pk_inf)
-        if (int rc = stage_in(ctx, SL_I, pk_inf, n, &d_inf)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n * 49, &d_out)) return rc;
-    k_compress<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, (uint8_t*)d_pk, (uint8_t*)d_inf, (uint8_t*)d_out);
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    void *d_pk, *d_inf, *d_out;
+    if (int rc = stage_in(ctx, {{pk96, n * 96, &d_pk}, {pk_inf, pk_inf ? n : 0, &d_inf}, {nullptr, n * 49, &d_out}})) return rc;
+    k_compress<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, (uint8_t*)d_pk, pk_inf ? (uint8_t*)d_inf : nullptr, (uint8_t*)d_out);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaMemcpyAsync(out49, d_out, n * 49, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2825,10 +2781,9 @@ int schnorr_b200_debug_field_ops(schnorr_b200_ctx* ctx, size_t n, const uint64_t
     if (!ctx || (n && (!a6 || !b6 || !out48))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_a, *d_b, *d_o;
-    if (int rc = stage_in(ctx, SL_D, a6, n * 48, &d_a)) return rc;
-    if (int rc = stage_in(ctx, SL_E, b6, n * 48, &d_b)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n * 48 * 8, &d_o)) return rc;
+    if (int rc = stage_in(ctx, {{a6, n * 48, &d_a}, {b6, n * 48, &d_b}, {nullptr, n * 48 * 8, &d_o}})) return rc;
     k_debug_field<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, (uint64_t*)d_a, (uint64_t*)d_b, (uint64_t*)d_o);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
@@ -2842,10 +2797,9 @@ int schnorr_b200_debug_lazy_ops(schnorr_b200_ctx* ctx, size_t n, const uint64_t*
     if (!ctx || (n && (!a6 || !b6 || !out48))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_a, *d_b, *d_o;
-    if (int rc = stage_in(ctx, SL_D, a6, n * 48, &d_a)) return rc;
-    if (int rc = stage_in(ctx, SL_E, b6, n * 48, &d_b)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n * 48 * 8, &d_o)) return rc;
+    if (int rc = stage_in(ctx, {{a6, n * 48, &d_a}, {b6, n * 48, &d_b}, {nullptr, n * 48 * 8, &d_o}})) return rc;
     k_debug_lazy<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, (uint64_t*)d_a, (uint64_t*)d_b, (uint64_t*)d_o);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
@@ -2859,9 +2813,9 @@ int schnorr_b200_debug_fp_core(schnorr_b200_ctx* ctx, int op, size_t n, const ui
     if (!ctx || op < 0 || op >= SCHNORR_B200_FP_OP_COUNT || (n && (!in16 || !out16))) return SCHNORR_B200_EARG;
     if (n == 0) return SCHNORR_B200_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void *d_in, *d_o;
-    if (int rc = stage_in(ctx, SL_D, in16, n * 64, &d_in)) return rc;
-    if (int rc = ensure_scratch(ctx, SL_H, n * 64, &d_o)) return rc;
+    if (int rc = stage_in(ctx, {{in16, n * 64, &d_in}, {nullptr, n * 64, &d_o}})) return rc;
     k_debug_fp_core<<<grid_for(n, 128), 128, 0, ctx->stream>>>(op, n, (uint32_t*)d_in, (uint32_t*)d_o);
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
@@ -2875,8 +2829,9 @@ int schnorr_b200_imad_peak(schnorr_b200_ctx* ctx, int iters, double* wide_mul_pe
     MULTI_DISPATCH(ctx, schnorr_b200_imad_peak(ctx->shards[0], iters, wide_mul_per_s, elapsed_ms));
     if (!ctx || iters <= 0 || !wide_mul_per_s) return SCHNORR_B200_EARG;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
     void* sink;
-    if (int rc = ensure_scratch(ctx, SL_H, 64, &sink)) return rc;
+    if (int rc = stage_in(ctx, {{nullptr, 64, &sink}})) return rc;
     int blocks = ctx->sm_count * 8;
     cudaEvent_t a, b;
     CUDA_TRY(ctx, cudaEventCreate(&a));
