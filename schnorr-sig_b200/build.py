@@ -6,7 +6,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-SO = os.path.join(CSRC, "libschnorr_b200%s.so" % os.environ.get("SB_SO_SUFFIX", ""))
+SO = os.path.join(CSRC, "libschnorr_b200.so")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC",
               "-diag-suppress", "550"]
@@ -31,8 +31,7 @@ def build(force=False, verbose=False):
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):
         raise RuntimeError("nvcc not found: the CUDA library cannot be built (there is no CPU fallback)")
-    extra = os.environ.get("SB_NVCC_EXTRA", "").split()   # experiment knobs, e.g. -DSB_FP6_INLINE=1
-    cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-o", SO, os.path.join(CSRC, "schnorr_b200.cu")]
+    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", SO, os.path.join(CSRC, "schnorr_b200.cu")]
     subprocess.check_call(cmd)
     return SO
 

@@ -142,10 +142,8 @@ SB_DEV void fp6_cofactor_norm(const fp6* d, fp6* c, fp_t* n) {
 }
 // The slope of a chord / tangent up to its base-field denominator: L = num * (n / d), n = norm(d).  Cofactor and product
 // in ONE out-of-line function (the fused doubling and addition both end in this pair): the cofactor never leaves the
-// registers and one call with its argument marshalling is saved per point operation.  L not canonical.
-#ifndef SB_SLOPE_FUSED
-#define SB_SLOPE_FUSED 1
-#endif
+// registers and one call with its argument marshalling is saved per point operation (k_verify_fast 74.61 against
+// 75.38 ms with two calls, profiles/r2_variants.md, v17).  L not canonical.
 SB_DEV_NOINLINE fp6_cof fp6_slope_nc(fp6 num, fp6 d) {
     fp6_cof r = fp6_cofactor_norm_body(d);
     fp6 L;
@@ -154,23 +152,16 @@ SB_DEV_NOINLINE fp6_cof fp6_slope_nc(fp6 num, fp6 d) {
     return r;
 }
 
+// The scaling helpers are inlined into jf_add / jf_dbl: 50.2 against 50.65 ms out of line (profiles/r1_variants.md).
 // a * s for s in Fp (any 64-bit representative)
-#ifndef SB_SCALE_INLINE
-#define SB_SCALE_INLINE 1  // measured: inlining the two scaling helpers into jf_add / jf_dbl is 1 % faster
-#endif
-#if SB_SCALE_INLINE
-#define SB_SCALE_FN SB_DEV
-#else
-#define SB_SCALE_FN SB_DEV_NOINLINE
-#endif
-SB_SCALE_FN fp6 fp6_scale(fp6 a, fp_t s) {
+SB_DEV fp6 fp6_scale(fp6 a, fp_t s) {
     fp6 r;
 #pragma unroll
     for (int i = 0; i < 6; i++) r.c[i] = fp_mul(a.c[i], s);
     return r;
 }
 // a * s - b * t  (s, t any 64-bit representatives; a, b canonical)
-SB_SCALE_FN fp6 fp6_scale_diff(fp6 a, fp_t s, fp6 b, fp_t t) {
+SB_DEV fp6 fp6_scale_diff(fp6 a, fp_t s, fp6 b, fp_t t) {
     fp6 r;
 #pragma unroll
     for (int i = 0; i < 6; i++) {
@@ -184,8 +175,8 @@ SB_SCALE_FN fp6 fp6_scale_diff(fp6 a, fp_t s, fp6 b, fp_t t) {
 }
 
 // a * s - b * t with non-canonical coefficients (feeds a multiplication only)
-SB_SCALE_FN fp6 fp6_scale_diff_nc(fp6 a, fp_t s, fp6 nb, fp_t t) {  // nb = a representative of -b (p - b, or b itself
-    fp6 r;                                                          // when the caller wants a s + b t)
+SB_DEV fp6 fp6_scale_diff_nc(fp6 a, fp_t s, fp6 nb, fp_t t) {  // nb = a representative of -b (p - b, or b itself
+    fp6 r;                                                     // when the caller wants a s + b t)
 #pragma unroll
     for (int i = 0; i < 6; i++) {
         wide_acc w;
@@ -217,14 +208,9 @@ SB_DEV_NOINLINE bool jf_dbl(jf_pt* p) {
         fp_t w4 = fp_mul(fp_sqr_nc(fp_sqr_nc(w)), inv3);
         fp6 num = fp6_sqr_nc(X);
         num.c[0] = fp_add(num.c[0], w4);    // (a non-canonical minuend is fine, fp_sub)
-#if SB_SLOPE_FUSED
         fp6_cof sl = fp6_slope_nc(num, Y);
         fp6 L = sl.c;                       // slope = L / (m w)
         n = sl.n;
-#else
-        fp6_cofactor_norm(&Y, &c, &n);
-        fp6 L = fp6_mul_nc(num, c);
-#endif
         fp_t m = fp_mul(n, two_thirds);
         fp_t m2 = fp_sqr_nc(m), m3 = fp_mul_nc(m2, m);
         fp6 A = fp6_scale(X, m2);
@@ -282,14 +268,9 @@ SB_DEV_NOINLINE bool jf_add(jf_pt* acc, const jf_pt* src, uint8_t mode) {
 #pragma unroll
         for (int i = 0; i < 6; i++) nY2.c[i] = negate ? Y2.c[i] : FP_P - Y2.c[i];
         fp6 num = fp6_scale_diff_nc(Y1, w2c, nY2, w1c);
-#if SB_SLOPE_FUSED
         fp6_cof sl = fp6_slope_nc(num, d);
         fp6 L = sl.c;                                // slope = L / (n w1 w2)
         n = sl.n;
-#else
-        fp6_cofactor_norm(&d, &c, &n);
-        fp6 L = fp6_mul_nc(num, c);
-#endif
         fp_t n2 = fp_sqr_nc(n), n3 = fp_mul_nc(n2, n);
         fp6 A = fp6_scale(X1, fp_mul_nc(n2, w2s));   // n^2 U1 = x1 w3^2
         fp6 X3 = fp6_sqr_sub_scaled(L, A, X2, fp_mul_nc(n2, w1s));            // L^2 - x1 w3^2 - x2 w3^2
@@ -346,15 +327,9 @@ SB_DEV_NOINLINE bool jf_madd(jf_pt* acc, const jf_pt* t, bool neg) {
         num.c[i] = wide_reduce_nc(w);
     }
     fp_t n;
-#if SB_SLOPE_FUSED
     fp6_cof sl = fp6_slope_nc(num, d);
     fp6 L = sl.c;                                     // slope = L / (n w1)
     n = sl.n;
-#else
-    fp6 c;
-    fp6_cofactor_norm(&d, &c, &n);
-    fp6 L = fp6_mul_nc(num, c);
-#endif
     fp_t n2 = fp_sqr_nc(n), n3 = fp_mul_nc(n2, n);
     fp6 A = fp6_scale(X1, n2);                        // x1 w3^2
     fp6 X3 = fp6_sqr_sub_scaled(L, A, X2, fp_mul_nc(n2, w1s));
@@ -408,11 +383,6 @@ SB_DEV void jf_dbl_exact(jf_pt* acc) {
     if (jf_dbl(acc)) acc->w = 0;
 }
 
-// block barrier every (mask + 1) steps of the doubling chain
-#ifndef SB_CHAIN_SYNC_MASK
-#define SB_CHAIN_SYNC_MASK 0  // measured: every step 45.37 ms, every 4th 45.61 ms at 2^19
-#endif
-
 enum fast_result : int {
     FAST_TORSION_FREE = 0,      // [q]P == O, h*P + e*G computed
     FAST_NOT_TORSION_FREE = 1,  // [q]P != O
@@ -429,14 +399,12 @@ enum fast_result : int {
 // indexed by the constant digits of q -- warp-uniform, hence coalesced -- and stay in thread-local memory, as does the
 // bucket of magnitude 8 (one digit in sixteen; two blocks of 128 threads x 8 slots fill the SM's shared memory).
 // On FAST_TORSION_FREE / FAST_NOT_TORSION_FREE, *R is the result (never the identity: that is reported as exceptional).
-#ifndef SB_FAST_BH_SHARED
-#define SB_FAST_BH_SHARED 7
-#endif
-static constexpr int FAST_BH_SHARED = SB_FAST_BH_SHARED;
+// 7 shared buckets: 79.73 ms against 80.25 with 6 and 82.59 with 8 (profiles/r2_variants.md, v12).
+static constexpr int FAST_BH_SHARED = 7;
 SB_DEV int verify_core_fast(const fp6& px, const fp6& py, const scalar& h, const scalar& e,
                             const uint64_t* __restrict__ gtab, jf_pt* R, jf_pt* Dp, jf_pt* Bh, int bh_stride) {
-    jf_pt Bq[8], Bhl[FAST_BH_SHARED < 8 ? 8 - FAST_BH_SHARED : 1];
-#define SB_BH(b) ((b) < FAST_BH_SHARED ? Bh + (size_t)(b) * bh_stride : &Bhl[(b) - (FAST_BH_SHARED < 8 ? FAST_BH_SHARED : 7)])
+    jf_pt Bq[8], Bhl[8 - FAST_BH_SHARED];
+#define SB_BH(b) ((b) < FAST_BH_SHARED ? Bh + (size_t)(b) * bh_stride : &Bhl[(b) - FAST_BH_SHARED])
     int h_carry = 0;  // signed 4-bit digits of h are recoded on the fly (recode_signed_w4), least significant first
     scalar hs = h;    // shifted right by one nibble per window: a dynamically indexed h.l[j >> 5] would live in local memory
     uint32_t q_seen = 0, h_seen = 0;
@@ -451,7 +419,7 @@ SB_DEV int verify_core_fast(const fp6& px, const fp6& py, const scalar& h, const
     Dp->w = 1;
 #pragma unroll 1
     for (int j = 0; j < SB_CHAIN_STEPS; j++) {
-        if ((j & SB_CHAIN_SYNC_MASK) == 0) SB_PHASE_SYNC(1);
+        SB_PHASE_SYNC();  // every step: 77.45 against 77.80 ms every 4th (profiles/r2_variants.md, v14)
         int dq = SB_QWNAF(j);
         if (dq != 0) {  // warp-uniform
             int idx = (dq < 0 ? -dq : dq) >> 1;
@@ -494,7 +462,7 @@ SB_DEV int verify_core_fast(const fp6& px, const fp6& py, const scalar& h, const
     bool same_h = !eRh;
 #pragma unroll 1
     for (int b = 6; b >= 0; b--) {
-        SB_PHASE_SYNC(1);
+        SB_PHASE_SYNC();
         bool eb = !((q_seen >> b) & 1);
         exc |= jf_add<true>(Rq, &Bq[b], jf_add_mode(eRq, eb, false));
         eRq = eRq && eb;
@@ -534,7 +502,7 @@ SB_DEV int verify_core_fast(const fp6& px, const fp6& py, const scalar& h, const
         T.w = 1;
 #pragma unroll 1
         for (int i = 0; i < GTAB_WINDOWS; i++) {
-            if ((i & 3) == 0) SB_PHASE_SYNC(1);
+            if ((i & 3) == 0) SB_PHASE_SYNC();
             int raw = (int)sc_bits(e, GTAB_W * i, GTAB_W) + carry;
             bool neg = raw > (1 << (GTAB_W - 1));
             carry = neg ? 1 : 0;

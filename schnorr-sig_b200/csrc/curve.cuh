@@ -198,41 +198,22 @@ SB_DEV jac_pt fixed_base_mul(const scalar& k, const uint64_t* __restrict__ gtab)
 // (252 doublings instead of 2 x 254), each scalar in signed 4-bit windows d_i in [-8, 8]:
 //     B[|d_i|] += sign(d_i) * D_i        then        k*P = sum_{m=1..8} m * B[m]   (14 additions)
 // q's digits are constants (warp-uniform additions); h's digits are per thread.
-#if defined(__CUDACC__)
-__constant__ int8_t c_q_wnaf4[256];  // CHEETAH_Q_WNAF4, filled at context creation
-#endif
-// width of the NAF used for q in the subgroup check: 5 -> 8 buckets (44 + 14 additions),
-// 4 -> 4 buckets (53 + 6 additions, 576 B less local memory per thread)
-#ifndef SB_Q_NAF_W
-#define SB_Q_NAF_W 5  // measured: width 5 = 7.84 M/s, width 4 = 7.74 M/s (profiles/r1_variants.md)
-#endif
+// q is taken in its width-5 NAF, 8 buckets of odd multiples (44 + 14 additions): 7.84 against 7.74 M/s at width 4
+// (profiles/r1_variants.md).
+static constexpr int SB_Q_BUCKETS = 8;
 // Steps of the shared doubling chain D_j = 2^j P: the last 4-bit window of the challenge starts at bit 252, and the
 // generated width-5 digits of q end at bit 251 (tools/gen_params.py: fold_top), so D_253..D_255 are never needed.
-#if SB_Q_NAF_W == 5
 static constexpr int SB_CHAIN_STEPS = 253;
 static_assert(CHEETAH_Q_WNAF5_LEN <= SB_CHAIN_STEPS, "digits of q above the last challenge window");
-#else
-static constexpr int SB_CHAIN_STEPS = 256;
-#endif
-#if SB_Q_NAF_W == 5
-#define SB_QNAF(i) SB_QWNAF(i)
-#elif defined(__CUDACC__)
-#define SB_QNAF(i) c_q_wnaf4[i]
-#else
-#define SB_QNAF(i) CHEETAH_Q_WNAF4[i]
-#endif
-static constexpr int SB_Q_BUCKETS = 1 << (SB_Q_NAF_W - 2);
 
 // Keeping the warps of a block in the same phase of the loop lets them share instruction-cache lines
 // (the point routines are ~4k instructions, larger than the cache): a block barrier per point
-// operation.  Exited threads do not take part in barriers, divergent branches contain none.
-#ifndef SB_PHASE_SYNC_LEVEL
-#define SB_PHASE_SYNC_LEVEL 1  // measured on B200: +11 % on k_verify (profiles/r1_variants.md)
-#endif
+// operation, +11 % on k_verify (profiles/r1_variants.md).  Exited threads do not take part in barriers, divergent
+// branches contain none.
 #if defined(__CUDA_ARCH__)
-#define SB_PHASE_SYNC(level) do { if (SB_PHASE_SYNC_LEVEL >= (level)) __syncthreads(); } while (0)
+#define SB_PHASE_SYNC() __syncthreads()
 #else
-#define SB_PHASE_SYNC(level) do { } while (0)
+#define SB_PHASE_SYNC() do { } while (0)
 #endif
 
 // k < 2^255  ->  64 signed digits, k = sum d_i 16^i, |d_i| <= 8
@@ -285,9 +266,9 @@ SB_DEV bool torsion_check_and_mul(const jac_pt& P, const scalar& h, jac_pt* hP, 
     *Dp = P;
 #pragma unroll 1
     for (int j = 0; j < SB_CHAIN_STEPS; j++) {
-        if ((j & 3) == 0) SB_PHASE_SYNC(1);
+        if ((j & 3) == 0) SB_PHASE_SYNC();
         if (j != 0) jac_dbl_mem(Dp);
-        int dq = SB_QNAF(j);
+        int dq = SB_QWNAF(j);
         if (dq != 0) jac_add_mem(&Bq[(dq < 0 ? -dq : dq) >> 1], Dp, dq < 0);  // warp-uniform
         if ((j & 3) == 0) {
             int dh = hd[j >> 2];

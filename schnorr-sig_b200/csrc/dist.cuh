@@ -251,7 +251,7 @@ __device__ int dverify_core(unsigned mask, fp_t px, fp_t py, const scalar& h, co
     D = dpt{px, py, 1};
 #pragma unroll 1
     for (int j = 0; j < SB_CHAIN_STEPS; j++) {
-        if ((j & 3) == 0) SB_PHASE_SYNC(1);
+        if ((j & 3) == 0) SB_PHASE_SYNC();
         int dq = SB_QWNAF(j);
         if (dq != 0) {
             int idx = (dq < 0 ? -dq : dq) >> 1;
@@ -277,7 +277,7 @@ __device__ int dverify_core(unsigned mask, fp_t px, fp_t py, const scalar& h, co
     bool same_h = !eRh;
 #pragma unroll 1
     for (int b = 6; b >= 0; b--) {
-        SB_PHASE_SYNC(1);
+        SB_PHASE_SYNC();
         bool eb = !((q_seen >> b) & 1);
         exc |= djf_add(mask, &Rq, &Bq[b], jf_add_mode(eRq, eb, false), k, gbase);
         eRq = eRq && eb;
@@ -314,7 +314,7 @@ __device__ int dverify_core(unsigned mask, fp_t px, fp_t py, const scalar& h, co
     T.w = 1;
 #pragma unroll 1
     for (int i = 0; i < GTAB_WINDOWS; i++) {
-        if ((i & 3) == 0) SB_PHASE_SYNC(1);
+        if ((i & 3) == 0) SB_PHASE_SYNC();
         int raw = (int)sc_bits(e, GTAB_W * i, GTAB_W) + carry;
         bool neg = raw > (1 << (GTAB_W - 1));
         carry = neg ? 1 : 0;

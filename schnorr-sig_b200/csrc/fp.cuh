@@ -3,8 +3,10 @@
 // canonical, not Montgomery -- SURVEY.md App. A).
 //
 // Device code is written on 32-bit halves: every 32x32->64 product is one IMAD.WIDE on the
-// integer-multiply pipe; the special-form reduction (2^64 = 2^32-1, 2^96 = -1 mod p) is
-// multiplier-free and runs on the ALU pipe.  Sums of 64x64 products are kept in a lazy accumulator
+// integer-multiply pipe.  The special-form reduction (2^64 = 2^32-1, 2^96 = -1 mod p) folds x2 (2^32-1)
+// in ONE multiply-add (IMAD.WIDE with carry-out) and applies the two wrap corrections together: 13.75
+// against 13.10 M/s with an add/subtract fold (profiles/r2_variants.md, v15).
+// Sums of 64x64 products are kept in a lazy accumulator
 // made of an "even" part E (words at bit 0,32,64,96,128: lo*lo and hi*hi products, one carry chain)
 // and an "odd" part O (words at bit 32,64,96: the two cross products).  A 64x64 product therefore
 // costs 4 IMAD.WIDE + 3 carry adds, and a whole dot product is reduced once.
@@ -20,13 +22,6 @@
 #else
 #define SB_DEV static inline __attribute__((always_inline))
 #define SB_DEV_NOINLINE static __attribute__((noinline))
-#endif
-
-// SB_FOLD_WIDE = 1: the fold x2 * (2^32 - 1) of a reduction is ONE multiply-add (IMAD.WIDE with carry-out) and the
-// two wrap corrections (carry of the fold, borrow of the 2^96 term) are applied together -- 3 instructions less per
-// reduction than the add/subtract form (the kernels are bound by instruction count, profiles/r2_variants.md).
-#ifndef SB_FOLD_WIDE
-#define SB_FOLD_WIDE 1
 #endif
 
 namespace sb {
@@ -77,7 +72,6 @@ SB_DEV fp_t fp_dbl(fp_t a) { return fp_add(a, a); }
 SB_DEV fp_t fp_reduce96_nc(uint32_t x0, uint32_t x1, uint32_t x2) {
 #if defined(__CUDA_ARCH__)
     uint32_t t0, t1;
-#if SB_FOLD_WIDE
     asm("{\n\t"
         ".reg .u32 c;\n\t"
         "mad.lo.cc.u32 %0, %4, 0xffffffff, %2;\n\t"   // (x1:x0) + x2 * (2^32 - 1)
@@ -89,21 +83,6 @@ SB_DEV fp_t fp_reduce96_nc(uint32_t x0, uint32_t x1, uint32_t x2) {
         "}"
         : "=&r"(t0), "=&r"(t1)
         : "r"(x0), "r"(x1), "r"(x2));
-#else
-    asm("{\n\t"
-        ".reg .u32 m0, m1, c;\n\t"
-        "sub.cc.u32 m0, 0, %4;\n\t"       // (m1:m0) = x2 * (2^32 - 1)
-        "subc.u32 m1, %4, 0;\n\t"
-        "add.cc.u32 %0, %2, m0;\n\t"
-        "addc.cc.u32 %1, %3, m1;\n\t"
-        "addc.u32 c, 0, 0;\n\t"           // wrapped 2^64 == EPS
-        "sub.u32 c, 0, c;\n\t"
-        "add.cc.u32 %0, %0, c;\n\t"
-        "addc.u32 %1, %1, 0;\n\t"
-        "}"
-        : "=&r"(t0), "=&r"(t1)
-        : "r"(x0), "r"(x1), "r"(x2));
-#endif
     return ((uint64_t)t1 << 32) | t0;
 #else
     uint64_t t = ((uint64_t)x1 << 32) | x0;
@@ -135,7 +114,7 @@ SB_DEV fp_t fp_reduce96(uint32_t x0, uint32_t x1, uint32_t x2) { return fp_canon
 // x4 must be small (< 2^31): it only ever holds the carries of a dot product.
 template <bool CANON>
 SB_DEV fp_t fp_reduce160_t(uint32_t x0, uint32_t x1, uint32_t x2, uint32_t x3, uint32_t x4) {
-#if defined(__CUDA_ARCH__) && SB_FOLD_WIDE
+#if defined(__CUDA_ARCH__)
     // V = (x1:x0) + x2 (2^32 - 1) - (x4:x3) lies in (-2^40, 2^65 - 2^33): the subtraction may borrow (m = -1), the fold
     // may carry (c = 1); the net multiple k = c + m of 2^64 = EPS (mod p) is applied once -- (t + k EPS) cannot wrap
     // again (k = 1: t <= 2^64 - 2^33; k = -1: t >= 2^64 - 2^40).  Subtracting first lets the fold's carry-out land
@@ -159,19 +138,6 @@ SB_DEV fp_t fp_reduce160_t(uint32_t x0, uint32_t x1, uint32_t x2, uint32_t x3, u
         : "r"(x0), "r"(x1), "r"(x2), "r"(x3), "r"(x4));
     fp_t r = ((uint64_t)t1 << 32) | t0;
     return CANON ? fp_canon_sel(r) : r;
-#elif defined(__CUDA_ARCH__)
-    uint32_t t0, t1;
-    asm("{\n\t"
-        ".reg .u32 m;\n\t"
-        "sub.cc.u32 %0, %2, %4;\n\t"      // (x1:x0) - (x4:x3)
-        "subc.cc.u32 %1, %3, %5;\n\t"
-        "subc.u32 m, 0, 0;\n\t"           // all ones on borrow: borrowed 2^64 == EPS too much
-        "sub.cc.u32 %0, %0, m;\n\t"
-        "subc.u32 %1, %1, 0;\n\t"
-        "}"
-        : "=&r"(t0), "=&r"(t1)
-        : "r"(x0), "r"(x1), "r"(x3), "r"(x4));
-    return CANON ? fp_reduce96(t0, t1, x2) : fp_reduce96_nc(t0, t1, x2);
 #else
     uint64_t lo = ((uint64_t)x1 << 32) | x0;
     uint64_t sub = ((uint64_t)x4 << 32) | x3;
@@ -321,7 +287,7 @@ SB_DEV fp_t fp_mul_nc(fp_t a, fp_t b) {
 #if defined(__CUDA_ARCH__)
     uint32_t a0 = (uint32_t)a, a1 = (uint32_t)(a >> 32), b0 = (uint32_t)b, b1 = (uint32_t)(b >> 32), t0, t1;
     asm("{\n\t"
-        ".reg .u32 p0, p1, p2, p3, m, m0, m1, c;\n\t"
+        ".reg .u32 p0, p1, p2, p3, m, m0, c;\n\t"
         "mul.lo.u32 p0, %2, %4;\n\t"
         "mul.hi.u32 p1, %2, %4;\n\t"
         "mul.lo.u32 p2, %3, %5;\n\t"
@@ -332,7 +298,6 @@ SB_DEV fp_t fp_mul_nc(fp_t a, fp_t b) {
         "mad.lo.cc.u32 p1, %3, %4, p1;\n\t"
         "madc.hi.cc.u32 p2, %3, %4, p2;\n\t"
         "addc.u32 p3, p3, 0;\n\t"
-#if SB_FOLD_WIDE
         "sub.cc.u32 %0, p0, p3;\n\t"                  // (p1:p0) - p3                [2^96 == -1]
         "subc.cc.u32 %1, p1, 0;\n\t"
         "subc.u32 m, 0, 0;\n\t"
@@ -343,21 +308,6 @@ SB_DEV fp_t fp_mul_nc(fp_t a, fp_t b) {
         "sub.cc.u32 %0, %0, m0;\n\t"
         "subc.u32 %1, %1, c;\n\t"
         "add.u32 %1, %1, m0;\n\t"
-#else
-        "sub.cc.u32 %0, p0, p3;\n\t"      // (p1:p0) - p3          [2^96 == -1]
-        "subc.cc.u32 %1, p1, 0;\n\t"
-        "subc.u32 m, 0, 0;\n\t"
-        "sub.cc.u32 %0, %0, m;\n\t"
-        "subc.u32 %1, %1, 0;\n\t"
-        "sub.cc.u32 m0, 0, p2;\n\t"       // + p2 * (2^32 - 1)     [2^64 == 2^32 - 1]
-        "subc.u32 m1, p2, 0;\n\t"
-        "add.cc.u32 %0, %0, m0;\n\t"
-        "addc.cc.u32 %1, %1, m1;\n\t"
-        "addc.u32 c, 0, 0;\n\t"
-        "sub.u32 c, 0, c;\n\t"
-        "add.cc.u32 %0, %0, c;\n\t"
-        "addc.u32 %1, %1, 0;\n\t"
-#endif
         "}"
         : "=&r"(t0), "=&r"(t1)
         : "r"(a0), "r"(a1), "r"(b0), "r"(b1));
@@ -371,7 +321,7 @@ SB_DEV fp_t fp_sqr_nc(fp_t a) {
 #if defined(__CUDA_ARCH__)
     uint32_t a0 = (uint32_t)a, a1 = (uint32_t)(a >> 32), t0, t1;
     asm("{\n\t"
-        ".reg .u32 p0, p1, p2, p3, c0, c1, c2, m, m0, m1, c;\n\t"
+        ".reg .u32 p0, p1, p2, p3, c0, c1, c2, m, m0, c;\n\t"
         "mul.lo.u32 p0, %2, %2;\n\t"
         "mul.hi.u32 p1, %2, %2;\n\t"
         "mul.lo.u32 p2, %3, %3;\n\t"
@@ -384,7 +334,6 @@ SB_DEV fp_t fp_sqr_nc(fp_t a) {
         "add.cc.u32 p1, p1, c0;\n\t"
         "addc.cc.u32 p2, p2, c1;\n\t"
         "addc.u32 p3, p3, c2;\n\t"
-#if SB_FOLD_WIDE
         "sub.cc.u32 %0, p0, p3;\n\t"
         "subc.cc.u32 %1, p1, 0;\n\t"
         "subc.u32 m, 0, 0;\n\t"
@@ -395,21 +344,6 @@ SB_DEV fp_t fp_sqr_nc(fp_t a) {
         "sub.cc.u32 %0, %0, m0;\n\t"
         "subc.u32 %1, %1, c;\n\t"
         "add.u32 %1, %1, m0;\n\t"
-#else
-        "sub.cc.u32 %0, p0, p3;\n\t"
-        "subc.cc.u32 %1, p1, 0;\n\t"
-        "subc.u32 m, 0, 0;\n\t"
-        "sub.cc.u32 %0, %0, m;\n\t"
-        "subc.u32 %1, %1, 0;\n\t"
-        "sub.cc.u32 m0, 0, p2;\n\t"
-        "subc.u32 m1, p2, 0;\n\t"
-        "add.cc.u32 %0, %0, m0;\n\t"
-        "addc.cc.u32 %1, %1, m1;\n\t"
-        "addc.u32 c, 0, 0;\n\t"
-        "sub.u32 c, 0, c;\n\t"
-        "add.cc.u32 %0, %0, c;\n\t"
-        "addc.u32 %1, %1, 0;\n\t"
-#endif
         "}"
         : "=&r"(t0), "=&r"(t1)
         : "r"(a0), "r"(a1));
@@ -437,28 +371,17 @@ SB_DEV fp_t fp_mul7_nc(fp_t a) {
 #if defined(__CUDA_ARCH__)
     uint32_t a0 = (uint32_t)a, a1 = (uint32_t)(a >> 32), t0, t1;
     asm("{\n\t"
-        ".reg .u32 x1, x2, m0, m1, c;\n\t"
+        ".reg .u32 x1, x2, c;\n\t"
         "mul.lo.u32 %0, %2, 7;\n\t"
         "mul.hi.u32 x1, %2, 7;\n\t"
         "mad.lo.cc.u32 %1, %3, 7, x1;\n\t"
         "madc.hi.u32 x2, %3, 7, 0;\n\t"
-#if SB_FOLD_WIDE
         "mad.lo.cc.u32 %0, x2, 0xffffffff, %0;\n\t"   // + x2 * (2^32 - 1)
         "madc.hi.cc.u32 %1, x2, 0xffffffff, %1;\n\t"
         "addc.u32 c, 0, 0;\n\t"
         "sub.cc.u32 %0, %0, c;\n\t"
         "subc.u32 %1, %1, 0;\n\t"
         "add.u32 %1, %1, c;\n\t"
-#else
-        "sub.cc.u32 m0, 0, x2;\n\t"       // + x2 * (2^32 - 1)
-        "subc.u32 m1, x2, 0;\n\t"
-        "add.cc.u32 %0, %0, m0;\n\t"
-        "addc.cc.u32 %1, %1, m1;\n\t"
-        "addc.u32 c, 0, 0;\n\t"
-        "sub.u32 c, 0, c;\n\t"
-        "add.cc.u32 %0, %0, c;\n\t"
-        "addc.u32 %1, %1, 0;\n\t"
-#endif
         "}"
         : "=&r"(t0), "=&r"(t1)
         : "r"(a0), "r"(a1));

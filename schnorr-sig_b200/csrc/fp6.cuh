@@ -128,23 +128,8 @@ SB_DEV void fp6_mul_sub_scaled_body(fp6& r, const fp6& a, const fp6& b, const fp
     }
 }
 
-#ifndef SB_FP6_INLINE
-#define SB_FP6_INLINE 0
-#endif
-#if SB_FP6_INLINE
-SB_DEV fp6 fp6_mul(const fp6& a, const fp6& b) {
-    fp6 r;
-    fp6_mul_body<true>(r, a, b);
-    return r;
-}
-SB_DEV fp6 fp6_sqr(const fp6& a) {
-    fp6 r;
-    fp6_sqr_body(r, a);
-    return r;
-}
-#else
 // Out-of-line: one copy of the ~500-instruction bodies per kernel keeps the hot loops inside the
-// instruction cache.
+// instruction cache (inlined: 3.65 against 4.78 M/s, profiles/r1_variants.md, v2-D).
 SB_DEV_NOINLINE fp6 fp6_mul(fp6 a, fp6 b) {
     fp6 r;
     fp6_mul_body<true>(r, a, b);
@@ -155,7 +140,6 @@ SB_DEV_NOINLINE fp6 fp6_sqr(fp6 a) {
     fp6_sqr_body(r, a);
     return r;
 }
-#endif
 // (helpers with TWO call sites per kernel stay out of line: duplicating them costs what the calls save,
 // profiles/r2_variants.md)
 SB_DEV_NOINLINE fp6 fp6_mul_sub_scaled(fp6 a, fp6 b, fp6 c, fp_t s) {
@@ -170,29 +154,22 @@ SB_DEV_NOINLINE fp6 fp6_mul_nc(fp6 a, fp6 b) {
     return r;
 }
 // The three squaring forms below have ONE call site per kernel (the fused doubling / addition, the mixed addition of
-// the MSM): inlined there they cost no code and save the argument marshalling of a call (SB_SQR_INLINE, measured).
-#ifndef SB_SQR_INLINE
-#define SB_SQR_INLINE 1
-#endif
-#if SB_SQR_INLINE
-#define SB_SQR_FN SB_DEV
-#else
-#define SB_SQR_FN SB_DEV_NOINLINE
-#endif
+// the MSM): inlined there they cost no code and save the argument marshalling of a call (k_verify_fast 75.21
+// against 76.33 ms out of line, profiles/r2_variants.md, v16).
 // a^2 with non-canonical coefficients
-SB_SQR_FN fp6 fp6_sqr_nc(fp6 a) {
+SB_DEV fp6 fp6_sqr_nc(fp6 a) {
     fp6 r;
     fp6_sqr_body_t<0, false>(r, a, nullptr, nullptr, 0);
     return r;
 }
 // a^2 - 2 A
-SB_SQR_FN fp6 fp6_sqr_sub2(fp6 a, fp6 A) {
+SB_DEV fp6 fp6_sqr_sub2(fp6 a, fp6 A) {
     fp6 r;
     fp6_sqr_body_t<1>(r, a, &A, nullptr, 0);
     return r;
 }
 // a^2 - A - B s
-SB_SQR_FN fp6 fp6_sqr_sub_scaled(fp6 a, fp6 A, fp6 B, fp_t s) {
+SB_DEV fp6 fp6_sqr_sub_scaled(fp6 a, fp6 A, fp6 B, fp_t s) {
     fp6 r;
     fp6_sqr_body_t<2>(r, a, &A, &B, s);
     return r;

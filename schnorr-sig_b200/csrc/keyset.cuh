@@ -17,10 +17,7 @@ namespace sb {
 
 // Window width of the per-key tables: ktab[key][KT_WINDOWS][KT_ENTRIES], entry d of window i = d * 2^(KT_W i) * P.
 // 8 bits: 32 windows x 129 entries x 96 B = 396 KB per key (profiles/r3_registered.md: 7 / 8 / 10 measured).
-#ifndef SB_KT_W
-#define SB_KT_W 8
-#endif
-static constexpr int KT_W = SB_KT_W;
+static constexpr int KT_W = 8;
 static constexpr int KT_WINDOWS = 255 / KT_W + 1;  // challenges are reduced mod q < 2^255
 static_assert(KT_WINDOWS * KT_W > 255, "the top window of a challenge must not carry out");
 static constexpr int KT_ENTRIES = (1 << (KT_W - 1)) + 1;
@@ -99,7 +96,7 @@ SB_DEV void jf_table_accumulate(jf_pt* acc, bool& acc_empty, bool& exc, const sc
     T.w = 1;
 #pragma unroll 1
     for (int i = 0; i < WINDOWS; i++) {
-        if ((i & 3) == 0) SB_PHASE_SYNC(1);
+        if ((i & 3) == 0) SB_PHASE_SYNC();
         int raw = (int)sc_bits(k, W * i, W) + carry;
         bool neg = raw > (1 << (W - 1));
         carry = neg ? 1 : 0;

@@ -110,12 +110,7 @@ SB_DEV fp_t rescue_inv_sbox(fp_t x) {
 // forward S-box group and of the inverse S-box group, driven by rolled loops over the two half-rounds and the two
 // groups of six state elements.
 // state elements per S-box group (independent chains interleaved for ILP; smaller = less code)
-#ifndef SB_SBOX_LANES
-#define SB_SBOX_LANES 6
-#endif
-#ifndef SB_RESCUE_COMPACT
-#define SB_RESCUE_COMPACT 1
-#endif
+static constexpr int SBOX_LANES = 6;
 // `sync`: block barrier per half-round.  Warps that run the permutation in step share instruction-cache lines (same
 // effect as SB_PHASE_SYNC in the point loops); only legal when EVERY live thread of the block runs the same number of
 // permutations -- the kernels vote on that (block_hash_vote, schnorr_b200.cu) and pass false otherwise; threads without work
@@ -126,35 +121,22 @@ SB_DEV fp_t rescue_inv_sbox(fp_t x) {
 #define SB_HASH_SYNC(flag) do { (void)(flag); } while (0)
 #endif
 SB_DEV_NOINLINE void rescue_permutation(fp_t* s, bool sync = false) {
-#if SB_RESCUE_COMPACT
 #pragma unroll 1
     for (int hr = 0; hr < 2 * RESCUE_ROUNDS; hr++) {
         SB_HASH_SYNC(sync);
         if ((hr & 1) == 0) {
 #pragma unroll 1
-            for (int g = 0; g < 12; g += SB_SBOX_LANES) {
+            for (int g = 0; g < 12; g += SBOX_LANES) {
 #pragma unroll
-                for (int i = 0; i < SB_SBOX_LANES; i++) s[g + i] = rescue_sbox(s[g + i]);
+                for (int i = 0; i < SBOX_LANES; i++) s[g + i] = rescue_sbox(s[g + i]);
             }
         } else {
             // inverse S-box: 6 independent chains at a time (ILP), one rolled copy of the code for both halves
 #pragma unroll 1
-            for (int g = 0; g < 12; g += SB_SBOX_LANES) rescue_inv_sbox_lanes<SB_SBOX_LANES>(s + g);
+            for (int g = 0; g < 12; g += SBOX_LANES) rescue_inv_sbox_lanes<SBOX_LANES>(s + g);
         }
         rescue_mds_ark(s, hr);
     }
-#else
-#pragma unroll 1
-    for (int r = 0; r < RESCUE_ROUNDS; r++) {
-#pragma unroll
-        for (int i = 0; i < 12; i++) s[i] = rescue_sbox(s[i]);
-        rescue_mds_ark(s, 2 * r);
-        // inverse S-box: 6 independent chains at a time (ILP), one rolled copy of the code for both halves
-#pragma unroll 1
-        for (int g = 0; g < 12; g += 6) rescue_inv_sbox_lanes<6>(s + g);
-        rescue_mds_ark(s, 2 * r + 1);
-    }
-#endif
 }
 
 // Streaming sponge = RescueHash::hash_field: additive absorption into state[0..8], permutation per

@@ -1162,7 +1162,6 @@ int schnorr_b200_create(int device, schnorr_b200_ctx** out) {
     CREATE_TRY(cudaEventCreate(&ctx->ev_k1));
     CREATE_TRY(cudaMemcpyToSymbol(c_ark, RESCUE_ARK, sizeof(uint64_t) * 2 * RESCUE_ROUNDS * 12));
     CREATE_TRY(cudaMemcpyToSymbol(c_q_wnaf5, CHEETAH_Q_WNAF5, sizeof(CHEETAH_Q_WNAF5)));  // the tail of the symbol stays zero
-    CREATE_TRY(cudaMemcpyToSymbol(c_q_wnaf4, CHEETAH_Q_WNAF4, 256));
     CREATE_TRY(cudaMalloc(&ctx->gtab, GTAB_U64 * sizeof(uint64_t)));
     CREATE_TRY(cudaMalloc(&ctx->exact_counters, schnorr_b200_ctx::MAX_CHUNKS * sizeof(uint32_t)));
     jac_pt* bases = nullptr;  // the GTAB_WINDOWS bases, then G itself (12 limbs)

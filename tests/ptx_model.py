@@ -2,7 +2,7 @@
 
 The host build of fp.cuh replaces every asm block with a portable fallback, so the CPU suite never runs the
 instruction sequences the kernels run.  This module preprocesses fp.cuh as the device compiler sees it
-(`__CUDA_ARCH__` defined, `SB_FOLD_WIDE` = 1 or 0), extracts every `asm(...)` block with the function around it,
+(`__CUDA_ARCH__` defined), extracts every `asm(...)` block with the function around it,
 and interprets the instructions on 32-bit words with one carry flag (CC.CF; a borrow for sub/subc).  Operands are
 bound by the C expressions of the constraint lists, not by position, so a block that passes a subset of its
 function's words is modelled correctly.  `FpCore` mirrors the C around the asm blocks, so it predicts the exact words
@@ -31,11 +31,10 @@ class ModelError(Exception):
 
 
 @functools.lru_cache(maxsize=None)
-def device_source(fold_wide):
+def device_source():
     """fp.cuh as the device compiler sees it (namespace sb only)."""
-    out = subprocess.check_output(["g++", "-E", "-P", "-x", "c++", "-D__CUDACC__", "-D__CUDA_ARCH__=1000",
-                                   "-DSB_FOLD_WIDE=%d" % fold_wide, FP_CUH], text=True,
-                                  stderr=subprocess.DEVNULL)   # "#pragma once in main file"
+    out = subprocess.check_output(["g++", "-E", "-P", "-x", "c++", "-D__CUDACC__", "-D__CUDA_ARCH__=1000", FP_CUH],
+                                  text=True, stderr=subprocess.DEVNULL)   # "#pragma once in main file"
     return out[out.index("namespace sb"):]
 
 
@@ -204,9 +203,9 @@ class AsmBlock:
 
 
 @functools.lru_cache(maxsize=None)
-def asm_blocks(fold_wide):
+def asm_blocks():
     """{function name: [AsmBlock]} of the device form of fp.cuh."""
-    src = device_source(fold_wide)
+    src = device_source()
     heads = [(m.start(), m.group(1)) for m in re.finditer(r"\b(?:fp_t|void)\s+(\w+)\s*\(", src)]
     blocks = {}
     for m in re.finditer(r"\basm\s*\(", src):
@@ -220,8 +219,8 @@ def asm_blocks(fold_wide):
     return blocks
 
 
-def count_asm(fold_wide):
-    return len(re.findall(r"\basm\s*\(", device_source(fold_wide)))
+def count_asm():
+    return len(re.findall(r"\basm\s*\(", device_source()))
 
 
 def lo(x):
@@ -236,7 +235,7 @@ def join(w0, w1):
     return (w1 << 32) | w0
 
 
-# ---- the paths a reduction takes (the SB_FOLD_WIDE = 1 order of fp_reduce160_t) ------------------------------------
+# ---- the paths a reduction takes (the order of fp_reduce160_t) ----------------------------------------------------
 def reduce_path(x0, x1, x2, x3=0, x4=0):
     """(m, c, k, t) of the reduction of x0 + x1 2^32 + x2 2^64 + x3 2^96 + x4 2^128: m = 1 when (x1:x0) - (x4:x3)
     borrows, c = 1 when the fold + x2 (2^32 - 1) carries, k = c - m the multiple of EPS applied, t the 64-bit value
@@ -277,11 +276,10 @@ def wide_state(E, O):
 
 
 class FpCore:
-    """The device field core, instruction for instruction, for one value of SB_FOLD_WIDE."""
+    """The device field core, instruction for instruction."""
 
-    def __init__(self, fold_wide=1):
-        self.fold_wide = fold_wide
-        self.blocks = asm_blocks(fold_wide)
+    def __init__(self):
+        self.blocks = asm_blocks()
 
     def _asm(self, fn, env):
         (block,) = self.blocks[fn]
@@ -315,10 +313,8 @@ class FpCore:
     def fp_reduce160_t(self, canon, x0, x1, x2, x3, x4):
         env = {"x0": x0, "x1": x1, "x2": x2, "x3": x3, "x4": x4}
         r = self._asm("fp_reduce160_t", env)
-        if self.fold_wide:
-            v = join(r["t0"], r["t1"])
-            return self.fp_canon_sel(v) if canon else v
-        return (self.fp_reduce96 if canon else self.fp_reduce96_nc)(r["t0"], r["t1"], x2)
+        v = join(r["t0"], r["t1"])
+        return self.fp_canon_sel(v) if canon else v
 
     def fp_canon(self, x):
         return x - P if x >= P else x

@@ -18,10 +18,9 @@ def cases():
     return fc.cases()
 
 
-@pytest.mark.parametrize("fold_wide", [1, 0])
 @pytest.mark.parametrize("op", OPS)
-def test_model_matches_integers(op, fold_wide, cases):
-    core = pm.FpCore(fold_wide)
+def test_model_matches_integers(op, cases):
+    core = pm.FpCore()
     bad = []
     for args in cases[op]:
         err = fc.check(op, args, core.op(op, args))
@@ -75,11 +74,10 @@ def test_cases_reach_every_path(op, need, cases):
 def test_model_covers_every_asm_block():
     """Every asm block of the device form of fp.cuh is modelled; a new block (or a new instruction in one) fails
     here until ptx_model.py is extended."""
-    for fold_wide in (1, 0):
-        blocks = pm.asm_blocks(fold_wide)
-        assert sorted(blocks) == sorted(pm.MODELLED), fold_wide
-        assert all(len(v) == 1 for v in blocks.values())
-        assert pm.count_asm(fold_wide) == len(pm.MODELLED)
+    blocks = pm.asm_blocks()
+    assert sorted(blocks) == sorted(pm.MODELLED)
+    assert all(len(v) == 1 for v in blocks.values())
+    assert pm.count_asm() == len(pm.MODELLED)
 
 
 def test_model_rejects_what_it_does_not_know():

@@ -3,8 +3,6 @@ inputs built to reach each carry and borrow path of its reductions (tests/fp_cor
 integers and, bit for bit, against the CPU model of the PTX (tests/ptx_model.py).  The model comparison pins the
 exact non-canonical representatives and accumulator states, and ties the model's reading of the PTX to the
 hardware: a wrong assumption about an instruction, or a miscompile, shows up as a mismatch."""
-import os
-
 import numpy as np
 import pytest
 
@@ -13,9 +11,6 @@ import ptx_model as pm
 from ptx_model import M64, P
 
 pytestmark = pytest.mark.gpu
-
-# the library is built with SB_FOLD_WIDE = 1 unless the build's extra flags say otherwise (build.py)
-FOLD_WIDE = 0 if "-DSB_FOLD_WIDE=0" in os.environ.get("SB_NVCC_EXTRA", "") else 1
 
 
 @pytest.fixture(scope="module")
@@ -36,7 +31,7 @@ def run(eng, op, items):
 
 @pytest.mark.parametrize("op", fc.OPS)
 def test_device_matches_integers_and_model(eng, cases, op):
-    core = pm.FpCore(FOLD_WIDE)
+    core = pm.FpCore()
     items = cases[op]
     wrong, differ = [], []
     for args, got in zip(items, run(eng, op, items)):

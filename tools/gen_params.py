@@ -100,8 +100,6 @@ def main():
     q_wnaf5 = fold_top(wnaf(Q, 5), 5, 251)
     assert sum(d << i for i, d in enumerate(q_wnaf5)) == Q and len(q_wnaf5) == 252
     assert all(d == 0 or (d & 1 and abs(d) < 16) for d in q_wnaf5) and sum(1 for d in q_wnaf5 if d) == 44
-    q_wnaf4 = wnaf(Q, 4)
-    assert sum(d << i for i, d in enumerate(q_wnaf4)) == Q and len(q_wnaf4) == 256
 
     params = {
         "_about": "constants of the Cheetah/Rescue Schnorr path with provenance tags; see tools/gen_params.py",
@@ -185,8 +183,6 @@ def main():
     h.append("/* width-5 NAF of q, least-significant digit first (uniform addition chain of the subgroup check) */\n")
     h.append("#define CHEETAH_Q_WNAF5_LEN %d\n" % len(q_wnaf5))
     h.append(arr8("CHEETAH_Q_WNAF5", q_wnaf5 + [0] * (256 - len(q_wnaf5))))   # zero-padded: the chain loops index up to 255
-    h.append("/* width-4 NAF of q (digits +-1,3,5,7), least-significant digit first */\n")
-    h.append(arr8("CHEETAH_Q_WNAF4", q_wnaf4))
     h.append("/* Frobenius: (u^i)^p = FP6_FROB[i] * u^i */\n")
     h.append(arr64("FP6_FROB", frob6))
     # Brace initialisers for constants that the device code keeps in __constant__ memory / constexpr tables: the kernels
