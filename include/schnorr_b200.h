@@ -467,6 +467,17 @@ enum {
 };
 int schnorr_b200_debug_fp_core(schnorr_b200_ctx *ctx, int op, size_t n, const uint32_t *in16, uint32_t *out16);
 
+/* Test hook (no reference counterpart): the point stage of Signature::verify (src/signature.rs:181-205) on a GIVEN
+ * challenge, so that exceptional group elements can be placed in chosen stages of one core.  n items of pk96 (affine
+ * x || y, not the identity), h32 and e32 (little-endian scalars below q), all n x ... host arrays.  CORE_EXACT runs the
+ * complete Jacobian routine (torsion_check_and_mul + fixed_base_accumulate), CORE_FAST the per-thread (X, Y, w) core of
+ * k_verify_fast (verify_core_fast), CORE_DIST its six-lane form of k_verify_dist (dverify_core).  result[i] = 0 when
+ * [q]P == O, 1 when not, 2 when the core met an exceptional case (never for CORE_EXACT); r97[i] = affine x || y of
+ * h*P + e*G and a byte 1 for the identity (meaningful unless result[i] == 2).  A bad core returns SCHNORR_B200_EARG. */
+enum { SCHNORR_B200_CORE_EXACT = 0, SCHNORR_B200_CORE_FAST, SCHNORR_B200_CORE_DIST, SCHNORR_B200_CORE_COUNT };
+int schnorr_b200_debug_verify_core(schnorr_b200_ctx *ctx, int core, size_t n, const uint8_t *pk96, const uint8_t *h32,
+                                   const uint8_t *e32, uint8_t *result, uint8_t *r97);
+
 /* Integer-multiply roofline calibration: runs a register-resident chain of `iters` dependent-free
  * 32x32->64 multiply-adds per thread on a full grid and returns wide multiplies per second. */
 int schnorr_b200_imad_peak(schnorr_b200_ctx *ctx, int iters, double *wide_mul_per_s, double *elapsed_ms);

@@ -981,6 +981,89 @@ __global__ void __launch_bounds__(128) k_debug_fp_core(int op, size_t n, const u
     for (int k = 0; k < 16; k++) out16[i * 16 + k] = y[k];
 }
 
+// test hook for the point stage of one verification on a given challenge: n items of (pk96, h32, e32) through one core
+// (SCHNORR_B200_CORE_*), each returning the core's result (fast_result) and R = h*P + e*G as affine x || y || identity
+// flag (97 bytes).  FAST runs verify_core_fast in the shared-memory layout of k_verify_fast, with stand-in inputs (G, zero
+// scalars) for the threads past n so that every thread reaches the barriers; DIST runs dverify_core five items per warp.
+template <int CORE>
+__global__ void __launch_bounds__(VERIFY_THREADS) k_debug_verify_core(size_t n, const uint8_t* __restrict__ pk96,
+                                                                      const uint8_t* __restrict__ h32,
+                                                                      const uint8_t* __restrict__ e32,
+                                                                      const uint64_t* __restrict__ gtab,
+                                                                      uint8_t* __restrict__ result, uint8_t* __restrict__ r97) {
+    extern __shared__ __align__(16) unsigned char s_core[];
+    size_t i;
+    int k = 0, gbase = 0;
+    if constexpr (CORE == SCHNORR_B200_CORE_DIST) {
+        int lane = threadIdx.x & 31, g = lane / 6;
+        if (g >= 5) return;
+        k = lane % 6;
+        gbase = 6 * g;
+        i = ((size_t)blockIdx.x * (VERIFY_THREADS / 32) + (threadIdx.x >> 5)) * 5 + g;
+        if (i >= n) return;
+    } else {
+        i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+        if (CORE == SCHNORR_B200_CORE_EXACT && i >= n) return;
+    }
+    bool live = i < n;
+    fp6 px, py;
+    scalar h = sc_zero(), e = sc_zero();
+    if (live) {
+        const uint64_t* p = reinterpret_cast<const uint64_t*>(pk96 + i * 96);
+        for (int c = 0; c < 6; c++) {
+            px.c[c] = p[c];
+            py.c[c] = p[6 + c];
+        }
+        h = sc_from_u64x4(load_u64_le(h32 + 32 * i), load_u64_le(h32 + 32 * i + 8), load_u64_le(h32 + 32 * i + 16),
+                          load_u64_le(h32 + 32 * i + 24));
+        e = sc_from_u64x4(load_u64_le(e32 + 32 * i), load_u64_le(e32 + 32 * i + 8), load_u64_le(e32 + 32 * i + 16),
+                          load_u64_le(e32 + 32 * i + 24));
+    } else {  // 1 * G, the first entry of the fixed-base table
+        for (int c = 0; c < 6; c++) {
+            px.c[c] = gtab[GTAB_ENTRY_U64 + c];
+            py.c[c] = gtab[GTAB_ENTRY_U64 + 6 + c];
+        }
+    }
+    int fr;
+    fp6 x, y;
+    bool inf;
+    if constexpr (CORE == SCHNORR_B200_CORE_EXACT) {
+        __shared__ jac_pt s_d[VERIFY_THREADS];
+        jac_pt r;
+        fr = torsion_check_and_mul(jac_from_affine(px, py, false), h, &r, &s_d[threadIdx.x]) ? FAST_TORSION_FREE
+                                                                                               : FAST_NOT_TORSION_FREE;
+        fixed_base_accumulate(&r, e, gtab);
+        jac_to_affine(r, x, y, inf);
+    } else if constexpr (CORE == SCHNORR_B200_CORE_FAST) {
+        jf_pt* s_d = reinterpret_cast<jf_pt*>(s_core);
+        jf_pt r;
+        fr = verify_core_fast(px, py, h, e, gtab, &r, s_d + threadIdx.x, s_d + VERIFY_THREADS + threadIdx.x, VERIFY_THREADS);
+        fp_t wi = fp_inv(fp_canon(r.w)), wi2 = fp_sqr(wi);
+        x = fp6_scale(r.X, wi2);
+        y = fp6_scale(r.Y, fp_mul(wi2, wi));
+        inf = r.w == 0;
+    } else {
+        dpt r;
+        fr = dverify_core(0x3fu << gbase, px.c[k], py.c[k], h, e, gtab, &r, k, gbase);
+        fp_t wi = fp_inv(fp_canon(r.w)), wi2 = fp_sqr(wi);
+        fp_t xk = fp_mul(r.X, wi2), yk = fp_mul(r.Y, fp_mul(wi2, wi));
+        for (int c = 0; c < 6; c++) {
+            x.c[c] = __shfl_sync(0x3fu << gbase, xk, gbase + c);
+            y.c[c] = __shfl_sync(0x3fu << gbase, yk, gbase + c);
+        }
+        inf = r.w == 0;
+    }
+    if (!live || k != 0) return;
+    result[i] = (uint8_t)fr;
+    uint8_t* o = r97 + i * 97;
+    for (int c = 0; c < 6; c++)
+        for (int b = 0; b < 8; b++) {
+            o[8 * c + b] = (uint8_t)(x.c[c] >> (8 * b));
+            o[48 + 8 * c + b] = (uint8_t)(y.c[c] >> (8 * b));
+        }
+    o[96] = inf;
+}
+
 // ------------------------------------------------------------------------------------------------
 // K6: integer-multiply roofline calibration.  8 independent accumulator chains per thread of
 // 32x32+64 -> 64 multiply-adds (IMAD.WIDE.U32), no memory traffic.
@@ -2819,6 +2902,38 @@ int schnorr_b200_debug_fp_core(schnorr_b200_ctx* ctx, int op, size_t n, const ui
     ctx->launches += 1;
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaMemcpyAsync(out16, d_o, n * 64, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return SCHNORR_B200_OK;
+}
+
+int schnorr_b200_debug_verify_core(schnorr_b200_ctx* ctx, int core, size_t n, const uint8_t* pk96, const uint8_t* h32,
+                                   const uint8_t* e32, uint8_t* result, uint8_t* r97) {
+    MULTI_DISPATCH(ctx, schnorr_b200_debug_verify_core(ctx->shards[0], core, n, pk96, h32, e32, result, r97));
+    if (!ctx || core < 0 || core >= SCHNORR_B200_CORE_COUNT || (n && (!pk96 || !h32 || !e32 || !result || !r97)))
+        return SCHNORR_B200_EARG;
+    if (n == 0) return SCHNORR_B200_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    scratch_scope scope(ctx->scratch, ctx->stream);
+    void *d_pk, *d_h, *d_e, *d_res, *d_r;
+    if (int rc = stage_in(ctx, {{pk96, n * 96, &d_pk}, {h32, n * 32, &d_h}, {e32, n * 32, &d_e}, {nullptr, n, &d_res},
+                                {nullptr, n * 97, &d_r}}))
+        return rc;
+    const uint8_t *p = (uint8_t*)d_pk, *hh = (uint8_t*)d_h, *ee = (uint8_t*)d_e;
+    if (core == SCHNORR_B200_CORE_EXACT)
+        k_debug_verify_core<SCHNORR_B200_CORE_EXACT><<<grid_for(n, VERIFY_THREADS), VERIFY_THREADS, 0, ctx->stream>>>(
+            n, p, hh, ee, ctx->gtab, (uint8_t*)d_res, (uint8_t*)d_r);
+    else if (core == SCHNORR_B200_CORE_FAST) {
+        CUDA_TRY(ctx, cudaFuncSetAttribute(k_debug_verify_core<SCHNORR_B200_CORE_FAST>,
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VERIFY_FAST_SMEM));
+        k_debug_verify_core<SCHNORR_B200_CORE_FAST><<<grid_for(n, VERIFY_THREADS), VERIFY_THREADS, VERIFY_FAST_SMEM,
+                                                      ctx->stream>>>(n, p, hh, ee, ctx->gtab, (uint8_t*)d_res, (uint8_t*)d_r);
+    } else
+        k_debug_verify_core<SCHNORR_B200_CORE_DIST><<<grid_for(n, DIST_SIGS_PER_BLOCK), VERIFY_THREADS, 0, ctx->stream>>>(
+            n, p, hh, ee, ctx->gtab, (uint8_t*)d_res, (uint8_t*)d_r);
+    ctx->launches += 1;
+    CUDA_TRY(ctx, cudaGetLastError());
+    CUDA_TRY(ctx, cudaMemcpyAsync(result, d_res, n, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(r97, d_r, n * 97, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return SCHNORR_B200_OK;
 }

@@ -642,6 +642,24 @@ class Engine:
         self._check(self._L.schnorr_b200_debug_fp_core(self._h, code, in16.shape[0], _ptr(in16), _ptr(out)), "debug_fp_core")
         return out
 
+    # core numbers of debug_verify_core (enum SCHNORR_B200_CORE_* of include/schnorr_b200.h)
+    VERIFY_CORES = ("exact", "fast", "dist")
+
+    def debug_verify_core(self, core, pk96, h32, e32):
+        """Test hook: the point stage of n verifications on given challenges through one core ("exact", "fast" or
+        "dist", or its number) -> (result uint8[n]: 0 torsion free, 1 not, 2 exceptional; R uint8[n, 97]: affine x || y
+        of h*P + e*G || identity flag)."""
+        code = self.VERIFY_CORES.index(core) if isinstance(core, str) else int(core)
+        pk96, h32, e32 = _u8(pk96, 96), _u8(h32, 32), _u8(e32, 32)
+        n = pk96.shape[0]
+        if h32.shape[0] != n or e32.shape[0] != n:
+            raise ValueError("one challenge and one e per key")
+        res = np.full(n, 255, dtype=np.uint8)
+        r97 = np.zeros((n, 97), dtype=np.uint8)
+        self._check(self._L.schnorr_b200_debug_verify_core(self._h, code, n, _ptr(pk96), _ptr(h32), _ptr(e32), _ptr(res),
+                                                           _ptr(r97)), "debug_verify_core")
+        return res, r97
+
     def imad_peak(self, iters=1 << 16):
         w = C.c_double(0)
         ms = C.c_double(0)
