@@ -268,7 +268,11 @@ int schnorr_b200_batch_finish(schnorr_b200_ctx *ctx, size_t n_partials, const ui
  * Bisection over partial MSMs (a range whose own random linear combination holds is clean), exact per-item check on the
  * failing slices: only items inside a failing slice can be flagged, so items whose non-identity terms cancel within a
  * slice (two torsion-shifted R with odd randomisers: T2 + T2 = O) are not.  flags[i] = 0 clean, 2 bad, 3 malformed (the reference panics on it); *n_bad (optional) = number of
- * non-zero flags.  rand32 as in verify_batch. */
+ * non-zero flags.  rand32 as in verify_batch.
+ * The slices are defined by n alone, so the flags and *n_bad do not depend on the device count: the host forms of this
+ * and of the three localisations below spread a multi-device context's work over up to 8 of its devices (one per 4096
+ * signatures), each holding only its own contiguous range of the batch, and return the bytes of a single-device
+ * context.  The _dev form (device buffers) needs a single-device context. */
 int schnorr_b200_locate_invalid(schnorr_b200_ctx *ctx, size_t n, const uint8_t *sigs81, const uint8_t *pk96,
                                 const uint8_t *pk_inf, const uint8_t *msgs, const uint64_t *msg_off,
                                 const uint8_t *rand32, uint8_t *flags, uint64_t *n_bad);
@@ -297,7 +301,8 @@ int schnorr_b200_verify_batch_registered_dev(schnorr_b200_ctx *ctx, const schnor
                                              const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
                                              const uint64_t *msg_off, const uint8_t *rand32, uint8_t *result216);
 /* locate_invalid (above) against a registered key set: the flags and *n_bad of locate_invalid on the gathered key
- * records; an index outside the set gets flag 3.  Runs on the first device.           src/batch.rs:102-129 */
+ * records; an index outside the set gets flag 3.  Each device gathers the records of its own range from its copy of
+ * the set; the flags do not depend on the device count.                          src/batch.rs:102-129 */
 int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
                                            const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
                                            const uint64_t *msg_off, const uint8_t *rand32, uint8_t *flags,
@@ -331,8 +336,9 @@ int schnorr_b200_verify_batch_keyed_registered_dev(schnorr_b200_ctx *ctx, const 
                                                    const uint8_t *keyed130, const uint8_t *msgs, const uint64_t *msg_off,
                                                    const uint8_t *rand32, uint8_t *result216);
 /* locate_invalid (above) over keyed records, without and with a registered key set: the flags and *n_bad of
- * locate_invalid on the front-end records of verify_batch_keyed; a record whose key does not decode gets flag 3.  Run on
- * the first device.                                  src/signature.rs:237-271, src/batch.rs:31-130 */
+ * locate_invalid on the front-end records of verify_batch_keyed; a record whose key does not decode gets flag 3.  Each
+ * device builds the records of its own range; the flags do not depend on the device count.
+ *                                                    src/signature.rs:237-271, src/batch.rs:31-130 */
 int schnorr_b200_locate_invalid_keyed(schnorr_b200_ctx *ctx, size_t n, const uint8_t *keyed130, const uint8_t *msgs,
                                       const uint64_t *msg_off, const uint8_t *rand32, uint8_t *flags, uint64_t *n_bad);
 int schnorr_b200_locate_invalid_keyed_registered(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
@@ -350,7 +356,8 @@ int schnorr_b200_locate_invalid_keyed_registered(schnorr_b200_ctx *ctx, const sc
  * batch_randomizers writes randomisers first_index ... first_index + n - 1 to rand32 (n x 32 B).  EARG for a NULL seed
  * and when the last index, first_index + n - 1, does not fit in a u64.  The host form's bytes do not depend on the
  * device count of the context; the _dev form (seed32 and rand32 on the device, no synchronisation) needs a single-device
- * context.  The randomisers of a failed seeded batch, batch_randomizers(seed32, 0, n), feed locate_invalid*. */
+ * context.  The randomisers of a failed seeded batch are batch_randomizers(seed32, 0, n); the seeded localisations below
+ * generate them on the devices. */
 int schnorr_b200_batch_randomizers(schnorr_b200_ctx *ctx, size_t n, const uint8_t *seed32, uint64_t first_index,
                                    uint8_t *rand32);
 int schnorr_b200_batch_randomizers_dev(schnorr_b200_ctx *ctx, size_t n, const uint8_t *seed32, uint64_t first_index,
@@ -374,6 +381,24 @@ int schnorr_b200_verify_batch_keyed_registered_seeded(schnorr_b200_ctx *ctx, con
                                                       const uint8_t *keyed130, const uint8_t *msgs,
                                                       const uint64_t *msg_off, const uint8_t *seed32, int *verdict,
                                                       uint8_t *lhs97, uint8_t *rhs97);
+/* Seeded host forms of the four localisations: the arguments of the parent entry point with a 32-byte seed in place of
+ * rand32.  flags and *n_bad are, byte for byte, the parent's given rand32 = batch_randomizers(seed32, 0, n); each device
+ * generates the randomisers of its own range, so a call sends 32 bytes of randomness instead of 32 per signature.  EARG
+ * for a NULL seed. */
+int schnorr_b200_locate_invalid_seeded(schnorr_b200_ctx *ctx, size_t n, const uint8_t *sigs81, const uint8_t *pk96,
+                                       const uint8_t *pk_inf, const uint8_t *msgs, const uint64_t *msg_off,
+                                       const uint8_t *seed32, uint8_t *flags, uint64_t *n_bad);
+int schnorr_b200_locate_invalid_registered_seeded(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                                  const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
+                                                  const uint64_t *msg_off, const uint8_t *seed32, uint8_t *flags,
+                                                  uint64_t *n_bad);
+int schnorr_b200_locate_invalid_keyed_seeded(schnorr_b200_ctx *ctx, size_t n, const uint8_t *keyed130, const uint8_t *msgs,
+                                             const uint64_t *msg_off, const uint8_t *seed32, uint8_t *flags,
+                                             uint64_t *n_bad);
+int schnorr_b200_locate_invalid_keyed_registered_seeded(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
+                                                        const uint8_t *keyed130, const uint8_t *msgs,
+                                                        const uint64_t *msg_off, const uint8_t *seed32, uint8_t *flags,
+                                                        uint64_t *n_bad);
 
 /* MSM points of the last batch verification on this context (all devices of a multi-device context): 2n for
  * verify_batch, n for a registered batch summed per key, 0 for the block-per-signature form of small batches; for

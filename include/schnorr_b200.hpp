@@ -226,8 +226,9 @@ public:
     std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                              const std::vector<std::vector<uint8_t>>& messages,
                                              const std::function<void(uint8_t*, size_t)>& rng) const;
-    // the same four with the randomisers generated on the device from a 32-byte seed (schnorr_b200_batch_randomizers):
-    // the seed must be fresh from a CSPRNG for every batch and unknown to the signers until the verdict
+    // the same four with the randomisers generated on the devices from a 32-byte seed (schnorr_b200_batch_randomizers;
+    // schnorr_b200_verify_batch_registered_seeded ... schnorr_b200_locate_invalid_keyed_registered_seeded): the seed must
+    // be fresh from a CSPRNG for every batch and unknown to the signers until the verdict
     Result verify_batch(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                         const std::vector<std::vector<uint8_t>>& messages, const std::array<uint8_t, 32>& seed) const;
     std::vector<size_t> locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
@@ -268,7 +269,7 @@ private:
     BatchInputs batch_records(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                               const std::vector<std::vector<uint8_t>>& messages) const;
     Result registered_verdict(const BatchInputs& in, const uint8_t* seed) const;
-    std::vector<size_t> registered_located(const BatchInputs& in) const;
+    std::vector<size_t> registered_located(const BatchInputs& in, const uint8_t* seed) const;
     Engine& eng_;
     schnorr_b200_keyset* ks_ = nullptr;
     std::vector<uint8_t> status_;
@@ -354,8 +355,7 @@ inline Result verify_batch(const std::vector<Signature>& signatures, const std::
     return result_from_verdict(verdict);
 }
 
-// the randomisers 0 ... n - 1 of a seed, as the seeded entry points generate them (schnorr_b200_batch_randomizers): the
-// rand32 that localises a failed seeded batch
+// the randomisers 0 ... n - 1 of a seed, as the seeded entry points generate them (schnorr_b200_batch_randomizers)
 inline std::vector<uint8_t> batch_randomizers(Engine& eng, size_t n, const std::array<uint8_t, 32>& seed) {
     std::vector<uint8_t> rand(n * 32);
     eng.check(schnorr_b200_batch_randomizers(eng.get(), n, seed.data(), 0, rand.data()), "batch_randomizers");
@@ -420,24 +420,28 @@ inline Result KeySet::verify_batch(const std::vector<size_t>& indices, const std
 
 inline std::vector<size_t> KeySet::locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                                                   const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
-    return registered_located(batch_inputs(indices, signatures, messages, rng));
+    return registered_located(batch_inputs(indices, signatures, messages, rng), nullptr);
 }
 
 inline std::vector<size_t> KeySet::locate_invalid(const std::vector<size_t>& indices, const std::vector<Signature>& signatures,
                                                   const std::vector<std::vector<uint8_t>>& messages,
                                                   const std::array<uint8_t, 32>& seed) const {
-    BatchInputs in = batch_records(indices, signatures, messages);
-    in.rand = batch_randomizers(eng_, in.idx.size(), seed);
-    return registered_located(in);
+    return registered_located(batch_records(indices, signatures, messages), seed.data());
 }
 
-inline std::vector<size_t> KeySet::registered_located(const BatchInputs& in) const {
+// the culprits of a registered batch: randomisers from in.rand, or generated on the devices from `seed` when it is not null
+inline std::vector<size_t> KeySet::registered_located(const BatchInputs& in, const uint8_t* seed) const {
     size_t n = in.idx.size();
     std::vector<uint8_t> flags(n, 0);
-    eng_.check(schnorr_b200_locate_invalid_registered(eng_.get(), ks_, n, in.sigs.data(), in.idx.data(),
-                                                      in.blob.empty() ? nullptr : in.blob.data(), in.off.data(),
-                                                      in.rand.data(), flags.data(), nullptr),
-               "locate_invalid_registered");
+    const uint8_t* msgs = in.blob.empty() ? nullptr : in.blob.data();
+    if (seed)
+        eng_.check(schnorr_b200_locate_invalid_registered_seeded(eng_.get(), ks_, n, in.sigs.data(), in.idx.data(), msgs,
+                                                                 in.off.data(), seed, flags.data(), nullptr),
+                   "locate_invalid_registered_seeded");
+    else
+        eng_.check(schnorr_b200_locate_invalid_registered(eng_.get(), ks_, n, in.sigs.data(), in.idx.data(), msgs,
+                                                          in.off.data(), in.rand.data(), flags.data(), nullptr),
+                   "locate_invalid_registered");
     std::vector<size_t> bad;
     for (size_t i = 0; i < n; i++) {
         if (flags[i] == 3) throw std::logic_error("called `Option::unwrap()` on a `None` value (non-canonical encoding)");
@@ -509,27 +513,29 @@ inline Result keyed_verdict(Engine& eng, const schnorr_b200_keyset* ks, const Ke
                   "verify_batch_keyed");
     return result_from_verdict(verdict);
 }
-// the culprits of locate_invalid_keyed (ks null) or of locate_invalid_keyed_registered on prepared records
-inline std::vector<size_t> keyed_culprits(Engine& eng, const schnorr_b200_keyset* ks, const KeyedBatchInputs& in) {
+// the culprits of locate_invalid_keyed (ks null) or of locate_invalid_keyed_registered on prepared records: randomisers
+// from in.rand, or generated on the devices from `seed` when it is not null
+inline std::vector<size_t> keyed_culprits(Engine& eng, const schnorr_b200_keyset* ks, const KeyedBatchInputs& in,
+                                          const uint8_t* seed) {
     std::vector<uint8_t> flags(in.n(), 0);
     const uint8_t* msgs = in.blob.empty() ? nullptr : in.blob.data();
-    if (ks)
+    if (ks && seed)
+        eng.check(schnorr_b200_locate_invalid_keyed_registered_seeded(eng.get(), ks, in.n(), in.recs.data(), msgs,
+                                                                      in.off.data(), seed, flags.data(), nullptr),
+                  "locate_invalid_keyed_registered_seeded");
+    else if (ks)
         eng.check(schnorr_b200_locate_invalid_keyed_registered(eng.get(), ks, in.n(), in.recs.data(), msgs, in.off.data(),
                                                                in.rand.data(), flags.data(), nullptr),
                   "locate_invalid_keyed_registered");
+    else if (seed)
+        eng.check(schnorr_b200_locate_invalid_keyed_seeded(eng.get(), in.n(), in.recs.data(), msgs, in.off.data(), seed,
+                                                           flags.data(), nullptr),
+                  "locate_invalid_keyed_seeded");
     else
         eng.check(schnorr_b200_locate_invalid_keyed(eng.get(), in.n(), in.recs.data(), msgs, in.off.data(), in.rand.data(),
                                                     flags.data(), nullptr),
                   "locate_invalid_keyed");
     return located(flags);
-}
-// keyed records with the randomisers 0 ... n - 1 of a seed: the inputs that localise a failed seeded batch
-inline KeyedBatchInputs keyed_seeded_inputs(Engine& eng, const std::vector<KeyedSignature>& keyed,
-                                            const std::vector<std::vector<uint8_t>>& messages,
-                                            const std::array<uint8_t, 32>& seed) {
-    KeyedBatchInputs in = keyed_batch_records(keyed, messages);
-    in.rand = batch_randomizers(eng, in.n(), seed);
-    return in;
 }
 
 // verify_batch([k.signature ...], [k.public_key ...], messages, rng) over KeyedSignature wire records, the keys decoded on
@@ -542,10 +548,10 @@ inline Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const
 // key or signature does not decode throws
 inline std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                                 const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) {
-    return keyed_culprits(Engine::instance(), nullptr, keyed_batch_inputs(keyed, messages, rng));
+    return keyed_culprits(Engine::instance(), nullptr, keyed_batch_inputs(keyed, messages, rng), nullptr);
 }
-// the same two with the randomisers generated on the device from a 32-byte seed (schnorr_b200_verify_batch_keyed_seeded,
-// schnorr_b200_batch_randomizers): the seed must be fresh from a CSPRNG for every batch and unknown to the signers until
+// the same two with the randomisers generated on the devices from a 32-byte seed (schnorr_b200_verify_batch_keyed_seeded,
+// schnorr_b200_locate_invalid_keyed_seeded): the seed must be fresh from a CSPRNG for every batch and unknown to the signers until
 // the verdict
 inline Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const std::vector<std::vector<uint8_t>>& messages,
                                  const std::array<uint8_t, 32>& seed) {
@@ -554,8 +560,7 @@ inline Result verify_batch_keyed(const std::vector<KeyedSignature>& keyed, const
 inline std::vector<size_t> locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                                 const std::vector<std::vector<uint8_t>>& messages,
                                                 const std::array<uint8_t, 32>& seed) {
-    Engine& eng = Engine::instance();
-    return keyed_culprits(eng, nullptr, keyed_seeded_inputs(eng, keyed, messages, seed));
+    return keyed_culprits(Engine::instance(), nullptr, keyed_batch_records(keyed, messages), seed.data());
 }
 inline Result KeySet::verify_batch_keyed(const std::vector<KeyedSignature>& keyed,
                                          const std::vector<std::vector<uint8_t>>& messages, const Rng& rng) const {
@@ -564,7 +569,7 @@ inline Result KeySet::verify_batch_keyed(const std::vector<KeyedSignature>& keye
 inline std::vector<size_t> KeySet::locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                                         const std::vector<std::vector<uint8_t>>& messages,
                                                         const Rng& rng) const {
-    return keyed_culprits(eng_, ks_, keyed_batch_inputs(keyed, messages, rng));
+    return keyed_culprits(eng_, ks_, keyed_batch_inputs(keyed, messages, rng), nullptr);
 }
 inline Result KeySet::verify_batch_keyed(const std::vector<KeyedSignature>& keyed,
                                          const std::vector<std::vector<uint8_t>>& messages,
@@ -574,7 +579,7 @@ inline Result KeySet::verify_batch_keyed(const std::vector<KeyedSignature>& keye
 inline std::vector<size_t> KeySet::locate_invalid_keyed(const std::vector<KeyedSignature>& keyed,
                                                         const std::vector<std::vector<uint8_t>>& messages,
                                                         const std::array<uint8_t, 32>& seed) const {
-    return keyed_culprits(eng_, ks_, keyed_seeded_inputs(eng_, keyed, messages, seed));
+    return keyed_culprits(eng_, ks_, keyed_batch_records(keyed, messages), seed.data());
 }
 
 }  // namespace schnorr_sig

@@ -59,14 +59,12 @@ pub fn verify_batch_seeded(signatures: &[Signature], public_keys: &[PublicKey], 
     }
 }
 
-/// `locate_invalid` with the randomisers of `verify_batch_seeded(.., seed)`: the culprits of that failed batch.
+/// `locate_invalid` with the randomisers of `verify_batch_seeded(.., seed)`, generated on the devices: the culprits of
+/// that failed batch.
 pub fn locate_invalid_seeded(signatures: &[Signature], public_keys: &[PublicKey], messages: &[&[u8]],
                              seed: &[u8; 32]) -> Vec<usize> {
     let (sigs, pks, infs) = records(signatures, public_keys);
-    let flags = ENGINE.with(|e| {
-        let rand = e.batch_randomizers(sigs.len(), seed, 0);
-        e.locate_invalid(&sigs, &pks, &infs, messages, &rand)
-    });
+    let flags = ENGINE.with(|e| e.locate_invalid_seeded(&sigs, &pks, &infs, messages, seed));
     assert!(flags.iter().all(|&f| f != 3), "called `Option::unwrap()` on a `None` value");
     flags.iter().enumerate().filter(|(_, &f)| f != 0).map(|(i, _)| i).collect()
 }

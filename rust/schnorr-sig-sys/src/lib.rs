@@ -61,6 +61,17 @@ extern "C" {
     pub fn schnorr_b200_verify_batch_keyed_registered_seeded(ctx: *mut schnorr_b200_ctx, ks: *const schnorr_b200_keyset,
         n: usize, keyed130: *const u8, msgs: *const u8, msg_off: *const u64, seed32: *const u8, verdict: *mut c_int,
         lhs97: *mut u8, rhs97: *mut u8) -> c_int;
+    pub fn schnorr_b200_locate_invalid_seeded(ctx: *mut schnorr_b200_ctx, n: usize, sigs81: *const u8, pk96: *const u8,
+        pk_inf: *const u8, msgs: *const u8, msg_off: *const u64, seed32: *const u8, flags: *mut u8,
+        n_bad: *mut u64) -> c_int;
+    pub fn schnorr_b200_locate_invalid_registered_seeded(ctx: *mut schnorr_b200_ctx, ks: *const schnorr_b200_keyset,
+        n: usize, sigs81: *const u8, key_idx: *const u32, msgs: *const u8, msg_off: *const u64, seed32: *const u8,
+        flags: *mut u8, n_bad: *mut u64) -> c_int;
+    pub fn schnorr_b200_locate_invalid_keyed_seeded(ctx: *mut schnorr_b200_ctx, n: usize, keyed130: *const u8,
+        msgs: *const u8, msg_off: *const u64, seed32: *const u8, flags: *mut u8, n_bad: *mut u64) -> c_int;
+    pub fn schnorr_b200_locate_invalid_keyed_registered_seeded(ctx: *mut schnorr_b200_ctx, ks: *const schnorr_b200_keyset,
+        n: usize, keyed130: *const u8, msgs: *const u8, msg_off: *const u64, seed32: *const u8, flags: *mut u8,
+        n_bad: *mut u64) -> c_int;
     pub fn schnorr_b200_keygen(ctx: *mut schnorr_b200_ctx, n: usize, sk32: *const u8, pk96: *mut u8, pk_inf: *mut u8) -> c_int;
     pub fn schnorr_b200_sign_many(ctx: *mut schnorr_b200_ctx, n: usize, sk32: *const u8, pk96: *const u8,
         pk_inf: *const u8, msgs: *const u8, msg_off: *const u64, nonce32: *const u8, sigs81: *mut u8) -> c_int;
@@ -175,6 +186,21 @@ impl Engine {
                                         core::ptr::null_mut())
         };
         self.check(rc, "schnorr_b200_locate_invalid");
+        flags
+    }
+
+    /// `locate_invalid` with randomisers `0 .. n` generated on the devices from a 32-byte seed: the flags of a failed
+    /// `verify_batch_seeded`.
+    pub fn locate_invalid_seeded(&self, sigs: &[[u8; 81]], pks: &[[u8; 96]], pk_inf: &[u8], messages: &[&[u8]],
+                                 seed: &[u8; 32]) -> Vec<u8> {
+        let (blob, off) = pack_messages(messages);
+        let mut flags = vec![0u8; sigs.len()];
+        let rc = unsafe {
+            schnorr_b200_locate_invalid_seeded(self.0, sigs.len(), sigs.as_ptr().cast(), pks.as_ptr().cast(),
+                                               pk_inf.as_ptr(), blob.as_ptr(), off.as_ptr(), seed.as_ptr(),
+                                               flags.as_mut_ptr(), core::ptr::null_mut())
+        };
+        self.check(rc, "schnorr_b200_locate_invalid_seeded");
         flags
     }
 

@@ -72,6 +72,12 @@ _SIGNATURES = {
     "schnorr_b200_verify_batch_keyed_seeded": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 4 + [C.POINTER(C.c_int), _u8p, _u8p]),
     "schnorr_b200_verify_batch_keyed_registered_seeded": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 4
                                                           + [C.POINTER(C.c_int), _u8p, _u8p]),
+    "schnorr_b200_locate_invalid_seeded": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 7 + [C.POINTER(C.c_uint64)]),
+    "schnorr_b200_locate_invalid_registered_seeded": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 6
+                                                      + [C.POINTER(C.c_uint64)]),
+    "schnorr_b200_locate_invalid_keyed_seeded": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 5 + [C.POINTER(C.c_uint64)]),
+    "schnorr_b200_locate_invalid_keyed_registered_seeded": (C.c_int, [C.c_void_p, C.c_void_p, _sz] + [_u8p] * 5
+                                                            + [C.POINTER(C.c_uint64)]),
     "schnorr_b200_last_batch_points": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "schnorr_b200_set_registered_batch_threshold": (C.c_int, [C.c_void_p, _sz]),
     "schnorr_b200_batch_partial_dev": (C.c_int, [C.c_void_p, _sz] + [_u8p] * 7),

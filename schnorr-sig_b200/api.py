@@ -106,15 +106,14 @@ def _random_scalar(rng) -> int:
     return int.from_bytes(rng.fill_bytes(64), "little") % _Q
 
 
-def _randomizers(n, rng, seed, materialise):
+def _randomizers(n, rng, seed):
     """The n x 32 randomiser bytes of a batch: one Scalar::random per signature from rng (OsRng by default); given a
-    32-byte seed instead, None -- the seeded entry points generate them on the device -- or, with materialise, the same
-    randomisers read back (Engine.batch_randomizers(n, seed)), which localise a failed seeded batch.  The seed must be
-    fresh from a CSPRNG for every batch and unknown to the signers until the verdict (include/schnorr_b200.h)."""
+    32-byte seed instead, None -- the seeded entry points generate them on the device.  The seed must be fresh from a
+    CSPRNG for every batch and unknown to the signers until the verdict (include/schnorr_b200.h)."""
     if seed is not None:
         if rng is not None:
             raise ValueError("a batch takes its randomisers from an rng or from a seed, not both")
-        return default_engine().batch_randomizers(n, seed) if materialise else None
+        return None
     rng = rng or OsRng()
     rand = np.zeros((n, 32), dtype=np.uint8)
     for i in range(n):
@@ -281,20 +280,20 @@ class KeySet:
                                                            blob, off)
         return _result_from_verdict(int(v[0]))
 
-    def _batch_inputs(self, indices, signatures, messages, rng, seed=None, materialise=True):
+    def _batch_inputs(self, indices, signatures, messages, rng, seed=None):
         n = len(signatures)
         assert len(indices) == n, "We should have the same number of signatures than public keys"
         assert len(messages) == n, "We should have the same number of messages than public keys"
         idx = np.array([int(i) if 0 <= int(i) < 2**32 else 2**32 - 1 for i in indices], dtype=np.uint32)
         sigs = np.frombuffer(b"".join(s.to_bytes() for s in signatures), dtype=np.uint8).reshape(n, 81)
         blob, off = _pack(messages)
-        return sigs, idx, blob, off, _randomizers(n, rng, seed, materialise)
+        return sigs, idx, blob, off, _randomizers(n, rng, seed)
 
     def verify_batch(self, indices, signatures, messages, rng=None, *, seed=None) -> Result:
         """verify_batch(signatures, [keys[i] for i in indices], messages, rng) (src/batch.rs:31-130) with the key side of
         the batch equation summed per key of the set; an index outside the set gives the malformed-batch error.  seed
         (32 bytes, instead of rng): the randomisers are generated on the device from it."""
-        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng, seed, materialise=False)
+        sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng, seed)
         if rand is None:
             v, _lhs, _rhs = default_engine().verify_batch_registered_seeded(self._handle, sigs, idx, blob, off, seed)
         else:
@@ -303,12 +302,16 @@ class KeySet:
 
     def locate_invalid(self, indices, signatures, messages, rng=None, *, seed=None):
         """locate_invalid(signatures, [keys[i] for i in indices], messages, rng): [(index, SignatureError), ...] in batch
-        semantics; a malformed item or an index outside the set panics."""
+        semantics; a malformed item or an index outside the set panics.  seed: that of verify_batch(..., seed=seed), to
+        localise that failed batch (the randomisers are generated on the devices)."""
         if len(signatures) == 0:
             assert len(indices) == 0 and len(messages) == 0
             return []
         sigs, idx, blob, off, rand = self._batch_inputs(indices, signatures, messages, rng, seed)
-        flags = default_engine().locate_invalid_registered(self._handle, sigs, idx, blob, off, rand)
+        if rand is None:
+            flags = default_engine().locate_invalid_registered_seeded(self._handle, sigs, idx, blob, off, seed)
+        else:
+            flags = default_engine().locate_invalid_registered(self._handle, sigs, idx, blob, off, rand)
         out = []
         for i in np.nonzero(flags)[0]:
             if flags[i] == MALFORMED:
@@ -319,7 +322,7 @@ class KeySet:
     def verify_batch_keyed(self, keyed_signatures, messages, rng=None, *, seed=None) -> Result:
         """verify_batch_keyed (below) with the records whose key is in the set taking its registered record and the
         key side summed per key: the same result."""
-        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed, materialise=False)
+        recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed)
         if rand is None:
             v, _lhs, _rhs = default_engine().verify_batch_keyed_registered_seeded(self._handle, recs, blob, off, seed)
         else:
@@ -332,6 +335,8 @@ class KeySet:
             assert len(messages) == 0
             return []
         recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed)
+        if rand is None:
+            return _keyed_located(default_engine().locate_invalid_keyed_registered_seeded(self._handle, recs, blob, off, seed))
         return _keyed_located(default_engine().locate_invalid_keyed_registered(self._handle, recs, blob, off, rand))
 
 
@@ -537,7 +542,7 @@ def verify_batch(signatures, public_keys, messages, rng=None, *, seed=None) -> R
     batch and unknown to the signers until the verdict."""
     assert len(signatures) == len(public_keys), "We should have the same number of signatures than public keys"
     assert len(messages) == len(public_keys), "We should have the same number of messages than public keys"
-    rand = _randomizers(len(signatures), rng, seed, materialise=False)
+    rand = _randomizers(len(signatures), rng, seed)
     if rand is None:
         v, _lhs, _rhs = default_engine().verify_batch_seeded(*_batch_arrays(signatures, public_keys, messages), seed)
         return _result_from_verdict(v)
@@ -551,7 +556,8 @@ def locate_invalid(signatures, public_keys, messages, rng=None, *, seed=None):
     public keys are not subgroup-checked.  A signature with a flipped y-sign flag is therefore reported here (it makes
     verify_batch fail) although Signature::verify accepts it.  Runs on the device: bisection over partial MSMs, then an
     exact per-item check of the failing slices (schnorr_b200_locate_invalid).  Malformed encodings panic as in
-    verify_batch.  seed: the randomisers of verify_batch(..., seed=seed), to localise that failed batch."""
+    verify_batch.  seed: that of verify_batch(..., seed=seed), to localise that failed batch (the randomisers are
+    generated on the devices)."""
     n = len(signatures)
     assert len(public_keys) == n and len(messages) == n
     if n == 0:
@@ -560,8 +566,11 @@ def locate_invalid(signatures, public_keys, messages, rng=None, *, seed=None):
     pks = np.frombuffer(b"".join(k.xy for k in public_keys), dtype=np.uint8).reshape(n, 96)
     inf = np.array([k.infinity for k in public_keys], dtype=np.uint8)
     blob, off = _pack(messages)
-    rand = _randomizers(n, rng, seed, materialise=True)
-    flags = default_engine().locate_invalid(sigs, pks, inf, blob, off, rand)
+    rand = _randomizers(n, rng, seed)
+    if rand is None:
+        flags = default_engine().locate_invalid_seeded(sigs, pks, inf, blob, off, seed)
+    else:
+        flags = default_engine().locate_invalid(sigs, pks, inf, blob, off, rand)
     out = []
     for i in np.nonzero(flags)[0]:
         if flags[i] == MALFORMED:
@@ -570,14 +579,14 @@ def locate_invalid(signatures, public_keys, messages, rng=None, *, seed=None):
     return out
 
 
-def _keyed_batch_inputs(keyed_signatures, messages, rng, seed=None, materialise=True):
+def _keyed_batch_inputs(keyed_signatures, messages, rng, seed=None):
     n = len(keyed_signatures)
     assert len(messages) == n, "We should have the same number of messages than signatures"
     recs = [k.to_bytes() if isinstance(k, KeyedSignature) else bytes(k) for k in keyed_signatures]
     assert all(len(b) == KEYED_SIGNATURE_LENGTH for b in recs)
     recs = np.frombuffer(b"".join(recs), dtype=np.uint8).reshape(n, KEYED_SIGNATURE_LENGTH)
     blob, off = _pack(messages)
-    return recs, blob, off, _randomizers(n, rng, seed, materialise)
+    return recs, blob, off, _randomizers(n, rng, seed)
 
 
 def _keyed_located(flags):
@@ -593,7 +602,7 @@ def verify_batch_keyed(keyed_signatures, messages, rng=None, *, seed=None) -> Re
     """verify_batch over KeyedSignature objects or their 130-byte records (src/signature.rs:237-271,
     src/batch.rs:31-130): verify_batch([k.signature ...], [k.public_key ...], messages, rng) with the keys decoded on
     the device.  A record whose key does not decode panics, as unwrapping KeyedSignature::from_bytes does."""
-    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed, materialise=False)
+    recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed)
     if rand is None:
         v, _lhs, _rhs = default_engine().verify_batch_keyed_seeded(recs, blob, off, seed)
     else:
@@ -608,6 +617,8 @@ def locate_invalid_keyed(keyed_signatures, messages, rng=None, *, seed=None):
         assert len(messages) == 0
         return []
     recs, blob, off, rand = _keyed_batch_inputs(keyed_signatures, messages, rng, seed)
+    if rand is None:
+        return _keyed_located(default_engine().locate_invalid_keyed_seeded(recs, blob, off, seed))
     return _keyed_located(default_engine().locate_invalid_keyed(recs, blob, off, rand))
 
 

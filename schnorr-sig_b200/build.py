@@ -13,7 +13,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
 
 
 def sources():
-    deps = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC)) if f.endswith((".cu", ".cuh"))]
+    deps = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC)) if f.endswith((".cu", ".cuh", ".h"))]
     deps += [os.path.join(HERE, "..", "include", f) for f in ("schnorr_b200.h", "cheetah_params.h")]
     return deps
 

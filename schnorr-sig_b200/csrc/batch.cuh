@@ -1527,130 +1527,6 @@ int schnorr_b200_verify_batch_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_t
     }, result216);
 }
 
-// Bisection over partial MSMs on DEVICE buffers.  A range whose own random linear combination
-//     sum_{i in range} s_i R_i - s_i h_i P_i  ==  (sum_{i in range} s_i e_i) G
-// holds is clean (up to the 2^-255 soundness error of the batch itself); a failing range is cut into LOCATE_FANOUT
-// sub-ranges, each checked by its own partial MSM; ranges of at most LOCATE_LEAF signatures -- or everything that is left
-// once the suspects stop shrinking -- go through k_batch_item_check.  One bad signature among 2^20 costs about two batch
-// verifications; a batch riddled with bad signatures degrades to one per-item pass.
-static constexpr size_t LOCATE_LEAF = 4096;
-static constexpr int LOCATE_FANOUT = 8;
-struct locate_range {
-    size_t lo, hi;
-};
-static int locate_items(schnorr_b200_ctx* ctx, const std::vector<locate_range>& ranges, const uint8_t* sigs81,
-                        const uint8_t* pk96, const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off,
-                        const uint8_t* rand32, uint8_t* flags) {
-    for (const locate_range& r : ranges) {
-        size_t cn = r.hi - r.lo;
-        if (cn == 0) continue;
-        scratch_scope scope(ctx->scratch, ctx->stream);
-        soa_batch soa;
-        if (int rc = alloc_soa(ctx, cn, &soa)) return rc;
-        k_ingest<<<grid_for(cn, INGEST_THREADS), INGEST_THREADS, 0, ctx->stream>>>(cn, sigs81 + 81 * r.lo, pk96 + 96 * r.lo,
-                                                                                   pk_inf ? pk_inf + r.lo : nullptr, soa);
-        k_batch_item_check<<<grid_for(cn, VERIFY_THREADS), VERIFY_THREADS, 0, ctx->stream>>>(soa, msgs, msg_off + r.lo,
-                                                                                           rand32 + 32 * r.lo, ctx->gtab,
-                                                                                           flags + r.lo);
-        ctx->launches += 2;
-        CUDA_TRY(ctx, cudaGetLastError());
-        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    }
-    return SCHNORR_B200_OK;
-}
-
-int schnorr_b200_locate_invalid_dev(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
-                                    const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off,
-                                    const uint8_t* rand32, uint8_t* flags) {
-    if (!ctx || (n && (!sigs81 || !pk96 || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
-    NOT_ON_MULTI(ctx);
-    if (n == 0) return SCHNORR_B200_OK;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, cudaMemsetAsync(flags, 0, n, ctx->stream));
-    std::vector<locate_range> suspects{{0, n}}, leaves;
-    scratch_scope scope(ctx->scratch, ctx->stream);
-    uint8_t* base;
-    const size_t slot = RESULT_BYTES + 192 + 40;   // result | partial, per sub-range
-    if (int rc = stage_in(ctx, {{nullptr, slot * LOCATE_FANOUT * 64, &base}})) return rc;
-    bool first = true;
-    while (!suspects.empty()) {
-        // cut every suspect range (the whole batch is first checked as it is: a batch that verifies has no culprit)
-        std::vector<locate_range> parts;
-        for (const locate_range& r : suspects) {
-            size_t len = r.hi - r.lo;
-            if (len <= LOCATE_LEAF) {
-                leaves.push_back(r);
-                continue;
-            }
-            int f = first ? 1 : LOCATE_FANOUT;
-            size_t step = (len + f - 1) / f;
-            for (size_t lo = r.lo; lo < r.hi; lo += step) parts.push_back({lo, lo + step < r.hi ? lo + step : r.hi});
-        }
-        first = false;
-        suspects.clear();
-        // too many pieces: the batch is riddled with bad signatures, finish item by item
-        if (parts.size() > (size_t)LOCATE_FANOUT * 64) {
-            for (const locate_range& r : parts) leaves.push_back(r);
-            break;
-        }
-        std::vector<uint8_t> host(parts.size() * slot);
-        for (size_t k = 0; k < parts.size(); k++) {
-            const locate_range& r = parts[k];
-            uint8_t* res = base + k * slot;
-            uint8_t* partial = res + RESULT_BYTES;
-            if (int rc = batch_partial_impl(ctx, r.hi - r.lo, sigs81 + 81 * r.lo, pk96 + 96 * r.lo, pk_inf ? pk_inf + r.lo : nullptr,
-                                            msgs, msg_off + r.lo, rand32 + 32 * r.lo, partial))
-                return rc;
-            k_batch_finish<<<1, 32, 0, ctx->stream>>>(1, (const uint64_t*)partial, ctx->gtab, res, nullptr);
-            ctx->launches += 1;
-        }
-        CUDA_TRY(ctx, cudaMemcpyAsync(host.data(), base, parts.size() * slot, cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-        for (size_t k = 0; k < parts.size(); k++)
-            if (host[k * slot] != VERDICT_OK) suspects.push_back(parts[k]);   // Err or malformed: look inside
-    }
-    return locate_items(ctx, leaves, sigs81, pk96, pk_inf, msgs, msg_off, rand32, flags);
-}
-
-// the host forms of localisation, on inputs staged on the first device of ctx: the flags into d_flags, copied back to
-// `flags` and counted; the error text of a shard is copied up to ctx
-static int locate_invalid_staged(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
-                                 const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
-                                 uint8_t* d_flags, uint8_t* flags, uint64_t* n_bad) {
-    schnorr_b200_ctx* c = device_ctx(ctx, 0);
-    if (int rc = schnorr_b200_locate_invalid_dev(c, n, sigs81, pk96, pk_inf, msgs, msg_off, rand32, d_flags)) {
-        if (c != ctx) ctx->err = c->err;
-        return rc;
-    }
-    CUDA_TRY(c, cudaMemcpyAsync(flags, d_flags, n, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
-    if (n_bad)
-        for (size_t i = 0; i < n; i++) *n_bad += flags[i] != 0;
-    return SCHNORR_B200_OK;
-}
-
-int schnorr_b200_locate_invalid(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs81, const uint8_t* pk96,
-                                const uint8_t* pk_inf, const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32,
-                                uint8_t* flags, uint64_t* n_bad) {
-    if (!ctx || (n && (!sigs81 || !pk96 || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
-    if (n_bad) *n_bad = 0;
-    if (n == 0) return SCHNORR_B200_OK;
-    schnorr_b200_ctx* c = device_ctx(ctx, 0);   // localisation runs on the first device
-    CUDA_TRY(c, cudaSetDevice(c->device));
-    CHECK_MSG_OFF(ctx, n, msg_off);
-    size_t mb = msg_off[n];
-    if (mb && !msgs) return SCHNORR_B200_EARG;
-    // the inputs stay resident across the bisection
-    scratch_scope scope(c->scratch, c->stream);
-    uint8_t *d_sig, *d_pk, *d_m, *d_off, *d_rand, *d_inf, *d_flags;
-    if (int rc = stage_in(c, {{sigs81, n * 81, &d_sig}, {pk96, n * 96, &d_pk}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                              {rand32, n * 32, &d_rand}, {pk_inf, n, &d_inf}, {nullptr, n, &d_flags}}))
-        return rc;
-    return locate_invalid_staged(ctx, n, d_sig, d_pk, pk_inf ? d_inf : nullptr, d_m, (const uint64_t*)d_off, d_rand, d_flags,
-                                 flags, n_bad);
-}
-
-
 int schnorr_b200_batch_finish(schnorr_b200_ctx* ctx, size_t n_partials, const uint8_t* partials192_host, int* verdict,
                               uint8_t* lhs97, uint8_t* rhs97) {
     if (!ctx || !partials192_host || !verdict || n_partials == 0) return SCHNORR_B200_EARG;

@@ -38,8 +38,8 @@ static std::vector<uint64_t> rebase_offsets(const uint64_t* msg_off, size_t lo, 
     for (size_t i = lo; i <= hi; i++) o[i - lo] = msg_off[i] - base;
     return o;
 }
-// runs fn(shard index, slice) on one host thread per slice; returns the first non-zero code and copies that shard's
-// error text into the parent context
+// runs fn(shard index, slice) on one host thread per slice (inline for one slice, which may be a single-device context
+// itself); returns the first non-zero code and copies that shard's error text into the parent context
 template <typename F>
 static int multi_run(schnorr_b200_ctx* ctx, const std::vector<shard_slice>& sl, F fn) {
     std::vector<int> rc(sl.size(), 0);
@@ -53,7 +53,8 @@ static int multi_run(schnorr_b200_ctx* ctx, const std::vector<shard_slice>& sl, 
     }
     for (size_t k = 0; k < sl.size(); k++)
         if (rc[k] != 0) {
-            ctx->err = "device " + std::to_string(ctx->shards[k]->device) + ": " + ctx->shards[k]->err;
+            schnorr_b200_ctx* sh = device_ctx(ctx, k);   // a single-device context (one slice) keeps its own text
+            if (sh != ctx) ctx->err = "device " + std::to_string(sh->device) + ": " + sh->err;
             return rc[k];
         }
     return SCHNORR_B200_OK;
@@ -115,14 +116,13 @@ static int multi_sign_many(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sk32,
     });
 }
 
-// verify_batch (and its registered-key-set form) over all devices: per-shard partials from `partial_fn`, one peer copy
-// each, finish on the first device.  A batch always uses every shard slice it is given (an empty slice contributes the
-// identity).
+// A batch over the given slices of a multi-device context: per-shard partials from partial_fn(k, slice, partial192),
+// one peer copy each, finish on the first device.  A batch always uses every shard slice it is given (an empty slice
+// contributes the identity).  multi_verify_batch cuts the call with multi_slices; localisation (locate.cuh) uses the
+// ranges the devices own.
 template <typename F>
-static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* msg_off, int* verdict, uint8_t* lhs97,
-                              uint8_t* rhs97, F partial_fn) {
-    if (n) CHECK_MSG_OFF(ctx, n, msg_off);
-    auto sl = multi_slices(ctx, n);
+static int multi_batch_partials(schnorr_b200_ctx* ctx, const std::vector<shard_slice>& sl, int* verdict, uint8_t* lhs97,
+                                uint8_t* rhs97, F partial_fn) {
     size_t g = sl.size();
     schnorr_b200_ctx* root = ctx->shards[0];
     CUDA_TRY(root, cudaSetDevice(root->device));
@@ -140,16 +140,7 @@ static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* m
         uint8_t* partial = gathered;  // the root writes its partial in place
         if (k != 0)
             if (int r2 = stage_in(sh, {{nullptr, 192, &partial}})) return r2;
-        size_t cn = s.hi - s.lo;
-        int r;
-        if (cn == 0) {
-            r = batch_partial_empty(sh, partial);
-        } else {
-            auto off = rebase_offsets(msg_off, s.lo, s.hi);
-            r = partial_fn(k, s, off.data(), partial);
-            // `off` must outlive the asynchronous copy that reads it: synchronise before it goes out of scope
-            if (r == 0 && cudaStreamSynchronize(sh->stream) != cudaSuccess) r = SCHNORR_B200_ECUDA;
-        }
+        int r = s.hi > s.lo ? partial_fn(k, s, partial) : batch_partial_empty(sh, partial);
         if (r) return r;
         if (k != 0) {  // the ONE exchange step of the batch path: 192 bytes over NVLink to the root device
             if (cudaMemcpyPeerAsync(gathered + 192 * (size_t)k, root->device, partial, sh->device, 192, sh->stream) != cudaSuccess) {
@@ -175,4 +166,19 @@ static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* m
     int r = read_result(root, res, verdict, lhs97, rhs97);
     if (r) ctx->err = root->err;
     return r;
+}
+
+// verify_batch (and its registered-key-set and keyed forms) over all devices: partial_fn(k, slice, rebased offsets,
+// partial192) reduces the non-empty slice of shard k to its partial on that shard's device
+template <typename F>
+static int multi_verify_batch(schnorr_b200_ctx* ctx, size_t n, const uint64_t* msg_off, int* verdict, uint8_t* lhs97,
+                              uint8_t* rhs97, F partial_fn) {
+    if (n) CHECK_MSG_OFF(ctx, n, msg_off);
+    return multi_batch_partials(ctx, multi_slices(ctx, n), verdict, lhs97, rhs97, [&](int k, shard_slice s, uint8_t* partial) {
+        auto off = rebase_offsets(msg_off, s.lo, s.hi);
+        int r = partial_fn(k, s, off.data(), partial);
+        // `off` must outlive the asynchronous copy that reads it: synchronise before it goes out of scope
+        if (r == 0 && cudaStreamSynchronize(ctx->shards[k]->stream) != cudaSuccess) r = SCHNORR_B200_ECUDA;
+        return r;
+    });
 }

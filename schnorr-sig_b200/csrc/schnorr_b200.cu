@@ -1143,6 +1143,7 @@ static int verify_many_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs
                             const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts, bool validate_offsets);
 #include "batch.cuh"
 #include "multi.cuh"
+#include "locate.cuh"
 // K2 for the smallest calls: one thread block per signature (uses the six-lane primitives of dist.cuh and the 24-lane
 // Jacobian toolkit of batch.cuh)
 #include "one.cuh"
@@ -2476,30 +2477,43 @@ int schnorr_b200_verify_batch_registered_dev(schnorr_b200_ctx* ctx, const schnor
     }, result216);
 }
 
-// localisation on the first device: the inputs staged, the items' key records gathered, then the per-signature bisection
-// of schnorr_b200_locate_invalid_dev
+// localisation against a registered key set: each device gathers the key records of its owned range from its copy of
+// the set, then the per-signature bisection of locate_invalid_host
+static int locate_invalid_registered_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
+                                          const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
+                                          const rand_source& rs, uint8_t* flags, uint64_t* n_bad) {
+    CHECK_KEYSET(ctx, ks);
+    return locate_invalid_host(ctx, n, msgs, msg_off, rs, flags, n_bad,
+                               [&](schnorr_b200_ctx* c, size_t k, size_t lo, size_t hi, locate_shard* s) {
+        size_t len = hi - lo;
+        const keyset_dev& kd = ks->devs[k];
+        uint8_t *d_sig, *d_idx, *d_pk, *d_inf;
+        if (int rc = stage_in(c, {{sigs81 + 81 * lo, len * 81, &d_sig}, {key_idx + lo, len * 4, &d_idx}, {nullptr, len * 96, &d_pk},
+                                  {nullptr, len, &d_inf}}))
+            return rc;
+        k_keyset_gather<<<grid_for(len, 128), 128, 0, c->stream>>>(len, (uint32_t*)d_idx, ks->n_keys, kd.pk12, kd.pk_inf,
+                                                                  (uint64_t*)d_pk, d_inf);
+        c->launches += 1;
+        s->sig = d_sig;
+        s->pk = d_pk;
+        s->inf = d_inf;
+        return 0;
+    });
+}
+
 int schnorr_b200_locate_invalid_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* sigs81,
                                            const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off,
                                            const uint8_t* rand32, uint8_t* flags, uint64_t* n_bad) {
     if (!ctx || !ks || (n && (!sigs81 || !key_idx || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
-    CHECK_KEYSET(ctx, ks);
-    if (n_bad) *n_bad = 0;
-    if (n == 0) return SCHNORR_B200_OK;
-    CHECK_MSG_OFF(ctx, n, msg_off);
-    size_t mb = msg_off[n];
-    if (mb && !msgs) return SCHNORR_B200_EARG;
-    schnorr_b200_ctx* c = device_ctx(ctx, 0);
-    const keyset_dev& kd = ks->devs[0];
-    CUDA_TRY(c, cudaSetDevice(c->device));
-    scratch_scope scope(c->scratch, c->stream);
-    uint8_t *d_sig, *d_idx, *d_m, *d_off, *d_rand, *d_flags, *d_pk, *d_inf;
-    if (int rc = stage_in(c, {{sigs81, n * 81, &d_sig}, {key_idx, n * 4, &d_idx}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                              {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}, {nullptr, n * 96, &d_pk}, {nullptr, n, &d_inf}}))
-        return rc;
-    k_keyset_gather<<<grid_for(n, 128), 128, 0, c->stream>>>(n, (uint32_t*)d_idx, ks->n_keys, kd.pk12, kd.pk_inf, (uint64_t*)d_pk,
-                                                            d_inf);
-    c->launches += 1;
-    return locate_invalid_staged(ctx, n, d_sig, d_pk, d_inf, d_m, (const uint64_t*)d_off, d_rand, d_flags, flags, n_bad);
+    return locate_invalid_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand_from_host(rand32), flags, n_bad);
+}
+
+int schnorr_b200_locate_invalid_registered_seeded(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                                  const uint8_t* sigs81, const uint32_t* key_idx, const uint8_t* msgs,
+                                                  const uint64_t* msg_off, const uint8_t* seed32, uint8_t* flags,
+                                                  uint64_t* n_bad) {
+    if (!ctx || !ks || !seed32 || (n && (!sigs81 || !key_idx || !msg_off || !flags))) return SCHNORR_B200_EARG;
+    return locate_invalid_registered_host(ctx, ks, n, sigs81, key_idx, msgs, msg_off, rand_from_seed(seed32), flags, n_bad);
 }
 
 }  // extern "C"
@@ -2589,29 +2603,22 @@ static int verify_batch_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_key
     }, verdict, lhs97, rhs97);
 }
 
-// localisation on the first device: the inputs staged, the front-end records, then the bisection of
-// schnorr_b200_locate_invalid_dev
+// localisation over keyed records (ks checked by the caller): each device builds the front-end records of its owned
+// range against its copy of the set, then the bisection of locate_invalid_host
 static int locate_invalid_keyed_host(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n, const uint8_t* keyed130,
-                                     const uint8_t* msgs, const uint64_t* msg_off, const uint8_t* rand32, uint8_t* flags,
+                                     const uint8_t* msgs, const uint64_t* msg_off, const rand_source& rs, uint8_t* flags,
                                      uint64_t* n_bad) {
-    if (n_bad) *n_bad = 0;
-    if (n == 0) return SCHNORR_B200_OK;
-    CHECK_MSG_OFF(ctx, n, msg_off);
-    size_t mb = msg_off[n];
-    if (mb && !msgs) return SCHNORR_B200_EARG;
-    schnorr_b200_ctx* c = device_ctx(ctx, 0);
-    CUDA_TRY(c, cudaSetDevice(c->device));
-    scratch_scope scope(c->scratch, c->stream);
-    uint8_t *d_rec, *d_m, *d_off, *d_rand, *d_flags;
-    if (int rc = stage_in(c, {{keyed130, n * 130, &d_rec}, {msgs, mb, &d_m}, {msg_off, (n + 1) * 8, &d_off},
-                              {rand32, n * 32, &d_rand}, {nullptr, n, &d_flags}}))
-        return rc;
-    keyed_front f;
-    if (int rc = keyed_front_end(c, ks, 0, n, d_rec, &f)) {
-        if (c != ctx) ctx->err = c->err;
-        return rc;
-    }
-    return locate_invalid_staged(ctx, n, f.sig, f.pk, f.inf, d_m, (const uint64_t*)d_off, d_rand, d_flags, flags, n_bad);
+    return locate_invalid_host(ctx, n, msgs, msg_off, rs, flags, n_bad,
+                               [&](schnorr_b200_ctx* c, size_t k, size_t lo, size_t hi, locate_shard* s) {
+        uint8_t* d_rec;
+        if (int rc = stage_in(c, {{keyed130 + 130 * lo, (hi - lo) * 130, &d_rec}})) return rc;
+        keyed_front f;
+        if (int rc = keyed_front_end(c, ks, k, hi - lo, d_rec, &f)) return rc;
+        s->sig = f.sig;
+        s->pk = f.pk;
+        s->inf = f.inf;
+        return 0;
+    });
 }
 
 extern "C" {
@@ -2671,7 +2678,13 @@ int schnorr_b200_verify_batch_keyed_registered_dev(schnorr_b200_ctx* ctx, const 
 int schnorr_b200_locate_invalid_keyed(schnorr_b200_ctx* ctx, size_t n, const uint8_t* keyed130, const uint8_t* msgs,
                                       const uint64_t* msg_off, const uint8_t* rand32, uint8_t* flags, uint64_t* n_bad) {
     if (!ctx || (n && (!keyed130 || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
-    return locate_invalid_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand32, flags, n_bad);
+    return locate_invalid_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand_from_host(rand32), flags, n_bad);
+}
+
+int schnorr_b200_locate_invalid_keyed_seeded(schnorr_b200_ctx* ctx, size_t n, const uint8_t* keyed130, const uint8_t* msgs,
+                                             const uint64_t* msg_off, const uint8_t* seed32, uint8_t* flags, uint64_t* n_bad) {
+    if (!ctx || !seed32 || (n && (!keyed130 || !msg_off || !flags))) return SCHNORR_B200_EARG;
+    return locate_invalid_keyed_host(ctx, nullptr, n, keyed130, msgs, msg_off, rand_from_seed(seed32), flags, n_bad);
 }
 
 int schnorr_b200_locate_invalid_keyed_registered(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
@@ -2679,7 +2692,15 @@ int schnorr_b200_locate_invalid_keyed_registered(schnorr_b200_ctx* ctx, const sc
                                                  const uint8_t* rand32, uint8_t* flags, uint64_t* n_bad) {
     if (!ctx || !ks || (n && (!keyed130 || !msg_off || !rand32 || !flags))) return SCHNORR_B200_EARG;
     CHECK_KEYSET(ctx, ks);
-    return locate_invalid_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand32, flags, n_bad);
+    return locate_invalid_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand_from_host(rand32), flags, n_bad);
+}
+
+int schnorr_b200_locate_invalid_keyed_registered_seeded(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t n,
+                                                        const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off,
+                                                        const uint8_t* seed32, uint8_t* flags, uint64_t* n_bad) {
+    if (!ctx || !ks || !seed32 || (n && (!keyed130 || !msg_off || !flags))) return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    return locate_invalid_keyed_host(ctx, ks, n, keyed130, msgs, msg_off, rand_from_seed(seed32), flags, n_bad);
 }
 
 // ---- keygen / sign ---------------------------------------------------------------------------

@@ -17,8 +17,9 @@
 // synchronisation.  The footprint is the deepest stack of any single call, except while a call grows the arena: the
 // old block and the overflow blocks then exist together until that call ends.
 //
-// A context is used by one host thread at a time.  multi_verify_batch opens a scope on its first shard on the calling
-// thread; that shard's worker thread then nests its own scopes inside it while the caller waits for it in join.
+// A context is used by one host thread at a time.  multi_batch_partials opens a scope on its first shard on the calling
+// thread, and the host localisations (locate.cuh) one on every shard they use; each shard's worker thread then nests
+// its own scopes inside it while the caller waits for it in join.
 #pragma once
 #include <cuda_runtime.h>
 

@@ -401,6 +401,59 @@ class Engine:
         self._check(rc, "verify_batch_keyed_seeded" if keyset is None else "verify_batch_keyed_registered_seeded")
         return verdict.value, lhs, rhs
 
+    def locate_invalid_seeded(self, sigs81, pk96, pk_inf, msgs, off, seed):
+        """locate_invalid with rand32 = batch_randomizers(n, seed), generated on the devices -> uint8[n]"""
+        sigs81, pk96, msgs, seed = _u8(sigs81, 81), _u8(pk96, 96), _u8(msgs), _seed32(seed)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = sigs81.shape[0]
+        self._check_offsets(n, pk96.shape[0], off, msgs)
+        inf = None if pk_inf is None else _u8(pk_inf)
+        self._check_inf(n, inf)
+        flags = np.zeros(n, dtype=np.uint8)
+        nb = C.c_uint64(0)
+        self._check(self._L.schnorr_b200_locate_invalid_seeded(self._h, n, _ptr(sigs81), _ptr(pk96), _ptr(inf), _ptr(msgs),
+                                                               _ptr(off), _ptr(seed), _ptr(flags), C.byref(nb)),
+                    "locate_invalid_seeded")
+        assert int(nb.value) == int(np.count_nonzero(flags))
+        return flags
+
+    def locate_invalid_registered_seeded(self, keyset, sigs81, key_idx, msgs, off, seed):
+        """locate_invalid_registered with rand32 = batch_randomizers(n, seed), generated on the devices."""
+        n, sigs81, key_idx, msgs, off = self._registered_inputs(sigs81, key_idx, msgs, off)
+        seed = _seed32(seed)
+        flags = np.zeros(n, dtype=np.uint8)
+        nb = C.c_uint64(0)
+        self._check(self._L.schnorr_b200_locate_invalid_registered_seeded(self._h, keyset.handle, n, _ptr(sigs81),
+                                                                          _ptr(key_idx), _ptr(msgs), _ptr(off), _ptr(seed),
+                                                                          _ptr(flags), C.byref(nb)),
+                    "locate_invalid_registered_seeded")
+        assert int(nb.value) == int(np.count_nonzero(flags))
+        return flags
+
+    def locate_invalid_keyed_seeded(self, keyed130, msgs, off, seed):
+        """locate_invalid_keyed with rand32 = batch_randomizers(n, seed), generated on the devices."""
+        return self._locate_keyed_seeded(None, keyed130, msgs, off, seed)
+
+    def locate_invalid_keyed_registered_seeded(self, keyset, keyed130, msgs, off, seed):
+        """locate_invalid_keyed_registered with rand32 = batch_randomizers(n, seed), generated on the devices."""
+        return self._locate_keyed_seeded(keyset, keyed130, msgs, off, seed)
+
+    def _locate_keyed_seeded(self, keyset, keyed130, msgs, off, seed):
+        n, keyed130, msgs, off = self._keyed_inputs(keyed130, msgs, off)
+        seed = _seed32(seed)
+        flags = np.zeros(n, dtype=np.uint8)
+        nb = C.c_uint64(0)
+        if keyset is None:
+            rc = self._L.schnorr_b200_locate_invalid_keyed_seeded(self._h, n, _ptr(keyed130), _ptr(msgs), _ptr(off),
+                                                                  _ptr(seed), _ptr(flags), C.byref(nb))
+        else:
+            rc = self._L.schnorr_b200_locate_invalid_keyed_registered_seeded(self._h, keyset.handle, n, _ptr(keyed130),
+                                                                             _ptr(msgs), _ptr(off), _ptr(seed), _ptr(flags),
+                                                                             C.byref(nb))
+        self._check(rc, "locate_invalid_keyed_seeded" if keyset is None else "locate_invalid_keyed_registered_seeded")
+        assert int(nb.value) == int(np.count_nonzero(flags))
+        return flags
+
     def _registered_batch_args(self, sigs81, key_idx, msgs, off, rand32):
         rand32 = _u8(rand32, 32)
         n, sigs81, key_idx, msgs, off = self._registered_inputs(sigs81, key_idx, msgs, off)
