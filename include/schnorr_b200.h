@@ -96,7 +96,11 @@ int schnorr_b200_set_dist_threshold(schnorr_b200_ctx *ctx, size_t max_signatures
  * chain, the challenge hash, e*G and then the sixteen bucket accumulations of one verification proceed side by side on
  * the block's warps (lowest latency for the reference's own Criterion case, a single Signature::verify,
  * benches/schnorr.rs:22-66).  0 disables it.  Default 512 (measured: 0.50-0.65 ms for 1..512 signatures against
- * 0.98-1.08 ms on six lanes; beyond ~1000 blocks the six-lane kernel is faster). */
+ * 0.98-1.08 ms on six lanes; beyond ~1000 blocks the six-lane kernel is faster).  The same threshold selects the
+ * block-per-signature form of calls against a registered key set (verify_registered_many, the host form of
+ * verify_keyed_registered_many): the challenge hash, e*G and a tree of the key's 32 table terms on the block's warps,
+ * with no doubling chain; larger registered calls run one signature per thread.  SIZE_MAX forces the block form, 0 the
+ * per-thread one (tests). */
 int schnorr_b200_set_one_threshold(schnorr_b200_ctx *ctx, size_t max_signatures);
 /* Batches of at most `max_signatures` compute their challenges with one signature per six lanes ahead of the (then
  * hash-free) prepare kernel; larger ones hash one signature per thread.  Default 2^18 (measured crossover). */
@@ -149,9 +153,12 @@ void schnorr_b200_keyset_destroy(schnorr_b200_keyset *ks);
 /* Signature::verify for n (signature, key, message) triples, key = key_idx[i] into the set: verdicts[i] is, byte for
  * byte, what verify_many returns for sigs81[i], message i and that key.  An index outside the set gives verdict 3
  * (indexing past the end of a slice panics in the reference).  A set from another context returns EARG.
- * last_exact_count, last_kernel_ms and set_exact_only apply as for verify_many.  The host form shards a multi-device
- * context in contiguous slices; the _dev form (device buffers, no synchronisation) needs a single-device context and a
- * non-NULL msgs even when every message is empty. */
+ * last_exact_count, last_kernel_ms and set_exact_only apply as for verify_many.  Calls (per device) of at most
+ * set_one_threshold signatures run one thread block per signature from the key's table, the latency form for a node
+ * that sees one vote or certificate at a time; larger calls one thread per signature.  The host form shards a
+ * multi-device context in contiguous slices, and each device picks its form by the size of its own slice; the _dev form
+ * (device buffers, no synchronisation) needs a single-device context and a non-NULL msgs even when every message is
+ * empty. */
 int schnorr_b200_verify_registered_many(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
                                         const uint8_t *sigs81, const uint32_t *key_idx, const uint8_t *msgs,
                                         const uint64_t *msg_off, uint8_t *verdicts);
@@ -215,10 +222,12 @@ int schnorr_b200_keyset_lookup_dev(schnorr_b200_ctx *ctx, const schnorr_b200_key
  * a registered key set: verdicts[i] is, byte for byte, what verify_keyed_many returns for record i.  A record whose key
  * bytes are the encoding of a findable key k takes the registered path of verify_registered_many with key k (the
  * decompressed key IS key k's record, so the verdict is verify_many's); every other record is decompressed and verified
- * as verify_keyed_many does (verdict 3 where the key does not decode).  Calls of at most 384 records run
- * verify_keyed_many.  Records whose key is not in the set cost more than in verify_keyed_many (the exact kernel): the
- * host form reads the miss count and runs verify_many on the decoded records when more than 40 % of them miss; the
- * _dev form does not synchronise and always takes the lookup path.  last_exact_count (misses count as exact items),
+ * as verify_keyed_many does (verdict 3 where the key does not decode).  Records whose key is not in the set cost more
+ * than in verify_keyed_many (the exact kernel): the host form reads the miss count and runs verify_many on the decoded
+ * records when more than 40 % of them miss; the _dev form does not synchronise and always takes the lookup path.  Calls
+ * (per device) of at most set_one_threshold records: the host form takes the lookup path with the block-per-signature
+ * kernel of verify_registered_many when every key was found and verify_many on the decoded records when any missed;
+ * the _dev form runs verify_keyed_many.  last_exact_count (misses count as exact items),
  * last_kernel_ms and set_exact_only apply.  The host form shards a multi-device context in contiguous slices, each with
  * that device's copy of the set; the _dev form needs a single-device context and a non-NULL msgs. */
 int schnorr_b200_verify_keyed_registered_many(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, size_t n,
@@ -502,6 +511,16 @@ int schnorr_b200_debug_fp_core(schnorr_b200_ctx *ctx, int op, size_t n, const ui
 enum { SCHNORR_B200_CORE_EXACT = 0, SCHNORR_B200_CORE_FAST, SCHNORR_B200_CORE_DIST, SCHNORR_B200_CORE_COUNT };
 int schnorr_b200_debug_verify_core(schnorr_b200_ctx *ctx, int core, size_t n, const uint8_t *pk96, const uint8_t *h32,
                                    const uint8_t *e32, uint8_t *result, uint8_t *r97);
+/* Test hook (no reference counterpart): the point stage of a verification against a registered key on a GIVEN
+ * challenge, key key_idx[i] of the set (EARG for an index at or beyond n_keys), h32 / e32 as in debug_verify_core.
+ * REG_CORE_THREAD runs the per-thread table core of verify_registered_many's large calls (verify_core_reg),
+ * REG_CORE_BLOCK the table tree, + e*G, of its block-per-signature form.  result[i] = 0, or 2 when the core met an
+ * exceptional case (the block core only for a collision in its e*G stage, never for e < q); r97 as in
+ * debug_verify_core.  Runs on the first device of a multi-device context.  A bad core returns SCHNORR_B200_EARG. */
+enum { SCHNORR_B200_REG_CORE_THREAD = 0, SCHNORR_B200_REG_CORE_BLOCK, SCHNORR_B200_REG_CORE_COUNT };
+int schnorr_b200_debug_verify_registered_core(schnorr_b200_ctx *ctx, const schnorr_b200_keyset *ks, int core, size_t n,
+                                              const uint32_t *key_idx, const uint8_t *h32, const uint8_t *e32,
+                                              uint8_t *result, uint8_t *r97);
 
 /* Integer-multiply roofline calibration: runs a register-resident chain of `iters` dependent-free
  * 32x32->64 multiply-adds per thread on a full grid and returns wide multiplies per second. */

@@ -150,7 +150,8 @@ public:
     // per key: 0 = in the prime-order subgroup (identity included), 1 = not, 3 = non-canonical limb
     const std::vector<uint8_t>& status() const { return status_; }
     size_t size() const { return status_.size(); }
-    // an index outside the set throws, as indexing past the end of a slice panics
+    // an index outside the set throws, as indexing past the end of a slice panics.  One signature runs one thread block
+    // over the key's table (the latency form, schnorr_b200_set_one_threshold): no doubling chain, no subgroup check
     Result verify_signature(size_t index, const Signature& signature, const std::vector<uint8_t>& message) const {
         auto sig = signature.to_bytes();
         uint64_t off[2] = {0, message.size()};
@@ -171,7 +172,8 @@ public:
     }
     std::optional<uint32_t> index_of(const PublicKey& key) const { return index_of(key.to_bytes()); }
     // KeyedSignature::verify(message) (schnorr_b200_verify_keyed_registered_many): the registered path when the key is
-    // in the set, what KeyedSignature::verify gives otherwise; a key or scalar that does not decode throws
+    // in the set (one thread block over the key's table, as verify_signature), what KeyedSignature::verify gives
+    // otherwise; a key or scalar that does not decode throws
     Result verify_keyed(const std::array<uint8_t, KEYED_SIGNATURE_LENGTH>& keyed, const std::vector<uint8_t>& message) const {
         uint64_t off[2] = {0, message.size()};
         uint8_t verdict = 255;

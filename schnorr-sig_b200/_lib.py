@@ -96,6 +96,7 @@ _SIGNATURES = {
     "schnorr_b200_debug_lazy_ops": (C.c_int, [C.c_void_p, _sz, _u8p, _u8p, _u8p]),
     "schnorr_b200_debug_fp_core": (C.c_int, [C.c_void_p, C.c_int, _sz, _u8p, _u8p]),
     "schnorr_b200_debug_verify_core": (C.c_int, [C.c_void_p, C.c_int, _sz] + [_u8p] * 5),
+    "schnorr_b200_debug_verify_registered_core": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, _sz] + [_u8p] * 5),
     "schnorr_b200_imad_peak": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 }
 

@@ -12,6 +12,7 @@
 //   k_keyset_scatter      replaced slots of a key set: records, status and tables from a compact registration
 //   k_keyset_gather       key records of the items of a registered call (ahead of k_ingest)
 //   k_verify_reg          Signature::verify against registered keys (table additions, no doubling chain)
+//   k_verify_reg_one      the same for calls of a few signatures: one thread block per signature (one_reg.cuh)
 //   k_keyset_encode       the lookup table of a key set's compressed encodings (sorted on the host)
 //   k_keyset_lookup       compressed keys -> indices into a registered key set (binary search)
 //   k_keyed_split_lookup  KeyedSignature records against a registered key set: registered record on a hit, decompressed
@@ -1149,6 +1150,77 @@ static int verify_many_host(schnorr_b200_ctx* ctx, size_t n, const uint8_t* sigs
 #include "one.cuh"
 // registration of a few keys: one thread block per key (the phases of k_verify_one)
 #include "keyset_block.cuh"
+// registered calls of a few signatures: one thread block per signature over the key's table
+#include "one_reg.cuh"
+
+// r97 of the verification-core hooks: affine x || y || identity flag
+__device__ void store_r97(uint8_t* o, const fp6& x, const fp6& y, bool inf) {
+    for (int c = 0; c < 6; c++)
+        for (int b = 0; b < 8; b++) {
+            o[8 * c + b] = (uint8_t)(x.c[c] >> (8 * b));
+            o[48 + 8 * c + b] = (uint8_t)(y.c[c] >> (8 * b));
+        }
+    o[96] = inf;
+}
+__device__ __forceinline__ scalar load_scalar_le(const uint8_t* p) {
+    return sc_from_u64x4(load_u64_le(p), load_u64_le(p + 8), load_u64_le(p + 16), load_u64_le(p + 24));
+}
+
+// test hooks for the point stage of a registered verification on a given challenge (schnorr_b200_debug_verify_registered_core):
+// item i = (key key_idx[i] of the set, h32[i], e32[i]), result and r97 as in k_debug_verify_core.
+// THREAD: verify_core_reg, the point stage of k_verify_reg, in its layout (one item per thread, key 0 and zero scalars
+// for the threads past n so that every thread reaches the barriers)
+__global__ void __launch_bounds__(VERIFY_THREADS) k_debug_reg_core_thread(size_t n, const uint32_t* __restrict__ key_idx,
+                                                                          const uint64_t* __restrict__ ktab,
+                                                                          const uint8_t* __restrict__ h32,
+                                                                          const uint8_t* __restrict__ e32,
+                                                                          const uint64_t* __restrict__ gtab,
+                                                                          uint8_t* __restrict__ result, uint8_t* __restrict__ r97) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool live = i < n;
+    scalar h = sc_zero(), e = sc_zero();
+    uint32_t key = 0;
+    if (live) {
+        key = key_idx[i];
+        h = load_scalar_le(h32 + 32 * i);
+        e = load_scalar_le(e32 + 32 * i);
+    }
+    jf_pt r;
+    int fr = verify_core_reg(h, e, ktab + (size_t)key * KT_KEY_U64, gtab, &r);
+    if (!live) return;
+    fp_t wi = fp_inv(fp_canon(r.w)), wi2 = fp_sqr(wi);
+    result[i] = (uint8_t)fr;
+    store_r97(r97 + 97 * i, fp6_scale(r.X, wi2), fp6_scale(r.Y, fp_mul(wi2, wi)), r.w == 0);
+}
+// BLOCK: phases B and C of k_verify_reg_one, one block per item (the digits of h recoded by thread 0)
+__global__ void __launch_bounds__(ONE_THREADS) k_debug_reg_core_block(const uint32_t* __restrict__ key_idx,
+                                                                      const uint64_t* __restrict__ ktab,
+                                                                      const uint8_t* __restrict__ h32,
+                                                                      const uint8_t* __restrict__ e32,
+                                                                      const uint64_t* __restrict__ gtab,
+                                                                      uint8_t* __restrict__ result, uint8_t* __restrict__ r97) {
+    __shared__ reg_one_shared S;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const size_t i = blockIdx.x;
+    if (tid == 0) recode_signed_kt(load_scalar_le(h32 + 32 * i), S.hd);
+    else if (warp == 1 && lane < 6) reg_one_e_stage(S, load_scalar_le(e32 + 32 * i), gtab, lane);
+    __syncthreads();
+    fp_t x, y, z;
+    reg_one_point_stage(S, ktab + (size_t)key_idx[i] * KT_KEY_U64, x, y, z);
+    if (warp == 0 && lane < 24) {
+        jac_pt R;
+        R.X = gather_fp6(x);
+        R.Y = gather_fp6(y);
+        R.Z = gather_fp6(z);
+        if (lane == 0) {
+            fp6 ax, ay;
+            bool inf;
+            jac_to_affine(R, ax, ay, inf);
+            result[i] = S.e_empty == 2 ? FAST_EXCEPTIONAL : FAST_TORSION_FREE;
+            store_r97(r97 + 97 * i, ax, ay, inf);
+        }
+    }
+}
 
 
 // Signature::verify over an ingested SoA batch: fast path (per-thread or warp-cooperative by call size), then the exact kernel over the handful of
@@ -1787,28 +1859,28 @@ static int keyset_build(schnorr_b200_ctx* ctx, schnorr_b200_keyset* ks, size_t k
     return 0;
 }
 
-// Calls of at most this many items run verify_many's kernels (launch_verify) on the gathered records: at these sizes
-// its block-per-signature kernel wins on latency.  Measured on a B200 (1000 W, 1965 MHz; profiles/r3_registered.md):
-// 1 / 128 / 384 signatures 0.47 / 0.47 / 0.58 ms there against 0.59 / 0.60 / 0.60 ms in k_verify_reg, 512 signatures
-// 0.61 against 0.60 ms.
-static constexpr size_t REG_SMALL_MAX = 384;
-
-// the fast kernel over an ingested batch of registered items, then the exact kernel over the items it handed back;
-// exact_only and small calls go through launch_verify (same verdicts: the planes hold each item's key record).
-// LOOKUP: key_idx may hold KEYSET_MISS (k_keyed_split_lookup); those items are finished by k_verify.  The work list is
-// taken in the caller's scope.
+// the fast kernel over an ingested batch of registered items, then the exact kernel over the items it handed back:
+// calls of at most one_max items (schnorr_b200_set_one_threshold) one thread block per signature (k_verify_reg_one),
+// larger ones one thread per signature (k_verify_reg); exact_only goes through launch_verify (same verdicts: the planes
+// hold each item's key record).  LOOKUP: key_idx may hold KEYSET_MISS (k_keyed_split_lookup); those items are finished
+// by k_verify.  The work list is taken in the caller's scope.
 template <bool LOOKUP>
 static int launch_verify_registered(schnorr_b200_ctx* ctx, const keyset_dev& kd, const soa_batch& soa,
                                     const uint32_t* key_idx, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts) {
     cudaStream_t st = ctx->stream;
-    if (ctx->exact_only || soa.n <= REG_SMALL_MAX) return launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, st);
+    if (ctx->exact_only) return launch_verify(ctx, soa, msgs, msg_off, verdicts, 0, st);
     uint32_t* list;
     if (int rc = stage_in(ctx, {{nullptr, 4 * soa.n, &list}})) return rc;
     uint32_t* counter = ctx->exact_counters;
     CUDA_TRY(ctx, cudaMemsetAsync(counter, 0, 4, st));
     ctx->exact_counters_used = 1;
     unsigned grid = grid_for(soa.n, VERIFY_THREADS);
-    k_verify_reg<LOOKUP><<<grid, VERIFY_THREADS, 0, st>>>(soa, key_idx, kd.status, kd.ktab, msgs, msg_off, ctx->gtab, verdicts, list, counter);
+    if (soa.n <= ctx->one_max)   // two blocks per SM at every size (one_reg.cuh: MINB)
+        k_verify_reg_one<2, LOOKUP><<<(unsigned)soa.n, ONE_THREADS, 0, st>>>(soa, key_idx, kd.status, kd.ktab, msgs, msg_off,
+                                                                              ctx->gtab, verdicts, list, counter);
+    else
+        k_verify_reg<LOOKUP><<<grid, VERIFY_THREADS, 0, st>>>(soa, key_idx, kd.status, kd.ktab, msgs, msg_off, ctx->gtab, verdicts,
+                                                              list, counter);
     k_verify<<<grid, VERIFY_THREADS, 0, st>>>(soa, msgs, msg_off, ctx->gtab, verdicts, list, counter);
     ctx->launches += 2;
     return 0;
@@ -2186,11 +2258,15 @@ int schnorr_b200_verify_registered_many_dev(schnorr_b200_ctx* ctx, const schnorr
 static constexpr double KEYED_REG_MAX_MISS_FRACTION = 0.4;
 
 // device buffers, single-device context, arguments checked by the caller.  `select`: read the miss count of the front
-// end (synchronises) and take verify_many above KEYED_REG_MAX_MISS_FRACTION.
+// end (synchronises) and take verify_many above KEYED_REG_MAX_MISS_FRACTION.  Calls of at most one_max records
+// (schnorr_b200_set_one_threshold): with `select`, the lookup path (k_verify_reg_one) only when every key was found,
+// since a miss in k_verify costs more than verify_many's block kernel; without it, which would have to synchronise to
+// learn the misses, verify_keyed_many.
 static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, size_t k, size_t n,
                                        const uint8_t* keyed130, const uint8_t* msgs, const uint64_t* msg_off, uint8_t* verdicts,
                                        bool select) {
-    if (n <= REG_SMALL_MAX) return schnorr_b200_verify_keyed_many_dev(ctx, n, keyed130, msgs, msg_off, verdicts);
+    const bool small = n <= ctx->one_max;
+    if (small && !select) return schnorr_b200_verify_keyed_many_dev(ctx, n, keyed130, msgs, msg_off, verdicts);
     const keyset_dev& kd = ks->devs[k];
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
@@ -2210,7 +2286,7 @@ static int verify_keyed_registered_dev(schnorr_b200_ctx* ctx, const schnorr_b200
         uint32_t misses = 0;
         CUDA_TRY(ctx, cudaMemcpyAsync(&misses, d_miss, 4, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(ctx, cudaStreamSynchronize(st));
-        lookup_path = misses <= KEYED_REG_MAX_MISS_FRACTION * (double)n;
+        lookup_path = small ? misses == 0 : misses <= KEYED_REG_MAX_MISS_FRACTION * (double)n;
     }
     if (lookup_path) {
         soa_batch soa;
@@ -2956,6 +3032,42 @@ int schnorr_b200_debug_verify_core(schnorr_b200_ctx* ctx, int core, size_t n, co
     CUDA_TRY(ctx, cudaMemcpyAsync(result, d_res, n, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaMemcpyAsync(r97, d_r, n * 97, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return SCHNORR_B200_OK;
+}
+
+int schnorr_b200_debug_verify_registered_core(schnorr_b200_ctx* ctx, const schnorr_b200_keyset* ks, int core, size_t n,
+                                              const uint32_t* key_idx, const uint8_t* h32, const uint8_t* e32, uint8_t* result,
+                                              uint8_t* r97) {
+    if (!ctx || !ks || core < 0 || core >= SCHNORR_B200_REG_CORE_COUNT || (n && (!key_idx || !h32 || !e32 || !result || !r97)))
+        return SCHNORR_B200_EARG;
+    CHECK_KEYSET(ctx, ks);
+    for (size_t i = 0; i < n; i++)
+        if (key_idx[i] >= ks->n_keys) {
+            ctx->err = "debug_verify_registered_core: a key index outside the set";
+            return SCHNORR_B200_EARG;
+        }
+    if (n == 0) return SCHNORR_B200_OK;
+    schnorr_b200_ctx* c = device_ctx(ctx, 0);
+    const keyset_dev& kd = ks->devs[0];
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    scratch_scope scope(c->scratch, c->stream);
+    void *d_idx, *d_h, *d_e, *d_res, *d_r;
+    if (int rc = stage_in(c, {{key_idx, n * 4, &d_idx}, {h32, n * 32, &d_h}, {e32, n * 32, &d_e}, {nullptr, n, &d_res},
+                              {nullptr, n * 97, &d_r}}))
+        return rc;
+    const uint32_t* idx = (uint32_t*)d_idx;
+    const uint8_t *hh = (uint8_t*)d_h, *ee = (uint8_t*)d_e;
+    if (core == SCHNORR_B200_REG_CORE_THREAD)
+        k_debug_reg_core_thread<<<grid_for(n, VERIFY_THREADS), VERIFY_THREADS, 0, c->stream>>>(n, idx, kd.ktab, hh, ee, c->gtab,
+                                                                                            (uint8_t*)d_res, (uint8_t*)d_r);
+    else
+        k_debug_reg_core_block<<<(unsigned)n, ONE_THREADS, 0, c->stream>>>(idx, kd.ktab, hh, ee, c->gtab, (uint8_t*)d_res,
+                                                                           (uint8_t*)d_r);
+    c->launches += 1;
+    CUDA_TRY(c, cudaGetLastError());
+    CUDA_TRY(c, cudaMemcpyAsync(result, d_res, n, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(c, cudaMemcpyAsync(r97, d_r, n * 97, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     return SCHNORR_B200_OK;
 }
 

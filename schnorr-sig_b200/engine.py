@@ -713,6 +713,26 @@ class Engine:
                                                            _ptr(r97)), "debug_verify_core")
         return res, r97
 
+    # core numbers of debug_verify_registered_core (enum SCHNORR_B200_REG_CORE_* of include/schnorr_b200.h)
+    REG_VERIFY_CORES = ("thread", "block")
+
+    def debug_verify_registered_core(self, keyset, core, key_idx, h32, e32):
+        """Test hook: the point stage of n verifications against keys key_idx of `keyset` on given challenges through the
+        per-thread table core ("thread") or the block-per-signature tree ("block"), or its number -> (result uint8[n]:
+        0, or 2 exceptional; R uint8[n, 97] as in debug_verify_core)."""
+        code = self.REG_VERIFY_CORES.index(core) if isinstance(core, str) else int(core)
+        key_idx = np.ascontiguousarray(key_idx, dtype=np.uint32).reshape(-1)
+        h32, e32 = _u8(h32, 32), _u8(e32, 32)
+        n = key_idx.shape[0]
+        if h32.shape[0] != n or e32.shape[0] != n:
+            raise ValueError("one challenge and one e per key index")
+        res = np.full(n, 255, dtype=np.uint8)
+        r97 = np.zeros((n, 97), dtype=np.uint8)
+        self._check(self._L.schnorr_b200_debug_verify_registered_core(self._h, keyset.handle, code, n, _ptr(key_idx),
+                                                                      _ptr(h32), _ptr(e32), _ptr(res), _ptr(r97)),
+                    "debug_verify_registered_core")
+        return res, r97
+
     def imad_peak(self, iters=1 << 16):
         w = C.c_double(0)
         ms = C.c_double(0)
